@@ -14,6 +14,10 @@ Prints ONE JSON line (rank 0).  `value` = pairs/s with inputs resident in HBM; `
 the public nn.Module call with pinned HOST inputs (decoded 8-bit HWC images -- the reference's inputs are PNG renders,
 README.md:73-74 -- H2D inside the timed region, voxels + IoU read back).
 
+--dump-outputs DIR writes what the last timed step of the resident loop returned (disp_left, disp_right, voxels, iou_counts)
+as DIR/<name>.npy, after that loop and outside every timed region.  Inputs and weights are seeded, so two builds run with the
+same arguments can be compared output for output.
+
 The same line carries the other BASELINE configs as extra keys, each measured briefly in the same run (N = 1):
   fp32_mode              configs[1] "fp32": the fast tensor-core mode that meets the 1e-3 tolerance ('bf16x3'), with its error
   latency                B = 1 / 8 through the CUDA-graph replay
@@ -46,6 +50,8 @@ def parse():
     p.add_argument('--precision', default='bf16', choices=['bf16', 'bf16x3', 'tf32', 'tf32x3', 'fp32'])
     p.add_argument('--no-cpu-baseline', action='store_true')
     p.add_argument('--no-extras', action='store_true', help='only the headline measurement (no secondary configs)')
+    p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                   help='write the outputs of the last timed step of the headline loop (rank 0) as DIR/<name>.npy')
     return p.parse_args()
 
 
@@ -428,6 +434,23 @@ def extra_peaks(dev):
     return out
 
 
+def dump_outputs(outdir, outputs, limit=64 * 2 ** 20):
+    """Writes `outputs` (name -> tensor, batch first) as outdir/<name>.npy: float tensors as float32, integer counts as
+    float64 (exact).  Above `limit` bytes in all, every array keeps the same seeded sample of batch entries, so two builds
+    run with the same arguments are compared pair for pair."""
+    import numpy as np
+    import torch
+    host = {k: (v.float() if v.is_floating_point() else v.double()).cpu().numpy() for k, v in outputs.items()}
+    B = next(iter(host.values())).shape[0]
+    keep = max(1, limit // sum(v[:1].nbytes for v in host.values()))
+    if keep < B:
+        idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values.numpy()
+        host = {k: v[idx] for k, v in host.items()}
+    os.makedirs(outdir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(outdir, k + '.npy'), v)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -465,10 +488,12 @@ def run_ours(args):
         dev_sets.append((l.to(dev), r.to(dev), g.to(dev)))
     T = len(cfg.TEST.VOXEL_THRESH)
     stats = torch.zeros(2 * T + 1, dtype=torch.int64, device=dev)
+    last_out = []            # outputs of the latest resident step: views of the model's workspace, valid until its next forward
 
     def step_resident(i):
         l, r, g = dev_sets[i % n_sets]
-        _, _, vox, iou = model(l, r, g)
+        last_out[:] = model(l, r, g)
+        _, _, vox, iou = last_out
         stats[:T] = iou[:, :, 0].sum(0)
         stats[T:2 * T] = iou[:, :, 1].sum(0)
         stats[2 * T] = B
@@ -648,6 +673,8 @@ def run_ours(args):
     n0 = lib.launches()
     with ClockSampler(local) as clk:
         ms = timed(step_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(('disp_left', 'disp_right', 'voxels', 'iou_counts'), last_out)))
     launches = (lib.launches() - n0) // (args.steps + args.warmup)        # kernels of this library per step
     n_dom = len(dom_events) // (args.steps + args.warmup)                 # plain aggregation launches per step
     dom_ms = [a.elapsed_time(b) for a, b in dom_events[n_dom * args.warmup:]]
