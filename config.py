@@ -85,3 +85,5 @@ __C.NETWORK.PRECISION = 'bf16'
 #
 __C.TEST = AttrDict()
 __C.TEST.VOXEL_THRESH = [0.2, 0.3, 0.4, 0.5]
+# bad-pixel thresholds of the disparity evaluation (forward(..., disp_gt=...)): |disp - gt| > t px at input resolution
+__C.TEST.DISP_THRESH = [1.0, 3.0]

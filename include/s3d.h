@@ -217,6 +217,16 @@ int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_out, int B, 
 /* disp_q fp32 [N,h,w] (1/4-res units) -> fp32 [N,H,W] = bilinear(scale*disp_q), align_corners=False. */
 int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h, int w, int H, int W,
                       float scale, void* stream);
+/* s3d_upsample_disp + evaluation against GT disparity.  disp_q fp32 [2B,h,w] (left-referenced first), disp fp32 [2B,H,W]
+ * (written bit-identically to s3d_upsample_disp), gt fp32 [B,2,H,W] (view 0 = left-referenced, 1 = right-referenced),
+ * thresholds: T <= 8 fp32 HOST values, stats int64 [B,2,2+T], ACCUMULATED (the caller zeroes it):
+ *   [n_valid, sum_valid q(|disp - gt|), count_valid(|disp - gt| > thresholds[t]) for t < T]
+ * valid: gt finite and 0 <= gt < max_gt.  q(e) = round-half-even(e * 65536) of the fp32 error (fixed point, 2^-16 px).
+ * Range: q < 2^26 per pixel while disparities are below 1024 px, so one image's sum stays below 2^50 for H*W <= 2^24 and
+ * int64 holds the sums of more than 2^12 such images.  Integer counters, one atomic per counter per block and no block
+ * spans two images: the stats do not depend on the launch order, batch split or number of GPUs. */
+int s3d_upsample_disp_eval(const float* disp_q, float* disp, const float* gt, const float* thresholds, int T,
+                           float max_gt, long long* stats, int B, int h, int w, int H, int W, float scale, void* stream);
 
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)

@@ -92,10 +92,16 @@ def main():
     if args.weights:
         load_checkpoint(model, args.weights)
     model.cuda().pack()
+    # one stats vector: the head's statistics, then the disparity counters of the same forwards
     if args.model == 'Stereo2Voxel':
-        res = T.iou_summary(T.test_voxel(cfg, model, n, bs, rank, world).cpu(), cfg.TEST.VOXEL_THRESH)
+        stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True).cpu()
+        nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
+        res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
     else:
-        res = T.chamfer_summary(T.test_point(cfg, model, n, bs, rank, world).cpu())
+        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True).cpu()
+        nh = 2
+        res = T.chamfer_summary(stats[:nh])
+    res['disparity'] = T.disp_summary(stats[nh:], cfg.TEST.DISP_THRESH)
     if rank == 0:
         res.update(model=args.model, precision=cfg.NETWORK.PRECISION, world_size=world, data='synthetic')
         print(json.dumps(res))

@@ -6,6 +6,9 @@ on disk).  Statistics are integer sums so that an N-GPU run is bit-identical to 
     per threshold t:  sum_b intersection(b,t), sum_b union(b,t)   (int64)
     n_samples                                                    (int64)
 Chamfer: sum_b CD(b) is accumulated in fp64 and reduced as a fixed-point int64 (2^-40 units).
+With eval_disp=True the same vector carries, per view (left-referenced, then right-referenced), the disparity counters the
+forward computes against the synthetic GT disparity (models.py, _StereoBase._upsample_disp):
+    n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) per t in TEST.DISP_THRESH   (int64)
 """
 import torch
 import torch.distributed as dist
@@ -13,6 +16,7 @@ import torch.distributed as dist
 from ..utils import synthetic
 
 _FX = float(1 << 40)
+_DISP_FX = float(1 << 16)
 
 
 def shard_range(n_total, rank, world):
@@ -38,12 +42,35 @@ def iou_summary(stats, thresholds):
             'intersection': [int(v) for v in stats[:T].tolist()], 'union': [int(v) for v in stats[T:2 * T].tolist()]}
 
 
-def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'):
+def disp_summary(stats_block, thresholds):
+    """Disparity counters [n_valid, epe_fx, bad_t...] x 2 views (int64 [2 * (2 + T)]) -> dict: end-point error
+    EPE = sum epe_fx / 2^16 / sum n_valid (px) and bad-pixel fractions, per view and over both views."""
+    T = len(thresholds)
+    v = [int(x) for x in stats_block.tolist()]
+    assert len(v) == 2 * (2 + T)
+
+    def one(n, epe_fx, bad):
+        return {'n_valid': n, 'epe': epe_fx / _DISP_FX / n if n else 0.0, 'bad': [b / n if n else 0.0 for b in bad]}
+    views = [v[:2 + T], v[2 + T:]]
+    out = {'thresholds': list(thresholds)}
+    for name, c in zip(('left', 'right'), views):
+        out[name] = one(c[0], c[1], c[2:])
+    out['all'] = one(views[0][0] + views[1][0], views[0][1] + views[1][1], [a + b for a, b in zip(views[0][2:], views[1][2:])])
+    return out
+
+
+def _disp_gt(pairs, H, W, device):
+    return torch.cat([synthetic.disparity_gt(p[2], H, W) for p in pairs]).to(device)
+
+
+def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
-    materialise exactly its own shard and the union over ranks is independent of `world`."""
+    materialise exactly its own shard and the union over ranks is independent of `world`.
+    eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring)."""
     th = list(cfg.TEST.VOXEL_THRESH)
     T = len(th)
-    stats = torch.zeros(2 * T + 1, dtype=torch.int64, device=device)
+    nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
+    stats = torch.zeros(2 * T + 1 + nd, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -53,16 +80,22 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.gt_volume(1, cfg.CONST.N_VOX, seed=100000 + i) for i in ids]).to(device)
-            _, _, _, iou = model(left, right, gt)
+            if eval_disp:
+                _, _, _, iou, ds = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device))
+                stats[2 * T + 1:] += ds.sum(0).flatten()
+            else:
+                _, _, _, iou = model(left, right, gt)
             stats[:T] += iou[:, :, 0].sum(0)
             stats[T:2 * T] += iou[:, :, 1].sum(0)
             stats[2 * T] += len(ids)
     return reduce_stats(stats)
 
 
-def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'):
+def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False):
+    """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, as for test_voxel)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
-    stats = torch.zeros(2, dtype=torch.int64, device=device)
+    nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
+    stats = torch.zeros(2 + nd, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -72,7 +105,11 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.point_clouds(1, 1, cfg.CONST.N_GT_POINTS, seed=200000 + i)[1] for i in ids]).to(device)
-            _, _, pts = model(left, right)
+            if eval_disp:
+                _, _, pts, ds = model(left, right, disp_gt=_disp_gt(pairs, H, W, device))
+                stats[2:] += ds.sum(0).flatten()
+            else:
+                _, _, pts = model(left, right)
             cd = chamfer_per_sample(pts.contiguous(), gt)
             stats[0] += torch.round(cd.sum() * _FX).to(torch.int64)
             stats[1] += len(ids)

@@ -56,6 +56,12 @@ Knobs& knobs();
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// Thresholds of the in-kernel evaluation counters (IoU in fuse_views, bad-pixel rates in upsample_disp_eval), passed by value.
+namespace {
+constexpr int kMaxThresh = 8;
+struct Thresh { float t[kMaxThresh]; };
+}  // namespace
+
 template <typename T> __device__ __forceinline__ float to_f32(T v);
 template <> __device__ __forceinline__ float to_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }

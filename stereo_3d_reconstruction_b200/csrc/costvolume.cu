@@ -317,8 +317,26 @@ corr_soft_argmin_kernel(const T* __restrict__ feat, float* __restrict__ disp, fl
 }
 
 // ------------------------------------------------------------------------------------------
-// bilinear upsample (align_corners = False), PyTorch index / weight convention
+// bilinear upsample (align_corners = False), PyTorch index / weight convention.  The formula lives in the two helpers
+// below, shared by the plain kernels and the evaluating ones, so both write the same bits.
 // ------------------------------------------------------------------------------------------
+struct UpRow { const float* p0; const float* p1; float ly, hy; };    // the two source rows of one output row + their weights
+
+__device__ __forceinline__ UpRow up_row(const float* __restrict__ q_img, int Y, int h, int w, float ry) {
+  float sy = ((float)Y + 0.5f) * ry - 0.5f;  if (sy < 0.f) sy = 0.f;
+  const int y0 = (int)sy, y1 = y0 + (y0 < h - 1 ? 1 : 0);
+  const float ly = sy - (float)y0;
+  return {q_img + (int64_t)y0 * w, q_img + (int64_t)y1 * w, ly, 1.f - ly};
+}
+
+__device__ __forceinline__ float up_px(const UpRow& r, int X, int w, float rx, float scale) {
+  float sx = ((float)X + 0.5f) * rx - 0.5f;  if (sx < 0.f) sx = 0.f;
+  const int x0 = (int)sx, x1 = x0 + (x0 < w - 1 ? 1 : 0);
+  const float lx = sx - (float)x0, hx = 1.f - lx;
+  const float v = r.hy * (hx * __ldg(r.p0 + x0) + lx * __ldg(r.p0 + x1)) + r.ly * (hx * __ldg(r.p1 + x0) + lx * __ldg(r.p1 + x1));
+  return v * scale;
+}
+
 __global__ void upsample_disp_kernel(const float* __restrict__ q, float* __restrict__ out, int N, int h, int w,
                                      int H, int W, float scale) {
   const int64_t total = (int64_t)N * H * W;
@@ -326,15 +344,7 @@ __global__ void upsample_disp_kernel(const float* __restrict__ q, float* __restr
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int X = (int)(i % W), Y = (int)((i / W) % H);
     const int64_t n = i / ((int64_t)W * H);
-    float sy = ((float)Y + 0.5f) * ry - 0.5f;  if (sy < 0.f) sy = 0.f;
-    float sx = ((float)X + 0.5f) * rx - 0.5f;  if (sx < 0.f) sx = 0.f;
-    const int y0 = (int)sy, x0 = (int)sx;
-    const int y1 = y0 + (y0 < h - 1 ? 1 : 0), x1 = x0 + (x0 < w - 1 ? 1 : 0);
-    const float ly = sy - (float)y0, lx = sx - (float)x0;
-    const float hy = 1.f - ly, hx = 1.f - lx;
-    const float* p = q + n * h * w;
-    const float v = hy * (hx * p[y0 * w + x0] + lx * p[y0 * w + x1]) + ly * (hx * p[y1 * w + x0] + lx * p[y1 * w + x1]);
-    out[i] = v * scale;
+    out[i] = up_px(up_row(q + n * h * w, Y, h, w, ry), X, w, rx, scale);
   }
 }
 
@@ -347,22 +357,98 @@ upsample_disp_v4_kernel(const float* __restrict__ q, float4* __restrict__ out, u
   if (i >= total4) return;
   const uint32_t X4 = i % (uint32_t)W4, row = i / (uint32_t)W4;
   const uint32_t Y = row % (uint32_t)H, n = row / (uint32_t)H;
-  float sy = ((float)Y + 0.5f) * ry - 0.5f;  if (sy < 0.f) sy = 0.f;
-  const int y0 = (int)sy, y1 = y0 + (y0 < h - 1 ? 1 : 0);
-  const float ly = sy - (float)y0, hy = 1.f - ly;
-  const float* p0 = q + ((int64_t)n * h + y0) * w;
-  const float* p1 = q + ((int64_t)n * h + y1) * w;
-  float r[4];
+  const UpRow r = up_row(q + (int64_t)n * h * w, (int)Y, h, w, ry);
+  float o[4];
 #pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int X = 4 * (int)X4 + k;
-    float sx = ((float)X + 0.5f) * rx - 0.5f;  if (sx < 0.f) sx = 0.f;
-    const int x0 = (int)sx, x1 = x0 + (x0 < w - 1 ? 1 : 0);
-    const float lx = sx - (float)x0, hx = 1.f - lx;
-    const float v = hy * (hx * __ldg(p0 + x0) + lx * __ldg(p0 + x1)) + ly * (hx * __ldg(p1 + x0) + lx * __ldg(p1 + x1));
-    r[k] = v * scale;
+  for (int k = 0; k < 4; ++k) o[k] = up_px(r, 4 * (int)X4 + k, w, rx, scale);
+  out[i] = make_float4(o[0], o[1], o[2], o[3]);
+}
+
+// ------------------------------------------------------------------------------------------
+// upsample + evaluation against GT disparity.  Each block covers part of ONE (sample, view) image (blockIdx.y = image),
+// so its counters belong to one row of `stats`; the per-thread counters are integers, reduced by warp shuffle ->
+// shared memory -> one 64-bit atomic per counter per block: any order of atomics gives the same sums.
+// ------------------------------------------------------------------------------------------
+struct DispCounters {
+  unsigned n_valid = 0;
+  unsigned long long epe_fx = 0;                 // sum of round-half-even(|disp - gt| * 2^16)
+  unsigned bad[kMaxThresh] = {};
+
+  __device__ __forceinline__ void add(float d, float g, float max_gt, const Thresh& th, int nT) {
+    if (!(isfinite(g) && g >= 0.f && g < max_gt)) return;
+    const float e = fabsf(__fsub_rn(d, g));      // the stored value: no contraction with the multiply that produced d
+    ++n_valid;
+    epe_fx += (unsigned long long)__float2ll_rn(e * 65536.f);    // exact scaling by 2^16, then round half to even
+#pragma unroll
+    for (int t = 0; t < kMaxThresh; ++t)
+      if (t < nT) bad[t] += e > th.t[t];
   }
-  out[i] = make_float4(r[0], r[1], r[2], r[3]);
+
+  // -> dst[0 .. 2+nT) of the block's image; every thread of the block calls it
+  __device__ __forceinline__ void flush(unsigned long long* __restrict__ dst, int nT) {
+    __shared__ unsigned long long blk[2 + kMaxThresh];
+    if (threadIdx.x < 2 + kMaxThresh) blk[threadIdx.x] = 0;
+    __syncthreads();
+    unsigned long long v[2 + kMaxThresh];
+    v[0] = n_valid;  v[1] = epe_fx;
+#pragma unroll
+    for (int t = 0; t < kMaxThresh; ++t) v[2 + t] = bad[t];
+#pragma unroll
+    for (int k = 0; k < 2 + kMaxThresh; ++k) {
+      if (k >= 2 + nT) break;
+      unsigned long long a = v[k];
+      for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+      if ((threadIdx.x & 31) == 0 && a) atomicAdd(&blk[k], a);
+    }
+    __syncthreads();
+    if ((int)threadIdx.x < 2 + nT && blk[threadIdx.x]) atomicAdd(dst + threadIdx.x, blk[threadIdx.x]);
+  }
+};
+
+// image n of [2B]: view = n / B (0 = left-referenced), sample b = n % B; gt [B,2,H,W], stats [B,2,2+nT]
+__device__ __forceinline__ int64_t eval_image_index(int n, int B) { return (int64_t)(n % B) * 2 + n / B; }
+
+__global__ void __launch_bounds__(256)
+upsample_disp_eval_v4_kernel(const float* __restrict__ q, float4* __restrict__ out, const float4* __restrict__ gt, int B, int h,
+                             int w, int H, int W4, float ry, float rx, float scale, Thresh th, int nT, float max_gt,
+                             unsigned long long* __restrict__ stats) {
+  const int n = blockIdx.y;
+  const int64_t img4 = (int64_t)H * W4;
+  const float* q_img = q + (int64_t)n * h * w;
+  float4* out_img = out + n * img4;
+  const float4* gt_img = gt + eval_image_index(n, B) * img4;
+  DispCounters c;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < (uint32_t)img4; i += gridDim.x * blockDim.x) {
+    const uint32_t X4 = i % (uint32_t)W4, Y = i / (uint32_t)W4;
+    const float4 g = __ldcs(gt_img + i);                            // read once: keep it out of L2
+    const UpRow r = up_row(q_img, (int)Y, h, w, ry);
+    float o[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) o[k] = up_px(r, 4 * (int)X4 + k, w, rx, scale);
+    out_img[i] = make_float4(o[0], o[1], o[2], o[3]);
+    c.add(o[0], g.x, max_gt, th, nT);  c.add(o[1], g.y, max_gt, th, nT);
+    c.add(o[2], g.z, max_gt, th, nT);  c.add(o[3], g.w, max_gt, th, nT);
+  }
+  c.flush(stats + eval_image_index(n, B) * (2 + nT), nT);
+}
+
+__global__ void __launch_bounds__(256)
+upsample_disp_eval_kernel(const float* __restrict__ q, float* __restrict__ out, const float* __restrict__ gt, int B, int h, int w,
+                          int H, int W, float scale, Thresh th, int nT, float max_gt, unsigned long long* __restrict__ stats) {
+  const int n = blockIdx.y;
+  const int img = H * W;                                            // < 2^31 (checked by the launcher)
+  const float ry = (float)h / (float)H, rx = (float)w / (float)W;
+  const float* q_img = q + (int64_t)n * h * w;
+  float* out_img = out + (int64_t)n * img;
+  const float* gt_img = gt + eval_image_index(n, B) * img;
+  DispCounters c;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < img; i += gridDim.x * blockDim.x) {
+    const int X = i % W, Y = i / W;
+    const float d = up_px(up_row(q_img, Y, h, w, ry), X, w, rx, scale);
+    out_img[i] = d;
+    c.add(d, __ldcs(gt_img + i), max_gt, th, nT);
+  }
+  c.flush(stats + eval_image_index(n, B) * (2 + nT), nT);
 }
 
 }  // namespace
@@ -465,6 +551,36 @@ extern "C" int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h,
   int64_t blocks = ceil_div64(total, 256);
   if (blocks > (int64_t)num_sms() * 16) blocks = (int64_t)num_sms() * 16;
   upsample_disp_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(disp_q, disp, N, h, w, H, W, scale);
+  S3D_LAUNCH_CHECK();
+  return S3D_OK;
+}
+
+extern "C" int s3d_upsample_disp_eval(const float* disp_q, float* disp, const float* gt, const float* thresholds, int T,
+                                      float max_gt, long long* stats, int B, int h, int w, int H, int W, float scale,
+                                      void* stream) {
+  if (!disp_q || !disp || !gt || !stats || (T > 0 && !thresholds)) {
+    set_error("upsample_disp_eval: null argument");
+    return S3D_ERR_INVALID;
+  }
+  S3D_CHECK_ARG(B > 0 && 2 * B < 65536 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31),
+                "upsample_disp_eval: bad shape");
+  S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "upsample_disp_eval: T must be in [0, 8]");
+  S3D_CHECK_ARG(max_gt > 0.f, "upsample_disp_eval: max_gt must be > 0");
+  Thresh th;
+  for (int t = 0; t < kMaxThresh; ++t) th.t[t] = t < T ? thresholds[t] : 0.f;
+  const int64_t img = (int64_t)H * W;
+  auto* st = reinterpret_cast<unsigned long long*>(stats);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (W % 4 == 0 && ((reinterpret_cast<uintptr_t>(disp) | reinterpret_cast<uintptr_t>(gt)) & 15) == 0) {
+    // 16 outputs per thread: 4x fewer blocks (and counter atomics) than one vector per thread
+    const dim3 grid((unsigned)ceil_div64(img / 4, 256 * 4), 2 * B);
+    upsample_disp_eval_v4_kernel<<<grid, 256, 0, s>>>(disp_q, reinterpret_cast<float4*>(disp), reinterpret_cast<const float4*>(gt),
+                                                      B, h, w, H, W / 4, (float)h / (float)H, (float)w / (float)W, scale, th, T,
+                                                      max_gt, st);
+    S3D_LAUNCH_CHECK();
+    return S3D_OK;
+  }
+  upsample_disp_eval_kernel<<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * B), 256, 0, s>>>(disp_q, disp, gt, B, h, w, H, W, scale, th, T, max_gt, st);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
 }

@@ -180,9 +180,6 @@ __global__ void pool_split_kernel(const __nv_bfloat16* __restrict__ x, __nv_bflo
   }
 }
 
-constexpr int kMaxThresh = 8;
-struct Thresh { float t[kMaxThresh]; };
-
 template <typename T>
 __global__ void __launch_bounds__(256)
 fuse_views_kernel(const T* __restrict__ score, int64_t sstride, const T* __restrict__ vol, int64_t vstride,

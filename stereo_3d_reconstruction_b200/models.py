@@ -134,14 +134,16 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt):
+    def __init__(self, model, left, right, gt, disp_gt=None):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
-        self.left.copy_(left);  self.right.copy_(right)
-        if gt is not None:
-            self.gt.copy_(gt)
-        run = (lambda: model._forward_impl(self.left, self.right, self.gt)) if gt is not None else \
-              (lambda: model._forward_impl(self.left, self.right))
+        self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
+        self._copy_in(left, right, gt, disp_gt)
+        args = (self.left, self.right) if gt is None else (self.left, self.right, self.gt)
+        kw = {} if disp_gt is None else {'disp_gt': self.disp_gt}
+
+        def run():                                    # zeroes its IoU / disparity counters itself: inside the graph
+            return model._forward_impl(*args, **kw)
         side = torch.cuda.Stream(device=left.device)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):                 # warm-up: workspace buffers and tensor maps exist before capture
@@ -152,11 +154,16 @@ class _GraphedForward:
         with torch.cuda.graph(self.graph):
             self.out = run()
 
-    def __call__(self, left, right, gt):
+    def _copy_in(self, left, right, gt, disp_gt):
         self.left.copy_(left, non_blocking=True)
         self.right.copy_(right, non_blocking=True)
         if self.gt is not None:
             self.gt.copy_(gt, non_blocking=True)
+        if self.disp_gt is not None:
+            self.disp_gt.copy_(disp_gt, non_blocking=True)
+
+    def __call__(self, left, right, gt, disp_gt=None):
+        self._copy_in(left, right, gt, disp_gt)
         self.graph.replay()
         return self.out
 
@@ -266,8 +273,9 @@ class _StereoBase(nn.Module):
     def _bhw(img):
         return (img.shape[0], img.shape[1], img.shape[2]) if img.dtype == torch.uint8 else (img.shape[0], img.shape[2], img.shape[3])
 
-    def _disparity(self, left, right):
-        """-> disp fp32 [2B,H,W] (left-referenced first), in input pixels."""
+    def _disparity(self, left, right, disp_gt=None):
+        """-> disp fp32 [2B,H,W] (left-referenced first), in input pixels, disp_q, and the disparity stats int64
+        [B,2,2+T] against disp_gt (None without it; see _upsample_disp)."""
         cfg = self.cfg
         B, H, W = self._bhw(left)
         D = cfg.NETWORK.MAX_DISP
@@ -345,8 +353,8 @@ class _StereoBase(nn.Module):
                 nb = ops.conv_cls_workspace_bytes(2 * B, D, h, w)
                 ops.conv_cls_soft_argmin(pa, a, self._packed['cls_b'].weight, -1.0, out=disp_q,
                                          workspace=self._buf('cls_ws', (nb,), torch.uint8))
-                disp = ops.upsample_disp(disp_q, H, W, 4.0, out=self._buf('disp', (2 * B, H, W), torch.float32))
-                return disp, disp_q
+                disp, stats = self._upsample_disp(disp_q, H, W, disp_gt)
+                return disp, disp_q, stats
             c = self._conv('cls_a', a, out=self._bufo('a0', 'cls_a', a))
             if self.precision == 'bf16' and c.shape[-1] in (16, 32, 64) and S == 32 and not _lib.KNOBS['no_cls_fused']:
                 # classifier + soft-argmin in one pass over the volume (csrc/cls_fused.cu)
@@ -359,8 +367,22 @@ class _StereoBase(nn.Module):
             if self._split:                                               # exact fp32 correlation on hi + lo
                 feat = ops.unsplit_bf16(feat, out=self._buf('feat32', feat.shape[:-1] + (feat.shape[-1] // 2,), torch.float32))
             ops.corr_soft_argmin(feat, B, D, out=disp_q, c_real=C)       # mean over the REAL channels (feat is padded)
-        disp = ops.upsample_disp(disp_q, H, W, 4.0, out=self._buf('disp', (2 * B, H, W), torch.float32))
-        return disp, disp_q
+        disp, stats = self._upsample_disp(disp_q, H, W, disp_gt)
+        return disp, disp_q, stats
+
+    def _upsample_disp(self, disp_q, H, W, disp_gt):
+        """Last kernel of the disparity stage: 1/4-res disparity -> input pixels [2B,H,W].  With disp_gt [B,2,H,W] the same
+        kernel also counts, per sample and view, [n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) for t in
+        TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> (disp, stats int64 [B,2,2+T]); else (disp, None)."""
+        B = disp_q.shape[0] // 2
+        out = self._buf('disp', (2 * B, H, W), torch.float32)
+        if disp_gt is None:
+            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None
+        th = list(self.cfg.TEST.DISP_THRESH)
+        stats = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64)
+        stats.zero_()
+        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, 4.0 * self.cfg.NETWORK.MAX_DISP, stats, out=out)
+        return out, stats
 
     def _bufo(self, name, layer, x):
         """Output buffer of `layer` for input x (channels-last, padded channels)."""
@@ -401,7 +423,7 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None):
+    def graphed(self, left, right, gt=None, *, disp_gt=None):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -409,15 +431,17 @@ class _StereoBase(nn.Module):
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
         left, right = self._check_inputs(left, right)
+        disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
-        key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype))
+        key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
+               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype))
         g = self._graphs.get(key)
         if g is None:
-            g = _GraphedForward(self, left, right, gt)
+            g = _GraphedForward(self, left, right, gt, disp_gt)
             self._graphs[key] = g
-        return g(left, right, gt)
+        return g(left, right, gt, disp_gt)
 
     def _check_inputs(self, left, right):
         if self._packed is None or self._packed_prec != self.precision:
@@ -433,10 +457,27 @@ class _StereoBase(nn.Module):
             raise ValueError('expected left/right of shape [B,3,H,W], got %s / %s' % (tuple(left.shape), tuple(right.shape)))
         return left.contiguous().float(), right.contiguous().float()
 
+    def _check_disp_gt(self, disp_gt, left):
+        """GT disparity of (checked) inputs `left`: fp32 [B,2,H,W] on their device, in input pixels, view 0 = left-referenced
+        (as disp_left), 1 = right-referenced; NaN marks pixels without GT."""
+        if disp_gt is None:
+            return None
+        B, H, W = self._bhw(left)
+        if not isinstance(disp_gt, torch.Tensor):
+            raise ValueError('disp_gt must be a tensor, got %s' % type(disp_gt).__name__)
+        if tuple(disp_gt.shape) != (B, 2, H, W):
+            raise ValueError('expected disp_gt of shape %s, got %s' % ((B, 2, H, W), tuple(disp_gt.shape)))
+        if disp_gt.dtype != torch.float32:
+            raise ValueError('disp_gt must be float32, got %s' % disp_gt.dtype)
+        if disp_gt.device != left.device:
+            raise ValueError('disp_gt must be on %s (the images\' device), got %s' % (left.device, disp_gt.device))
+        return disp_gt.contiguous()
+
 
 class Stereo2Voxel(_StereoBase):
-    """forward(left, right[, gt]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W], voxels [B,32,32,32]
-    [, iou_counts int64 [B,T,2]]).  Outputs are views of the module's workspace: clone to keep them."""
+    """forward(left, right[, gt][, disp_gt=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W], voxels [B,32,32,32]
+    [, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']]).  Outputs are views of the module's workspace: clone to
+    keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views (NaN = none); disp_stats: _StereoBase._upsample_disp."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -475,26 +516,28 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None):
+    def forward(self, left, right, gt=None, *, disp_gt=None):
         left, right = self._check_inputs(left, right)
+        disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
             outs = []
             for s in range(0, B, mb):
-                o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb])
+                o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
+                                        None if disp_gt is None else disp_gt[s:s + mb])
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_chunk(left, right, gt)
+        return self._forward_chunk(left, right, gt, disp_gt)
 
-    def _forward_impl(self, left, right, gt=None):
-        return self._forward_chunk(left, right, gt)
+    def _forward_impl(self, left, right, gt=None, disp_gt=None):
+        return self._forward_chunk(left, right, gt, disp_gt)
 
-    def _forward_chunk(self, left, right, gt):
+    def _forward_chunk(self, left, right, gt, disp_gt=None):
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
-        disp, _ = self._disparity(left, right)
+        disp, _, dstats = self._disparity(left, right, disp_gt)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         k0 = cfg.NETWORK.DEC_CHANNELS[0]
@@ -534,11 +577,14 @@ class Stereo2Voxel(_StereoBase):
                        thresholds=list(cfg.TEST.VOXEL_THRESH) if gt is not None else None, iou=iou, out=fused,
                        score_lo=s.shape[-1] // 2 if self._split else 0, vol_lo=split_lo)
         out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), fused.view(B, nv, nv, nv))
-        return out + (iou,) if gt is not None else out
+        if gt is not None:
+            out += (iou,)
+        return out + (dstats,) if disp_gt is not None else out
 
 
 class Stereo2Point(_StereoBase):
-    """forward(left, right) -> (disp_left, disp_right, points [B,N_POINTS,3])."""
+    """forward(left, right[, disp_gt=]) -> (disp_left, disp_right, points [B,N_POINTS,3][, disp_stats int64 [B,2,2+T]])
+    (disp_gt / disp_stats as for Stereo2Voxel)."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -551,14 +597,14 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right):
+    def forward(self, left, right, *, disp_gt=None):
         left, right = self._check_inputs(left, right)
-        return self._forward_impl(left, right)
+        return self._forward_impl(left, right, disp_gt=self._check_disp_gt(disp_gt, left))
 
-    def _forward_impl(self, left, right):
+    def _forward_impl(self, left, right, disp_gt=None):
         cfg = self.cfg
         B = left.shape[0]
-        disp, _ = self._disparity(left, right)
+        disp, _, dstats = self._disparity(left, right, disp_gt)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         if x.shape[2] != L or x.shape[3] != L:
@@ -577,7 +623,8 @@ class Stereo2Point(_StereoBase):
         npts = cfg.CONST.N_POINTS
         pts = self._buf('pts', (B, 1, 1, 1, pad_to(npts * 3)), torch.float32)
         self._conv('pt_fc2', y, out=pts)
-        return disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3)
+        out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3))
+        return out + (dstats,) if disp_gt is not None else out
 
 
 def build_model(name, cfg, seed=None):

@@ -346,6 +346,26 @@ def upsample_disp(disp_q, H, W, scale, out=None):
     return out
 
 
+def upsample_disp_eval(disp_q, H, W, scale, gt, thresholds, max_gt, stats, out=None):
+    """upsample_disp + evaluation against GT disparity (include/s3d.h, s3d_upsample_disp_eval).  disp_q fp32 [2B,h,w] (left-
+    referenced first) -> disp fp32 [2B,H,W], bit-identical to upsample_disp.  gt fp32 [B,2,H,W] (NaN = no GT).  The per-image
+    counters [n_valid, sum of |disp - gt| in 2^-16 px, count(|disp - gt| > t) per threshold] are ADDED to stats int64
+    [B,2,2+T]."""
+    _chk(disp_q, gt, stats, out)
+    assert disp_q.dtype == torch.float32 and gt.dtype == torch.float32 and stats.dtype == torch.int64
+    N, h, w = disp_q.shape
+    B, T = N // 2, len(thresholds)
+    assert N == 2 * B and tuple(gt.shape) == (B, 2, H, W) and tuple(stats.shape) == (B, 2, 2 + T)
+    if out is None:
+        out = torch.empty((N, H, W), dtype=torch.float32, device=disp_q.device)
+    th = (ctypes.c_float * max(T, 1))(*[float(t) for t in thresholds])
+    rc = _lib.load().s3d_upsample_disp_eval(disp_q.data_ptr(), out.data_ptr(), gt.data_ptr(), th, T, float(max_gt),
+                                            stats.data_ptr(), B, h, w, H, W, float(scale), _stream())
+    _lib.check(rc, 's3d_upsample_disp_eval')
+    _lib.count_launch()
+    return out
+
+
 def latent_to_vox(x, L, out=None, split=False):
     """[N,1,H,W,C] -> pooled to LxL -> [N,2,2,2,C*L*L/8] (oracle's NCHW .view order).  split: hi | lo pairs in and out."""
     _chk(x, out)

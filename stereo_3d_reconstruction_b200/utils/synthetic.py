@@ -18,6 +18,20 @@ def stereo_pair(B, H, W, max_disp_px, seed=0, device='cpu'):
     return left.to(device), right.to(device), d.to(device)
 
 
+def disparity_gt(d, H, W):
+    """GT disparity fp32 [B,2,H,W] of a stereo_pair with per-row disparity d [B,H], in the orientation of the models'
+    disp_left / disp_right; NaN where a pixel has no match in the other view:
+      view 0 (left-referenced):  left[y, x] == right[y, x - d], valid where x - d >= 0;
+      view 1 (right-referenced): right[y, x] == left[y, x + d], valid where x + d < W (stereo_pair zeroes the other pixels)."""
+    B = d.shape[0]
+    assert tuple(d.shape) == (B, H)
+    dd = d.to(torch.float32).view(B, H, 1).expand(B, H, W)
+    x = torch.arange(W, device=d.device).view(1, 1, W)
+    dv = d.view(B, H, 1)
+    nan = torch.full_like(dd, float('nan'))
+    return torch.stack([torch.where(x - dv >= 0, dd, nan), torch.where(x + dv < W, dd, nan)], 1)
+
+
 def gt_volume(B, n_vox=32, p=0.1, seed=1, device='cpu'):
     g = torch.Generator().manual_seed(seed)
     return (torch.rand(B, n_vox, n_vox, n_vox, generator=g) < p).to(torch.uint8).to(device)
