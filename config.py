@@ -87,3 +87,6 @@ __C.TEST = AttrDict()
 __C.TEST.VOXEL_THRESH = [0.2, 0.3, 0.4, 0.5]
 # bad-pixel thresholds of the disparity evaluation (forward(..., disp_gt=...)): |disp - gt| > t px at input resolution
 __C.TEST.DISP_THRESH = [1.0, 3.0]
+# left-right consistency check (forward(..., lr_check=True)): a pixel is kept when its disparity d and the other view's
+# disparity at the pixel it points to (x -/+ round(d)) differ by at most this many px; finite, >= 0
+__C.TEST.LR_THRESH = 1.0

@@ -227,6 +227,18 @@ int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h, int w, int
  * spans two images: the stats do not depend on the launch order, batch split or number of GPUs. */
 int s3d_upsample_disp_eval(const float* disp_q, float* disp, const float* gt, const float* thresholds, int T,
                            float max_gt, long long* stats, int B, int h, int w, int H, int W, float scale, void* stream);
+/* s3d_upsample_disp (+ s3d_upsample_disp_eval when gt is set) + the left-right consistency check of the two views, in one
+ * launch.  disp is bit-identical to s3d_upsample_disp, disp_stats to what s3d_upsample_disp_eval adds.  With D0 / D1 the
+ * left- / right-referenced maps of a sample and d = Dv[y,x] finite, k = round-half-even(d), xo = x - k (view 0) or x + k
+ * (view 1): the pixel is KEPT iff 0 <= xo < W and |d - D(1-v)[y,xo]| <= lr_thresh (fp32 subtraction, one rounding; a NaN
+ * on the other side is not kept).  A non-finite d is not kept; |d| >= W + 1 is out of range.  lr_mask uint8 [B,2,H,W]
+ * (1 = kept).  lr_stats int64 [B,2,3+T], ACCUMULATED:
+ *   [n_kept, n_valid_kept, sum_{valid & kept} q(|disp - gt|), count_{valid & kept}(|disp - gt| > thresholds[t]) for t < T]
+ * (valid and q as for s3d_upsample_disp_eval).  gt == NULL needs disp_stats == NULL and adds column 0 only; T still sets the
+ * row length.  lr_thresh must be >= 0. */
+int s3d_upsample_disp_lr(const float* disp_q, float* disp, uint8_t* lr_mask, float lr_thresh, const float* gt,
+                         const float* thresholds, int T, float max_gt, long long* disp_stats, long long* lr_stats,
+                         int B, int h, int w, int H, int W, float scale, void* stream);
 
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)

@@ -26,6 +26,8 @@ def get_args():
     p.add_argument('--precision', default=None, choices=['bf16', 'bf16x3', 'tf32', 'tf32x3', 'fp32'])
     p.add_argument('--batch-size', type=int, default=None)
     p.add_argument('--n-samples', type=int, default=None, help='synthetic test-set size (default: one batch per rank)')
+    p.add_argument('--lr-check', action='store_true',
+                   help='also run the left-right disparity consistency check and report it as lr_consistency')
     return p.parse_args()
 
 
@@ -94,14 +96,19 @@ def main():
     model.cuda().pack()
     # one stats vector: the head's statistics, then the disparity counters of the same forwards
     if args.model == 'Stereo2Voxel':
-        stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True).cpu()
+        stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check).cpu()
         nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
         res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
     else:
-        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True).cpu()
+        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check).cpu()
         nh = 2
         res = T.chamfer_summary(stats[:nh])
-    res['disparity'] = T.disp_summary(stats[nh:], cfg.TEST.DISP_THRESH)
+    nd = 2 * (2 + len(cfg.TEST.DISP_THRESH))
+    res['disparity'] = T.disp_summary(stats[nh:nh + nd], cfg.TEST.DISP_THRESH)
+    if args.lr_check:
+        res['lr_consistency'] = T.lr_summary(stats[nh + nd:], cfg.TEST.DISP_THRESH,
+                                             res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
+        res['lr_consistency']['lr_thresh'] = float(cfg.TEST.LR_THRESH)
     if rank == 0:
         res.update(model=args.model, precision=cfg.NETWORK.PRECISION, world_size=world, data='synthetic')
         print(json.dumps(res))

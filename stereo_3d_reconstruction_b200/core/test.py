@@ -9,6 +9,8 @@ Chamfer: sum_b CD(b) is accumulated in fp64 and reduced as a fixed-point int64 (
 With eval_disp=True the same vector carries, per view (left-referenced, then right-referenced), the disparity counters the
 forward computes against the synthetic GT disparity (models.py, _StereoBase._upsample_disp):
     n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) per t in TEST.DISP_THRESH   (int64)
+With eval_lr=True (needs eval_disp) the left-right consistency counters of the same forwards follow, per view:
+    n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the kept valid pixels  (int64)
 """
 import torch
 import torch.distributed as dist
@@ -59,18 +61,50 @@ def disp_summary(stats_block, thresholds):
     return out
 
 
+def lr_summary(stats_block, thresholds, n_pixels, disp_block):
+    """LR-check counters [n_kept, n_valid_kept, epe_fx, bad_t...] x 2 views (int64 [2 * (3 + T)]) -> dict, per view and over
+    both views: density = n_kept / n_pixels (n_pixels: pixels of one view over the run), kept_of_valid = n_valid_kept /
+    n_valid (n_valid from the disparity counters `disp_block`, as for disp_summary), and EPE / bad-pixel fractions over the
+    kept valid pixels."""
+    T = len(thresholds)
+    v = [int(x) for x in stats_block.tolist()]
+    nv = [int(x) for x in disp_block.tolist()]
+    assert len(v) == 2 * (3 + T) and len(nv) == 2 * (2 + T)
+
+    def one(pix, n_valid, c):
+        nk, nvk, epe_fx, bad = c[0], c[1], c[2], c[3:]
+        return {'n_kept': nk, 'density': nk / pix if pix else 0.0, 'n_valid_kept': nvk,
+                'kept_of_valid': nvk / n_valid if n_valid else 0.0, 'epe': epe_fx / _DISP_FX / nvk if nvk else 0.0,
+                'bad': [b / nvk if nvk else 0.0 for b in bad]}
+    views = [v[:3 + T], v[3 + T:]]
+    valid = [nv[0], nv[2 + T]]
+    out = {'thresholds': list(thresholds)}
+    for name, c, n in zip(('left', 'right'), views, valid):
+        out[name] = one(n_pixels, n, c)
+    out['all'] = one(2 * n_pixels, valid[0] + valid[1], [a + b for a, b in zip(views[0], views[1])])
+    return out
+
+
 def _disp_gt(pairs, H, W, device):
     return torch.cat([synthetic.disparity_gt(p[2], H, W) for p in pairs]).to(device)
 
 
-def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False):
+def _lr_len(cfg, eval_disp, eval_lr):
+    if eval_lr and not eval_disp:
+        raise ValueError('eval_lr=True needs eval_disp=True')
+    return 2 * (3 + len(cfg.TEST.DISP_THRESH)) if eval_lr else 0
+
+
+def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
-    eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring)."""
+    eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
+    eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones."""
     th = list(cfg.TEST.VOXEL_THRESH)
     T = len(th)
+    nl = _lr_len(cfg, eval_disp, eval_lr)
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    stats = torch.zeros(2 * T + 1 + nd, dtype=torch.int64, device=device)
+    stats = torch.zeros(2 * T + 1 + nd + nl, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -80,7 +114,11 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.gt_volume(1, cfg.CONST.N_VOX, seed=100000 + i) for i in ids]).to(device)
-            if eval_disp:
+            if eval_lr:
+                _, _, _, iou, ds, _, ls = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
+                stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
+                stats[2 * T + 1 + nd:] += ls.sum(0).flatten()
+            elif eval_disp:
                 _, _, _, iou, ds = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device))
                 stats[2 * T + 1:] += ds.sum(0).flatten()
             else:
@@ -91,11 +129,13 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
     return reduce_stats(stats)
 
 
-def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False):
-    """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, as for test_voxel)."""
+def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False):
+    """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, as
+    for test_voxel)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
+    nl = _lr_len(cfg, eval_disp, eval_lr)
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    stats = torch.zeros(2 + nd, dtype=torch.int64, device=device)
+    stats = torch.zeros(2 + nd + nl, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -105,7 +145,11 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.point_clouds(1, 1, cfg.CONST.N_GT_POINTS, seed=200000 + i)[1] for i in ids]).to(device)
-            if eval_disp:
+            if eval_lr:
+                _, _, pts, ds, _, ls = model(left, right, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
+                stats[2:2 + nd] += ds.sum(0).flatten()
+                stats[2 + nd:] += ls.sum(0).flatten()
+            elif eval_disp:
                 _, _, pts, ds = model(left, right, disp_gt=_disp_gt(pairs, H, W, device))
                 stats[2:] += ds.sum(0).flatten()
             else:

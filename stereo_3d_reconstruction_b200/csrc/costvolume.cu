@@ -365,9 +365,10 @@ upsample_disp_v4_kernel(const float* __restrict__ q, float4* __restrict__ out, u
 }
 
 // ------------------------------------------------------------------------------------------
-// upsample + evaluation against GT disparity.  Each block covers part of ONE (sample, view) image (blockIdx.y = image),
-// so its counters belong to one row of `stats`; the per-thread counters are integers, reduced by warp shuffle ->
-// shared memory -> one 64-bit atomic per counter per block: any order of atomics gives the same sums.
+// upsample + evaluation against GT disparity (kEval) and / or the left-right consistency check (kLR).  Each block covers
+// part of ONE (sample, view) image (blockIdx.y = image), so its counters belong to one row of `stats` / `lr_stats`; the
+// per-thread counters are integers, reduced by warp shuffle -> shared memory -> one 64-bit atomic per counter per block:
+// any order of atomics gives the same sums.
 // ------------------------------------------------------------------------------------------
 struct DispCounters {
   unsigned n_valid = 0;
@@ -384,71 +385,151 @@ struct DispCounters {
       if (t < nT) bad[t] += e > th.t[t];
   }
 
-  // -> dst[0 .. 2+nT) of the block's image; every thread of the block calls it
-  __device__ __forceinline__ void flush(unsigned long long* __restrict__ dst, int nT) {
-    __shared__ unsigned long long blk[2 + kMaxThresh];
-    if (threadIdx.x < 2 + kMaxThresh) blk[threadIdx.x] = 0;
+  // -> dst[0 .. n) of the block's image, n <= kLead + 2 + nT, as [lead (kLead = 1 only), n_valid, epe_fx, bad...]; every
+  // thread of the block calls it.  The shared array belongs to the instantiation, so a kernel may flush a <0> and a <1> set
+  // back to back.
+  template <int kLead = 0>
+  __device__ __forceinline__ void flush(unsigned long long* __restrict__ dst, int n, unsigned lead = 0) {
+    constexpr int kN = kLead + 2 + kMaxThresh;
+    __shared__ unsigned long long blk[kN];
+    if (threadIdx.x < kN) blk[threadIdx.x] = 0;
     __syncthreads();
-    unsigned long long v[2 + kMaxThresh];
-    v[0] = n_valid;  v[1] = epe_fx;
+    unsigned long long v[kN];
+    v[0] = lead;
+    v[kLead] = n_valid;  v[kLead + 1] = epe_fx;
 #pragma unroll
-    for (int t = 0; t < kMaxThresh; ++t) v[2 + t] = bad[t];
+    for (int t = 0; t < kMaxThresh; ++t) v[kLead + 2 + t] = bad[t];
 #pragma unroll
-    for (int k = 0; k < 2 + kMaxThresh; ++k) {
-      if (k >= 2 + nT) break;
+    for (int k = 0; k < kN; ++k) {
+      if (k >= n) break;
       unsigned long long a = v[k];
       for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
       if ((threadIdx.x & 31) == 0 && a) atomicAdd(&blk[k], a);
     }
     __syncthreads();
-    if ((int)threadIdx.x < 2 + nT && blk[threadIdx.x]) atomicAdd(dst + threadIdx.x, blk[threadIdx.x]);
+    if ((int)threadIdx.x < n && blk[threadIdx.x]) atomicAdd(dst + threadIdx.x, blk[threadIdx.x]);
   }
 };
 
-// image n of [2B]: view = n / B (0 = left-referenced), sample b = n % B; gt [B,2,H,W], stats [B,2,2+nT]
+// image n of [2B]: view = n / B (0 = left-referenced), sample b = n % B; gt / lr_mask [B,2,H,W], stats [B,2,2+nT],
+// lr_stats [B,2,3+nT]
 __device__ __forceinline__ int64_t eval_image_index(int n, int B) { return (int64_t)(n % B) * 2 + n / B; }
 
+// Left-right consistency of the pixel at column X whose stored disparity is d (include/s3d.h, s3d_upsample_disp_lr).  `ro`:
+// the OTHER view's source rows of the same output row, so up_px gives the value the other image's blocks store at xo.
+// dir = -1 for view 0 (xo = X - k), +1 for view 1 (xo = X + k).
+__device__ __forceinline__ bool lr_kept(float d, int X, const UpRow& ro, int w, int W, float rx, float scale, int dir,
+                                        float tau) {
+  if (!(fabsf(d) < (float)(W + 1))) return false;       // NaN / inf, or |k| > W: xo out of range (and no int overflow)
+  const int xo = X + dir * __float2int_rn(d);            // round half to even
+  if (xo < 0 || xo >= W) return false;
+  return fabsf(__fsub_rn(d, up_px(ro, xo, w, rx, scale))) <= tau;     // NaN on the other side: not kept
+}
+
+template <bool kEval, bool kLR>
 __global__ void __launch_bounds__(256)
 upsample_disp_eval_v4_kernel(const float* __restrict__ q, float4* __restrict__ out, const float4* __restrict__ gt, int B, int h,
                              int w, int H, int W4, float ry, float rx, float scale, Thresh th, int nT, float max_gt,
-                             unsigned long long* __restrict__ stats) {
+                             unsigned long long* __restrict__ stats, uint32_t* __restrict__ lr_mask, float lr_thresh,
+                             unsigned long long* __restrict__ lr_stats) {
   const int n = blockIdx.y;
   const int64_t img4 = (int64_t)H * W4;
   const float* q_img = q + (int64_t)n * h * w;
+  const int64_t q_other = (int64_t)(n < B ? B : -B) * h * w;        // the other view's 1/4-res image, relative to q_img
+  const int dir = n < B ? -1 : 1;
   float4* out_img = out + n * img4;
-  const float4* gt_img = gt + eval_image_index(n, B) * img4;
-  DispCounters c;
+  const float4* gt_img = kEval ? gt + eval_image_index(n, B) * img4 : nullptr;
+  uint32_t* mask_img = kLR ? lr_mask + eval_image_index(n, B) * img4 : nullptr;
+  DispCounters c, kc;                                               // all pixels / the kept ones (kLR)
+  unsigned n_kept = 0;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < (uint32_t)img4; i += gridDim.x * blockDim.x) {
     const uint32_t X4 = i % (uint32_t)W4, Y = i / (uint32_t)W4;
-    const float4 g = __ldcs(gt_img + i);                            // read once: keep it out of L2
+    float4 g4 = {};
+    if (kEval) g4 = __ldcs(gt_img + i);                             // read once: keep it out of L2
     const UpRow r = up_row(q_img, (int)Y, h, w, ry);
     float o[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) o[k] = up_px(r, 4 * (int)X4 + k, w, rx, scale);
     out_img[i] = make_float4(o[0], o[1], o[2], o[3]);
-    c.add(o[0], g.x, max_gt, th, nT);  c.add(o[1], g.y, max_gt, th, nT);
-    c.add(o[2], g.z, max_gt, th, nT);  c.add(o[3], g.w, max_gt, th, nT);
+    const float g[4] = {g4.x, g4.y, g4.z, g4.w};
+    if (kEval) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) c.add(o[k], g[k], max_gt, th, nT);
+    }
+    if (kLR) {
+      const UpRow ro = {r.p0 + q_other, r.p1 + q_other, r.ly, r.hy};  // same output row Y, same weights
+      uint32_t m = 0;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const bool keep = lr_kept(o[k], 4 * (int)X4 + k, ro, w, 4 * W4, rx, scale, dir, lr_thresh);
+        m |= (uint32_t)keep << (8 * k);
+        n_kept += keep;
+        if (kEval && keep) kc.add(o[k], g[k], max_gt, th, nT);
+      }
+      mask_img[i] = m;                                              // four mask bytes, one 32-bit store
+    }
   }
-  c.flush(stats + eval_image_index(n, B) * (2 + nT), nT);
+  if (kEval) c.flush(stats + eval_image_index(n, B) * (2 + nT), 2 + nT);
+  if (kLR) kc.flush<1>(lr_stats + eval_image_index(n, B) * (3 + nT), kEval ? 3 + nT : 1, n_kept);
 }
 
+template <bool kEval, bool kLR>
 __global__ void __launch_bounds__(256)
 upsample_disp_eval_kernel(const float* __restrict__ q, float* __restrict__ out, const float* __restrict__ gt, int B, int h, int w,
-                          int H, int W, float scale, Thresh th, int nT, float max_gt, unsigned long long* __restrict__ stats) {
+                          int H, int W, float scale, Thresh th, int nT, float max_gt, unsigned long long* __restrict__ stats,
+                          uint8_t* __restrict__ lr_mask, float lr_thresh, unsigned long long* __restrict__ lr_stats) {
   const int n = blockIdx.y;
   const int img = H * W;                                            // < 2^31 (checked by the launcher)
   const float ry = (float)h / (float)H, rx = (float)w / (float)W;
   const float* q_img = q + (int64_t)n * h * w;
+  const int64_t q_other = (int64_t)(n < B ? B : -B) * h * w;
+  const int dir = n < B ? -1 : 1;
   float* out_img = out + (int64_t)n * img;
-  const float* gt_img = gt + eval_image_index(n, B) * img;
-  DispCounters c;
+  const float* gt_img = kEval ? gt + eval_image_index(n, B) * img : nullptr;
+  uint8_t* mask_img = kLR ? lr_mask + eval_image_index(n, B) * img : nullptr;
+  DispCounters c, kc;
+  unsigned n_kept = 0;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < img; i += gridDim.x * blockDim.x) {
     const int X = i % W, Y = i / W;
-    const float d = up_px(up_row(q_img, Y, h, w, ry), X, w, rx, scale);
+    const UpRow r = up_row(q_img, Y, h, w, ry);
+    const float d = up_px(r, X, w, rx, scale);
     out_img[i] = d;
-    c.add(d, __ldcs(gt_img + i), max_gt, th, nT);
+    const float g = kEval ? __ldcs(gt_img + i) : 0.f;
+    if (kEval) c.add(d, g, max_gt, th, nT);
+    if (kLR) {
+      const UpRow ro = {r.p0 + q_other, r.p1 + q_other, r.ly, r.hy};
+      const bool keep = lr_kept(d, X, ro, w, W, rx, scale, dir, lr_thresh);
+      mask_img[i] = keep;
+      n_kept += keep;
+      if (kEval && keep) kc.add(d, g, max_gt, th, nT);
+    }
   }
-  c.flush(stats + eval_image_index(n, B) * (2 + nT), nT);
+  if (kEval) c.flush(stats + eval_image_index(n, B) * (2 + nT), 2 + nT);
+  if (kLR) kc.flush<1>(lr_stats + eval_image_index(n, B) * (3 + nT), kEval ? 3 + nT : 1, n_kept);
+}
+
+// Shared launcher of s3d_upsample_disp_eval (kEval) and s3d_upsample_disp_lr (kLR, kEval when it has GT); arguments checked.
+template <bool kEval, bool kLR>
+int launch_upsample_eval(const float* disp_q, float* disp, const float* gt, const Thresh& th, int T, float max_gt,
+                         long long* stats, uint8_t* lr_mask, float lr_thresh, long long* lr_stats, int B, int h, int w, int H,
+                         int W, float scale, cudaStream_t s) {
+  const int64_t img = (int64_t)H * W;
+  auto* st = reinterpret_cast<unsigned long long*>(stats);
+  auto* lst = reinterpret_cast<unsigned long long*>(lr_stats);
+  if (W % 4 == 0 && ((reinterpret_cast<uintptr_t>(disp) | reinterpret_cast<uintptr_t>(gt)) & 15) == 0 &&
+      (reinterpret_cast<uintptr_t>(lr_mask) & 3) == 0) {
+    // 16 outputs per thread: 4x fewer blocks (and counter atomics) than one vector per thread
+    const dim3 grid((unsigned)ceil_div64(img / 4, 256 * 4), 2 * B);
+    upsample_disp_eval_v4_kernel<kEval, kLR><<<grid, 256, 0, s>>>(
+        disp_q, reinterpret_cast<float4*>(disp), reinterpret_cast<const float4*>(gt), B, h, w, H, W / 4, (float)h / (float)H,
+        (float)w / (float)W, scale, th, T, max_gt, st, reinterpret_cast<uint32_t*>(lr_mask), lr_thresh, lst);
+    S3D_LAUNCH_CHECK();
+    return S3D_OK;
+  }
+  upsample_disp_eval_kernel<kEval, kLR><<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * B), 256, 0, s>>>(
+      disp_q, disp, gt, B, h, w, H, W, scale, th, T, max_gt, st, lr_mask, lr_thresh, lst);
+  S3D_LAUNCH_CHECK();
+  return S3D_OK;
 }
 
 }  // namespace
@@ -568,21 +649,31 @@ extern "C" int s3d_upsample_disp_eval(const float* disp_q, float* disp, const fl
   S3D_CHECK_ARG(max_gt > 0.f, "upsample_disp_eval: max_gt must be > 0");
   Thresh th;
   for (int t = 0; t < kMaxThresh; ++t) th.t[t] = t < T ? thresholds[t] : 0.f;
-  const int64_t img = (int64_t)H * W;
-  auto* st = reinterpret_cast<unsigned long long*>(stats);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (W % 4 == 0 && ((reinterpret_cast<uintptr_t>(disp) | reinterpret_cast<uintptr_t>(gt)) & 15) == 0) {
-    // 16 outputs per thread: 4x fewer blocks (and counter atomics) than one vector per thread
-    const dim3 grid((unsigned)ceil_div64(img / 4, 256 * 4), 2 * B);
-    upsample_disp_eval_v4_kernel<<<grid, 256, 0, s>>>(disp_q, reinterpret_cast<float4*>(disp), reinterpret_cast<const float4*>(gt),
-                                                      B, h, w, H, W / 4, (float)h / (float)H, (float)w / (float)W, scale, th, T,
-                                                      max_gt, st);
-    S3D_LAUNCH_CHECK();
-    return S3D_OK;
+  return launch_upsample_eval<true, false>(disp_q, disp, gt, th, T, max_gt, stats, nullptr, 0.f, nullptr, B, h, w, H, W, scale,
+                                           static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int s3d_upsample_disp_lr(const float* disp_q, float* disp, uint8_t* lr_mask, float lr_thresh, const float* gt,
+                                    const float* thresholds, int T, float max_gt, long long* disp_stats, long long* lr_stats,
+                                    int B, int h, int w, int H, int W, float scale, void* stream) {
+  if (!disp_q || !disp || !lr_mask || !lr_stats || (gt && T > 0 && !thresholds)) {
+    set_error("upsample_disp_lr: null argument");
+    return S3D_ERR_INVALID;
   }
-  upsample_disp_eval_kernel<<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * B), 256, 0, s>>>(disp_q, disp, gt, B, h, w, H, W, scale, th, T, max_gt, st);
-  S3D_LAUNCH_CHECK();
-  return S3D_OK;
+  S3D_CHECK_ARG(!gt == !disp_stats, "upsample_disp_lr: gt and disp_stats must be both set or both NULL");
+  S3D_CHECK_ARG(B > 0 && 2 * B < 65536 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31),
+                "upsample_disp_lr: bad shape");
+  S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "upsample_disp_lr: T must be in [0, 8]");
+  S3D_CHECK_ARG(lr_thresh >= 0.f, "upsample_disp_lr: lr_thresh must be >= 0 (and not NaN)");
+  S3D_CHECK_ARG(!gt || max_gt > 0.f, "upsample_disp_lr: max_gt must be > 0");
+  Thresh th;
+  for (int t = 0; t < kMaxThresh; ++t) th.t[t] = gt && t < T ? thresholds[t] : 0.f;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (gt)
+    return launch_upsample_eval<true, true>(disp_q, disp, gt, th, T, max_gt, disp_stats, lr_mask, lr_thresh, lr_stats, B, h, w,
+                                            H, W, scale, s);
+  return launch_upsample_eval<false, true>(disp_q, disp, nullptr, th, T, 0.f, nullptr, lr_mask, lr_thresh, lr_stats, B, h, w, H,
+                                           W, scale, s);
 }
 
 extern "C" int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* cost_out, int N, int D, int h, int w,

@@ -11,6 +11,7 @@ The torch.nn layers below are PARAMETER CONTAINERS only -- their forward is neve
 folds BatchNorm and re-lays every weight for the tcgen05 implicit-GEMM engine once; `forward()` is a
 sequence of C-ABI calls (include/s3d.h) on the current CUDA stream, with no torch math on the path.
 """
+import math
 import os
 
 import torch
@@ -134,15 +135,17 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt, disp_gt=None):
+    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
         self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
         self._copy_in(left, right, gt, disp_gt)
         args = (self.left, self.right) if gt is None else (self.left, self.right, self.gt)
         kw = {} if disp_gt is None else {'disp_gt': self.disp_gt}
+        if lr_check:
+            kw['lr_check'] = True
 
-        def run():                                    # zeroes its IoU / disparity counters itself: inside the graph
+        def run():                                    # zeroes its IoU / disparity / LR counters itself: inside the graph
             return model._forward_impl(*args, **kw)
         side = torch.cuda.Stream(device=left.device)
         side.wait_stream(torch.cuda.current_stream())
@@ -273,9 +276,9 @@ class _StereoBase(nn.Module):
     def _bhw(img):
         return (img.shape[0], img.shape[1], img.shape[2]) if img.dtype == torch.uint8 else (img.shape[0], img.shape[2], img.shape[3])
 
-    def _disparity(self, left, right, disp_gt=None):
-        """-> disp fp32 [2B,H,W] (left-referenced first), in input pixels, disp_q, and the disparity stats int64
-        [B,2,2+T] against disp_gt (None without it; see _upsample_disp)."""
+    def _disparity(self, left, right, disp_gt=None, lr_check=False):
+        """-> disp fp32 [2B,H,W] (left-referenced first), in input pixels, disp_q, the disparity stats int64 [B,2,2+T]
+        against disp_gt (None without it) and the LR check's (lr_mask, lr_stats) (None without lr_check; see _upsample_disp)."""
         cfg = self.cfg
         B, H, W = self._bhw(left)
         D = cfg.NETWORK.MAX_DISP
@@ -353,8 +356,8 @@ class _StereoBase(nn.Module):
                 nb = ops.conv_cls_workspace_bytes(2 * B, D, h, w)
                 ops.conv_cls_soft_argmin(pa, a, self._packed['cls_b'].weight, -1.0, out=disp_q,
                                          workspace=self._buf('cls_ws', (nb,), torch.uint8))
-                disp, stats = self._upsample_disp(disp_q, H, W, disp_gt)
-                return disp, disp_q, stats
+                disp, stats, lr = self._upsample_disp(disp_q, H, W, disp_gt, lr_check)
+                return disp, disp_q, stats, lr
             c = self._conv('cls_a', a, out=self._bufo('a0', 'cls_a', a))
             if self.precision == 'bf16' and c.shape[-1] in (16, 32, 64) and S == 32 and not _lib.KNOBS['no_cls_fused']:
                 # classifier + soft-argmin in one pass over the volume (csrc/cls_fused.cu)
@@ -367,22 +370,39 @@ class _StereoBase(nn.Module):
             if self._split:                                               # exact fp32 correlation on hi + lo
                 feat = ops.unsplit_bf16(feat, out=self._buf('feat32', feat.shape[:-1] + (feat.shape[-1] // 2,), torch.float32))
             ops.corr_soft_argmin(feat, B, D, out=disp_q, c_real=C)       # mean over the REAL channels (feat is padded)
-        disp, stats = self._upsample_disp(disp_q, H, W, disp_gt)
-        return disp, disp_q, stats
+        disp, stats, lr = self._upsample_disp(disp_q, H, W, disp_gt, lr_check)
+        return disp, disp_q, stats, lr
 
-    def _upsample_disp(self, disp_q, H, W, disp_gt):
+    def _upsample_disp(self, disp_q, H, W, disp_gt, lr_check=False):
         """Last kernel of the disparity stage: 1/4-res disparity -> input pixels [2B,H,W].  With disp_gt [B,2,H,W] the same
         kernel also counts, per sample and view, [n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) for t in
-        TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> (disp, stats int64 [B,2,2+T]); else (disp, None)."""
+        TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> stats int64 [B,2,2+T] (else None).  With lr_check it
+        also runs the left-right consistency check (include/s3d.h, s3d_upsample_disp_lr; tolerance TEST.LR_THRESH px) ->
+        lr = (lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T]: [n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and
+        count(|disp - gt| > t) over the kept valid pixels]; GT columns zero without disp_gt) (else None).
+        -> (disp, stats, lr)."""
         B = disp_q.shape[0] // 2
         out = self._buf('disp', (2 * B, H, W), torch.float32)
-        if disp_gt is None:
-            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None
         th = list(self.cfg.TEST.DISP_THRESH)
-        stats = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64)
-        stats.zero_()
-        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, 4.0 * self.cfg.NETWORK.MAX_DISP, stats, out=out)
-        return out, stats
+        stats = None
+        if disp_gt is not None:
+            stats = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64)
+            stats.zero_()
+        max_gt = 4.0 * self.cfg.NETWORK.MAX_DISP
+        if lr_check:
+            tau = float(self.cfg.TEST.LR_THRESH)
+            if not (math.isfinite(tau) and tau >= 0):
+                raise ValueError('TEST.LR_THRESH must be finite and >= 0, got %r' % self.cfg.TEST.LR_THRESH)
+            mask = self._buf('lr_mask', (B, 2, H, W), torch.uint8)
+            lr_stats = self._buf('lr_stats', (B, 2, 3 + len(th)), torch.int64)
+            lr_stats.zero_()
+            ops.upsample_disp_lr(disp_q, H, W, 4.0, tau, mask, lr_stats, gt=disp_gt, thresholds=th, max_gt=max_gt, stats=stats,
+                                 out=out)
+            return out, stats, (mask, lr_stats)
+        if disp_gt is None:
+            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None, None
+        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, max_gt, stats, out=out)
+        return out, stats, None
 
     def _bufo(self, name, layer, x):
         """Output buffer of `layer` for input x (channels-last, padded channels)."""
@@ -423,7 +443,7 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -436,10 +456,10 @@ class _StereoBase(nn.Module):
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
         key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
-               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype))
+               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check))
         g = self._graphs.get(key)
         if g is None:
-            g = _GraphedForward(self, left, right, gt, disp_gt)
+            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check))
             self._graphs[key] = g
         return g(left, right, gt, disp_gt)
 
@@ -475,9 +495,11 @@ class _StereoBase(nn.Module):
 
 
 class Stereo2Voxel(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W], voxels [B,32,32,32]
-    [, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']]).  Outputs are views of the module's workspace: clone to
-    keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views (NaN = none); disp_stats: _StereoBase._upsample_disp."""
+    """forward(left, right[, gt][, disp_gt=][, lr_check=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W], voxels [B,32,32,32]
+    [, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T']]).
+    Outputs are views of the module's workspace: clone to keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views
+    (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; disp_stats, lr_mask, lr_stats:
+    _StereoBase._upsample_disp."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -516,7 +538,7 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False):
         left, right = self._check_inputs(left, right)
         disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
@@ -525,19 +547,19 @@ class Stereo2Voxel(_StereoBase):
             outs = []
             for s in range(0, B, mb):
                 o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
-                                        None if disp_gt is None else disp_gt[s:s + mb])
+                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check)
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_chunk(left, right, gt, disp_gt)
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check)
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None):
-        return self._forward_chunk(left, right, gt, disp_gt)
+    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False):
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check)
 
-    def _forward_chunk(self, left, right, gt, disp_gt=None):
+    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False):
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
-        disp, _, dstats = self._disparity(left, right, disp_gt)
+        disp, _, dstats, lr = self._disparity(left, right, disp_gt, lr_check)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         k0 = cfg.NETWORK.DEC_CHANNELS[0]
@@ -579,12 +601,14 @@ class Stereo2Voxel(_StereoBase):
         out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), fused.view(B, nv, nv, nv))
         if gt is not None:
             out += (iou,)
-        return out + (dstats,) if disp_gt is not None else out
+        if disp_gt is not None:
+            out += (dstats,)
+        return out + lr if lr_check else out
 
 
 class Stereo2Point(_StereoBase):
-    """forward(left, right[, disp_gt=]) -> (disp_left, disp_right, points [B,N_POINTS,3][, disp_stats int64 [B,2,2+T]])
-    (disp_gt / disp_stats as for Stereo2Voxel)."""
+    """forward(left, right[, disp_gt=][, lr_check=]) -> (disp_left, disp_right, points [B,N_POINTS,3]
+    [, disp_stats int64 [B,2,2+T]][, lr_mask, lr_stats]) (disp_gt, lr_check and the extra outputs as for Stereo2Voxel)."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -597,14 +621,14 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, *, disp_gt=None):
+    def forward(self, left, right, *, disp_gt=None, lr_check=False):
         left, right = self._check_inputs(left, right)
-        return self._forward_impl(left, right, disp_gt=self._check_disp_gt(disp_gt, left))
+        return self._forward_impl(left, right, disp_gt=self._check_disp_gt(disp_gt, left), lr_check=lr_check)
 
-    def _forward_impl(self, left, right, disp_gt=None):
+    def _forward_impl(self, left, right, disp_gt=None, lr_check=False):
         cfg = self.cfg
         B = left.shape[0]
-        disp, _, dstats = self._disparity(left, right, disp_gt)
+        disp, _, dstats, lr = self._disparity(left, right, disp_gt, lr_check)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         if x.shape[2] != L or x.shape[3] != L:
@@ -624,7 +648,9 @@ class Stereo2Point(_StereoBase):
         pts = self._buf('pts', (B, 1, 1, 1, pad_to(npts * 3)), torch.float32)
         self._conv('pt_fc2', y, out=pts)
         out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3))
-        return out + (dstats,) if disp_gt is not None else out
+        if disp_gt is not None:
+            out += (dstats,)
+        return out + lr if lr_check else out
 
 
 def build_model(name, cfg, seed=None):

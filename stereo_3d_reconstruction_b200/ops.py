@@ -366,6 +366,34 @@ def upsample_disp_eval(disp_q, H, W, scale, gt, thresholds, max_gt, stats, out=N
     return out
 
 
+def upsample_disp_lr(disp_q, H, W, scale, lr_thresh, mask, lr_stats, gt=None, thresholds=(), max_gt=0.0, stats=None, out=None):
+    """upsample_disp + the left-right consistency check of the two views (include/s3d.h, s3d_upsample_disp_lr), and with gt
+    the evaluation of upsample_disp_eval, in one launch.  disp_q fp32 [2B,h,w] (left-referenced first) -> disp fp32 [2B,H,W],
+    bit-identical to upsample_disp.  mask uint8 [B,2,H,W] <- 1 where the pixel is kept.  lr_stats int64 [B,2,3+T] (T =
+    len(thresholds)) += [n_kept, n_valid_kept, sum of |disp - gt| in 2^-16 px over valid & kept, count(|disp - gt| > t) over
+    valid & kept]; without gt only column 0.  gt fp32 [B,2,H,W] and stats int64 [B,2,2+T] come together (stats += what
+    upsample_disp_eval adds)."""
+    _chk(disp_q, mask, lr_stats, gt, stats, out)
+    assert disp_q.dtype == torch.float32 and mask.dtype == torch.uint8 and lr_stats.dtype == torch.int64
+    assert (gt is None) == (stats is None)
+    N, h, w = disp_q.shape
+    B, T = N // 2, len(thresholds)
+    assert N == 2 * B and tuple(mask.shape) == (B, 2, H, W) and tuple(lr_stats.shape) == (B, 2, 3 + T)
+    if gt is not None:
+        assert gt.dtype == torch.float32 and stats.dtype == torch.int64
+        assert tuple(gt.shape) == (B, 2, H, W) and tuple(stats.shape) == (B, 2, 2 + T)
+    if out is None:
+        out = torch.empty((N, H, W), dtype=torch.float32, device=disp_q.device)
+    th = (ctypes.c_float * max(T, 1))(*[float(t) for t in thresholds])
+    rc = _lib.load().s3d_upsample_disp_lr(disp_q.data_ptr(), out.data_ptr(), mask.data_ptr(), float(lr_thresh),
+                                          None if gt is None else gt.data_ptr(), th, T, float(max_gt),
+                                          None if stats is None else stats.data_ptr(), lr_stats.data_ptr(), B, h, w, H, W,
+                                          float(scale), _stream())
+    _lib.check(rc, 's3d_upsample_disp_lr')
+    _lib.count_launch()
+    return out
+
+
 def latent_to_vox(x, L, out=None, split=False):
     """[N,1,H,W,C] -> pooled to LxL -> [N,2,2,2,C*L*L/8] (oracle's NCHW .view order).  split: hi | lo pairs in and out."""
     _chk(x, out)
