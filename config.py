@@ -90,3 +90,7 @@ __C.TEST.DISP_THRESH = [1.0, 3.0]
 # left-right consistency check (forward(..., lr_check=True)): a pixel is kept when its disparity d and the other view's
 # disparity at the pixel it points to (x -/+ round(d)) differ by at most this many px; finite, >= 0
 __C.TEST.LR_THRESH = 1.0
+# F-score thresholds of the point-cloud evaluation (Stereo2Point forward(..., gt)): a point counts when its nearest neighbour
+# in the other cloud is closer than t, a Euclidean distance in the points' units (0.01 = F-Score@1% on unit-scale shapes);
+# at most 8, each finite and > 0
+__C.TEST.FSCORE_THRESH = [0.01]

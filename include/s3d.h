@@ -287,6 +287,20 @@ int64_t s3d_chamfer_workspace_bytes(int B, int N, int M);
 int s3d_chamfer_forward_ws(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1,
                            float* dist2, int32_t* idx2, int B, int N, int M, void* workspace,
                            int64_t workspace_bytes, void* stream);
+/* Chamfer search of s3d_chamfer_forward_ws (same dist / idx outputs, bit for bit) + per-sample point-cloud metrics.
+ * xyz1 = predicted [B,N,3], xyz2 = GT [B,M,3].  stats int64 [B,2,3+T] is ADDED to (caller zeroes):
+ *   direction 0 = xyz1 -> xyz2 (dist1), direction 1 = xyz2 -> xyz1 (dist2); per direction
+ *   [ sum q(d), sum q(sqrt_rn(d)), n_out, count(sqrt_rn(d) < tau_t) for t < T ]   over the points with d in range.
+ * d is the squared distance written to dist1 / dist2.  In range: d finite and d < 2^8; every other point (a NaN point gets
+ * d = +inf) counts in n_out only.  q(x) = round-half-even(x * 2^32) as int64 (the product is exact in fp32); sqrt_rn is the
+ * correctly rounded fp32 square root.  A point counts at tau_t when sqrt_rn(d) < tau_t in fp32, strictly: the thresholds
+ * are Euclidean distances in the points' units.  tau: T <= 8 HOST values, each finite and > 0.  N, M < 2^22, so a
+ * (sample, direction) sum of q < 2^40 stays inside int64.  The counters are integers summed with one atomic per counter
+ * per block, no block spanning two (sample, direction) slices: they do not depend on the launch order or batch split.
+ * One kernel after the search, over the distances it has just written. */
+int s3d_chamfer_eval(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2, int32_t* idx2,
+                     int B, int N, int M, const float* tau, int T, long long* stats,
+                     void* workspace, int64_t workspace_bytes, void* stream);
 
 /* Measurement aid (bench.py): a launch of independent fp32 FMA chains that is bound by the FMA issue rate only;
  * *fma_count (HOST) receives the number of thread-level FMAs the launch executes.  Timed with CUDA events it gives the

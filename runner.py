@@ -100,15 +100,20 @@ def main():
         nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
         res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
     else:
-        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check).cpu()
+        # + the point-cloud counters (Chamfer L2 / L1, precision, recall, F-score) of the same forwards, at the very end
+        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check, eval_points=True).cpu()
         nh = 2
         res = T.chamfer_summary(stats[:nh])
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH))
+    nl = 2 * (3 + len(cfg.TEST.DISP_THRESH)) if args.lr_check else 0
     res['disparity'] = T.disp_summary(stats[nh:nh + nd], cfg.TEST.DISP_THRESH)
     if args.lr_check:
-        res['lr_consistency'] = T.lr_summary(stats[nh + nd:], cfg.TEST.DISP_THRESH,
+        res['lr_consistency'] = T.lr_summary(stats[nh + nd:nh + nd + nl], cfg.TEST.DISP_THRESH,
                                              res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
         res['lr_consistency']['lr_thresh'] = float(cfg.TEST.LR_THRESH)
+    if args.model == 'Stereo2Point':
+        res['points'] = T.points_summary(stats[nh + nd + nl:], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
+                                         cfg.CONST.N_GT_POINTS)
     if rank == 0:
         res.update(model=args.model, precision=cfg.NETWORK.PRECISION, world_size=world, data='synthetic')
         print(json.dumps(res))

@@ -11,14 +11,22 @@ forward computes against the synthetic GT disparity (models.py, _StereoBase._ups
     n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) per t in TEST.DISP_THRESH   (int64)
 With eval_lr=True (needs eval_disp) the left-right consistency counters of the same forwards follow, per view:
     n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the kept valid pixels  (int64)
+With eval_points=True (test_point) the point-cloud counters of the same forwards come last (models.py,
+Stereo2Point._point_stats), per direction (predicted -> GT, then GT -> predicted), then per threshold t in
+TEST.FSCORE_THRESH:
+    sum q(d), sum q(sqrt d), n_out, count(sqrt d < t) per t                                    (int64)
+    sum_b q(F_b(t)),  F_b = 2 P R / (P + R) (0 when both are 0), P = count_pred / N, R = count_gt / M   (int64)
+with q(x) = round-half-even(x * 2^32); F_b is computed elementwise in fp64 on the device, so the vector stays integer.
 """
 import torch
 import torch.distributed as dist
 
+from ..models import fscore_thresholds
 from ..utils import synthetic
 
 _FX = float(1 << 40)
 _DISP_FX = float(1 << 16)
+_PT_FX = float(1 << 32)
 
 
 def shard_range(n_total, rank, world):
@@ -85,6 +93,46 @@ def lr_summary(stats_block, thresholds, n_pixels, disp_block):
     return out
 
 
+def point_block(point_stats, N, M):
+    """Per-batch increment of the point block from the forward's point_stats int64 [B,2,3+T] (N predicted, M GT points per
+    sample): the counters summed over the batch, then sum_b round-half-even(F_b(t) * 2^32) per threshold, in fp64."""
+    c = point_stats[:, :, 3:].double()
+    p, r = c[:, 0] / N, c[:, 1] / M
+    f = torch.where(p + r > 0, 2 * p * r / (p + r), torch.zeros_like(p))
+    return torch.cat([point_stats.sum(0).flatten(), torch.round(f * _PT_FX).to(torch.int64).sum(0)])
+
+
+def points_summary(block, thresholds, n_samples, N, M):
+    """Point counters (int64 [2 * (3 + T) + T], as point_block sums them) -> dict:
+    chamfer_l2 = (sum q(d1) / N + sum q(d2) / M) / 2^32 / n (squared distances: GRNet's ChamferDistance, the mean of dist1
+    plus the mean of dist2), chamfer_l1 = (sum q(sqrt d1) / N + sum q(sqrt d2) / M) / 2 / 2^32 / n (GRNet's
+    ChamferDistanceL1), both inf when a point was out of range (n_out > 0); per threshold the precision (predicted points
+    within t of the GT), recall (GT points within t of the prediction) and the mean per-sample F-score."""
+    T = len(thresholds)
+    v = [int(x) for x in block.tolist()]
+    assert len(v) == 2 * (3 + T) + T
+    pred, gt, f = v[:3 + T], v[3 + T:2 * (3 + T)], v[2 * (3 + T):]
+    n = n_samples
+    n_out = pred[2] + gt[2]
+    if n_out:
+        l2 = l1 = float('inf')
+    elif n:
+        l2 = (pred[0] / N + gt[0] / M) / _PT_FX / n
+        l1 = 0.5 * (pred[1] / N + gt[1] / M) / _PT_FX / n
+    else:
+        l2 = l1 = 0.0
+    return {'n_samples': n, 'n_pred': N, 'n_gt': M, 'thresholds': list(thresholds), 'chamfer_l2': l2, 'chamfer_l1': l1,
+            'n_out': n_out, 'precision': [c / (N * n) if n else 0.0 for c in pred[3:]],
+            'recall': [c / (M * n) if n else 0.0 for c in gt[3:]], 'fscore': [x / _PT_FX / n if n else 0.0 for x in f]}
+
+
+def _point_len(cfg, eval_points):
+    if not eval_points:
+        return 0
+    T = len(fscore_thresholds(cfg))                     # ValueError on a bad TEST.FSCORE_THRESH, before any forward
+    return 2 * (3 + T) + T
+
+
 def _disp_gt(pairs, H, W, device):
     return torch.cat([synthetic.disparity_gt(p[2], H, W) for p in pairs]).to(device)
 
@@ -129,13 +177,15 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
     return reduce_stats(stats)
 
 
-def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False):
+def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
+               eval_points=False):
     """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, as
-    for test_voxel)."""
+    for test_voxel, + the point-cloud counters with eval_points: module docstring)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
     nl = _lr_len(cfg, eval_disp, eval_lr)
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    stats = torch.zeros(2 + nd + nl, dtype=torch.int64, device=device)
+    npt = _point_len(cfg, eval_points)
+    stats = torch.zeros(2 + nd + nl + npt, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -145,15 +195,20 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.point_clouds(1, 1, cfg.CONST.N_GT_POINTS, seed=200000 + i)[1] for i in ids]).to(device)
+            head = (gt,) if eval_points else ()
             if eval_lr:
-                _, _, pts, ds, _, ls = model(left, right, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
+                out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
+                ds, ls = out[-3], out[-1]
                 stats[2:2 + nd] += ds.sum(0).flatten()
-                stats[2 + nd:] += ls.sum(0).flatten()
+                stats[2 + nd:2 + nd + nl] += ls.sum(0).flatten()
             elif eval_disp:
-                _, _, pts, ds = model(left, right, disp_gt=_disp_gt(pairs, H, W, device))
-                stats[2:] += ds.sum(0).flatten()
+                out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device))
+                stats[2:2 + nd] += out[-1].sum(0).flatten()
             else:
-                _, _, pts = model(left, right)
+                out = model(left, right, *head)
+            pts = out[2]
+            if eval_points:
+                stats[2 + nd + nl:] += point_block(out[3], pts.shape[1], gt.shape[1])
             cd = chamfer_per_sample(pts.contiguous(), gt)
             stats[0] += torch.round(cd.sum() * _FX).to(torch.int64)
             stats[1] += len(ids)

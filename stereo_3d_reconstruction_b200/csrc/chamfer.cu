@@ -28,6 +28,8 @@
 //     (distance bits << 32 | 256-point block): non-negative floats order like their bit patterns, so the key's minimum is
 //     the minimum distance at the lowest block; chamfer_sym_finish_kernel rescans that one block for the lowest index.
 // About 9.6 issued instructions per pair for BOTH directions against 2 x 11, and 8 of them are the exact arithmetic.
+#include <cmath>
+
 #include "common.cuh"
 
 namespace s3d {
@@ -326,6 +328,61 @@ int launch_dir(const float* q, const float* r, float* dist, int32_t* idx, int B,
   return S3D_OK;
 }
 
+// ---- point-cloud metrics over the search's distances (s3d_chamfer_eval) ------------------------------------------------
+// A separate pass over dist1 / dist2 (just written, read from L2), so the search kernels above stay as they are.  Blocks
+// [0, B * c0) cover direction 0 (dist1, c0 blocks per sample), the rest direction 1 (dist2, c1 per sample); a block never
+// spans two (sample, direction) slices.  Integer counters: warp shuffle -> shared memory -> one 64-bit atomic per counter
+// per block, so the sums do not depend on the launch order.
+constexpr int kEvalThreads = 256;
+constexpr int kEvalPts = 4 * kEvalThreads;   // distances per block
+constexpr float kEvalMaxD = 256.f;           // in range: d finite and d < 2^8, so q(d) < 2^40
+constexpr float kFx = 4294967296.f;          // 2^32: q(x) = round-half-even(x * 2^32), the product exact in fp32
+
+__global__ void __launch_bounds__(kEvalThreads)
+chamfer_eval_kernel(const float* __restrict__ dist1, const float* __restrict__ dist2, int N, int M, int c0, int c1, int B,
+                    Thresh th, int nT, unsigned long long* __restrict__ stats) {
+  const int64_t blk0 = (int64_t)B * c0;
+  const bool d1 = blockIdx.x < blk0;
+  const int64_t k = d1 ? blockIdx.x : blockIdx.x - blk0;
+  const int c = d1 ? c0 : c1, n = d1 ? N : M;
+  const int b = (int)(k / c), chunk = (int)(k % c);
+  const float* d = (d1 ? dist1 : dist2) + (int64_t)b * n;
+  unsigned long long sum_d = 0, sum_s = 0;
+  unsigned n_out = 0, cnt[kMaxThresh] = {};
+#pragma unroll
+  for (int j = 0; j < kEvalPts / kEvalThreads; ++j) {
+    const int i = chunk * kEvalPts + j * kEvalThreads + threadIdx.x;
+    if (i >= n) break;
+    const float v = d[i];
+    if (!(v < kEvalMaxD)) { ++n_out; continue; }                 // +inf (NaN point or nothing compared less), NaN, >= 2^8
+    const float s = __fsqrt_rn(v);
+    sum_d += (unsigned long long)__float2ll_rn(v * kFx);
+    sum_s += (unsigned long long)__float2ll_rn(s * kFx);
+#pragma unroll
+    for (int t = 0; t < kMaxThresh; ++t)
+      if (t < nT) cnt[t] += s < th.t[t];
+  }
+  constexpr int kN = 3 + kMaxThresh;
+  __shared__ unsigned long long acc[kN];
+  if (threadIdx.x < kN) acc[threadIdx.x] = 0;
+  __syncthreads();
+  unsigned long long v[kN];
+  v[0] = sum_d;  v[1] = sum_s;  v[2] = n_out;
+#pragma unroll
+  for (int t = 0; t < kMaxThresh; ++t) v[3 + t] = cnt[t];
+  const int nc = 3 + nT;
+#pragma unroll
+  for (int j = 0; j < kN; ++j) {
+    if (j >= nc) break;
+    unsigned long long a = v[j];
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    if ((threadIdx.x & 31) == 0 && a) atomicAdd(&acc[j], a);
+  }
+  __syncthreads();
+  if ((int)threadIdx.x < nc && acc[threadIdx.x])
+    atomicAdd(stats + ((int64_t)b * 2 + (d1 ? 0 : 1)) * nc + threadIdx.x, acc[threadIdx.x]);
+}
+
 }  // namespace
 }  // namespace s3d
 
@@ -390,6 +447,28 @@ extern "C" int s3d_chamfer_forward_ws(const float* xyz1, const float* xyz2, floa
   int rc = launch_dir(xyz1, xyz2, dist1, idx1, B, N, M, st);
   if (rc != S3D_OK) return rc;
   return launch_dir(xyz2, xyz1, dist2, idx2, B, M, N, st);
+}
+
+extern "C" int s3d_chamfer_eval(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2, int32_t* idx2,
+                                int B, int N, int M, const float* tau, int T, long long* stats, void* workspace,
+                                int64_t workspace_bytes, void* stream) {
+  using namespace s3d;
+  if (!stats || (T > 0 && !tau)) { set_error("chamfer_eval: null argument"); return S3D_ERR_INVALID; }
+  S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "chamfer_eval: T must be in [0, %d], got %d", kMaxThresh, T);
+  Thresh th;
+  for (int t = 0; t < kMaxThresh; ++t) {
+    th.t[t] = t < T ? tau[t] : 0.f;
+    S3D_CHECK_ARG(t >= T || (std::isfinite(th.t[t]) && th.t[t] > 0.f),"chamfer_eval: threshold %d must be finite and > 0", t);
+  }
+  S3D_CHECK_ARG(N < (1 << 22) && M < (1 << 22), "chamfer_eval: N and M must be below 2^22 (N=%d, M=%d)", N, M);
+  const int c0 = N > 0 ? ceil_div(N, kEvalPts) : 0, c1 = M > 0 ? ceil_div(M, kEvalPts) : 0;
+  S3D_CHECK_ARG((int64_t)B * (c0 + c1) < (1ll << 31), "chamfer_eval: grid too large");
+  const int rc = s3d_chamfer_forward_ws(xyz1, xyz2, dist1, idx1, dist2, idx2, B, N, M, workspace, workspace_bytes, stream);
+  if (rc != S3D_OK || B == 0) return rc;
+  chamfer_eval_kernel<<<(unsigned)((int64_t)B * (c0 + c1)), kEvalThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      dist1, dist2, N, M, c0, c1, B, th, T, reinterpret_cast<unsigned long long*>(stats));
+  S3D_LAUNCH_CHECK();
+  return S3D_OK;
 }
 
 extern "C" int s3d_chamfer_forward(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2,

@@ -80,6 +80,7 @@ SIGNATURES = {
     's3d_chamfer_forward': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp], _i),
     's3d_chamfer_workspace_bytes': ([_i, _i, _i], ctypes.c_int64),
     's3d_chamfer_forward_ws': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _i64, _vp], _i),
+    's3d_chamfer_eval': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, ctypes.POINTER(_f), _i, _vp, _vp, _i64, _vp], _i),
     's3d_fma_probe': ([_vp, _i, ctypes.POINTER(ctypes.c_int64), _vp], _i),
 }
 

@@ -451,6 +451,7 @@ class _StereoBase(nn.Module):
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
         left, right = self._check_inputs(left, right)
+        gt = self._check_gt(gt, left)
         disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
@@ -476,6 +477,10 @@ class _StereoBase(nn.Module):
         if left.shape != right.shape or left.dim() != 4 or left.shape[1] != 3:
             raise ValueError('expected left/right of shape [B,3,H,W], got %s / %s' % (tuple(left.shape), tuple(right.shape)))
         return left.contiguous().float(), right.contiguous().float()
+
+    def _check_gt(self, gt, left):
+        """The head's GT as the head takes it (Stereo2Point validates its point cloud)."""
+        return gt
 
     def _check_disp_gt(self, disp_gt, left):
         """GT disparity of (checked) inputs `left`: fp32 [B,2,H,W] on their device, in input pixels, view 0 = left-referenced
@@ -606,13 +611,46 @@ class Stereo2Voxel(_StereoBase):
         return out + lr if lr_check else out
 
 
+def fscore_thresholds(cfg):
+    """TEST.FSCORE_THRESH as floats: at most 8 (the kernel's limit) Euclidean distances in the points' units, each finite
+    and > 0; anything else is a ValueError."""
+    th = cfg.TEST.get('FSCORE_THRESH')
+    try:
+        th = [float(t) for t in th]
+    except (TypeError, ValueError):
+        raise ValueError('TEST.FSCORE_THRESH must be a list of numbers, got %r' % (th,)) from None
+    if len(th) > 8 or not all(math.isfinite(t) and t > 0 for t in th):
+        raise ValueError('TEST.FSCORE_THRESH must hold at most 8 finite distances > 0, got %r' % (cfg.TEST.FSCORE_THRESH,))
+    return th
+
+
 class Stereo2Point(_StereoBase):
-    """forward(left, right[, disp_gt=][, lr_check=]) -> (disp_left, disp_right, points [B,N_POINTS,3]
-    [, disp_stats int64 [B,2,2+T]][, lr_mask, lr_stats]) (disp_gt, lr_check and the extra outputs as for Stereo2Voxel)."""
+    """forward(left, right[, gt][, disp_gt=][, lr_check=]) -> (disp_left, disp_right, points [B,N_POINTS,3]
+    [, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats]) (disp_gt, lr_check and their
+    outputs as for Stereo2Voxel).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
+    `points` against it and counts, per sample and direction (0: predicted -> GT, 1: GT -> predicted), [sum of squared
+    distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
+    (include/s3d.h, s3d_chamfer_eval)."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
         self.point_decoder = _PointDecoder(cfg)
+
+    def _check_gt(self, gt, left):
+        """GT point cloud of (checked) inputs `left`: fp32 [B,M,3], M >= 1, on their device."""
+        if gt is None:
+            return None
+        B = left.shape[0]
+        if not isinstance(gt, torch.Tensor):
+            raise ValueError('gt must be a tensor, got %s' % type(gt).__name__)
+        if gt.dim() != 3 or gt.shape[0] != B or gt.shape[1] < 1 or gt.shape[2] != 3:
+            raise ValueError('expected gt of shape [%d, M, 3], got %s' % (B, tuple(gt.shape)))
+        if gt.dtype != torch.float32:
+            raise ValueError('gt must be float32, got %s' % gt.dtype)
+        if gt.device != left.device:
+            raise ValueError('gt must be on %s (the images\' device), got %s' % (left.device, gt.device))
+        fscore_thresholds(self.cfg)                    # a bad TEST.FSCORE_THRESH fails before anything is launched
+        return gt.contiguous()
 
     def _pack_head(self, P, dc, dev):
         pd = self.point_decoder
@@ -621,11 +659,12 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, *, disp_gt=None, lr_check=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False):
         left, right = self._check_inputs(left, right)
-        return self._forward_impl(left, right, disp_gt=self._check_disp_gt(disp_gt, left), lr_check=lr_check)
+        return self._forward_impl(left, right, self._check_gt(gt, left), disp_gt=self._check_disp_gt(disp_gt, left),
+                                  lr_check=lr_check)
 
-    def _forward_impl(self, left, right, disp_gt=None, lr_check=False):
+    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False):
         cfg = self.cfg
         B = left.shape[0]
         disp, _, dstats, lr = self._disparity(left, right, disp_gt, lr_check)
@@ -647,10 +686,28 @@ class Stereo2Point(_StereoBase):
         npts = cfg.CONST.N_POINTS
         pts = self._buf('pts', (B, 1, 1, 1, pad_to(npts * 3)), torch.float32)
         self._conv('pt_fc2', y, out=pts)
-        out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3))
+        points = pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3)
+        out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), points)
+        if gt is not None:
+            out += (self._point_stats(points, gt),)
         if disp_gt is not None:
             out += (dstats,)
         return out + lr if lr_check else out
+
+    def _point_stats(self, points, gt):
+        """Chamfer search of points [B,N,3] against gt [B,M,3] + the metric counters -> point_stats int64 [B,2,3+T], zeroed
+        here (so a graph replay starts from zero).  Every buffer comes from the workspace: no allocation on this path."""
+        th = fscore_thresholds(self.cfg)
+        B, N, M = points.shape[0], points.shape[1], gt.shape[1]
+        if not points.is_contiguous():                 # the fc2 output row is padded: copy the points out of it
+            points = self._buf('pts_xyz', (B, N, 3), torch.float32).copy_(points)
+        stats = self._buf('point_stats', (B, 2, 3 + len(th)), torch.int64)
+        stats.zero_()
+        nb = ops.chamfer_workspace_bytes(B, N, M)
+        ops.chamfer_eval(points, gt, th, stats, workspace=self._buf('cd_ws', (nb,), torch.uint8) if nb else None,
+                         out=(self._buf('cd_d1', (B, N), torch.float32), self._buf('cd_d2', (B, M), torch.float32),
+                              self._buf('cd_i1', (B, N), torch.int32), self._buf('cd_i2', (B, M), torch.int32)))
+        return stats
 
 
 def build_model(name, cfg, seed=None):

@@ -463,7 +463,7 @@ def chamfer_forward(xyz1, xyz2, workspace=None):
     idx1 = torch.empty((B, N), dtype=torch.int32, device=dev)
     idx2 = torch.empty((B, M), dtype=torch.int32, device=dev)
     L = _lib.load()
-    need = int(L.s3d_chamfer_workspace_bytes(B, N, M)) if min(B, N, M) > 0 else 0
+    need = chamfer_workspace_bytes(B, N, M)
     if need and (workspace is None or workspace.numel() * workspace.element_size() < need):
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
     rc = L.s3d_chamfer_forward_ws(xyz1.data_ptr(), xyz2.data_ptr(), dist1.data_ptr(), idx1.data_ptr(),
@@ -471,4 +471,46 @@ def chamfer_forward(xyz1, xyz2, workspace=None):
                                   workspace.data_ptr() if need else None, need, _stream())
     _lib.check(rc, 's3d_chamfer_forward_ws')
     _lib.count_launch(2)
+    return dist1, dist2, idx1, idx2
+
+
+def chamfer_workspace_bytes(B, N, M):
+    return int(_lib.load().s3d_chamfer_workspace_bytes(B, N, M)) if min(B, N, M) > 0 else 0
+
+
+def chamfer_eval(xyz1, xyz2, tau, stats, workspace=None, out=None):
+    """chamfer_forward + per-sample point-cloud metrics (include/s3d.h, s3d_chamfer_eval).  xyz1 = predicted [B,N,3], xyz2 =
+    GT [B,M,3], fp32.  stats int64 [B,2,3+T] (T = len(tau)) += per direction (0: xyz1 -> xyz2, 1: xyz2 -> xyz1)
+    [sum q(d), sum q(sqrt d), n_out, count(sqrt d < tau_t) per t], q(x) = round-half-even(x * 2^32), over the points with
+    finite d < 2^8 (the others are n_out).  out: optional (dist1 [B,N], dist2 [B,M], idx1 [B,N], idx2 [B,M]) buffers (fp32,
+    fp32, int32, int32) to write into.  -> (dist1, dist2, idx1, idx2), bit-identical to chamfer_forward."""
+    _chk(xyz1, xyz2, stats, workspace)
+    if xyz1.dtype != torch.float32 or xyz2.dtype != torch.float32:
+        raise ValueError('chamfer_eval: point clouds must be float32')
+    B, N, three = xyz1.shape
+    B2, M, three2 = xyz2.shape
+    if three != 3 or three2 != 3 or B != B2:
+        raise ValueError('chamfer_eval: expected [B,N,3] and [B,M,3]')
+    T = len(tau)
+    if stats.dtype != torch.int64 or tuple(stats.shape) != (B, 2, 3 + T):
+        raise ValueError('chamfer_eval: stats must be int64 [%d, 2, %d]' % (B, 3 + T))
+    dev = xyz1.device
+    if out is None:
+        out = (torch.empty((B, N), dtype=torch.float32, device=dev), torch.empty((B, M), dtype=torch.float32, device=dev),
+               torch.empty((B, N), dtype=torch.int32, device=dev), torch.empty((B, M), dtype=torch.int32, device=dev))
+    dist1, dist2, idx1, idx2 = out
+    _chk(dist1, dist2, idx1, idx2)
+    for t, shape, dt in ((dist1, (B, N), torch.float32), (dist2, (B, M), torch.float32), (idx1, (B, N), torch.int32),
+                         (idx2, (B, M), torch.int32)):
+        if tuple(t.shape) != shape or t.dtype != dt:
+            raise ValueError('chamfer_eval: out buffer %s %s, expected %s %s' % (tuple(t.shape), t.dtype, shape, dt))
+    need = chamfer_workspace_bytes(B, N, M)
+    if need and (workspace is None or workspace.numel() * workspace.element_size() < need):
+        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
+    th = (ctypes.c_float * max(T, 1))(*[float(t) for t in tau])
+    rc = _lib.load().s3d_chamfer_eval(xyz1.data_ptr(), xyz2.data_ptr(), dist1.data_ptr(), idx1.data_ptr(), dist2.data_ptr(),
+                                      idx2.data_ptr(), B, N, M, th, T, stats.data_ptr(),
+                                      workspace.data_ptr() if need else None, need, _stream())
+    _lib.check(rc, 's3d_chamfer_eval')
+    _lib.count_launch(3)                       # the two search kernels + chamfer_eval_kernel
     return dist1, dist2, idx1, idx2
