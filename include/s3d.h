@@ -91,6 +91,20 @@ typedef struct S3dConvParams {
    * (the slice that carries input plane p into output plane z = p+1-kz, which accumulates in slot z % 3 == s).
    * Rotation 3 is rotation 0 with block 2 zeroed (p = 0: there is no output plane -1). */
   const void* w_nstack;
+  /* Optional constant-region descriptor (dz_nref = 0: none), used by the plane-scatter kernel with bf16 operands and
+   * ignored by every other engine.  The input is N = 2 * dz_nref volumes descending from a concat cost volume (in the
+   * order of s3d_cost_volume_concat: [0, dz_nref) left-referenced, [dz_nref, N) right-referenced), and input plane z of
+   * pixel column x is the same, bit for bit, for every z in [xr + dz_c, iD - 1 - dz_e], xr = x (left-referenced) or
+   * iW - 1 - x (right-referenced).  The output then repeats along z on [xr + dz_c + 2, oD - 2 - dz_e]; the kernel computes
+   * such a run once per column and stores it as copies (same results, fewer MMAs).  Not used with z-split columns.
+   * dz_sched (may be NULL): int32 DEVICE table that pairs the columns for the CTA pairs of the kernel and balances their
+   * planes, dz_pairs pairs: [dz_pairs + 1 offsets into the items][items x 2 column indices]; column index
+   * (n * ceil(oH / 32) + y0 / 32) * ceil(oW / 8) + x0 / 8 for the 32 x 8 patch at (y0, x0), an index >= the column
+   * count is an empty column.  Built by layers.py (dz_schedule); every column must appear exactly once.
+   * dz_planes (may be NULL): int64 DEVICE counter, ADDED the number of input planes the kernel's CTAs marched. */
+  int32_t dz_nref, dz_c, dz_e, dz_pairs;
+  const int32_t* dz_sched;
+  long long* dz_planes;
 } S3dConvParams;
 
 const char* s3d_version(void);
@@ -99,7 +113,7 @@ const char* s3d_last_error(void);
 /* 0 if device `dev` is usable (compute capability 10.x), else a negative code. */
 int s3d_device_check(int dev);
 /* A/B switches of the launchers ("no_scatter", "scatter_no_pair", "scatter_generic", "scatter_tps3", "scatter_ring",
- * "scatter_res_transpose", "scatter_no_transpose", "no_corr_tc", "scatter_zsplit", "scatter_no_rm", "igemm_ts1", "igemm_one_cta", "scatter_one_cta", "no_conv_first_tc", "chamfer_sym", "chamfer_sym_r"; all 0 by default = the shipped path).  They are
+ * "scatter_res_transpose", "scatter_no_transpose", "no_corr_tc", "scatter_zsplit", "scatter_no_rm", "igemm_ts1", "igemm_one_cta", "scatter_one_cta", "no_conv_first_tc", "chamfer_sym", "chamfer_sym_r", "no_dz_skip"; all 0 by default = the shipped path).  They are
  * initialised ONCE from the environment variables S3D_<NAME> when the library is first used and are never read from
  * the environment on the launch path; s3d_set_knob overrides one at run time.  Process-wide, not thread-safe against
  * concurrent launches. */

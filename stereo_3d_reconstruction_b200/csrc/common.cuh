@@ -50,6 +50,7 @@ struct Knobs {
   int chamfer_sym;            // S3D_CHAMFER_SYM: 1 = symmetric one-pass Chamfer kernel at every size (given a workspace), -1 = never (0: when it fills the chip)
   int chamfer_sym_r;          // S3D_CHAMFER_SYM_R: resident points per lane of the symmetric Chamfer kernel, 4 or 8 (0: automatic)
   int scatter_no_rm;          // S3D_SCATTER_NO_RM: residual added by the epilogue threads instead of an identity tap on the tensor core
+  int no_dz_skip;             // S3D_NO_DZ_SKIP: the plane-scatter kernel ignores S3dConvParams' constant-region descriptor (dz_nref)
 };
 Knobs& knobs();
 

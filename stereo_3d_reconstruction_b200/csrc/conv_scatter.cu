@@ -91,6 +91,17 @@ int conv_scatter_launch(const S3dConvParams* p_in, const void* in, const float* 
     grid -= grid % 2;
     a.ncols_max = (int)((total + grid - 1) / grid);
   } else if ((int64_t)grid > total) grid = (int)total;
+  // constant-region skip (include/s3d.h dz_nref; conv_scatter.cuh, Item): bf16 operands and whole columns only -- a z-split
+  // chunk marches its own few planes, so the skip is off there.  The schedule table replaces the round-robin column order
+  // of CTA pairs and sets the grid; single CTAs skip on their own columns without it.
+  const bool dz = p.dz_nref > 0 && !tf32 && !split && a.nz == 1 && !knobs().no_dz_skip;
+  if (dz) S3D_CHECK_ARG(p.N == 2 * p.dz_nref && p.dz_c >= 0 && p.dz_e >= 0, "scatter: constant-region descriptor");
+  if (!dz) a.p.dz_nref = 0;
+  if (!dz || !a.pair) a.p.dz_sched = nullptr;
+  if (a.p.dz_sched) {
+    S3D_CHECK_ARG(p.dz_pairs >= 1, "scatter: dz_pairs");
+    grid = 2 * p.dz_pairs;
+  }
   const int w_rows = a.pair ? 3 * a.cp / 2 : 3 * a.cp;          // weight rows staged per CTA
   a.w_tx = a.tps * w_rows * a.row_bytes;
   a.w_bytes = (a.w_tx + 1023) / 1024 * 1024;

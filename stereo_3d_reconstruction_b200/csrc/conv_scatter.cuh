@@ -120,10 +120,48 @@ __device__ __forceinline__ Col decode_col(const ScArgs& a, int c) {
 }
 
 // Columns this CTA walks.  The two CTAs of a pair run the same MMAs, so in pair mode every CTA walks ncols_max
-// columns; a column index >= total_cols decodes to n >= N (TMA zero fill, nothing stored).
+// columns (or its pair's list in the schedule table, include/s3d.h dz_sched); a column index >= total_cols decodes to
+// n >= N (TMA zero fill, nothing stored).
 __device__ __forceinline__ int cta_cols(const ScArgs& a) {
+  if (a.p.dz_sched) return __ldg(a.p.dz_sched + (blockIdx.x >> 1) + 1) - __ldg(a.p.dz_sched + (blockIdx.x >> 1));
   return a.pair ? a.ncols_max : (a.total_cols - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
 }
+
+// Constant-region skip (include/s3d.h, dz_nref).  Output planes [zs, zs + J] of a work item are equal: once input plane
+// zs + 1 is done (out plane zs drained), the slots of out planes zs + 1 and zs + 2 hold exactly the partial sums that out
+// planes zs + 1 + J and zs + 2 + J need (their input planes are the same), so the march continues at input plane
+// zs + 2 + J and the epilogue stores plane zs J more times.  J % 3 == 0 keeps every slot (z % 3) and weight rotation
+// (p % 3) where it was.  The two CTAs of a pair issue the same MMAs: both take the intersection of their columns' runs.
+struct Item { Col c; int zs, J; };
+
+__device__ __forceinline__ int dz_first(const ScArgs& a, const Col& c) {      // first plane of the column's repeating run
+  if (c.n >= a.p.N) return 0;                                                 // empty column: no constraint
+  const int xr = c.n < a.p.dz_nref ? min(c.x0 + kTX - 1, a.p.oW - 1) : a.p.oW - 1 - c.x0;
+  return xr + a.p.dz_c + 2;
+}
+
+__device__ __forceinline__ Item cta_item(const ScArgs& a, int ci) {
+  int mine, other;
+  if (a.p.dz_sched) {
+    const int r = blockIdx.x & 1;
+    const int32_t* e = a.p.dz_sched + a.p.dz_pairs + 1 + 2 * (__ldg(a.p.dz_sched + (blockIdx.x >> 1)) + ci);
+    mine = __ldg(e + r);  other = __ldg(e + (r ^ 1));
+  } else {
+    mine = blockIdx.x + ci * gridDim.x;  other = a.pair ? (mine ^ 1) : mine;   // pair mode: grid even, partner = blockIdx ^ 1
+  }
+  Item it;
+  it.c = decode_col(a, mine);
+  it.zs = 0;  it.J = 0;
+  if (a.p.dz_nref > 0) {
+    const int zs = max(dz_first(a, it.c), dz_first(a, decode_col(a, other))), ze = a.p.oD - 2 - a.p.dz_e;
+    it.zs = zs;
+    it.J = ze - zs >= 3 ? (ze - zs) / 3 * 3 : 0;
+  }
+  return it;
+}
+
+// The input planes of a work item, in march order: 0 .. D-1 with zs + 2 .. zs + 1 + J left out.
+__device__ __forceinline__ int next_plane(const Item& it, int p) { return p == it.zs + 1 ? p + 1 + it.J : p + 1; }
 
 __device__ __forceinline__ uint64_t desc_hi(uint32_t sbo, int row_bytes) {
   const uint64_t layout = row_bytes == 128 ? 2ull : (row_bytes == 64 ? 4ull : 6ull);
@@ -150,7 +188,9 @@ __device__ __forceinline__ void sc_produce(const ScArgs& a, ScCtrl& ctrl, uint32
   int ws = 0;  uint32_t wphase = 0;
   int pslot = 0;  uint32_t pphase = 0;
   int pci = 0, pj = 0, issued = 0;
-  Col pc = decode_col(a, blockIdx.x);
+  Item pit{};
+  if (ncols > 0) pit = cta_item(a, 0);
+  const Col& pc = pit.c;
   auto issue_plane = [&](bool blocking) -> bool {
     if (pci >= ncols) return false;
     const uint32_t be = bar_pe + 8 * pslot, bf = bar_pf + 8 * pslot;
@@ -172,9 +212,10 @@ __device__ __forceinline__ void sc_produce(const ScArgs& a, ScCtrl& ctrl, uint32
     __syncwarp();
     ++issued;
     if (++pslot == ring) { pslot = 0; pphase ^= 1; }
-    if (++pj == D) {
+    pj = next_plane(pit, pj);
+    if (pj >= D) {
       pj = 0;  ++pci;
-      if (pci < ncols) pc = decode_col(a, blockIdx.x + pci * gridDim.x);
+      if (pci < ncols) pit = cta_item(a, pci);
     }
     return true;
   };
@@ -199,10 +240,11 @@ __device__ __forceinline__ void sc_produce(const ScArgs& a, ScCtrl& ctrl, uint32
     rphase ^= 1;
   };
   for (int ci = 0; ci < ncols; ++ci) {
-    int rot = 3;                                 // weight rotation: 3 for p = 0, then p % 3
-    [[maybe_unused]] const Col rc = decode_col(a, blockIdx.x + ci * gridDim.x);
+    int rot = 3;                                 // weight rotation: 3 for p = 0, then p % 3 (a skip keeps p % 3)
+    const Item it = cta_item(a, ci);
+    [[maybe_unused]] const Col& rc = it.c;
     if constexpr (kRM) load_res(rc, 0);
-    for (int p = 0; p < D; ++p, ++gp) {
+    for (int p = 0; p < D; p = next_plane(it, p), ++gp) {
       while (issued <= gp) issue_plane(true);
       const int ahead = gp + ring;               // planes that may be in flight while plane gp is being read
 #pragma unroll
@@ -224,9 +266,13 @@ __device__ __forceinline__ void sc_produce(const ScArgs& a, ScCtrl& ctrl, uint32
         __syncwarp();
         if (++ws == w_stages) { ws = 0; wphase ^= 1; }
       }
-      if constexpr (kRM) { if (p + 1 < D) load_res(rc, p + 1); }       // one plane ahead (see load_res)
+      if constexpr (kRM) { const int pn = next_plane(it, p); if (pn < D) load_res(rc, pn); }       // one plane ahead (see load_res)
       rot = (p == 0) ? 1 : (rot == 2 ? 0 : rot + 1);
     }
+  }
+  if (a.p.dz_planes) {
+    if (ptx::elect_one()) atomicAdd(reinterpret_cast<unsigned long long*>(a.p.dz_planes), (unsigned long long)issued);
+    __syncwarp();
   }
 }
 
@@ -243,6 +289,7 @@ struct ScIssue {
   uint32_t rb16, tap_step, tile_off, chunk_step; // 16-byte units
   uint32_t idesc;
   int D, ncols;
+  const ScArgs* args = nullptr;                  // work items (cta_item); only sc_issue reads it
 };
 
 template <bool kPair>
@@ -327,7 +374,8 @@ __device__ __forceinline__ void sc_issue(const ScIssue& z, const ScRes* rs = nul
   const uint32_t x_lo0 = desc_lo(z.planes_u32), x_lo_step = z.slot_bytes >> 4;
   const uint32_t d0 = z.tmem_base, d1 = z.tmem_base + kTP;
   for (int ci = 0; ci < z.ncols; ++ci) {
-    for (int p = 0; p < z.D; ++p) {
+    const Item it = cta_item(*z.args, ci);
+    for (int p = 0; p < z.D; p = next_plane(it, p)) {
       ptx::mbar_wait_u32(z.bar_pf + 8 * pw, pwphase);
       const uint64_t xd0 = z.x_hi | (x_lo0 + pw * x_lo_step);
       const uint64_t xd1 = xd0 + z.tile_off;
@@ -430,9 +478,11 @@ __device__ __forceinline__ void sc_res_load(const ScEpi& e, int64_t grp_off, int
 
 // kAct: 0 ReLU, 2 general slope (none / leaky).  (An identity variant that skips the three slope instructions was
 // measured SLOWER on the residual layer, 2.85 vs 2.70 ms, and grew the kernel; it is not instantiated.)
+// ncopy > 0: the same values are stored again at ncopy more planes, zstep elements apart.
 template <int CP, typename TOut, bool kRes, int kAct>
 __device__ __forceinline__ void sc_fast_store(const ScEpi& e, int64_t grp_off, int lane, uint32_t okmask,
-                                              const uint32_t (&v)[CP / 16][16], uint4 (&r)[CP * sizeof(TOut) / 16]) {
+                                              const uint32_t (&v)[CP / 16][16], uint4 (&r)[CP * sizeof(TOut) / 16],
+                                              int ncopy = 0, int64_t zstep = 0) {
   constexpr int NCH = CP * sizeof(TOut) / 16;
   constexpr int CPC = 16 / sizeof(TOut);          // channels per chunk
   uint4 c[NCH];
@@ -483,21 +533,24 @@ __device__ __forceinline__ void sc_fast_store(const ScEpi& e, int64_t grp_off, i
   chunk_transpose<NCH>(c, lane);
   const int j = lane & (NCH - 1);
   TOut* o = reinterpret_cast<TOut*>(e.out) + grp_off + j * CPC;
+  for (int i = 0; i <= ncopy; ++i, o += zstep) {
 #pragma unroll
-  for (int k = 0; k < NCH; ++k)
-    if ((okmask >> k) & 1u) *reinterpret_cast<uint4*>(o + k * e.osW) = c[k];
+    for (int k = 0; k < NCH; ++k)
+      if ((okmask >> k) & 1u) *reinterpret_cast<uint4*>(o + k * e.osW) = c[k];
+  }
 }
 
 // One drained plane: residual chunks `r` (already loaded, still in group order) + accumulators -> coalesced stores.
 template <int CP, typename TOut>
 __device__ __forceinline__ void sc_fast_plane(const ScEpi& e, int64_t grp_off, int lane, uint32_t okmask,
-                                              const uint32_t (&v)[CP / 16][16], uint4 (&r)[CP * sizeof(TOut) / 16]) {
+                                              const uint32_t (&v)[CP / 16][16], uint4 (&r)[CP * sizeof(TOut) / 16],
+                                              int ncopy, int64_t zstep) {
   if (e.slope == 0.f) {                             // ReLU (the aggregation layers): one instruction per value
-    if (e.residual) sc_fast_store<CP, TOut, true, 0>(e, grp_off, lane, okmask, v, r);
-    else            sc_fast_store<CP, TOut, false, 0>(e, grp_off, lane, okmask, v, r);
+    if (e.residual) sc_fast_store<CP, TOut, true, 0>(e, grp_off, lane, okmask, v, r, ncopy, zstep);
+    else            sc_fast_store<CP, TOut, false, 0>(e, grp_off, lane, okmask, v, r, ncopy, zstep);
   } else {
-    if (e.residual) sc_fast_store<CP, TOut, true, 2>(e, grp_off, lane, okmask, v, r);
-    else            sc_fast_store<CP, TOut, false, 2>(e, grp_off, lane, okmask, v, r);
+    if (e.residual) sc_fast_store<CP, TOut, true, 2>(e, grp_off, lane, okmask, v, r, ncopy, zstep);
+    else            sc_fast_store<CP, TOut, false, 2>(e, grp_off, lane, okmask, v, r, ncopy, zstep);
   }
 }
 
@@ -519,7 +572,8 @@ __device__ __forceinline__ void sc_epilogue(const ScArgs& a, ScCtrl& ctrl, uint3
   uint32_t aphase = 0;
   const int ncols = cta_cols(a);
   for (int ci = 0; ci < ncols; ++ci) {
-    const Col c = decode_col(a, blockIdx.x + ci * gridDim.x);
+    const Item it = cta_item(a, ci);
+    const Col& c = it.c;
     const bool rowok = c.y0 + yl < a.p.oH && c.n < a.p.N;
     const bool ok = rowok && c.x0 + xl < a.p.oW;
     const int64_t row_off = (int64_t)c.n * a.p.osN + (int64_t)(c.y0 + yl) * a.p.osH + (int64_t)c.x0 * a.p.osW;
@@ -529,7 +583,7 @@ __device__ __forceinline__ void sc_epilogue(const ScArgs& a, ScCtrl& ctrl, uint3
 #pragma unroll
     for (int k = 0; k < NCH; ++k) okmask |= (rowok && c.x0 + xb + k < a.p.oW) ? (1u << k) : 0u;
     int slot = 0, z = 0;                              // next output plane to drain and its slot (z % 3)
-    for (int p = 0; p < D; ++p) {
+    for (int p = 0; p < D; p = next_plane(it, p)) {
       // input plane p done => out plane p-1 is complete; after the last input plane so is out plane D-1
       const int ndrain = (p >= 1 ? 1 : 0) + (p == D - 1 ? 1 : 0);
       uint4 r[NCH];
@@ -562,17 +616,21 @@ __device__ __forceinline__ void sc_epilogue(const ScArgs& a, ScCtrl& ctrl, uint3
         const int64_t zo = (int64_t)(c.zb + z) * a.p.osD;
         const bool stz = z >= zs0 && z < zs1 && c.zb + z < a.p.oD;       // z-split: a chunk's border planes are not stored
         const uint32_t om = stz ? okmask : 0u;
+        const int ncopy = z == it.zs ? it.J : 0;      // out planes zs + 1 .. zs + J are copies of plane zs (never z-split)
         if constexpr (kFast) {
           // (second drain of the last plane: its residual could not be prefetched)
           if (i == 1 && a.residual) sc_res_load<NCH, TOut>(fe, grp_off + zo, fe.osW, lane, om, r);
-          if constexpr (kSRes >= 0) sc_fast_store<CP, TOut, kSRes != 0, kSAct>(fe, grp_off + zo, lane, om, v, r);
-          else sc_fast_plane<CP, TOut>(fe, grp_off + zo, lane, om, v, r);
+          if constexpr (kSRes >= 0) sc_fast_store<CP, TOut, kSRes != 0, kSAct>(fe, grp_off + zo, lane, om, v, r, ncopy, a.p.osD);
+          else sc_fast_plane<CP, TOut>(fe, grp_off + zo, lane, om, v, r, ncopy, a.p.osD);
         } else {
           if (ok && stz) {
+            for (int k = 0; k <= ncopy; ++k) {
 #pragma unroll
-            for (int j = 0; j < CP / 16; ++j) epilogue_store16(ep, pix_off + zo, 16 * j, v[j]);
+              for (int j = 0; j < CP / 16; ++j) epilogue_store16(ep, pix_off + zo + k * a.p.osD, 16 * j, v[j]);
+            }
           }
         }
+        z += ncopy;                                   // ncopy % 3 == 0: the slot stays
         ++z;
         if (++slot == 3) slot = 0;
       }
@@ -801,7 +859,7 @@ conv_scatter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_cons
                         ptx::smem_u32(&ctrl.w_empty[0]), ptx::smem_u32(&ctrl.acc_full[0]), ptx::smem_u32(&ctrl.acc_empty[0]),
                         desc_hi(kHX * rb, rb), desc_hi(8 * rb, rb), a.slot_bytes, a.w_bytes, a.w_stages, a.ring,
                         (uint32_t)(rb >> 4), (uint32_t)(((kPair ? 3 * a.cp / 2 : 3 * a.cp) * rb) >> 4), (uint32_t)((kTileY * kHX * rb) >> 4), (uint32_t)(a.chunk_stride >> 4), a.idesc,
-                        a.dl, cta_cols(a)};
+                        a.dl, cta_cols(a), &a};
     if constexpr (kSplit) {
       // kPer counts the MMAs of one operand HALF here
       if constexpr (RB == 256) sc_issue<false, 1, 4, kPair, 2, true>(zi);

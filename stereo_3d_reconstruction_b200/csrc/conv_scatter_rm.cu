@@ -69,7 +69,7 @@ conv_scatter_rm_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_c
                         ptx::smem_u32(&ctrl.w_empty[0]), ptx::smem_u32(&ctrl.acc_full[0]), ptx::smem_u32(&ctrl.acc_empty[0]),
                         desc_hi(kHX * rb, rb), desc_hi(8 * rb, rb), a.slot_bytes, a.w_bytes, a.w_stages, a.ring,
                         (uint32_t)(rb >> 4), (uint32_t)(((3 * a.cp / 2) * rb) >> 4), (uint32_t)((kTileY * kHX * rb) >> 4),
-                        (uint32_t)(a.chunk_stride >> 4), a.idesc, a.dl, cta_cols(a)};
+                        (uint32_t)(a.chunk_stride >> 4), a.idesc, a.dl, cta_cols(a), &a};
     sc_issue<false, 1, 4, kPair, 1, false, true>(zi, &rs);
   } else if (warp >= 4) {
     sc_epilogue<CP, __nv_bfloat16, true, 0, kSAct>(a, ctrl, tmem_base, warp, lane);

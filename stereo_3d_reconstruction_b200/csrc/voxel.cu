@@ -43,6 +43,7 @@ const KnobName kKnobNames[] = {
     {"igemm_one_cta", "S3D_IGEMM_ONE_CTA", &Knobs::igemm_one_cta},
     {"chamfer_sym", "S3D_CHAMFER_SYM", &Knobs::chamfer_sym},
     {"chamfer_sym_r", "S3D_CHAMFER_SYM_R", &Knobs::chamfer_sym_r},
+    {"no_dz_skip", "S3D_NO_DZ_SKIP", &Knobs::no_dz_skip},
 };
 }  // namespace
 

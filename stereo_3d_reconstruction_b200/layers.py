@@ -103,6 +103,63 @@ def _choose_bn(cout_pad, m_tiles=None, n_sms=148):
     return divs[-1]
 
 
+# ---- constant-region skip of the plane-scatter kernel (include/s3d.h dz_nref, csrc/conv_scatter.cuh Item) ------------
+# A column is a 32 x 8 pixel patch of one volume marching over the D planes.  Its output planes [zs, zs + J] repeat: the
+# kernel marches the input planes dz_march(zs, J, D) and stores out plane zs J more times.  These functions mirror the
+# kernel's arithmetic so that the schedule (and the tests) can reason about it without a GPU.
+
+plane_counter = None      # int64 CUDA tensor [1] or None: every conv launch ADDS the input planes its scatter CTAs marched
+
+
+def dz_first(col, N, nref, oH, oW, c):
+    """First output plane of the repeating run of column `col` (conv_scatter.cuh dz_first); 0 for an empty column."""
+    cy, cx = -(-oH // 32), -(-oW // 8)
+    if col >= N * cy * cx:
+        return 0
+    n, x0 = col // (cy * cx), (col % cx) * 8
+    xr = min(x0 + 7, oW - 1) if n < nref else oW - 1 - x0
+    return xr + c + 2
+
+
+def dz_jump(zs, D, e):
+    """Planes skipped by a run starting at zs: the largest multiple of 3 <= (D - 2 - e) - zs (0 below 3)."""
+    ze = D - 2 - e
+    return (ze - zs) // 3 * 3 if ze - zs >= 3 else 0
+
+
+def dz_march(zs, J, D):
+    """Input planes a work item marches, in order (conv_scatter.cuh next_plane)."""
+    out, p = [], 0
+    while p < D:
+        out.append(p)
+        p = p + 1 + J if p == zs + 1 else p + 1
+    return out
+
+
+def dz_schedule(N, nref, oH, oW, D, c, e, npairs):
+    """Pairing + balance table of the CTA pairs (include/s3d.h dz_sched) -> (int32 list, planes marched per pair).
+
+    Partners issue the same MMAs, so they walk the intersection of their runs: columns are sorted by their first repeating
+    plane and paired neighbour by neighbour (equal runs except at group borders; an odd column gets an empty partner).
+    The pairs of columns are then dealt out longest first, each to the least loaded CTA pair."""
+    total = N * -(-oH // 32) * -(-oW // 8)
+    first = [dz_first(k, N, nref, oH, oW, c) for k in range(total)]
+    cols = sorted(range(total), key=lambda k: (first[k], k))
+    items = [(cols[i], cols[i + 1] if i + 1 < total else total) for i in range(0, total, 2)]
+    cost = [D - dz_jump(max(first[a], first[b] if b < total else 0), D, e) for a, b in items]
+    load, lists = [0] * npairs, [[] for _ in range(npairs)]
+    for i in sorted(range(len(items)), key=lambda i: (-cost[i], i)):
+        q = min(range(npairs), key=lambda q: (load[q], q))
+        load[q] += cost[i]
+        lists[q].append(items[i])
+    offs, ent = [0], []
+    for lst in lists:
+        offs.append(offs[-1] + len(lst))
+        for a, b in lst:
+            ent += [a, b]
+    return offs + ent, load
+
+
 class PackedConv:
     """One folded + packed conv-like layer.  `taps`: list (per class) of lists of (dz,dy,dx)."""
 
@@ -361,8 +418,8 @@ class PackedConv:
             return iD, iH, iW
         return tuple((i + 2 * p - k) // s + 1 for i, k, p, s in zip((iD, iH, iW), self.ksize, self.pad, self.stride))
 
-    def params(self, N, iD, iH, iW, out_strides, out_dtype_code, cout_store=None, os_lo=0):
-        key = (N, iD, iH, iW, tuple(out_strides), out_dtype_code, cout_store, os_lo)
+    def params(self, N, iD, iH, iW, out_strides, out_dtype_code, cout_store=None, os_lo=0, region=None):
+        key = (N, iD, iH, iW, tuple(out_strides), out_dtype_code, cout_store, os_lo, region)
         p = self._cache.get(key)
         if p is not None:
             return p
@@ -390,11 +447,24 @@ class PackedConv:
         p.w_nstack = self.weight_ns.data_ptr() if self.weight_ns is not None else None
         if self.proj is not None:
             p.proj_w, p.proj_channel, p.proj_act = self.proj[0].data_ptr(), self.proj[1], self.proj[2]
+        if region is not None:
+            # the table lives as long as the cached params (built once per shape: graph replay reuses it)
+            p.dz_nref, p.dz_c, p.dz_e = region
+            dev = self.weight.device
+            ncols = N * -(-oH // 32) * -(-oW // 8)
+            p.dz_pairs = max(1, min(torch.cuda.get_device_properties(dev).multi_processor_count // 2, -(-ncols // 2)))
+            table, _ = dz_schedule(N, p.dz_nref, oH, oW, oD, p.dz_c, p.dz_e, p.dz_pairs)
+            sched = torch.tensor(table, dtype=torch.int32).to(dev)
+            p.dz_sched, p.dz_sched_keep = sched.data_ptr(), sched
         self._cache[key] = p
         return p
 
-    def __call__(self, x, out=None, residual=None, out_dtype=None, cout_store=None, out_view=None, engine='igemm'):
+    def __call__(self, x, out=None, residual=None, out_dtype=None, cout_store=None, out_view=None, engine='igemm', dz=None):
         """x: channels-last [N,D,H,W,Cin_pad] contiguous CUDA tensor ([.., hi(Cin_pad) | lo(Cin_pad)] for a split layer).
+
+        dz: None or (nref, c, e): x is N = 2 * nref volumes whose plane z is the same for z in [xr + c, D - 1 - e]
+        (include/s3d.h dz_nref; xr = x for the first nref volumes, W - 1 - x for the others).  Only a hint: the
+        plane-scatter kernel computes the repeating output planes once, every other engine ignores it.
 
         out: destination tensor (allocated if None) -- `out_view` optionally gives
         (data_ptr_offset_elems, (osN, osD, osH, osW[, osC])) to write into a channel slice of a wider buffer
@@ -434,7 +504,8 @@ class PackedConv:
             off, strides = out_view[:2]
             os_lo = out_view[2] if len(out_view) > 2 else 0
             assert code != _lib.DTYPE_BF16X2 or os_lo > 0, 'a split output view needs its hi -> lo offset'
-        p = self.params(N, iD, iH, iW, strides, code, cout_store, os_lo)
+        p = self.params(N, iD, iH, iW, strides, code, cout_store, os_lo, dz)
+        p.dz_planes = None if plane_counter is None else plane_counter.data_ptr()
         L = _lib.load()
         fn = L.s3d_conv_igemm if engine == 'igemm' else L.s3d_conv_direct
         esz = out.element_size()

@@ -37,6 +37,8 @@ class S3dConvParams(ctypes.Structure):
         ('bn', ctypes.c_int32),
         ('proj_w', ctypes.c_void_p), ('proj_channel', ctypes.c_int32), ('proj_act', ctypes.c_int32),
         ('w_nstack', ctypes.c_void_p),
+        ('dz_nref', ctypes.c_int32), ('dz_c', ctypes.c_int32), ('dz_e', ctypes.c_int32), ('dz_pairs', ctypes.c_int32),
+        ('dz_sched', ctypes.c_void_p), ('dz_planes', ctypes.c_void_p),
     ]
 
 
@@ -121,7 +123,7 @@ def check(rc, what):
 # at run time (tests, A/B scripts) -- a model picks host-side knobs up at its next pack().
 HOST_KNOBS = ('no_vol2d', 'no_concat_fuse', 'no_cls_fused', 'no_conv_first', 'no_d2s', 'no_ref_once', 'no_cls_chain', 'no_sheared', 'no_map_conv', 'no_conv2d_halo')
 LIB_KNOBS = ('no_scatter', 'scatter_tps3', 'scatter_no_pair', 'scatter_ring', 'scatter_res_transpose',
-             'scatter_no_transpose', 'scatter_generic', 'no_corr_tc', 'scatter_zsplit', 'scatter_no_rm', 'igemm_ts1', 'igemm_one_cta', 'scatter_one_cta', 'no_conv_first_tc', 'chamfer_sym', 'chamfer_sym_r')
+             'scatter_no_transpose', 'scatter_generic', 'no_corr_tc', 'scatter_zsplit', 'scatter_no_rm', 'igemm_ts1', 'igemm_one_cta', 'scatter_one_cta', 'no_conv_first_tc', 'chamfer_sym', 'chamfer_sym_r', 'no_dz_skip')
 KNOBS = {k: int(os.environ.get('S3D_' + k.upper()) is not None) for k in HOST_KNOBS}
 KNOBS['no_scatter'] = int(os.environ.get('S3D_NO_SCATTER') is not None)        # both sides look at this one
 

@@ -343,9 +343,13 @@ class _StereoBase(nn.Module):
                 assert feat.shape[-1] == cm * C, 'FEAT_CHANNELS must be a multiple of 16'
                 vol = ops.cost_volume_concat(feat, B, D, out=self._buf('vol', (2 * B, D, h, w, 2 * cm * C), dt), split=self._split)
                 a = self._conv('dres0a', vol, out=self._bufo('a0', 'dres0a', vol))
-            a = self._conv('dres0b', a, out=self._bufo('a1', 'dres0b', a))
-            y = self._conv('dres1a', a, out=self._bufo('a2', 'dres1a', a))
-            a = self._conv('dres1b', y, residual=a, out=self._bufo('a3', 'dres1b', y))
+            # Where the target half of the concat volume is zero around a pixel (d > x + 1 left-referenced, d > w - 2 - x
+            # right-referenced), a0 is the same on every plane up to D - 2: the layers below compute such planes once
+            # (include/s3d.h dz_nref).  Each 3x3x3 layer moves the region one plane in from both ends.  bf16 only.
+            bf = self.precision == 'bf16'
+            a = self._conv('dres0b', a, out=self._bufo('a1', 'dres0b', a), dz=(B, 3, 1) if bf else None)
+            y = self._conv('dres1a', a, out=self._bufo('a2', 'dres1a', a), dz=(B, 5, 2) if bf else None)
+            a = self._conv('dres1b', y, residual=a, out=self._bufo('a3', 'dres1b', y), dz=(B, 7, 3) if bf else None)
             S = self._packed['cls_b'].cout_pad                      # 27 taps padded to 32 planes
             pa = self._packed['cls_a']
             if (self.precision == 'bf16' and isinstance(pa, PackedConv) and pa.weight_ns is not None and pa.cin_pad == 64 and
