@@ -913,5 +913,77 @@ KernFn split_kernel(bool lean, bool pair, int phys_row_bytes, int cp, bool resid
 typedef void (*KernFnR)(CUtensorMap, CUtensorMap, CUtensorMap, ScArgs);
 KernFnR rm_kernel(bool relu);
 
+// ---- host side: the decisions every plane-scatter launcher shares (conv_scatter.cu, conv_scatter_concat.cu,
+// conv_scatter_cls.cu).  Shared-memory budgets, ring depths, weight stages and kernel choices stay with each launcher.
+
+// Plane slots, weight stages and the kernels' shared-memory base are 1024-byte aligned (the 128B-swizzle atom pattern).
+inline int align1024(int bytes) { return (bytes + 1023) / 1024 * 1024; }
+
+// A layer the plane-scatter kernels compute: stride 1, the 27 taps of a 3x3x3 kernel in canonical order (dz major, dx
+// fastest), output grid = input grid, one class, and a plain output (no coordinate multipliers, projection or planar
+// channel stride).
+inline bool plane_scatter_layer(const S3dConvParams& p) {
+  if (p.n_classes != 1 || p.sx != 1 || p.sy != 1 || p.sz != 1 || p.ntaps != 27) return false;
+  if (p.omx != 1 || p.omy != 1 || p.omz != 1 || p.osC != 1 || p.proj_w) return false;
+  if (p.oD != p.iD || p.oH != p.iH || p.oW != p.iW) return false;
+  for (int t = 0; t < 27; ++t)
+    if (p.dz[t] != t / 9 - 1 || p.dy[t] != (t % 9) / 3 - 1 || p.dx[t] != t % 3 - 1) return false;
+  return true;
+}
+
+// Plane slots of nchunks K chunks of row_bytes bytes (kc channels) each, the kTY x kTX columns of a.p's output grid and
+// no z-split (a work item marches its whole column).  -> the column count.
+inline int64_t plane_geometry(ScArgs& a, int row_bytes, int kc, int nchunks) {
+  a.row_bytes = row_bytes;  a.kc = kc;  a.nchunks = nchunks;
+  a.chunk_stride = align1024(kPlaneRows * row_bytes);
+  a.slot_bytes = nchunks * a.chunk_stride;
+  a.cols_x = ceil_div(a.p.oW, kTX);  a.cols_y = ceil_div(a.p.oH, kTY);
+  a.nz = 1;  a.zc = a.p.oD;  a.dl = a.p.oD;
+  return (int64_t)a.p.N * a.cols_x * a.cols_y;
+}
+
+// Deals `total` work items to at most `grid` CTAs (a.pair decided): CTA pairs take an even grid and each walks
+// ncols_max items (cta_cols), single CTAs stride over the items.  -> the grid to launch.
+inline int deal_columns(ScArgs& a, int64_t total, int grid) {
+  a.total_cols = (int)total;
+  if (a.pair) {
+    if ((int64_t)grid > total) grid = (int)((total + 1) / 2 * 2);
+    grid -= grid % 2;
+    a.ncols_max = (int)((total + grid - 1) / grid);
+  } else if ((int64_t)grid > total) grid = (int)total;
+  return grid;
+}
+
+// The transposed (coalesced) epilogue stores: 16-byte aligned out / residual (nullptr: none), 16-byte multiples as
+// pixel strides, osW < 2^24, a bias, every channel stored, a none / ReLU / LeakyReLU activation.
+inline bool coalesced_store_ok(const S3dConvParams& p, const float* bias, const void* out, const void* residual, int out_elem_size) {
+  const bool simple_act = p.act == S3D_ACT_NONE || p.act == S3D_ACT_RELU || p.act == S3D_ACT_LEAKY;
+  auto aligned = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+  auto dense16 = [&](int64_t st) { return (st * out_elem_size) % 16 == 0; };
+  return simple_act && bias != nullptr && p.cout_store == p.Cout && aligned(out) && aligned(residual) &&
+         dense16(p.osW) && dense16(p.osH) && dense16(p.osD) && dense16(p.osN) && p.osW < (1ll << 24);
+}
+
+// Launches a plane-scatter kernel with `smem` bytes of dynamic shared memory: as clusters of two CTAs when `pair`
+// (cta_group::2), plainly otherwise.
+template <typename... KArgs, typename... Args>
+int launch_plane_scatter(void (*kern)(KArgs...), int grid, int smem, bool pair, cudaStream_t stream, const Args&... args) {
+  S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  if (pair) {
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3(grid);  cfg.blockDim = dim3(kThreads);  cfg.dynamicSmemBytes = smem;  cfg.stream = stream;
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = 2;  attr.val.clusterDim.y = 1;  attr.val.clusterDim.z = 1;
+    cfg.attrs = &attr;  cfg.numAttrs = 1;
+    S3D_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
+  } else {
+    kern<<<grid, kThreads, smem, stream>>>(args...);
+  }
+  S3D_LAUNCH_CHECK();
+  return S3D_OK;
+}
+
 }  // namespace scatter
 }  // namespace s3d

@@ -387,11 +387,8 @@ extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p_in, const void* i
   if (!p_in || !in || !bias || !w_taps || !workspace || !disp) { set_error("conv_cls_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   const S3dConvParams& p = *p_in;
   S3D_CHECK_ARG(p.w_nstack != nullptr, "conv_cls_soft_argmin: the layer needs host-packed rotations (w_nstack)");
-  S3D_CHECK_ARG(p.in_dtype == S3D_DTYPE_BF16 && p.Cin == 64 && p.Cout == 64 && p.act == S3D_ACT_RELU && p.n_classes == 1 &&
-                p.ntaps == 27 && p.sx == 1 && p.sy == 1 && p.sz == 1 && p.oD == p.iD && p.oH == p.iH && p.oW == p.iW,
-                "conv_cls_soft_argmin: needs a bf16 stride-1 3x3x3 64 -> 64 ReLU layer");
-  for (int t = 0; t < 27; ++t)
-    S3D_CHECK_ARG(p.dz[t] == t / 9 - 1 && p.dy[t] == (t % 9) / 3 - 1 && p.dx[t] == t % 3 - 1, "conv_cls_soft_argmin: tap order");
+  S3D_CHECK_ARG(plane_scatter_layer(p) && p.in_dtype == S3D_DTYPE_BF16 && p.Cin == 64 && p.Cout == 64 && p.act == S3D_ACT_RELU,
+                "conv_cls_soft_argmin: needs a bf16 stride-1 3x3x3 64 -> 64 ReLU layer in canonical tap order");
   S3D_CHECK_ARG(((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(w_taps) | reinterpret_cast<uintptr_t>(workspace)) & 15) == 0,
                 "conv_cls_soft_argmin: pointers must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -401,23 +398,14 @@ extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p_in, const void* i
   ScArgs& a = ca.a;
   a.p = p;  a.bias = bias;  a.residual = nullptr;  a.out = nullptr;
   ca.partials = static_cast<float*>(workspace);
-  a.nchunks = 1;  a.row_bytes = 128;  a.kc = 64;
-  a.chunk_stride = (kPlaneRows * 128 + 1023) / 1024 * 1024;
-  a.slot_bytes = a.chunk_stride;
+  const int64_t total = plane_geometry(a, 128, 64, 1);
   a.cp = 64;  a.tps = 1;
-  a.nz = 1;  a.zc = p.oD;  a.dl = p.oD;
-  a.cols_x = ceil_div(p.oW, kTX);  a.cols_y = ceil_div(p.oH, kTY);
-  const int64_t total = (int64_t)p.N * a.cols_x * a.cols_y;
   S3D_CHECK_ARG(total >= 2 && total < (1ll << 31), "conv_cls_soft_argmin: needs at least two columns (CTA pairs)");
-  a.total_cols = (int)total;
-  int grid = num_sms();
   a.pair = 1;
-  if ((int64_t)grid > total) grid = (int)((total + 1) / 2 * 2);
-  grid -= grid % 2;
-  a.ncols_max = (int)((total + grid - 1) / grid);
+  const int grid = deal_columns(a, total, num_sms());
   const int w_rows = 3 * a.cp / 2;
   a.w_tx = w_rows * 128;
-  a.w_bytes = (a.w_tx + 1023) / 1024 * 1024;
+  a.w_bytes = align1024(a.w_tx);
   const int extra = kYBytes + 2048;
   const int budget = 227 * 1024 - 1024 - 640 - extra;
   a.ring = 3;
@@ -438,17 +426,8 @@ extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p_in, const void* i
   if (rc != S3D_OK) return rc;
 
   const int smem_bytes = a.ring * a.slot_bytes + a.w_stages * a.w_bytes + extra + 1024;
-  auto kern = conv_scatter_cls_kernel<true>;
-  S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid);  cfg.blockDim = dim3(kThreads);  cfg.dynamicSmemBytes = smem_bytes;  cfg.stream = st;
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeClusterDimension;
-  attr.val.clusterDim.x = 2;  attr.val.clusterDim.y = 1;  attr.val.clusterDim.z = 1;
-  cfg.attrs = &attr;  cfg.numAttrs = 1;
-  S3D_CUDA(cudaLaunchKernelEx(&cfg, kern, map_x, map_w, map_wb, ca));
-  S3D_LAUNCH_CHECK();
+  rc = launch_plane_scatter(conv_scatter_cls_kernel<true>, grid, smem_bytes, a.pair, st, map_x, map_w, map_wb, ca);
+  if (rc != S3D_OK) return rc;
   const int64_t npix = (int64_t)p.N * p.oH * p.oW;
   partials_soft_argmin_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(ca.partials, disp, p.N, p.oD, p.oH, p.oW, a.cols_x, a.cols_y, sign);
   S3D_LAUNCH_CHECK();

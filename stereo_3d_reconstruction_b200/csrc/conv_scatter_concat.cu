@@ -1063,10 +1063,7 @@ static int launch_concat_ros(const S3dConvParams& p, const void* feat, int feat_
   using namespace s3d::scatter;
   S3D_CHECK_ARG(w_refonce != nullptr, "conv_concat_volume: split (BF16X2) operands need the reference-once form (s3d_conv_concat_volume_ro)");
   S3D_CHECK_ARG(p.w_nstack != nullptr && bias != nullptr, "conv_concat_volume_ro: the layer needs host-packed rotations (w_nstack) and a bias");
-  S3D_CHECK_ARG(p.n_classes == 1 && p.ntaps == 27 && p.sx == 1 && p.sy == 1 && p.sz == 1 && p.omx == 1 && p.omy == 1 && p.omz == 1 &&
-                p.osC == 1 && !p.proj_w && p.oD == p.iD && p.oH == p.iH && p.oW == p.iW, "conv_concat_volume_ro: not a stride-1 3x3x3 layer");
-  for (int t = 0; t < 27; ++t)
-    S3D_CHECK_ARG(p.dz[t] == t / 9 - 1 && p.dy[t] == (t % 9) / 3 - 1 && p.dx[t] == t % 3 - 1, "conv_concat_volume_ro: tap order");
+  S3D_CHECK_ARG(plane_scatter_layer(p), "conv_concat_volume_ro: not a stride-1 3x3x3 layer in canonical tap order");
   S3D_CHECK_ARG(p.N % 2 == 0 && p.Cin == 64 && p.Cout == 64 && p.cout_store == 64 && p.out_dtype == S3D_DTYPE_BF16X2 && p.act == S3D_ACT_RELU,
                 "conv_concat_volume_ro (split): needs C = 32 feature channels, Cout = 64, a split output and ReLU");
   const int C = 32, B = p.N / 2, D = p.iD, h = p.iH, w = p.iW, rb = 128;
@@ -1081,23 +1078,14 @@ static int launch_concat_ros(const S3dConvParams& p, const void* feat, int feat_
   a.p = p;  a.bias = bias;  a.residual = nullptr;  a.out = out;
   a.split = 1;  a.os_lo = p.os_lo ? p.os_lo : (int64_t)p.Cout;
   ca.n_half = B;  ca.D = D;
-  a.nchunks = 1;  a.row_bytes = rb;  a.kc = C;
-  a.chunk_stride = (kPlaneRows * rb + 1023) / 1024 * 1024;
-  a.slot_bytes = a.chunk_stride;
+  const int64_t total = plane_geometry(a, rb, C, 1);
   a.cp = 64;  a.tps = 1;
-  a.nz = 1;  a.zc = D;  a.dl = D;
-  a.cols_x = ceil_div(w, kTX);  a.cols_y = ceil_div(h, kTY);
-  const int64_t total = (int64_t)p.N * a.cols_x * a.cols_y;
   S3D_CHECK_ARG(total >= 2 && total < (1ll << 31), "conv_concat_volume_ro: column count out of range");
-  a.total_cols = (int)total;
-  int grid = num_sms();
   a.pair = 1;
-  if ((int64_t)grid > total) grid = (int)((total + 1) / 2 * 2);
-  grid -= grid % 2;
-  a.ncols_max = (int)((total + grid - 1) / grid);
+  const int grid = deal_columns(a, total, num_sms());
   const int w_rows = 3 * a.cp / 2;
   a.w_tx = 2 * w_rows * 64;                                     // [w_hi | w_lo] tiles of 64-byte rows
-  a.w_bytes = (a.w_tx + 1023) / 1024 * 1024;
+  a.w_bytes = align1024(a.w_tx);
   ra.w_tx_r = (a.cp / 2) * 128;
   ra.idesc_r = ptx::make_instr_desc(1, 256, a.cp);
   const int budget = 227 * 1024 - 1024 - 640;
@@ -1107,11 +1095,8 @@ static int launch_concat_ros(const S3dConvParams& p, const void* feat, int feat_
   S3D_CHECK_ARG(a.w_stages >= 3, "conv_concat_volume_ro (split): not enough shared memory");
   a.idesc = ptx::make_instr_desc(1, 256, 3 * a.cp);
   a.res_direct = 1;
-  {
-    auto dense16 = [&](int64_t s_) { return (s_ * 2) % 16 == 0; };
-    a.fast_store = dense16(p.osW) && dense16(p.osH) && dense16(p.osD) && dense16(p.osN) && dense16(a.os_lo) && p.osW < (1ll << 24);
-    S3D_CHECK_ARG(a.fast_store, "conv_concat_volume_ro (split): output strides must be multiples of 16 bytes");
-  }
+  a.fast_store = coalesced_store_ok(p, bias, out, nullptr, 2) && (a.os_lo * 2) % 16 == 0;
+  S3D_CHECK_ARG(a.fast_store, "conv_concat_volume_ro (split): output strides must be multiples of 16 bytes");
   const uint8_t* fb = static_cast<const uint8_t*>(feat);
   const cuuint64_t px = 2 * C * 2, row = (cuuint64_t)feat_pitch * px, img = (cuuint64_t)h * row;
   CUtensorMap map_ref, map_tl, map_tr, map_w, map_wr;
@@ -1137,18 +1122,8 @@ static int launch_concat_ros(const S3dConvParams& p, const void* feat, int feat_
   rc = encode_weight_map(&map_wr, w_refonce, 2, false, 2 * C, a.cp, 27, 2 * C, a.cp / 2, CU_TENSOR_MAP_SWIZZLE_128B, 1);
   if (rc != S3D_OK) return rc;
   const int smem_bytes = (2 + a.ring) * a.slot_bytes + a.w_stages * a.w_bytes + 1024;
-  auto kern = conv_scatter_concat_ros_kernel<true>;
-  S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid);  cfg.blockDim = dim3(kThreads);  cfg.dynamicSmemBytes = smem_bytes;  cfg.stream = st;
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeClusterDimension;
-  attr.val.clusterDim.x = 2;  attr.val.clusterDim.y = 1;  attr.val.clusterDim.z = 1;
-  cfg.attrs = &attr;  cfg.numAttrs = 1;
-  S3D_CUDA(cudaLaunchKernelEx(&cfg, kern, map_ref, map_tl, map_tr, map_w, map_wr, ra));
-  S3D_LAUNCH_CHECK();
-  return S3D_OK;
+  return launch_plane_scatter(conv_scatter_concat_ros_kernel<true>, grid, smem_bytes, a.pair, st, map_ref, map_tl, map_tr, map_w,
+                              map_wr, ra);
 }
 
 // w_refonce != nullptr: reference-once mode (bf16, CTA pairs, Cout = 64, ReLU, coalesced stores only).
@@ -1163,10 +1138,7 @@ static int launch_concat(const S3dConvParams* p_in, const void* feat, int feat_p
   const bool tf32 = p.in_dtype == S3D_DTYPE_F32;
   const int esz = tf32 ? 4 : 2;
   S3D_CHECK_ARG(p.w_nstack != nullptr, "conv_concat_volume: the layer needs host-packed rotations (w_nstack)");
-  S3D_CHECK_ARG(p.n_classes == 1 && p.ntaps == 27 && p.sx == 1 && p.sy == 1 && p.sz == 1 && p.omx == 1 && p.omy == 1 && p.omz == 1 &&
-                p.osC == 1 && !p.proj_w && p.oD == p.iD && p.oH == p.iH && p.oW == p.iW, "conv_concat_volume: not a stride-1 3x3x3 layer");
-  for (int t = 0; t < 27; ++t)
-    S3D_CHECK_ARG(p.dz[t] == t / 9 - 1 && p.dy[t] == (t % 9) / 3 - 1 && p.dx[t] == t % 3 - 1, "conv_concat_volume: tap order");
+  S3D_CHECK_ARG(plane_scatter_layer(p), "conv_concat_volume: not a stride-1 3x3x3 layer in canonical tap order");
   S3D_CHECK_ARG(p.N % 2 == 0 && p.Cin % 2 == 0, "conv_concat_volume: N = 2B volumes, Cin = 2C channels");
   const int C = p.Cin / 2, B = p.N / 2, D = p.iD, h = p.iH, w = p.iW;
   const int rb = C * esz;
@@ -1183,26 +1155,17 @@ static int launch_concat(const S3dConvParams* p_in, const void* feat, int feat_p
   ScArgs& a = ca.a;
   a.p = p;  a.bias = bias;  a.residual = nullptr;  a.out = out;
   ca.n_half = B;  ca.D = D;
-  a.nchunks = 2;  a.row_bytes = rb;  a.kc = C;
-  a.chunk_stride = (kPlaneRows * rb + 1023) / 1024 * 1024;
+  const int64_t total = plane_geometry(a, rb, C, 2);          // (no z-split here: small batches take the unfused path)
   a.slot_bytes = a.chunk_stride;                               // a slot holds ONE half (reference buffers / target ring)
   a.cp = p.Cout;  a.tps = 1;
-  a.nz = 1;  a.zc = D;  a.dl = D;                              // (no z-split here: small batches take the unfused path)
-  a.cols_x = ceil_div(w, kTX);  a.cols_y = ceil_div(h, kTY);
-  const int64_t total = (int64_t)p.N * a.cols_x * a.cols_y;
   S3D_CHECK_ARG(total > 0 && total < (1ll << 31), "conv_concat_volume: column count out of range");
-  a.total_cols = (int)total;
   int grid = num_sms();
   a.pair = ((3 * a.cp / 2) % 8 == 0 && total >= 2 && grid >= 2 && !knobs().scatter_no_pair) ? 1 : 0;
-  if (a.pair) {
-    if ((int64_t)grid > total) grid = (int)((total + 1) / 2 * 2);
-    grid -= grid % 2;
-    a.ncols_max = (int)((total + grid - 1) / grid);
-  } else if ((int64_t)grid > total) grid = (int)total;
+  grid = deal_columns(a, total, grid);
   const int w_rows = a.pair ? 3 * a.cp / 2 : 3 * a.cp;
   // one stage = one tap, both K chunks; reference-once: kTps taps of the target chunk
   a.w_tx = ro ? kTps * w_rows * rb : 2 * w_rows * rb;
-  a.w_bytes = (a.w_tx + 1023) / 1024 * 1024;
+  a.w_bytes = align1024(a.w_tx);
   const int budget = 227 * 1024 - 1024 - 640;
   int ring = 4;
   while (ring > 2 && (2 + ring) * a.slot_bytes + 4 * a.w_bytes > budget) --ring;
@@ -1212,13 +1175,7 @@ static int launch_concat(const S3dConvParams* p_in, const void* feat, int feat_p
   S3D_CHECK_ARG(a.w_stages >= 2 && (a.pair || rb < 128), "conv_concat_volume: not enough shared memory (128-byte halves need CTA pairs)");
   a.idesc = ptx::make_instr_desc(tf32 ? 2 : 1, a.pair ? 256 : 128, 3 * a.cp);
   a.res_direct = 1;
-  {
-    const int oesz = p.out_dtype == S3D_DTYPE_BF16 ? 2 : 4;
-    const bool simple_act = p.act == S3D_ACT_NONE || p.act == S3D_ACT_RELU || p.act == S3D_ACT_LEAKY;
-    auto dense16 = [&](int64_t s_) { return (s_ * oesz) % 16 == 0; };
-    a.fast_store = simple_act && bias != nullptr && p.cout_store == p.Cout && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
-                   dense16(p.osW) && dense16(p.osH) && dense16(p.osD) && dense16(p.osN) && p.osW < (1ll << 24);
-  }
+  a.fast_store = coalesced_store_ok(p, bias, out, nullptr, p.out_dtype == S3D_DTYPE_BF16 ? 2 : 4);
 
   const CUtensorMapSwizzle sw = rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
   const uint8_t* fb = static_cast<const uint8_t*>(feat);
@@ -1248,13 +1205,6 @@ static int launch_concat(const S3dConvParams* p_in, const void* feat, int feat_p
   if (rc != S3D_OK) return rc;
 
   const int smem_bytes = (2 + a.ring) * a.slot_bytes + a.w_stages * a.w_bytes + 1024;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid);  cfg.blockDim = dim3(kThreads);  cfg.dynamicSmemBytes = smem_bytes;  cfg.stream = st;
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeClusterDimension;
-  attr.val.clusterDim.x = 2;  attr.val.clusterDim.y = 1;  attr.val.clusterDim.z = 1;
-  cfg.attrs = &attr;  cfg.numAttrs = 1;
   if (ro) {
     const bool simple = a.pair && !tf32 && p.out_dtype == S3D_DTYPE_BF16 && a.fast_store && a.cp == 64 && p.act == S3D_ACT_RELU;
     S3D_CHECK_ARG(simple && rb <= 64 && a.w_stages >= 4,
@@ -1270,10 +1220,7 @@ static int launch_concat(const S3dConvParams* p_in, const void* feat, int feat_p
     if (rc != S3D_OK) return rc;
     typedef void (*KernR)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, RoArgs);
     KernR kern = rb == 64 ? conv_scatter_concat_ro_kernel<true, 2> : conv_scatter_concat_ro_kernel<true, 1>;
-    S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-    S3D_CUDA(cudaLaunchKernelEx(&cfg, kern, map_ref, map_tl, map_tr, map_w, map_wr, ra));
-    S3D_LAUNCH_CHECK();
-    return S3D_OK;
+    return launch_plane_scatter(kern, grid, smem_bytes, a.pair, st, map_ref, map_tl, map_tr, map_w, map_wr, ra);
   }
   typedef void (*Kern)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CcArgs);
   const bool lean = a.pair && !tf32 && p.out_dtype == S3D_DTYPE_BF16 && a.fast_store && a.cp == 64 && p.act == S3D_ACT_RELU && rb == 64;
@@ -1288,14 +1235,7 @@ static int launch_concat(const S3dConvParams* p_in, const void* feat, int feat_p
     kern = tf32 ? conv_scatter_concat_kernel<true, false, 2, false>
                 : (rb == 64 ? conv_scatter_concat_kernel<false, false, 2, false> : conv_scatter_concat_kernel<false, false, 1, false>);
   }
-  S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-  if (a.pair) {
-    S3D_CUDA(cudaLaunchKernelEx(&cfg, kern, map_ref, map_tl, map_tr, map_w, ca));
-  } else {
-    kern<<<grid, kThreads, smem_bytes, st>>>(map_ref, map_tl, map_tr, map_w, ca);
-  }
-  S3D_LAUNCH_CHECK();
-  return S3D_OK;
+  return launch_plane_scatter(kern, grid, smem_bytes, a.pair, st, map_ref, map_tl, map_tr, map_w, ca);
 }
 
 extern "C" int s3d_conv_concat_volume(const S3dConvParams* p, const void* feat, int feat_pitch, int feat_pad, const float* bias,

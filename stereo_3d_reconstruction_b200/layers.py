@@ -111,6 +111,17 @@ def _choose_bn(cout_pad, m_tiles=None, n_sms=148):
 plane_counter = None      # int64 CUDA tensor [1] or None: every conv launch ADDS the input planes its scatter CTAs marched
 
 
+def scatter_columns(N, h, w):
+    """Columns of the plane-scatter kernel over N volumes of h x w planes: 32 (y) x 8 (x) patches (conv_scatter.cuh kTY, kTX)."""
+    return N * -(-h // 32) * -(-w // 8)
+
+
+def more_columns_than_pairs(N, h, w):
+    """More plane-scatter columns than a B200's 74 CTA pairs (148 SMs): the launcher runs whole columns, no z-split
+    (conv_scatter.cu, conv_scatter_launch)."""
+    return scatter_columns(N, h, w) > 74
+
+
 def dz_first(col, N, nref, oH, oW, c):
     """First output plane of the repeating run of column `col` (conv_scatter.cuh dz_first); 0 for an empty column."""
     cy, cx = -(-oH // 32), -(-oW // 8)
@@ -142,7 +153,7 @@ def dz_schedule(N, nref, oH, oW, D, c, e, npairs):
     Partners issue the same MMAs, so they walk the intersection of their runs: columns are sorted by their first repeating
     plane and paired neighbour by neighbour (equal runs except at group borders; an odd column gets an empty partner).
     The pairs of columns are then dealt out longest first, each to the least loaded CTA pair."""
-    total = N * -(-oH // 32) * -(-oW // 8)
+    total = scatter_columns(N, oH, oW)
     first = [dz_first(k, N, nref, oH, oW, c) for k in range(total)]
     cols = sorted(range(total), key=lambda k: (first[k], k))
     items = [(cols[i], cols[i + 1] if i + 1 < total else total) for i in range(0, total, 2)]
@@ -451,7 +462,7 @@ class PackedConv:
             # the table lives as long as the cached params (built once per shape: graph replay reuses it)
             p.dz_nref, p.dz_c, p.dz_e = region
             dev = self.weight.device
-            ncols = N * -(-oH // 32) * -(-oW // 8)
+            ncols = scatter_columns(N, oH, oW)
             p.dz_pairs = max(1, min(torch.cuda.get_device_properties(dev).multi_processor_count // 2, -(-ncols // 2)))
             table, _ = dz_schedule(N, p.dz_nref, oH, oW, oD, p.dz_c, p.dz_e, p.dz_pairs)
             sched = torch.tensor(table, dtype=torch.int32).to(dev)
@@ -555,7 +566,7 @@ class PackedConv:
     def _call_as_volume(self, x, out, residual, cout_store, out_view):
         """Run a batch of images [N,1,H,W,C] through the 27-tap twin as G volumes of N/G planes (see __init__)."""
         N, _, H, W, C = x.shape
-        patches = -(-H // 32) * -(-W // 8)                     # columns per volume in conv_scatter.cu
+        patches = scatter_columns(1, H, W)                     # columns per volume
         # G volumes of N/G images: minimise waves x (planes per column + pipeline fill/drain), 148 columns per wave
         G = min((g for g in range(1, N + 1) if N % g == 0),
                 key=lambda g: (-(-g * patches // 148) * (N // g + 2), g))

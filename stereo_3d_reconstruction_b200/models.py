@@ -19,7 +19,7 @@ import torch.nn as nn
 
 from . import lib as _lib
 from . import ops
-from .layers import PackedConv, SplitConv, pad_to, torch_dtype, cmult
+from .layers import PackedConv, SplitConv, pad_to, torch_dtype, cmult, more_columns_than_pairs
 
 A = _lib  # activation / dtype codes
 
@@ -306,7 +306,7 @@ class _StereoBase(nn.Module):
                        not _lib.KNOBS['no_concat_fuse'] and not _lib.KNOBS['no_scatter'] and
                        # small batches: fewer columns than SMs -> unfused volume + the z-split plane-scatter kernel (a column of
                        # D planes would be a serial chain on a fraction of the chip; csrc/conv_scatter.cuh, ScArgs::nz)
-                       (sheared or 2 * B * (-(-h // 32)) * (-(-w // 8)) > 74))
+                       (sheared or more_columns_than_pairs(2 * B, h, w)))
         cm = cmult(self._dtype_code())                           # physical channels per logical channel (2 when split)
         if fuse_volume:
             # features go into rows with D zero pixels on both sides: the fused cost-volume + dres0a kernel reads the shifted
@@ -354,7 +354,7 @@ class _StereoBase(nn.Module):
             pa = self._packed['cls_a']
             if (self.precision == 'bf16' and isinstance(pa, PackedConv) and pa.weight_ns is not None and pa.cin_pad == 64 and
                     pa.cout_pad == 64 and pa.act == _lib.ACT_RELU and S == 32 and a.shape[-1] == 64 and
-                    2 * B * (-(-h // 32)) * (-(-w // 8)) > 74 and
+                    more_columns_than_pairs(2 * B, h, w) and
                     not _lib.KNOBS['no_cls_chain'] and not _lib.KNOBS['no_cls_fused'] and not _lib.KNOBS['no_scatter']):
                 # cls_a + classifier + soft-argmin in one march, cls_a's 2.1 GB output never written (csrc/conv_scatter_cls.cu)
                 nb = ops.conv_cls_workspace_bytes(2 * B, D, h, w)
