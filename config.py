@@ -90,6 +90,9 @@ __C.TEST.DISP_THRESH = [1.0, 3.0]
 # left-right consistency check (forward(..., lr_check=True)): a pixel is kept when its disparity d and the other view's
 # disparity at the pixel it points to (x -/+ round(d)) differ by at most this many px; finite, >= 0
 __C.TEST.LR_THRESH = 1.0
+# disparity uncertainty (forward(..., uncertainty=True)): a pixel counts as confident at t when the standard deviation of its
+# soft-argmin distribution, in input px, is <= t; at most 4, each finite and >= 0
+__C.TEST.UNC_THRESH = [1.0, 2.0, 4.0]
 # F-score thresholds of the point-cloud evaluation (Stereo2Point forward(..., gt)): a point counts when its nearest neighbour
 # in the other cloud is closer than t, a Euclidean distance in the points' units (0.01 = F-Score@1% on unit-scale shapes);
 # at most 8, each finite and > 0

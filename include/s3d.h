@@ -254,6 +254,38 @@ int s3d_upsample_disp_lr(const float* disp_q, float* disp, uint8_t* lr_mask, flo
                          const float* thresholds, int T, float max_gt, long long* disp_stats, long long* lr_stats,
                          int B, int h, int w, int H, int W, float scale, void* stream);
 
+/* --- disparity uncertainty ------------------------------------------------------------------------------------------------
+ * The *_std entry points below take the arguments of their siblings plus disp_std_q fp32 [N,h,w] (non-NULL).  They write the
+ * same disp bit for bit, and into disp_std_q the standard deviation of each pixel's soft-argmin distribution, in planes:
+ * with p_d = softmax_d(sign * cost_d) the weights whose mean is disp_q,
+ *   sigma_q = sqrt(sum_d p_d (d - disp_q)^2)     (fp32, >= 0; NaN where disp_q is not finite).
+ * The corr kernels include the cost-0 planes outside the image, as for the mean.  Accuracy: |sigma_q - sigma_ref| <= 1e-4 *
+ * (1 + sigma_ref) against sigma_ref computed in fp64 from the same costs, also for sharp peaks at large d (the online kernels
+ * accumulate the moments about the running arg-max plane, the corr kernels take a second pass about the mean). */
+int s3d_tap_gather_soft_argmin_std(const float* taps, float* disp, float* disp_std_q, float* cost_out, int N, int D, int h, int w,
+                                   int tap_stride, float sign, void* stream);
+int s3d_cls_soft_argmin_std(const void* x, const void* w_taps, float* disp, float* disp_std_q, int N, int D, int h, int w, int C,
+                            float sign, void* stream);
+int s3d_conv_cls_soft_argmin_std(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps, void* workspace,
+                                 float* disp, float* disp_std_q, float sign, void* stream);
+int s3d_corr_soft_argmin_std(const void* feat, float* disp, float* disp_std_q, float* cost_out, int B, int h, int w,
+                             int C, int c_real, int D, int dtype, void* stream);
+/* s3d_upsample_disp (+ s3d_upsample_disp_eval when gt is set, + s3d_upsample_disp_lr when lr_mask is set) + the upsampled
+ * standard deviation and confidence-filtered counters, in one launch.  disp, disp_stats, lr_mask and lr_stats are what the
+ * siblings write / add, bit for bit.  disp_std_q fp32 [2B,h,w] (from a *_std entry point) -> disp_std fp32 [B,2,H,W] (view 0
+ * = left-referenced) = bilinear(scale * disp_std_q), bit-identical to s3d_upsample_disp(disp_std_q, scale) of the image.
+ * unc_thresh: K <= 4 HOST values in input pixels, finite and >= 0.  unc_stats int64 [B,2,K,3+T], ACCUMULATED: per view and
+ * threshold k, over the CONFIDENT pixels (disp_std <= unc_thresh[k] in fp32; a non-finite disp_std never is)
+ *   [n_conf, n_valid_conf, sum_{valid & conf} q(|disp - gt|), count_{valid & conf}(|disp - gt| > thresholds[t]) for t < T]
+ * (valid and q as for s3d_upsample_disp_eval; the range argument there holds for these sums, which run over fewer pixels).
+ * gt == NULL needs disp_stats == NULL and adds column 0 only; T still sets the row length.  lr_mask and lr_stats come together
+ * (NULL: no LR check), lr_thresh as for s3d_upsample_disp_lr.  disp_std is bit-identical to s3d_upsample_disp where both take the
+ * same (16-byte or scalar) path: W % 4 == 0 and 16-byte aligned outputs, or neither. */
+int s3d_upsample_disp_std(const float* disp_q, float* disp, const float* disp_std_q, float* disp_std, const float* unc_thresh,
+                          int K, long long* unc_stats, const float* gt, const float* thresholds, int T, float max_gt,
+                          long long* disp_stats, uint8_t* lr_mask, float lr_thresh, long long* lr_stats, int B, int h, int w,
+                          int H, int W, float scale, void* stream);
+
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)
  * re-indexing of the oracle, written channels-last as [N,2,2,2,C*L*L/8].

@@ -28,6 +28,8 @@ def get_args():
     p.add_argument('--n-samples', type=int, default=None, help='synthetic test-set size (default: one batch per rank)')
     p.add_argument('--lr-check', action='store_true',
                    help='also run the left-right disparity consistency check and report it as lr_consistency')
+    p.add_argument('--uncertainty', action='store_true',
+                   help='also compute the per-pixel disparity uncertainty and report the confidence-filtered metrics as uncertainty')
     return p.parse_args()
 
 
@@ -96,23 +98,29 @@ def main():
     model.cuda().pack()
     # one stats vector: the head's statistics, then the disparity counters of the same forwards
     if args.model == 'Stereo2Voxel':
-        stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check).cpu()
+        stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check,
+                             eval_unc=args.uncertainty).cpu()
         nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
         res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
     else:
         # + the point-cloud counters (Chamfer L2 / L1, precision, recall, F-score) of the same forwards, at the very end
-        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check, eval_points=True).cpu()
+        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check, eval_points=True,
+                             eval_unc=args.uncertainty).cpu()
         nh = 2
         res = T.chamfer_summary(stats[:nh])
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH))
     nl = 2 * (3 + len(cfg.TEST.DISP_THRESH)) if args.lr_check else 0
+    nu = 2 * len(cfg.TEST.UNC_THRESH) * (3 + len(cfg.TEST.DISP_THRESH)) if args.uncertainty else 0
     res['disparity'] = T.disp_summary(stats[nh:nh + nd], cfg.TEST.DISP_THRESH)
     if args.lr_check:
         res['lr_consistency'] = T.lr_summary(stats[nh + nd:nh + nd + nl], cfg.TEST.DISP_THRESH,
                                              res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
         res['lr_consistency']['lr_thresh'] = float(cfg.TEST.LR_THRESH)
+    if args.uncertainty:
+        res['uncertainty'] = T.unc_summary(stats[nh + nd + nl:nh + nd + nl + nu], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH,
+                                           res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
     if args.model == 'Stereo2Point':
-        res['points'] = T.points_summary(stats[nh + nd + nl:], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
+        res['points'] = T.points_summary(stats[nh + nd + nl + nu:], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
                                          cfg.CONST.N_GT_POINTS)
     if rank == 0:
         res.update(model=args.model, precision=cfg.NETWORK.PRECISION, world_size=world, data='synthetic')

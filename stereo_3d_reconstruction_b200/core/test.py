@@ -11,6 +11,9 @@ forward computes against the synthetic GT disparity (models.py, _StereoBase._ups
     n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) per t in TEST.DISP_THRESH   (int64)
 With eval_lr=True (needs eval_disp) the left-right consistency counters of the same forwards follow, per view:
     n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the kept valid pixels  (int64)
+With eval_unc=True (needs eval_disp) the uncertainty counters of the same forwards follow, per view, then per threshold k in
+TEST.UNC_THRESH (models.py, _StereoBase._upsample_disp):
+    n_conf, n_valid_conf, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the confident valid pixels  (int64)
 With eval_points=True (test_point) the point-cloud counters of the same forwards come last (models.py,
 Stereo2Point._point_stats), per direction (predicted -> GT, then GT -> predicted), then per threshold t in
 TEST.FSCORE_THRESH:
@@ -21,7 +24,7 @@ with q(x) = round-half-even(x * 2^32); F_b is computed elementwise in fp64 on th
 import torch
 import torch.distributed as dist
 
-from ..models import fscore_thresholds
+from ..models import fscore_thresholds, unc_thresholds
 from ..utils import synthetic
 
 _FX = float(1 << 40)
@@ -93,6 +96,31 @@ def lr_summary(stats_block, thresholds, n_pixels, disp_block):
     return out
 
 
+def unc_summary(stats_block, unc_thresh, thresholds, n_pixels, disp_block):
+    """Uncertainty counters [n_conf, n_valid_conf, epe_fx, bad_t...] x K thresholds x 2 views (int64 [2 * K * (3 + T)]) -> dict,
+    per view and over both views a list over the K thresholds tau (the sparsification curve at those points): density =
+    n_conf / n_pixels (n_pixels: pixels of one view over the run), conf_of_valid = n_valid_conf / n_valid (n_valid from the
+    disparity counters `disp_block`, as for lr_summary), and EPE / bad-pixel fractions over the confident valid pixels."""
+    K, T = len(unc_thresh), len(thresholds)
+    v = [int(x) for x in stats_block.tolist()]
+    nv = [int(x) for x in disp_block.tolist()]
+    assert len(v) == 2 * K * (3 + T) and len(nv) == 2 * (2 + T)
+
+    def one(pix, n_valid, c):
+        nc, nvc, epe_fx, bad = c[0], c[1], c[2], c[3:]
+        return {'n_conf': nc, 'density': nc / pix if pix else 0.0, 'n_valid_conf': nvc,
+                'conf_of_valid': nvc / n_valid if n_valid else 0.0, 'epe': epe_fx / _DISP_FX / nvc if nvc else 0.0,
+                'bad': [b / nvc if nvc else 0.0 for b in bad]}
+    r = 3 + T
+    views = [[v[(vi * K + k) * r:(vi * K + k + 1) * r] for k in range(K)] for vi in range(2)]
+    valid = [nv[0], nv[2 + T]]
+    out = {'unc_thresh': list(unc_thresh), 'thresholds': list(thresholds)}
+    for name, rows, n in zip(('left', 'right'), views, valid):
+        out[name] = [one(n_pixels, n, c) for c in rows]
+    out['all'] = [one(2 * n_pixels, valid[0] + valid[1], [a + b for a, b in zip(views[0][k], views[1][k])]) for k in range(K)]
+    return out
+
+
 def point_block(point_stats, N, M):
     """Per-batch increment of the point block from the forward's point_stats int64 [B,2,3+T] (N predicted, M GT points per
     sample): the counters summed over the batch, then sum_b round-half-even(F_b(t) * 2^32) per threshold, in fp64."""
@@ -143,16 +171,26 @@ def _lr_len(cfg, eval_disp, eval_lr):
     return 2 * (3 + len(cfg.TEST.DISP_THRESH)) if eval_lr else 0
 
 
-def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False):
+def _unc_len(cfg, eval_disp, eval_unc):
+    if eval_unc and not eval_disp:
+        raise ValueError('eval_unc=True needs eval_disp=True')
+    # ValueError on a bad TEST.UNC_THRESH, before any forward
+    return 2 * len(unc_thresholds(cfg)) * (3 + len(cfg.TEST.DISP_THRESH)) if eval_unc else 0
+
+
+def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
+               eval_unc=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
-    eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones."""
+    eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
+    eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones."""
     th = list(cfg.TEST.VOXEL_THRESH)
     T = len(th)
     nl = _lr_len(cfg, eval_disp, eval_lr)
+    nu = _unc_len(cfg, eval_disp, eval_unc)
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    stats = torch.zeros(2 * T + 1 + nd + nl, dtype=torch.int64, device=device)
+    stats = torch.zeros(2 * T + 1 + nd + nl + nu, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -162,7 +200,14 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.gt_volume(1, cfg.CONST.N_VOX, seed=100000 + i) for i in ids]).to(device)
-            if eval_lr:
+            if eval_unc:
+                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=eval_lr, uncertainty=True)
+                iou, ds = out[3], out[4]
+                stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
+                if eval_lr:
+                    stats[2 * T + 1 + nd:2 * T + 1 + nd + nl] += out[6].sum(0).flatten()
+                stats[2 * T + 1 + nd + nl:] += out[-1].sum(0).flatten()
+            elif eval_lr:
                 _, _, _, iou, ds, _, ls = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
                 stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
                 stats[2 * T + 1 + nd:] += ls.sum(0).flatten()
@@ -178,14 +223,15 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
 
 
 def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_points=False):
-    """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, as
-    for test_voxel, + the point-cloud counters with eval_points: module docstring)."""
+               eval_points=False, eval_unc=False):
+    """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, the
+    uncertainty counters with eval_unc, as for test_voxel, + the point-cloud counters with eval_points: module docstring)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
     nl = _lr_len(cfg, eval_disp, eval_lr)
+    nu = _unc_len(cfg, eval_disp, eval_unc)
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
     npt = _point_len(cfg, eval_points)
-    stats = torch.zeros(2 + nd + nl + npt, dtype=torch.int64, device=device)
+    stats = torch.zeros(2 + nd + nl + nu + npt, dtype=torch.int64, device=device)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -196,7 +242,14 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.point_clouds(1, 1, cfg.CONST.N_GT_POINTS, seed=200000 + i)[1] for i in ids]).to(device)
             head = (gt,) if eval_points else ()
-            if eval_lr:
+            if eval_unc:
+                out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device), lr_check=eval_lr, uncertainty=True)
+                k = 3 + len(head)                                  # disp_stats, then [lr_mask, lr_stats], disp_std, unc_stats
+                stats[2:2 + nd] += out[k].sum(0).flatten()
+                if eval_lr:
+                    stats[2 + nd:2 + nd + nl] += out[k + 2].sum(0).flatten()
+                stats[2 + nd + nl:2 + nd + nl + nu] += out[-1].sum(0).flatten()
+            elif eval_lr:
                 out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
                 ds, ls = out[-3], out[-1]
                 stats[2:2 + nd] += ds.sum(0).flatten()
@@ -208,7 +261,7 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
                 out = model(left, right, *head)
             pts = out[2]
             if eval_points:
-                stats[2 + nd + nl:] += point_block(out[3], pts.shape[1], gt.shape[1])
+                stats[2 + nd + nl + nu:] += point_block(out[3], pts.shape[1], gt.shape[1])
             cd = chamfer_per_sample(pts.contiguous(), gt)
             stats[0] += torch.round(cd.sum() * _FX).to(torch.int64)
             stats[1] += len(ids)

@@ -42,6 +42,7 @@ struct ClsArgs {
   int row_bytes, slot_bytes, ring;
   int cols_x, cols_y, total_cols;
   uint32_t idesc;
+  float* std_q;        // kStd: the distribution's standard deviation [N,h,w]
 };
 
 struct ClsCtrl {
@@ -60,7 +61,7 @@ __device__ __forceinline__ Col decode_col(const ClsArgs& a, int c) {
   return r;
 }
 
-template <int kPer>                              // MMAs per tile = row_bytes / 32
+template <int kPer, bool kStd>                   // MMAs per tile = row_bytes / 32; kStd: also write std_q (common.cuh, SoftSpread)
 __global__ void __launch_bounds__(kThreads, 1)
 cls_fused_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w,
                  const __grid_constant__ ClsArgs a) {
@@ -161,11 +162,16 @@ cls_fused_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
     for (int ci = 0; ci < ncols; ++ci) {
       const Col c = decode_col(a, blockIdx.x + ci * gridDim.x);
       float m = -INFINITY, s = 0.f, t = 0.f;
+      SoftSpread u;
       float c0 = 0.f, c1 = 0.f, c2 = 0.f;          // partial costs of output planes p-1, p, p+1
       auto retire = [&](int z, float cst) {
         const float v = a.sign * cst;
-        if (v > m) { const float sc = expf(m - v); s *= sc; t *= sc; m = v; }
+        if (v > m) {
+          const float sc = expf(m - v); s *= sc; t *= sc; m = v;
+          if (kStd) { u.scale(sc);  u.move(z, s); }
+        }
         const float e = expf(v - m);  s += e;  t += e * (float)z;
+        if (kStd) u.add(e, z);
       };
       for (int p = 0; p < D; ++p) {
         ptx::mbar_wait_u32(bar_af + 8 * buf, aphase);
@@ -212,7 +218,10 @@ cls_fused_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
       }
       retire(D - 1, c0);
       const int y = c.y0 + yl, x = c.x0 + xl;
-      if (y < a.h && x < a.w) a.disp[((int64_t)c.n * a.h + y) * a.w + x] = t / s;
+      if (y < a.h && x < a.w) {
+        a.disp[((int64_t)c.n * a.h + y) * a.w + x] = t / s;
+        if (kStd) a.std_q[((int64_t)c.n * a.h + y) * a.w + x] = u.sigma(t / s, s);
+      }
     }
   }
 
@@ -227,8 +236,9 @@ cls_fused_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
 }  // namespace
 }  // namespace s3d
 
-extern "C" int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, int N, int D, int h, int w, int C,
-                                   float sign, void* stream) {
+// s3d_cls_soft_argmin (std_q == NULL) and s3d_cls_soft_argmin_std
+static int cls_soft_argmin(const void* x, const void* w_taps, float* disp, float* std_q, int N, int D, int h, int w, int C,
+                           float sign, void* stream) {
   using namespace s3d;
   if (!x || !w_taps || !disp) { set_error("cls_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(N > 0 && D > 0 && h > 0 && w > 0, "cls_soft_argmin: bad shape");
@@ -237,7 +247,7 @@ extern "C" int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* dis
                 "cls_soft_argmin: pointers must be 16-byte aligned");
   ClsArgs a;
   memset(&a, 0, sizeof(a));
-  a.disp = disp;  a.sign = sign;  a.N = N;  a.D = D;  a.h = h;  a.w = w;
+  a.disp = disp;  a.std_q = std_q;  a.sign = sign;  a.N = N;  a.D = D;  a.h = h;  a.w = w;
   a.row_bytes = C * 2;
   a.slot_bytes = kTiles * 128 * a.row_bytes;                // 384 rows; multiple of 1024
   const int fixed = 4096 + kTaps * kTS * 4 + 1024;          // weights + projection buffer + alignment slack
@@ -261,11 +271,23 @@ extern "C" int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* dis
   rc = encode_weight_map(&map_w, w_taps, 2, false, C, kN, 1, C, kN, sw, 1);
   if (rc != S3D_OK) return rc;
   const int smem_bytes = a.ring * a.slot_bytes + fixed;
-  auto kern = a.row_bytes == 128 ? cls_fused_kernel<4> : (a.row_bytes == 64 ? cls_fused_kernel<2> : cls_fused_kernel<1>);
+  auto kern = std_q ? (a.row_bytes == 128 ? cls_fused_kernel<4, true> : (a.row_bytes == 64 ? cls_fused_kernel<2, true> : cls_fused_kernel<1, true>))
+                    : (a.row_bytes == 128 ? cls_fused_kernel<4, false> : (a.row_bytes == 64 ? cls_fused_kernel<2, false> : cls_fused_kernel<1, false>));
   S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   int grid = num_sms();
   if (grid > a.total_cols) grid = a.total_cols;
   kern<<<grid, kThreads, smem_bytes, static_cast<cudaStream_t>(stream)>>>(map_x, map_w, a);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
+}
+
+extern "C" int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, int N, int D, int h, int w, int C,
+                                   float sign, void* stream) {
+  return cls_soft_argmin(x, w_taps, disp, nullptr, N, D, h, w, C, sign, stream);
+}
+
+extern "C" int s3d_cls_soft_argmin_std(const void* x, const void* w_taps, float* disp, float* disp_std_q, int N, int D, int h,
+                                       int w, int C, float sign, void* stream) {
+  if (!disp_std_q) { s3d::set_error("cls_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
+  return cls_soft_argmin(x, w_taps, disp, disp_std_q, N, D, h, w, C, sign, stream);
 }

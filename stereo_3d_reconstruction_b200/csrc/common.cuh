@@ -89,4 +89,35 @@ __device__ __forceinline__ float apply_act(float v, int act, float a) {
 // Out-of-line copy for epilogues that must stay small: 16 calls instead of 16 inlined switch bodies.
 static __device__ __noinline__ float apply_act_slow(float v, int act, float a) { return apply_act(v, act, a); }
 
+// sigma_q = sqrt(var) of a soft-argmin distribution; a non-finite mean gives NaN.
+__device__ __forceinline__ float soft_std(float var, float mu) {
+  return isfinite(mu) ? sqrtf(fmaxf(var, 0.f)) : __int_as_float(0x7fffffff);
+}
+
+// Spread of the soft-argmin distribution for the online (max, sum e, sum e*d) marches: the first and second moments of the
+// weights about the running arg-max plane r, s1 = sum e (d - r), s2 = sum e (d - r)^2, shifted when the max moves.  About 0,
+// sum e d^2 / sum e - mu^2 cancels in fp32 when mu is large and the peak sharp (D = 128, peak at 120, sigma 0.05: wrong in the
+// second digit).  About r it cannot: p_r >= 1/D, so s2 / s <= (D + 1) var.
+struct SoftSpread {
+  float s1 = 0.f, s2 = 0.f;
+  int r = 0;
+  // the max moved to plane z and s1, s2 and s (the sum of the weights) were rescaled to it
+  __device__ __forceinline__ void move(int z, float s) {
+    const float dl = (float)(r - z);
+    s2 = fmaf(dl * dl, s, fmaf(2.f * dl, s1, s2));
+    s1 = fmaf(dl, s, s1);
+    r = z;
+  }
+  __device__ __forceinline__ void scale(float sc) { s1 *= sc;  s2 *= sc; }
+  __device__ __forceinline__ void add(float e, int z) {
+    const float dz = (float)(z - r);
+    s1 = fmaf(e, dz, s1);
+    s2 = fmaf(e * dz, dz, s2);
+  }
+  __device__ __forceinline__ float sigma(float mu, float s) const {
+    const float a = s1 / s;
+    return soft_std(s2 / s - a * a, mu);
+  }
+};
+
 }  // namespace s3d

@@ -340,9 +340,11 @@ conv_scatter_cls_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
 // ---- partial cost planes -> disparity -------------------------------------------------------------------------------------------
 // One thread per pixel: cost[z] = own patch's cell + the cells of the neighbouring patches whose halo ring covers the pixel (left /
 // right, up / down, diagonal -- always in this order), then the online soft-argmin over z (cls_fused.cu's arithmetic).
+// kStd: also the distribution's standard deviation -> std_q (common.cuh, SoftSpread); disp is the same either way.
+template <bool kStd>
 __global__ void __launch_bounds__(256)
 partials_soft_argmin_kernel(const float* __restrict__ partials, float* __restrict__ disp, int N, int D, int h, int w, int cols_x,
-                            int cols_y, float sign) {
+                            int cols_y, float sign, float* __restrict__ std_q) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= (int64_t)N * h * w) return;
   const int x = (int)(idx % w), y = (int)((idx / w) % h), n = (int)(idx / ((int64_t)w * h));
@@ -359,6 +361,7 @@ partials_soft_argmin_kernel(const float* __restrict__ partials, float* __restric
   const float* p2 = hy ? cell_ptr(py + dyn, px, dyn > 0 ? -1 : kTY, xi) : nullptr;
   const float* p3 = (hx && hy) ? cell_ptr(py + dyn, px + dxn, dyn > 0 ? -1 : kTY, dxn > 0 ? -1 : kTX) : nullptr;
   float m = -INFINITY, s = 0.f, tt = 0.f;
+  SoftSpread u;
   for (int z = 0; z < D; ++z) {
     const int64_t o = (int64_t)z * kCells;
     float c = p0[o];
@@ -366,10 +369,15 @@ partials_soft_argmin_kernel(const float* __restrict__ partials, float* __restric
     if (p2) c += p2[o];
     if (p3) c += p3[o];
     const float v = sign * c;
-    if (v > m) { const float sc = expf(m - v); s *= sc; tt *= sc; m = v; }
+    if (v > m) {
+      const float sc = expf(m - v); s *= sc; tt *= sc; m = v;
+      if (kStd) { u.scale(sc);  u.move(z, s); }
+    }
     const float e = expf(v - m);  s += e;  tt += e * (float)z;
+    if (kStd) u.add(e, z);
   }
   disp[idx] = tt / s;
+  if (kStd) std_q[idx] = u.sigma(tt / s, s);
 }
 
 }  // namespace scatter
@@ -380,8 +388,9 @@ extern "C" int64_t s3d_conv_cls_workspace_bytes(int N, int D, int h, int w) {
   return (int64_t)N * ((h + kTY - 1) / kTY) * ((w + kTX - 1) / kTX) * D * kCells * 4;
 }
 
-extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p_in, const void* in, const float* bias, const void* w_taps,
-                                        void* workspace, float* disp, float sign, void* stream) {
+// s3d_conv_cls_soft_argmin (std_q == NULL) and s3d_conv_cls_soft_argmin_std
+static int conv_cls_soft_argmin(const S3dConvParams* p_in, const void* in, const float* bias, const void* w_taps, void* workspace,
+                                float* disp, float* std_q, float sign, void* stream) {
   using namespace s3d;
   using namespace s3d::scatter;
   if (!p_in || !in || !bias || !w_taps || !workspace || !disp) { set_error("conv_cls_soft_argmin: null argument"); return S3D_ERR_INVALID; }
@@ -429,7 +438,23 @@ extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p_in, const void* i
   rc = launch_plane_scatter(conv_scatter_cls_kernel<true>, grid, smem_bytes, a.pair, st, map_x, map_w, map_wb, ca);
   if (rc != S3D_OK) return rc;
   const int64_t npix = (int64_t)p.N * p.oH * p.oW;
-  partials_soft_argmin_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(ca.partials, disp, p.N, p.oD, p.oH, p.oW, a.cols_x, a.cols_y, sign);
+  const unsigned blocks = (unsigned)((npix + 255) / 256);
+  if (std_q)
+    partials_soft_argmin_kernel<true><<<blocks, 256, 0, st>>>(ca.partials, disp, p.N, p.oD, p.oH, p.oW, a.cols_x, a.cols_y, sign, std_q);
+  else
+    partials_soft_argmin_kernel<false><<<blocks, 256, 0, st>>>(ca.partials, disp, p.N, p.oD, p.oH, p.oW, a.cols_x, a.cols_y, sign,
+                                                               nullptr);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
+}
+
+extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps,
+                                        void* workspace, float* disp, float sign, void* stream) {
+  return conv_cls_soft_argmin(p, in, bias, w_taps, workspace, disp, nullptr, sign, stream);
+}
+
+extern "C" int s3d_conv_cls_soft_argmin_std(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps,
+                                            void* workspace, float* disp, float* disp_std_q, float sign, void* stream) {
+  if (!disp_std_q) { s3d::set_error("conv_cls_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
+  return conv_cls_soft_argmin(p, in, bias, w_taps, workspace, disp, disp_std_q, sign, stream);
 }

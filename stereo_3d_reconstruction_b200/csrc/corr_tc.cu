@@ -45,6 +45,7 @@ struct CorrArgs {
   int tiles_per_img, pair_tiles;   // pair tile = (stereo pair, two image rows): one load, two accumulators (left / right reference)
   float inv_c;
   uint32_t idesc;
+  float* std_q;        // kStd: the distribution's standard deviation [2B,h,w]
 };
 
 struct CorrCtrl {
@@ -57,6 +58,9 @@ struct CorrCtrl {
 // weight does not need): <= 2 ulp, results below 2^-126 flush to zero.
 __device__ __forceinline__ float ex2_approx(float x) { float r;  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));  return r; }
 
+// kStd: also the standard deviation of each pixel's distribution, from a third pass over the held exponentials about the mean
+// (exact two-pass variance; the zero-cost tail in closed form).
+template <bool kStd>
 __global__ void __launch_bounds__(kThreads, 1)
 corr_tc_kernel(const __grid_constant__ CUtensorMap map_f, const __grid_constant__ CorrArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -223,6 +227,27 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_f, const __grid_constant_
         t = fmaf(e0, tail_d, t);
       }
       if (x < w && y < a.h) a.disp[((int64_t)n * a.h + y) * w + x] = __fdividef(t, s);
+      if (kStd) {
+        // sum e (d - mu)^2 with d = x - xt (left view) or xt - x (right view): the same (xt - x - sgn mu)^2 for both
+        const float mu = __fdividef(t, s), c0 = (float)x + sgn * mu;
+        float v4[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          if (c >= c_lo && c <= c_hi) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const float dd = (float)(c * 16 + i) - c0;
+              v4[i & 3] = fmaf(__uint_as_float(u[c][i]) * dd, dd, v4[i & 3]);
+            }
+          }
+        }
+        float v2 = (v4[0] + v4[1]) + (v4[2] + v4[3]);
+        if (dz0 < D) {                                      // the tail: tail_cnt planes, mean tail_d, variance (cnt^2 - 1) / 12
+          const float dt = tail_d - mu;
+          v2 = fmaf(ex2_approx(-m) * tail_cnt, fmaf(dt, dt, (tail_cnt * tail_cnt - 1.f) * (1.f / 12.f)), v2);
+        }
+        if (x < w && y < a.h) a.std_q[((int64_t)n * a.h + y) * w + x] = soft_std(v2 / s, mu);
+      }
       img += step_img;  yt += step_row;
       if (yt >= a.tiles_per_img) { yt -= a.tiles_per_img;  ++img; }
     }
@@ -242,10 +267,10 @@ bool corr_tc_eligible(int w, int C, int D, int dtype) {
   return dtype == S3D_DTYPE_BF16 && w <= kWP && (C * 2) % 32 == 0 && C <= 6 * 64 && D >= 1 && !knobs().no_corr_tc;
 }
 
-int corr_tc_launch(const void* feat, float* disp, int B, int h, int w, int C, int D, float inv_c, cudaStream_t stream) {
+int corr_tc_launch(const void* feat, float* disp, float* std_q, int B, int h, int w, int C, int D, float inv_c, cudaStream_t stream) {
   CorrArgs a;
   memset(&a, 0, sizeof(a));
-  a.disp = disp;  a.B = B;  a.h = h;  a.w = w;  a.C = C;  a.D = D;
+  a.disp = disp;  a.std_q = std_q;  a.B = B;  a.h = h;  a.w = w;  a.C = C;  a.D = D;
   const int cb = C * 2;
   a.row_bytes = cb % 128 == 0 ? 128 : (cb % 64 == 0 ? 64 : 32);
   a.kc = a.row_bytes / 2;
@@ -272,10 +297,11 @@ int corr_tc_launch(const void* feat, float* disp, int B, int h, int w, int C, in
   int rc = encode_act_map(&map_f, feat, 2, false, C, w, h, B, 2, box, estr, sw);
   if (rc != S3D_OK) return rc;
   const int smem_bytes = a.stages * a.stage_bytes + 1024;
-  S3D_CUDA(cudaFuncSetAttribute(corr_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  auto kern = std_q ? corr_tc_kernel<true> : corr_tc_kernel<false>;
+  S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   int grid = num_sms();
   if (grid > a.pair_tiles) grid = a.pair_tiles;
-  corr_tc_kernel<<<grid, kThreads, smem_bytes, stream>>>(map_f, a);
+  kern<<<grid, kThreads, smem_bytes, stream>>>(map_f, a);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
 }

@@ -168,10 +168,12 @@ soft_argmin_v4_kernel(const float4* __restrict__ cost, float4* __restrict__ disp
 // fused with the soft-argmin over z so the cost volume itself never reaches HBM.
 // One thread per (n, y, x); marching over the input plane z' it keeps the three partial sums of the
 // output planes z'-1, z', z'+1 in registers and retires plane z'-1 into an online softmax.
+// kStd: also the distribution's standard deviation -> std_q (common.cuh, SoftSpread).
 // ------------------------------------------------------------------------------------------
+template <bool kStd>
 __global__ void __launch_bounds__(128)
 tap_gather_soft_argmin_kernel(const float* __restrict__ P, float* __restrict__ disp, float* __restrict__ cost_out,
-                              int N, int D, int h, int w, int ts, float sign) {
+                              int N, int D, int h, int w, int ts, float sign, float* __restrict__ std_q) {
   // taps are LINE-PLANAR: P[n][z][y][t][x]: for a fixed tap the lanes of a warp (consecutive x) read
   // consecutive floats (one coalesced wavefront per load, neighbours reuse L1), while the producer
   // writes each image line as one contiguous ts*w*4-byte block (DRAM-friendly).
@@ -182,12 +184,17 @@ tap_gather_soft_argmin_kernel(const float* __restrict__ P, float* __restrict__ d
   const float* Pn = P + (int64_t)n * D * ts * plane;
   const int64_t tstride = w, lstride = (int64_t)ts * w;      // tap stride, line stride
   float m = -INFINITY, s = 0.f, t = 0.f;
+  SoftSpread u;
   float c0 = 0.f, c1 = 0.f, c2 = 0.f;            // partial costs of output planes z'-1, z', z'+1
   auto retire = [&](int z, float c) {
     if (cost_out) cost_out[((int64_t)n * D + z) * plane + (int64_t)y * w + x] = c;
     const float v = sign * c;
-    if (v > m) { const float sc = expf(m - v); s *= sc; t *= sc; m = v; }
+    if (v > m) {
+      const float sc = expf(m - v); s *= sc; t *= sc; m = v;
+      if (kStd) { u.scale(sc);  u.move(z, s); }
+    }
     const float e = expf(v - m);  s += e;  t += e * (float)z;
+    if (kStd) u.add(e, z);
   };
   for (int zi = 0; zi < D; ++zi) {
     const float* Pz = Pn + (int64_t)zi * ts * plane;
@@ -212,6 +219,7 @@ tap_gather_soft_argmin_kernel(const float* __restrict__ P, float* __restrict__ d
   }
   retire(D - 1, c0);
   disp[(int64_t)n * plane + (int64_t)y * w + x] = t / s;
+  if (kStd) std_q[(int64_t)n * plane + (int64_t)y * w + x] = u.sigma(t / s, s);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -220,10 +228,13 @@ tap_gather_soft_argmin_kernel(const float* __restrict__ P, float* __restrict__ d
 constexpr int kXG = 4;   // x per thread
 constexpr int kDG = 8;   // d per thread
 
-template <typename T, bool kLeftRef>
+// kStd: also the standard deviation of each pixel's distribution -> std_row, in a second pass over the held costs about the
+// mean the first pass reduced (exact two-pass variance: one more value in the warp-shuffle reduction).
+template <typename T, bool kLeftRef, bool kStd>
 __device__ __forceinline__ void corr_row(const T* __restrict__ ref_g, const T* __restrict__ tgt_g,
                                          float* __restrict__ disp_row, float* __restrict__ cost_row,
-                                         int64_t cost_plane, int w, int C, int D, float inv_c, float* smem) {
+                                         int64_t cost_plane, int w, int C, int D, float inv_c, float* smem,
+                                         float* __restrict__ std_row) {
   const int WP = ((w + 3) & ~3);
   const int rs = WP + 4;                       // ref row stride (floats); +4 spreads banks
   const int ts = WP + D + 12 + 4;              // tgt row stride: zero pad D + window slack
@@ -267,7 +278,7 @@ __device__ __forceinline__ void corr_row(const T* __restrict__ ref_g, const T* _
 #pragma unroll
         for (int j = 0; j < kDG; ++j) acc[i][j] = fmaf(r[i], t[kLeftRef ? (8 + i - j) : (i + j)], acc[i][j]);
     }
-    float res[kXG];
+    float res[kXG], sd[kXG];
 #pragma unroll
     for (int i = 0; i < kXG; ++i) {
       float m = -INFINITY;
@@ -282,11 +293,25 @@ __device__ __forceinline__ void corr_row(const T* __restrict__ ref_g, const T* _
         tt += __shfl_xor_sync(0xffffffffu, tt, o);
       }
       res[i] = tt / s;
+      if (kStd) {
+        float v2 = 0.f;
+#pragma unroll
+        for (int j = 0; j < kDG; ++j) {
+          const float dd = (float)(d0 + j) - res[i];
+          v2 = fmaf(__expf(acc[i][j] - m) * dd, dd, v2);
+        }
+        for (int o = ndg >> 1; o > 0; o >>= 1) v2 += __shfl_xor_sync(0xffffffffu, v2, o);
+        sd[i] = soft_std(v2 / s, res[i]);
+      }
     }
     if (active) {
       if (dgi == 0) {
 #pragma unroll
         for (int i = 0; i < kXG; ++i) if (x0 + i < w) disp_row[x0 + i] = res[i];
+        if (kStd) {
+#pragma unroll
+          for (int i = 0; i < kXG; ++i) if (x0 + i < w) std_row[x0 + i] = sd[i];
+        }
       }
       if (cost_row) {
 #pragma unroll
@@ -299,10 +324,10 @@ __device__ __forceinline__ void corr_row(const T* __restrict__ ref_g, const T* _
   }
 }
 
-template <typename T>
+template <typename T, bool kStd>
 __global__ void __launch_bounds__(256)
 corr_soft_argmin_kernel(const T* __restrict__ feat, float* __restrict__ disp, float* __restrict__ cost_out,
-                        int B, int h, int w, int C, int D, float inv_c) {
+                        int B, int h, int w, int C, int D, float inv_c, float* __restrict__ std_q) {
   extern __shared__ float smem_f[];
   const int n = blockIdx.x / h, y = blockIdx.x % h;
   const bool left_ref = n < B;
@@ -312,8 +337,9 @@ corr_soft_argmin_kernel(const T* __restrict__ feat, float* __restrict__ disp, fl
   float* disp_row = disp + ((int64_t)n * h + y) * w;
   const int64_t plane = (int64_t)h * w;
   float* cost_row = cost_out ? cost_out + (int64_t)n * D * plane + (int64_t)y * w : nullptr;
-  if (left_ref) corr_row<T, true>(ref_g, tgt_g, disp_row, cost_row, plane, w, C, D, inv_c, smem_f);
-  else          corr_row<T, false>(ref_g, tgt_g, disp_row, cost_row, plane, w, C, D, inv_c, smem_f);
+  float* std_row = kStd ? std_q + ((int64_t)n * h + y) * w : nullptr;
+  if (left_ref) corr_row<T, true, kStd>(ref_g, tgt_g, disp_row, cost_row, plane, w, C, D, inv_c, smem_f, std_row);
+  else          corr_row<T, false, kStd>(ref_g, tgt_g, disp_row, cost_row, plane, w, C, D, inv_c, smem_f, std_row);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -335,6 +361,17 @@ __device__ __forceinline__ float up_px(const UpRow& r, int X, int w, float rx, f
   const float lx = sx - (float)x0, hx = 1.f - lx;
   const float v = r.hy * (hx * __ldg(r.p0 + x0) + lx * __ldg(r.p0 + x1)) + r.ly * (hx * __ldg(r.p1 + x0) + lx * __ldg(r.p1 + x1));
   return v * scale;
+}
+
+// up_px with its roundings spelled out: the contraction ptxas picks for upsample_disp_kernel.  Inlined next to other work it may
+// contract the same expression the other way round (1 ulp apart), so the scalar kStd path uses this to stay bit-identical.
+__device__ __forceinline__ float up_px_rn(const UpRow& r, int X, int w, float rx, float scale) {
+  float sx = ((float)X + 0.5f) * rx - 0.5f;  if (sx < 0.f) sx = 0.f;
+  const int x0 = (int)sx, x1 = x0 + (x0 < w - 1 ? 1 : 0);
+  const float lx = sx - (float)x0, hx = 1.f - lx;
+  const float a = __fmaf_rn(lx, __ldg(r.p0 + x1), __fmul_rn(hx, __ldg(r.p0 + x0)));
+  const float b = __fmaf_rn(lx, __ldg(r.p1 + x1), __fmul_rn(hx, __ldg(r.p1 + x0)));
+  return __fmul_rn(__fmaf_rn(r.hy, a, __fmul_rn(r.ly, b)), scale);
 }
 
 __global__ void upsample_disp_kernel(const float* __restrict__ q, float* __restrict__ out, int N, int h, int w,
@@ -411,8 +448,36 @@ struct DispCounters {
   }
 };
 
-// image n of [2B]: view = n / B (0 = left-referenced), sample b = n % B; gt / lr_mask [B,2,H,W], stats [B,2,2+nT],
-// lr_stats [B,2,3+nT]
+// Confidence-filtered counters (kStd): per threshold k < nU, the pixels whose upsampled standard deviation is <= ut.t[k]
+// (a non-finite one never is), and with kEval the disparity counters over those of them with valid GT.
+constexpr int kMaxUnc = 4;
+struct UncCounters {
+  unsigned n_conf[kMaxUnc] = {};
+  DispCounters c[kMaxUnc];
+
+  template <bool kEval>
+  __device__ __forceinline__ void add(float sd, float d, float g, const Thresh& ut, int nU, float max_gt, const Thresh& th,
+                                      int nT) {
+#pragma unroll
+    for (int k = 0; k < kMaxUnc; ++k) {
+      if (k < nU && sd <= ut.t[k]) {
+        ++n_conf[k];
+        if (kEval) c[k].add(d, g, max_gt, th, nT);
+      }
+    }
+  }
+
+  // -> rows [k][3 + nT] of the block's image, [n_conf, n_valid_conf, epe_fx, bad...] (column 0 only without kEval)
+  template <bool kEval>
+  __device__ __forceinline__ void flush(unsigned long long* __restrict__ dst, int nU, int nT) {
+#pragma unroll
+    for (int k = 0; k < kMaxUnc; ++k)
+      if (k < nU) c[k].flush<1>(dst + k * (3 + nT), kEval ? 3 + nT : 1, n_conf[k]);
+  }
+};
+
+// image n of [2B]: view = n / B (0 = left-referenced), sample b = n % B; gt / lr_mask / disp_std [B,2,H,W], stats
+// [B,2,2+nT], lr_stats [B,2,3+nT], unc_stats [B,2,nU,3+nT]
 __device__ __forceinline__ int64_t eval_image_index(int n, int B) { return (int64_t)(n % B) * 2 + n / B; }
 
 // Left-right consistency of the pixel at column X whose stored disparity is d (include/s3d.h, s3d_upsample_disp_lr).  `ro`:
@@ -426,12 +491,14 @@ __device__ __forceinline__ bool lr_kept(float d, int X, const UpRow& ro, int w, 
   return fabsf(__fsub_rn(d, up_px(ro, xo, w, rx, scale))) <= tau;     // NaN on the other side: not kept
 }
 
-template <bool kEval, bool kLR>
+// kStd: the same interpolation of the standard deviation std_q -> std_out, and the confidence-filtered counters (UncCounters).
+template <bool kEval, bool kLR, bool kStd>
 __global__ void __launch_bounds__(256)
 upsample_disp_eval_v4_kernel(const float* __restrict__ q, float4* __restrict__ out, const float4* __restrict__ gt, int B, int h,
                              int w, int H, int W4, float ry, float rx, float scale, Thresh th, int nT, float max_gt,
                              unsigned long long* __restrict__ stats, uint32_t* __restrict__ lr_mask, float lr_thresh,
-                             unsigned long long* __restrict__ lr_stats) {
+                             unsigned long long* __restrict__ lr_stats, const float* __restrict__ std_q,
+                             float4* __restrict__ std_out, Thresh ut, int nU, unsigned long long* __restrict__ unc_stats) {
   const int n = blockIdx.y;
   const int64_t img4 = (int64_t)H * W4;
   const float* q_img = q + (int64_t)n * h * w;
@@ -440,7 +507,10 @@ upsample_disp_eval_v4_kernel(const float* __restrict__ q, float4* __restrict__ o
   float4* out_img = out + n * img4;
   const float4* gt_img = kEval ? gt + eval_image_index(n, B) * img4 : nullptr;
   uint32_t* mask_img = kLR ? lr_mask + eval_image_index(n, B) * img4 : nullptr;
+  const float* std_img = kStd ? std_q + (int64_t)n * h * w : nullptr;
+  float4* std_out_img = kStd ? std_out + eval_image_index(n, B) * img4 : nullptr;
   DispCounters c, kc;                                               // all pixels / the kept ones (kLR)
+  UncCounters uc;                                                   // the confident ones (kStd)
   unsigned n_kept = 0;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < (uint32_t)img4; i += gridDim.x * blockDim.x) {
     const uint32_t X4 = i % (uint32_t)W4, Y = i / (uint32_t)W4;
@@ -468,16 +538,28 @@ upsample_disp_eval_v4_kernel(const float* __restrict__ q, float4* __restrict__ o
       }
       mask_img[i] = m;                                              // four mask bytes, one 32-bit store
     }
+    if (kStd) {
+      const UpRow rs = up_row(std_img, (int)Y, h, w, ry);
+      float sd[4];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) sd[k] = up_px(rs, 4 * (int)X4 + k, w, rx, scale);
+      std_out_img[i] = make_float4(sd[0], sd[1], sd[2], sd[3]);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) uc.add<kEval>(sd[k], o[k], g[k], ut, nU, max_gt, th, nT);
+    }
   }
   if (kEval) c.flush(stats + eval_image_index(n, B) * (2 + nT), 2 + nT);
   if (kLR) kc.flush<1>(lr_stats + eval_image_index(n, B) * (3 + nT), kEval ? 3 + nT : 1, n_kept);
+  if (kStd) uc.flush<kEval>(unc_stats + eval_image_index(n, B) * nU * (3 + nT), nU, nT);
 }
 
-template <bool kEval, bool kLR>
+template <bool kEval, bool kLR, bool kStd>
 __global__ void __launch_bounds__(256)
 upsample_disp_eval_kernel(const float* __restrict__ q, float* __restrict__ out, const float* __restrict__ gt, int B, int h, int w,
                           int H, int W, float scale, Thresh th, int nT, float max_gt, unsigned long long* __restrict__ stats,
-                          uint8_t* __restrict__ lr_mask, float lr_thresh, unsigned long long* __restrict__ lr_stats) {
+                          uint8_t* __restrict__ lr_mask, float lr_thresh, unsigned long long* __restrict__ lr_stats,
+                          const float* __restrict__ std_q, float* __restrict__ std_out, Thresh ut, int nU,
+                          unsigned long long* __restrict__ unc_stats) {
   const int n = blockIdx.y;
   const int img = H * W;                                            // < 2^31 (checked by the launcher)
   const float ry = (float)h / (float)H, rx = (float)w / (float)W;
@@ -487,7 +569,10 @@ upsample_disp_eval_kernel(const float* __restrict__ q, float* __restrict__ out, 
   float* out_img = out + (int64_t)n * img;
   const float* gt_img = kEval ? gt + eval_image_index(n, B) * img : nullptr;
   uint8_t* mask_img = kLR ? lr_mask + eval_image_index(n, B) * img : nullptr;
+  const float* std_img = kStd ? std_q + (int64_t)n * h * w : nullptr;
+  float* std_out_img = kStd ? std_out + eval_image_index(n, B) * img : nullptr;
   DispCounters c, kc;
+  UncCounters uc;
   unsigned n_kept = 0;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < img; i += gridDim.x * blockDim.x) {
     const int X = i % W, Y = i / W;
@@ -503,31 +588,50 @@ upsample_disp_eval_kernel(const float* __restrict__ q, float* __restrict__ out, 
       n_kept += keep;
       if (kEval && keep) kc.add(d, g, max_gt, th, nT);
     }
+    if (kStd) {
+      const float sd = up_px_rn(up_row(std_img, Y, h, w, ry), X, w, rx, scale);
+      std_out_img[i] = sd;
+      uc.add<kEval>(sd, d, g, ut, nU, max_gt, th, nT);
+    }
   }
   if (kEval) c.flush(stats + eval_image_index(n, B) * (2 + nT), 2 + nT);
   if (kLR) kc.flush<1>(lr_stats + eval_image_index(n, B) * (3 + nT), kEval ? 3 + nT : 1, n_kept);
+  if (kStd) uc.flush<kEval>(unc_stats + eval_image_index(n, B) * nU * (3 + nT), nU, nT);
 }
 
-// Shared launcher of s3d_upsample_disp_eval (kEval) and s3d_upsample_disp_lr (kLR, kEval when it has GT); arguments checked.
-template <bool kEval, bool kLR>
+// The standard-deviation arguments of launch_upsample_eval (kStd)
+struct UncArgs {
+  const float* std_q = nullptr;
+  float* std_out = nullptr;
+  Thresh ut = {};
+  int nU = 0;
+  long long* stats = nullptr;
+};
+
+// Shared launcher of s3d_upsample_disp_eval (kEval), s3d_upsample_disp_lr (kLR, kEval when it has GT) and
+// s3d_upsample_disp_std (kStd, with kEval / kLR when it has GT / a mask); arguments checked.
+template <bool kEval, bool kLR, bool kStd = false>
 int launch_upsample_eval(const float* disp_q, float* disp, const float* gt, const Thresh& th, int T, float max_gt,
                          long long* stats, uint8_t* lr_mask, float lr_thresh, long long* lr_stats, int B, int h, int w, int H,
-                         int W, float scale, cudaStream_t s) {
+                         int W, float scale, cudaStream_t s, const UncArgs& u = UncArgs()) {
   const int64_t img = (int64_t)H * W;
   auto* st = reinterpret_cast<unsigned long long*>(stats);
   auto* lst = reinterpret_cast<unsigned long long*>(lr_stats);
-  if (W % 4 == 0 && ((reinterpret_cast<uintptr_t>(disp) | reinterpret_cast<uintptr_t>(gt)) & 15) == 0 &&
+  auto* ust = reinterpret_cast<unsigned long long*>(u.stats);
+  if (W % 4 == 0 && ((reinterpret_cast<uintptr_t>(disp) | reinterpret_cast<uintptr_t>(gt) | reinterpret_cast<uintptr_t>(u.std_out)) &
+                     15) == 0 &&
       (reinterpret_cast<uintptr_t>(lr_mask) & 3) == 0) {
     // 16 outputs per thread: 4x fewer blocks (and counter atomics) than one vector per thread
     const dim3 grid((unsigned)ceil_div64(img / 4, 256 * 4), 2 * B);
-    upsample_disp_eval_v4_kernel<kEval, kLR><<<grid, 256, 0, s>>>(
+    upsample_disp_eval_v4_kernel<kEval, kLR, kStd><<<grid, 256, 0, s>>>(
         disp_q, reinterpret_cast<float4*>(disp), reinterpret_cast<const float4*>(gt), B, h, w, H, W / 4, (float)h / (float)H,
-        (float)w / (float)W, scale, th, T, max_gt, st, reinterpret_cast<uint32_t*>(lr_mask), lr_thresh, lst);
+        (float)w / (float)W, scale, th, T, max_gt, st, reinterpret_cast<uint32_t*>(lr_mask), lr_thresh, lst, u.std_q,
+        reinterpret_cast<float4*>(u.std_out), u.ut, u.nU, ust);
     S3D_LAUNCH_CHECK();
     return S3D_OK;
   }
-  upsample_disp_eval_kernel<kEval, kLR><<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * B), 256, 0, s>>>(
-      disp_q, disp, gt, B, h, w, H, W, scale, th, T, max_gt, st, lr_mask, lr_thresh, lst);
+  upsample_disp_eval_kernel<kEval, kLR, kStd><<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * B), 256, 0, s>>>(
+      disp_q, disp, gt, B, h, w, H, W, scale, th, T, max_gt, st, lr_mask, lr_thresh, lst, u.std_q, u.std_out, u.ut, u.nU, ust);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
 }
@@ -539,7 +643,7 @@ using namespace s3d;
 
 namespace s3d {
 bool corr_tc_eligible(int w, int C, int D, int dtype);
-int corr_tc_launch(const void* feat, float* disp, int B, int h, int w, int C, int D, float inv_c, cudaStream_t stream);
+int corr_tc_launch(const void* feat, float* disp, float* std_q, int B, int h, int w, int C, int D, float inv_c, cudaStream_t stream);
 }
 
 extern "C" int s3d_cost_volume_concat(const void* feat, void* vol, int B, int h, int w, int C, int D, int dtype,
@@ -583,8 +687,9 @@ extern "C" int s3d_soft_argmin(const float* cost, float* disp, int N, int D, int
   return S3D_OK;
 }
 
-extern "C" int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_out, int B, int h, int w, int C, int c_real,
-                                    int D, int dtype, void* stream) {
+// s3d_corr_soft_argmin (std_q == NULL) and s3d_corr_soft_argmin_std
+static int corr_soft_argmin(const void* feat, float* disp, float* std_q, float* cost_out, int B, int h, int w, int C, int c_real,
+                            int D, int dtype, void* stream) {
   if (!feat || !disp) { set_error("corr_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(dtype == S3D_DTYPE_F32 || dtype == S3D_DTYPE_BF16, "corr_soft_argmin: bad dtype");
   S3D_CHECK_ARG(B > 0 && h > 0 && w > 0 && C > 0 && D > 0, "corr_soft_argmin: bad shape");
@@ -593,7 +698,7 @@ extern "C" int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_o
   const float inv_c = 1.f / (float)(c_real > 0 ? c_real : C);
   // bf16 features, rows of up to 64 pixels, no debug cost output: Gram-matrix kernel on the tensor cores (corr_tc.cu)
   if (!cost_out && corr_tc_eligible(w, C, D, dtype))
-    return corr_tc_launch(feat, disp, B, h, w, C, D, inv_c, static_cast<cudaStream_t>(stream));
+    return corr_tc_launch(feat, disp, std_q, B, h, w, C, D, inv_c, static_cast<cudaStream_t>(stream));
   S3D_CHECK_ARG(D >= 8 && D <= 128 && (D & (D - 1)) == 0, "corr_soft_argmin (SIMT path): D must be a power of two in [8,128]");
   const int WP = (w + 3) & ~3;
   const size_t smem = (size_t)C * ((WP + 4) + (WP + D + 16)) * sizeof(float);
@@ -604,17 +709,29 @@ extern "C" int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_o
   if (threads > 256) threads = 256;
   if (threads < 32) threads = 32;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  auto launch = [&](auto kern, const auto* f) -> int {
+    S3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    kern<<<2 * B * h, threads, smem, st>>>(f, disp, cost_out, B, h, w, C, D, inv_c, std_q);
+    S3D_LAUNCH_CHECK();
+    return S3D_OK;
+  };
   if (dtype == S3D_DTYPE_BF16) {
-    S3D_CUDA(cudaFuncSetAttribute(corr_soft_argmin_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    corr_soft_argmin_kernel<__nv_bfloat16><<<2 * B * h, threads, smem, st>>>(
-        static_cast<const __nv_bfloat16*>(feat), disp, cost_out, B, h, w, C, D, inv_c);
-  } else {
-    S3D_CUDA(cudaFuncSetAttribute(corr_soft_argmin_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    corr_soft_argmin_kernel<float><<<2 * B * h, threads, smem, st>>>(
-        static_cast<const float*>(feat), disp, cost_out, B, h, w, C, D, inv_c);
+    const auto* f = static_cast<const __nv_bfloat16*>(feat);
+    return std_q ? launch(corr_soft_argmin_kernel<__nv_bfloat16, true>, f) : launch(corr_soft_argmin_kernel<__nv_bfloat16, false>, f);
   }
-  S3D_LAUNCH_CHECK();
-  return S3D_OK;
+  const auto* f = static_cast<const float*>(feat);
+  return std_q ? launch(corr_soft_argmin_kernel<float, true>, f) : launch(corr_soft_argmin_kernel<float, false>, f);
+}
+
+extern "C" int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_out, int B, int h, int w, int C, int c_real,
+                                    int D, int dtype, void* stream) {
+  return corr_soft_argmin(feat, disp, nullptr, cost_out, B, h, w, C, c_real, D, dtype, stream);
+}
+
+extern "C" int s3d_corr_soft_argmin_std(const void* feat, float* disp, float* disp_std_q, float* cost_out, int B, int h, int w,
+                                        int C, int c_real, int D, int dtype, void* stream) {
+  if (!disp_std_q) { set_error("corr_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
+  return corr_soft_argmin(feat, disp, disp_std_q, cost_out, B, h, w, C, c_real, D, dtype, stream);
 }
 
 extern "C" int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h, int w, int H, int W, float scale,
@@ -676,15 +793,68 @@ extern "C" int s3d_upsample_disp_lr(const float* disp_q, float* disp, uint8_t* l
                                            W, scale, s);
 }
 
-extern "C" int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* cost_out, int N, int D, int h, int w,
-                                          int tap_stride, float sign, void* stream) {
+extern "C" int s3d_upsample_disp_std(const float* disp_q, float* disp, const float* disp_std_q, float* disp_std,
+                                     const float* unc_thresh, int K, long long* unc_stats, const float* gt, const float* thresholds,
+                                     int T, float max_gt, long long* disp_stats, uint8_t* lr_mask, float lr_thresh,
+                                     long long* lr_stats, int B, int h, int w, int H, int W, float scale, void* stream) {
+  if (!disp_q || !disp || !disp_std_q || !disp_std || (K > 0 && (!unc_thresh || !unc_stats)) || (gt && T > 0 && !thresholds)) {
+    set_error("upsample_disp_std: null argument");
+    return S3D_ERR_INVALID;
+  }
+  S3D_CHECK_ARG(!gt == !disp_stats, "upsample_disp_std: gt and disp_stats must be both set or both NULL");
+  S3D_CHECK_ARG(!lr_mask == !lr_stats, "upsample_disp_std: lr_mask and lr_stats must be both set or both NULL");
+  S3D_CHECK_ARG(B > 0 && 2 * B < 65536 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31),
+                "upsample_disp_std: bad shape");
+  S3D_CHECK_ARG(K >= 0 && K <= kMaxUnc, "upsample_disp_std: K must be in [0, 4]");
+  S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "upsample_disp_std: T must be in [0, 8]");
+  S3D_CHECK_ARG(!lr_mask || lr_thresh >= 0.f, "upsample_disp_std: lr_thresh must be >= 0 (and not NaN)");
+  S3D_CHECK_ARG(!gt || max_gt > 0.f, "upsample_disp_std: max_gt must be > 0");
+  UncArgs u;
+  u.std_q = disp_std_q;  u.std_out = disp_std;  u.nU = K;  u.stats = unc_stats;
+  for (int k = 0; k < K; ++k) {
+    S3D_CHECK_ARG(unc_thresh[k] >= 0.f && unc_thresh[k] < INFINITY, "upsample_disp_std: unc_thresh must be finite and >= 0");
+    u.ut.t[k] = unc_thresh[k];
+  }
+  Thresh th;
+  for (int t = 0; t < kMaxThresh; ++t) th.t[t] = gt && t < T ? thresholds[t] : 0.f;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (gt && lr_mask)
+    return launch_upsample_eval<true, true, true>(disp_q, disp, gt, th, T, max_gt, disp_stats, lr_mask, lr_thresh, lr_stats, B, h,
+                                                  w, H, W, scale, s, u);
+  if (gt)
+    return launch_upsample_eval<true, false, true>(disp_q, disp, gt, th, T, max_gt, disp_stats, nullptr, 0.f, nullptr, B, h, w, H,
+                                                   W, scale, s, u);
+  if (lr_mask)
+    return launch_upsample_eval<false, true, true>(disp_q, disp, nullptr, th, T, 0.f, nullptr, lr_mask, lr_thresh, lr_stats, B, h,
+                                                   w, H, W, scale, s, u);
+  return launch_upsample_eval<false, false, true>(disp_q, disp, nullptr, th, T, 0.f, nullptr, nullptr, 0.f, nullptr, B, h, w, H, W,
+                                                  scale, s, u);
+}
+
+// s3d_tap_gather_soft_argmin (std_q == NULL) and s3d_tap_gather_soft_argmin_std
+static int tap_gather_soft_argmin(const float* taps, float* disp, float* std_q, float* cost_out, int N, int D, int h, int w,
+                                  int tap_stride, float sign, void* stream) {
   if (!taps || !disp) { set_error("tap_gather_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(N > 0 && D > 0 && h > 0 && w > 0 && tap_stride >= 27 && h < 65536 && N < 65536,
                 "tap_gather_soft_argmin: bad shape");
   const int threads = w <= 32 ? 32 : (w <= 64 ? 64 : 128);
   dim3 grid(ceil_div(w, threads), h, N);
-  tap_gather_soft_argmin_kernel<<<grid, threads, 0, static_cast<cudaStream_t>(stream)>>>(taps, disp, cost_out, N, D, h, w,
-                                                                                      tap_stride, sign);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (std_q)
+    tap_gather_soft_argmin_kernel<true><<<grid, threads, 0, st>>>(taps, disp, cost_out, N, D, h, w, tap_stride, sign, std_q);
+  else
+    tap_gather_soft_argmin_kernel<false><<<grid, threads, 0, st>>>(taps, disp, cost_out, N, D, h, w, tap_stride, sign, nullptr);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
+}
+
+extern "C" int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* cost_out, int N, int D, int h, int w,
+                                          int tap_stride, float sign, void* stream) {
+  return tap_gather_soft_argmin(taps, disp, nullptr, cost_out, N, D, h, w, tap_stride, sign, stream);
+}
+
+extern "C" int s3d_tap_gather_soft_argmin_std(const float* taps, float* disp, float* disp_std_q, float* cost_out, int N, int D,
+                                              int h, int w, int tap_stride, float sign, void* stream) {
+  if (!disp_std_q) { set_error("tap_gather_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
+  return tap_gather_soft_argmin(taps, disp, disp_std_q, cost_out, N, D, h, w, tap_stride, sign, stream);
 }

@@ -72,6 +72,12 @@ SIGNATURES = {
     's3d_upsample_disp': ([_vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
     's3d_upsample_disp_eval': ([_vp, _vp, _vp, ctypes.POINTER(_f), _i, _f, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
     's3d_upsample_disp_lr': ([_vp, _vp, _vp, _f, _vp, ctypes.POINTER(_f), _i, _f, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
+    's3d_tap_gather_soft_argmin_std': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
+    's3d_cls_soft_argmin_std': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
+    's3d_conv_cls_soft_argmin_std': ([ctypes.POINTER(S3dConvParams), _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp], _i),
+    's3d_corr_soft_argmin_std': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),
+    's3d_upsample_disp_std': ([_vp, _vp, _vp, _vp, ctypes.POINTER(_f), _i, _vp, _vp, ctypes.POINTER(_f), _i, _f, _vp, _vp, _f, _vp,
+                               _i, _i, _i, _i, _i, _f, _vp], _i),
     's3d_latent_to_vox': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_avg_pool': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_depth_to_space': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),

@@ -135,7 +135,7 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False):
+    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
         self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
@@ -144,8 +144,10 @@ class _GraphedForward:
         kw = {} if disp_gt is None else {'disp_gt': self.disp_gt}
         if lr_check:
             kw['lr_check'] = True
+        if uncertainty:
+            kw['uncertainty'] = True
 
-        def run():                                    # zeroes its IoU / disparity / LR counters itself: inside the graph
+        def run():                                    # zeroes its IoU / disparity / LR / uncertainty counters itself: inside the graph
             return model._forward_impl(*args, **kw)
         side = torch.cuda.Stream(device=left.device)
         side.wait_stream(torch.cuda.current_stream())
@@ -276,9 +278,10 @@ class _StereoBase(nn.Module):
     def _bhw(img):
         return (img.shape[0], img.shape[1], img.shape[2]) if img.dtype == torch.uint8 else (img.shape[0], img.shape[2], img.shape[3])
 
-    def _disparity(self, left, right, disp_gt=None, lr_check=False):
+    def _disparity(self, left, right, disp_gt=None, lr_check=False, uncertainty=False):
         """-> disp fp32 [2B,H,W] (left-referenced first), in input pixels, disp_q, the disparity stats int64 [B,2,2+T]
-        against disp_gt (None without it) and the LR check's (lr_mask, lr_stats) (None without lr_check; see _upsample_disp)."""
+        against disp_gt (None without it), the LR check's (lr_mask, lr_stats) (None without lr_check) and with uncertainty
+        (disp_std, unc_stats) (else None; see _upsample_disp)."""
         cfg = self.cfg
         B, H, W = self._bhw(left)
         D = cfg.NETWORK.MAX_DISP
@@ -320,6 +323,9 @@ class _StereoBase(nn.Module):
         else:
             feat = self._conv('enc5', x, out=self._bufo('e5', 'enc5', x))
         disp_q = self._buf('disp_q', (2 * B, h, w), torch.float32)
+        # the standard deviation of each pixel's soft-argmin distribution, from the same kernel as disp_q
+        std_q = self._buf('disp_std_q', (2 * B, h, w), torch.float32) if uncertainty else None
+        std_kw = {} if std_q is None else {'std_out': std_q}           # the plain calls keep their plain signature
         if cfg.NETWORK.COST_VOLUME == 'concat':
             if fuse_volume:
                 # bf16: reference-once form -- the d-independent reference half is convolved once per column, the planes run
@@ -359,32 +365,36 @@ class _StereoBase(nn.Module):
                 # cls_a + classifier + soft-argmin in one march, cls_a's 2.1 GB output never written (csrc/conv_scatter_cls.cu)
                 nb = ops.conv_cls_workspace_bytes(2 * B, D, h, w)
                 ops.conv_cls_soft_argmin(pa, a, self._packed['cls_b'].weight, -1.0, out=disp_q,
-                                         workspace=self._buf('cls_ws', (nb,), torch.uint8))
-                disp, stats, lr = self._upsample_disp(disp_q, H, W, disp_gt, lr_check)
-                return disp, disp_q, stats, lr
+                                         workspace=self._buf('cls_ws', (nb,), torch.uint8), **std_kw)
+                disp, stats, lr, unc = self._upsample_disp(disp_q, H, W, disp_gt, lr_check, std_q)
+                return disp, disp_q, stats, lr, unc
             c = self._conv('cls_a', a, out=self._bufo('a0', 'cls_a', a))
             if self.precision == 'bf16' and c.shape[-1] in (16, 32, 64) and S == 32 and not _lib.KNOBS['no_cls_fused']:
                 # classifier + soft-argmin in one pass over the volume (csrc/cls_fused.cu)
-                ops.cls_soft_argmin(c, self._packed['cls_b'].weight, -1.0, out=disp_q)
+                ops.cls_soft_argmin(c, self._packed['cls_b'].weight, -1.0, out=disp_q, **std_kw)
             else:
                 taps = self._buf('taps', (2 * B, D, h, S, w), torch.float32)   # line-planar: [.., y, tap, x]
                 self._conv('cls_b', c, out=taps, out_view=(0, (D * h * S * w, h * S * w, S * w, 1, w)), cout_store=S)
-                ops.tap_gather_soft_argmin(taps, -1.0, out=disp_q)
+                ops.tap_gather_soft_argmin(taps, -1.0, out=disp_q, **std_kw)
         else:
             if self._split:                                               # exact fp32 correlation on hi + lo
                 feat = ops.unsplit_bf16(feat, out=self._buf('feat32', feat.shape[:-1] + (feat.shape[-1] // 2,), torch.float32))
-            ops.corr_soft_argmin(feat, B, D, out=disp_q, c_real=C)       # mean over the REAL channels (feat is padded)
-        disp, stats, lr = self._upsample_disp(disp_q, H, W, disp_gt, lr_check)
-        return disp, disp_q, stats, lr
+            ops.corr_soft_argmin(feat, B, D, out=disp_q, c_real=C, **std_kw)        # mean over the REAL channels (feat is padded)
+        disp, stats, lr, unc = self._upsample_disp(disp_q, H, W, disp_gt, lr_check, std_q)
+        return disp, disp_q, stats, lr, unc
 
-    def _upsample_disp(self, disp_q, H, W, disp_gt, lr_check=False):
+    def _upsample_disp(self, disp_q, H, W, disp_gt, lr_check=False, std_q=None):
         """Last kernel of the disparity stage: 1/4-res disparity -> input pixels [2B,H,W].  With disp_gt [B,2,H,W] the same
         kernel also counts, per sample and view, [n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) for t in
         TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> stats int64 [B,2,2+T] (else None).  With lr_check it
         also runs the left-right consistency check (include/s3d.h, s3d_upsample_disp_lr; tolerance TEST.LR_THRESH px) ->
         lr = (lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T]: [n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and
-        count(|disp - gt| > t) over the kept valid pixels]; GT columns zero without disp_gt) (else None).
-        -> (disp, stats, lr)."""
+        count(|disp - gt| > t) over the kept valid pixels]; GT columns zero without disp_gt) (else None).  With std_q (the
+        1/4-res standard deviation) the same kernel also upsamples it and counts the confident pixels (include/s3d.h,
+        s3d_upsample_disp_std; thresholds TEST.UNC_THRESH px) -> unc = (disp_std fp32 [B,2,H,W], unc_stats int64
+        [B,2,K,3+T]: per threshold [n_conf, n_valid_conf, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the
+        confident valid pixels]; GT columns zero without disp_gt) (else None).
+        -> (disp, stats, lr, unc)."""
         B = disp_q.shape[0] // 2
         out = self._buf('disp', (2 * B, H, W), torch.float32)
         th = list(self.cfg.TEST.DISP_THRESH)
@@ -393,6 +403,7 @@ class _StereoBase(nn.Module):
             stats = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64)
             stats.zero_()
         max_gt = 4.0 * self.cfg.NETWORK.MAX_DISP
+        lr = None
         if lr_check:
             tau = float(self.cfg.TEST.LR_THRESH)
             if not (math.isfinite(tau) and tau >= 0):
@@ -400,13 +411,24 @@ class _StereoBase(nn.Module):
             mask = self._buf('lr_mask', (B, 2, H, W), torch.uint8)
             lr_stats = self._buf('lr_stats', (B, 2, 3 + len(th)), torch.int64)
             lr_stats.zero_()
-            ops.upsample_disp_lr(disp_q, H, W, 4.0, tau, mask, lr_stats, gt=disp_gt, thresholds=th, max_gt=max_gt, stats=stats,
+            lr = (mask, lr_stats)
+        if std_q is not None:
+            ut = unc_thresholds(self.cfg)
+            unc_stats = self._buf('unc_stats', (B, 2, len(ut), 3 + len(th)), torch.int64)
+            unc_stats.zero_()
+            _, disp_std = ops.upsample_disp_std(disp_q, std_q, H, W, 4.0, ut, unc_stats, gt=disp_gt, thresholds=th, max_gt=max_gt,
+                                                stats=stats, lr_thresh=tau if lr_check else 0.0, mask=None if lr is None else lr[0],
+                                                lr_stats=None if lr is None else lr[1], out=out,
+                                                std_out=self._buf('disp_std', (B, 2, H, W), torch.float32))
+            return out, stats, lr, (disp_std, unc_stats)
+        if lr_check:
+            ops.upsample_disp_lr(disp_q, H, W, 4.0, tau, lr[0], lr[1], gt=disp_gt, thresholds=th, max_gt=max_gt, stats=stats,
                                  out=out)
-            return out, stats, (mask, lr_stats)
+            return out, stats, lr, None
         if disp_gt is None:
-            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None, None
+            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None, None, None
         ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, max_gt, stats, out=out)
-        return out, stats, None
+        return out, stats, None, None
 
     def _bufo(self, name, layer, x):
         """Output buffer of `layer` for input x (channels-last, padded channels)."""
@@ -447,13 +469,15 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
         ~0.12 ms per aggregation layer), so the graph only removes the launch gaps.
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
+        if uncertainty:
+            unc_thresholds(self.cfg)
         left, right = self._check_inputs(left, right)
         gt = self._check_gt(gt, left)
         disp_gt = self._check_disp_gt(disp_gt, left)
@@ -461,10 +485,10 @@ class _StereoBase(nn.Module):
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
         key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
-               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check))
+               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check), bool(uncertainty))
         g = self._graphs.get(key)
         if g is None:
-            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check))
+            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check), bool(uncertainty))
             self._graphs[key] = g
         return g(left, right, gt, disp_gt)
 
@@ -504,11 +528,13 @@ class _StereoBase(nn.Module):
 
 
 class Stereo2Voxel(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W], voxels [B,32,32,32]
-    [, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T']]).
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W],
+    voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64
+    [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']]).
     Outputs are views of the module's workspace: clone to keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views
-    (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; disp_stats, lr_mask, lr_stats:
-    _StereoBase._upsample_disp."""
+    (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; uncertainty=True: the standard
+    deviation of each pixel's soft-argmin distribution in input pixels, and counters over the pixels it marks as confident
+    (K = len(TEST.UNC_THRESH)); disp_stats, lr_mask, lr_stats, disp_std, unc_stats: _StereoBase._upsample_disp."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -547,7 +573,9 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False):
+        if uncertainty:
+            unc_thresholds(self.cfg)                   # a bad TEST.UNC_THRESH fails before anything is launched
         left, right = self._check_inputs(left, right)
         disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
@@ -556,19 +584,19 @@ class Stereo2Voxel(_StereoBase):
             outs = []
             for s in range(0, B, mb):
                 o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
-                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check)
+                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check, uncertainty)
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check)
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty)
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False):
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check)
+    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False):
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty)
 
-    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False):
+    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False):
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
-        disp, _, dstats, lr = self._disparity(left, right, disp_gt, lr_check)
+        disp, _, dstats, lr, unc = self._disparity(left, right, disp_gt, lr_check, uncertainty)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         k0 = cfg.NETWORK.DEC_CHANNELS[0]
@@ -612,7 +640,20 @@ class Stereo2Voxel(_StereoBase):
             out += (iou,)
         if disp_gt is not None:
             out += (dstats,)
-        return out + lr if lr_check else out
+        return out + (lr or ()) + (unc or ())
+
+
+def unc_thresholds(cfg):
+    """TEST.UNC_THRESH as floats: at most 4 (the kernel's limit) standard deviations in input pixels, each finite and >= 0 (a
+    pixel with disp_std <= t counts as confident at t); anything else is a ValueError."""
+    th = cfg.TEST.get('UNC_THRESH')
+    try:
+        th = [float(t) for t in th]
+    except (TypeError, ValueError):
+        raise ValueError('TEST.UNC_THRESH must be a list of numbers, got %r' % (th,)) from None
+    if len(th) > 4 or not all(math.isfinite(t) and t >= 0 for t in th):
+        raise ValueError('TEST.UNC_THRESH must hold at most 4 finite values >= 0, got %r' % (cfg.TEST.UNC_THRESH,))
+    return th
 
 
 def fscore_thresholds(cfg):
@@ -629,9 +670,9 @@ def fscore_thresholds(cfg):
 
 
 class Stereo2Point(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=]) -> (disp_left, disp_right, points [B,N_POINTS,3]
-    [, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats]) (disp_gt, lr_check and their
-    outputs as for Stereo2Voxel).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left, disp_right, points [B,N_POINTS,3]
+    [, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats][, disp_std, unc_stats]) (disp_gt,
+    lr_check, uncertainty and their outputs as for Stereo2Voxel).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
     `points` against it and counts, per sample and direction (0: predicted -> GT, 1: GT -> predicted), [sum of squared
     distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
     (include/s3d.h, s3d_chamfer_eval)."""
@@ -663,15 +704,17 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False):
+        if uncertainty:
+            unc_thresholds(self.cfg)
         left, right = self._check_inputs(left, right)
         return self._forward_impl(left, right, self._check_gt(gt, left), disp_gt=self._check_disp_gt(disp_gt, left),
-                                  lr_check=lr_check)
+                                  lr_check=lr_check, uncertainty=uncertainty)
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False):
+    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False):
         cfg = self.cfg
         B = left.shape[0]
-        disp, _, dstats, lr = self._disparity(left, right, disp_gt, lr_check)
+        disp, _, dstats, lr, unc = self._disparity(left, right, disp_gt, lr_check, uncertainty)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         if x.shape[2] != L or x.shape[3] != L:
@@ -696,7 +739,7 @@ class Stereo2Point(_StereoBase):
             out += (self._point_stats(points, gt),)
         if disp_gt is not None:
             out += (dstats,)
-        return out + lr if lr_check else out
+        return out + (lr or ()) + (unc or ())
 
     def _point_stats(self, points, gt):
         """Chamfer search of points [B,N,3] against gt [B,M,3] + the metric counters -> point_stats int64 [B,2,3+T], zeroed
