@@ -316,6 +316,24 @@ int s3d_unsplit_bf16(const void* x, float* out, int64_t npix, int C, void* strea
 int s3d_fuse_views(const void* score, int64_t score_stride, const void* vol, int64_t vol_stride,
                    int dtype, float* fused, int B, int V, int nvox, const uint8_t* gt,
                    const float* thresholds, int T, long long* iou, int64_t score_lo, int64_t vol_lo, void* stream);
+/* Voxel-surface metrics of predicted occupancy against GT occupancy: exact voxel-face Chamfer and F-score counters.
+ * fused fp32 [B,n,n,n], gt uint8 [B,n,n,n]; 1 <= n <= 64.  Occupied: fused >= thresholds[t] in fp32 (NaN is empty, as for
+ * the IoU of s3d_fuse_views), gt != 0; outside the grid is empty.  Surface = the centres of the faces between an occupied and
+ * an empty voxel, in doubled integer coordinates (voxel centre 2i+1, a face at an even coordinate 0..2n on its axis), so each
+ * is a site of the (2n+1)^3 lattice.  s = squared distance in doubled units to the nearest point of the other surface, an
+ * integer <= 3 (2n)^2: exact, no ties problem.  stats int64 [B,T,2,3+F] is ADDED to (caller zeroes); per sample, t and
+ * direction (0: predicted -> GT, 1: GT -> predicted)
+ *   [ n_pts, sum s, sum q(sqrt_rn(s)), count(s < kbound[f]) for f < F ]
+ * q(x) = round-half-even(x * 2^32) (exact product), sqrt_rn = the correctly rounded fp32 square root of (float)s.  When the
+ * other surface is empty only n_pts is counted.  kbound: F <= 8 HOST ints in [0, 3 (2n)^2 + 1]; an F-score threshold tau in
+ * unit-cube units (the grid spans a unit cube) is kbound = min(ceil((2n tau)^2), 3 (2n)^2 + 1).  thresholds: T <= 8 HOST
+ * values.  workspace: >= s3d_voxel_surface_workspace_bytes(B, T, n) bytes, 8-byte aligned (one uint16 distance grid per
+ * sample and surface).  Two kernels: the in-plane passes of the distance transform, then the third pass at the query sites
+ * fused with the counters (one atomic per counter per block, no block spanning two slices: the sums do not depend on the
+ * launch order or the batch split). */
+int64_t s3d_voxel_surface_workspace_bytes(int B, int T, int n);
+int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
+                           const int* kbound, int F, long long* stats, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* --- Chamfer distance (row C; replaces extensions/chamfer_dist, README.md:62-65) ------- */
 /* xyz1 fp32 [B,N,3], xyz2 fp32 [B,M,3] -> dist1 fp32 [B,N], idx1 int32 [B,N] (nearest in

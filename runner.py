@@ -30,6 +30,9 @@ def get_args():
                    help='also run the left-right disparity consistency check and report it as lr_consistency')
     p.add_argument('--uncertainty', action='store_true',
                    help='also compute the per-pixel disparity uncertainty and report the confidence-filtered metrics as uncertainty')
+    p.add_argument('--surface', action='store_true',
+                   help='Stereo2Voxel: also evaluate the voxel-face surfaces against GT and report Chamfer L2 / L1 and '
+                        'F-score as surface')
     return p.parse_args()
 
 
@@ -78,6 +81,8 @@ def main():
     from config import cfg
     if not args.test:
         sys.exit('Only `runner.py --test` is implemented: this is the inference-tier build (training is out of scope).')
+    if args.surface and args.model != 'Stereo2Voxel':
+        sys.exit('--surface evaluates voxel surfaces: Stereo2Voxel only')
     if not torch.cuda.is_available():
         sys.exit('runner.py --test needs a CUDA device (sm_100a); there is no CPU fallback.')
     from stereo_3d_reconstruction_b200 import models
@@ -99,7 +104,7 @@ def main():
     # one stats vector: the head's statistics, then the disparity counters of the same forwards
     if args.model == 'Stereo2Voxel':
         stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check,
-                             eval_unc=args.uncertainty).cpu()
+                             eval_unc=args.uncertainty, eval_surface=args.surface).cpu()
         nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
         res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
     else:
@@ -119,6 +124,9 @@ def main():
     if args.uncertainty:
         res['uncertainty'] = T.unc_summary(stats[nh + nd + nl:nh + nd + nl + nu], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH,
                                            res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
+    if args.surface:
+        res['surface'] = T.surface_summary(stats[nh + nd + nl + nu:], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH,
+                                           res['n_samples'])
     if args.model == 'Stereo2Point':
         res['points'] = T.points_summary(stats[nh + nd + nl + nu:], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
                                          cfg.CONST.N_GT_POINTS)

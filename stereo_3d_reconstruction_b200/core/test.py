@@ -20,6 +20,11 @@ TEST.FSCORE_THRESH:
     sum q(d), sum q(sqrt d), n_out, count(sqrt d < t) per t                                    (int64)
     sum_b q(F_b(t)),  F_b = 2 P R / (P + R) (0 when both are 0), P = count_pred / N, R = count_gt / M   (int64)
 with q(x) = round-half-even(x * 2^32); F_b is computed elementwise in fp64 on the device, so the vector stays integer.
+With eval_surface=True (test_voxel) the voxel-surface counters of the same forwards come last (models.py,
+Stereo2Voxel._surface_stats), per t in TEST.VOXEL_THRESH (surface_block):
+    n_both, sum_b q(CD_L2_b), sum_b q(CD_L1_b), then per tau in TEST.FSCORE_THRESH sum_b q(P_b), sum_b q(R_b), sum_b q(F_b)
+                                                                                               (int64)
+again computed per batch in fp64 on the device.
 """
 import torch
 import torch.distributed as dist
@@ -154,6 +159,59 @@ def points_summary(block, thresholds, n_samples, N, M):
             'recall': [c / (M * n) if n else 0.0 for c in gt[3:]], 'fscore': [x / _PT_FX / n if n else 0.0 for x in f]}
 
 
+def surface_block(surf_stats, n):
+    """Per-batch increment of the surface block from the forward's surf_stats int64 [B,T,2,3+F] (n = N_VOX) -> int64
+    [T * (3 + 3F)]: per t [n_both, sum_b q(CD_L2_b), sum_b q(CD_L1_b), then per tau sum_b q(P_b), sum_b q(R_b), sum_b q(F_b)],
+    q(x) = round-half-even(x * 2^32), in fp64.  Direction 0 = predicted -> GT (n_0 points), 1 = GT -> predicted (n_1):
+    CD_L2_b = (sum s_0 / n_0 + sum s_1 / n_1) / (2n)^2 and CD_L1_b = (sum q_0 / n_0 + sum q_1 / n_1) / 2 / 2^32 / (2n), both
+    over the n_both samples where both surfaces are non-empty (0 elsewhere); P_b = count_0 / n_0, R_b = count_1 / n_1 (0 when
+    the denominator is 0), F_b = 2 P R / (P + R) (0 when P + R = 0)."""
+    c = surf_stats.double()
+    n0, n1 = c[:, :, 0, 0], c[:, :, 1, 0]
+    both = (n0 > 0) & (n1 > 0)
+    z = torch.zeros_like(n0)
+    l2 = torch.where(both, (c[:, :, 0, 1] / n0 + c[:, :, 1, 1] / n1) / (2 * n) ** 2, z)
+    l1 = torch.where(both, (c[:, :, 0, 2] / n0 + c[:, :, 1, 2] / n1) / 2 / _PT_FX / (2 * n), z)
+    p = torch.where(n0[..., None] > 0, c[:, :, 0, 3:] / n0[..., None], torch.zeros_like(c[:, :, 0, 3:]))
+    r = torch.where(n1[..., None] > 0, c[:, :, 1, 3:] / n1[..., None], torch.zeros_like(c[:, :, 1, 3:]))
+    f = torch.where(p + r > 0, 2 * p * r / (p + r), torch.zeros_like(p))
+
+    def q(x):
+        return torch.round(x * _PT_FX).to(torch.int64).sum(0)
+    T = c.shape[1]
+    prf = torch.stack([q(p), q(r), q(f)], -1).reshape(T, -1)
+    return torch.cat([both.sum(0, dtype=torch.int64)[:, None], q(l2)[:, None], q(l1)[:, None], prf], 1).flatten()
+
+
+def surface_summary(block, voxel_thresh, fscore_thresh, n_samples):
+    """Surface counters (int64 [T * (3 + 3F)], as surface_block sums them) -> dict with one entry per t in voxel_thresh:
+    n_both, chamfer_l2 / chamfer_l1 (means over the n_both samples whose two surfaces are non-empty, in unit-cube units;
+    inf when n_both = 0) and per tau the precision, recall and F-score as means over all n_samples."""
+    T, F = len(voxel_thresh), len(fscore_thresh)
+    v = [int(x) for x in block.tolist()]
+    assert len(v) == T * (3 + 3 * F)
+    n = n_samples
+    per = []
+    for t in range(T):
+        r = v[t * (3 + 3 * F):(t + 1) * (3 + 3 * F)]
+        nb = r[0]
+        per.append({'voxel_thresh': float(voxel_thresh[t]), 'n_both': nb,
+                    'chamfer_l2': r[1] / _PT_FX / nb if nb else float('inf'),
+                    'chamfer_l1': r[2] / _PT_FX / nb if nb else float('inf'),
+                    'precision': [r[3 + 3 * f] / _PT_FX / n if n else 0.0 for f in range(F)],
+                    'recall': [r[4 + 3 * f] / _PT_FX / n if n else 0.0 for f in range(F)],
+                    'fscore': [r[5 + 3 * f] / _PT_FX / n if n else 0.0 for f in range(F)]})
+    return {'n_samples': n, 'thresholds': [float(t) for t in voxel_thresh], 'fscore_thresh': list(fscore_thresh),
+            'by_thresh': per}
+
+
+def _surface_len(cfg, eval_surface):
+    if not eval_surface:
+        return 0
+    F = len(fscore_thresholds(cfg))                     # ValueError on a bad TEST.FSCORE_THRESH, before any forward
+    return len(cfg.TEST.VOXEL_THRESH) * (3 + 3 * F)
+
+
 def _point_len(cfg, eval_points):
     if not eval_points:
         return 0
@@ -179,18 +237,21 @@ def _unc_len(cfg, eval_disp, eval_unc):
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_unc=False):
+               eval_unc=False, eval_surface=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
     eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
-    eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones."""
+    eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones.
+    eval_surface: the same forward also evaluates the voxel surfaces; their block comes last."""
     th = list(cfg.TEST.VOXEL_THRESH)
     T = len(th)
     nl = _lr_len(cfg, eval_disp, eval_lr)
     nu = _unc_len(cfg, eval_disp, eval_unc)
     nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    stats = torch.zeros(2 * T + 1 + nd + nl + nu, dtype=torch.int64, device=device)
+    ns = _surface_len(cfg, eval_surface)
+    stats = torch.zeros(2 * T + 1 + nd + nl + nu + ns, dtype=torch.int64, device=device)
+    sk = {'surface': True} if eval_surface else {}
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -201,21 +262,26 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.gt_volume(1, cfg.CONST.N_VOX, seed=100000 + i) for i in ids]).to(device)
             if eval_unc:
-                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=eval_lr, uncertainty=True)
+                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=eval_lr, uncertainty=True, **sk)
                 iou, ds = out[3], out[4]
                 stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
                 if eval_lr:
                     stats[2 * T + 1 + nd:2 * T + 1 + nd + nl] += out[6].sum(0).flatten()
-                stats[2 * T + 1 + nd + nl:] += out[-1].sum(0).flatten()
+                stats[2 * T + 1 + nd + nl:2 * T + 1 + nd + nl + nu] += out[-1 - bool(sk)].sum(0).flatten()   # before surf_stats
             elif eval_lr:
-                _, _, _, iou, ds, _, ls = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
+                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True, **sk)
+                iou, ds, ls = out[3], out[4], out[6]
                 stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
-                stats[2 * T + 1 + nd:] += ls.sum(0).flatten()
+                stats[2 * T + 1 + nd:2 * T + 1 + nd + nl] += ls.sum(0).flatten()
             elif eval_disp:
-                _, _, _, iou, ds = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device))
-                stats[2 * T + 1:] += ds.sum(0).flatten()
+                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), **sk)
+                iou, ds = out[3], out[4]
+                stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
             else:
-                _, _, _, iou = model(left, right, gt)
+                out = model(left, right, gt, **sk)
+                iou = out[3]
+            if eval_surface:
+                stats[2 * T + 1 + nd + nl + nu:] += surface_block(out[-1], cfg.CONST.N_VOX)
             stats[:T] += iou[:, :, 0].sum(0)
             stats[T:2 * T] += iou[:, :, 1].sum(0)
             stats[2 * T] += len(ids)

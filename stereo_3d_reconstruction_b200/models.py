@@ -135,7 +135,7 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False):
+    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
         self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
@@ -146,8 +146,10 @@ class _GraphedForward:
             kw['lr_check'] = True
         if uncertainty:
             kw['uncertainty'] = True
+        if surface:
+            kw['surface'] = True
 
-        def run():                                    # zeroes its IoU / disparity / LR / uncertainty counters itself: inside the graph
+        def run():                                    # zeroes its IoU / disparity / LR / uncertainty / surface counters itself: inside the graph
             return model._forward_impl(*args, **kw)
         side = torch.cuda.Stream(device=left.device)
         side.wait_stream(torch.cuda.current_stream())
@@ -469,7 +471,7 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -478,6 +480,7 @@ class _StereoBase(nn.Module):
         are overwritten by the next call with the same signature."""
         if uncertainty:
             unc_thresholds(self.cfg)
+        self._check_surface(surface, gt)
         left, right = self._check_inputs(left, right)
         gt = self._check_gt(gt, left)
         disp_gt = self._check_disp_gt(disp_gt, left)
@@ -485,10 +488,11 @@ class _StereoBase(nn.Module):
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
         key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
-               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check), bool(uncertainty))
+               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check), bool(uncertainty),
+               bool(surface))
         g = self._graphs.get(key)
         if g is None:
-            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check), bool(uncertainty))
+            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check), bool(uncertainty), bool(surface))
             self._graphs[key] = g
         return g(left, right, gt, disp_gt)
 
@@ -510,6 +514,11 @@ class _StereoBase(nn.Module):
         """The head's GT as the head takes it (Stereo2Point validates its point cloud)."""
         return gt
 
+    def _check_surface(self, surface, gt):
+        """surface=True (the voxel-surface metrics) is a Stereo2Voxel option."""
+        if surface:
+            raise ValueError('surface=True evaluates voxel surfaces: Stereo2Voxel only')
+
     def _check_disp_gt(self, disp_gt, left):
         """GT disparity of (checked) inputs `left`: fp32 [B,2,H,W] on their device, in input pixels, view 0 = left-referenced
         (as disp_left), 1 = right-referenced; NaN marks pixels without GT."""
@@ -530,11 +539,15 @@ class _StereoBase(nn.Module):
 class Stereo2Voxel(_StereoBase):
     """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W],
     voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64
-    [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']]).
+    [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, surf_stats int64 [B,T,2,3+F]]).
     Outputs are views of the module's workspace: clone to keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views
     (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; uncertainty=True: the standard
     deviation of each pixel's soft-argmin distribution in input pixels, and counters over the pixels it marks as confident
-    (K = len(TEST.UNC_THRESH)); disp_stats, lr_mask, lr_stats, disp_std, unc_stats: _StereoBase._upsample_disp."""
+    (K = len(TEST.UNC_THRESH)); disp_stats, lr_mask, lr_stats, disp_std, unc_stats: _StereoBase._upsample_disp.
+    surface=True (needs gt): the voxel-face surfaces of the prediction at each t in TEST.VOXEL_THRESH and of gt, evaluated
+    against each other; surf_stats per sample, t and direction (0: predicted -> GT, 1: GT -> predicted) = [n_pts, sum s,
+    sum q(sqrt s), count(s < k) per tau in TEST.FSCORE_THRESH] with s the exact squared distance to the other surface in
+    doubled lattice units (include/s3d.h, s3d_voxel_surface_eval; two more launches)."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -573,9 +586,17 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False):
+    def _check_surface(self, surface, gt):
+        """surface=True needs the GT occupancy and a valid TEST.FSCORE_THRESH: checked before anything is launched."""
+        if surface:
+            if gt is None:
+                raise ValueError('surface=True needs the GT occupancy gt')
+            fscore_thresholds(self.cfg)
+
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
         if uncertainty:
             unc_thresholds(self.cfg)                   # a bad TEST.UNC_THRESH fails before anything is launched
+        self._check_surface(surface, gt)
         left, right = self._check_inputs(left, right)
         disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
@@ -584,15 +605,15 @@ class Stereo2Voxel(_StereoBase):
             outs = []
             for s in range(0, B, mb):
                 o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
-                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check, uncertainty)
+                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check, uncertainty, surface)
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty)
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface)
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False):
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty)
+    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface)
 
-    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False):
+    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
@@ -640,7 +661,20 @@ class Stereo2Voxel(_StereoBase):
             out += (iou,)
         if disp_gt is not None:
             out += (dstats,)
-        return out + (lr or ()) + (unc or ())
+        out += (lr or ()) + (unc or ())
+        if surface:
+            out += (self._surface_stats(fused, gt8),)
+        return out
+
+    def _surface_stats(self, fused, gt8):
+        """Voxel-surface counters of fused [B,n^3] against gt8 [B,n^3] -> surf_stats int64 [B,T,2,3+F], zeroed here (so a
+        graph replay starts from zero).  Every buffer comes from the workspace: no allocation on this path."""
+        th, fth = list(self.cfg.TEST.VOXEL_THRESH), fscore_thresholds(self.cfg)
+        B, nv = fused.shape[0], self.cfg.CONST.N_VOX
+        stats = self._buf('surf_stats', (B, len(th), 2, 3 + len(fth)), torch.int64)
+        stats.zero_()
+        nb = ops.voxel_surface_workspace_bytes(B, len(th), nv)
+        return ops.voxel_surface_eval(fused, gt8, th, fth, stats, workspace=self._buf('surf_ws', (max(nb, 1),), torch.uint8))
 
 
 def unc_thresholds(cfg):

@@ -3,6 +3,7 @@
 device / dtype / contiguity, allocates outputs with torch, passes raw pointers and the current
 CUDA stream, and raises on a non-zero return code.  None of them computes anything in Python."""
 import ctypes
+import math
 
 import torch
 
@@ -585,3 +586,54 @@ def chamfer_eval(xyz1, xyz2, tau, stats, workspace=None, out=None):
     _lib.check(rc, 's3d_chamfer_eval')
     _lib.count_launch(3)                       # the two search kernels + chamfer_eval_kernel
     return dist1, dist2, idx1, idx2
+
+
+def voxel_kbound(tau, n):
+    """F-score threshold tau (Euclidean distance in unit-cube units; the n^3 grid spans the unit cube) -> the integer bound
+    k of s3d_voxel_surface_eval, in float64: a surface point counts when its squared distance s in doubled lattice units is
+    < k, i.e. exactly when sqrt(s) / (2n) < tau."""
+    return min(math.ceil((2 * n * float(tau)) ** 2), 3 * (2 * n) ** 2 + 1)
+
+
+def voxel_surface_workspace_bytes(B, T, n):
+    return int(_lib.load().s3d_voxel_surface_workspace_bytes(B, T, n))
+
+
+def voxel_surface_eval(fused, gt8, voxel_thresh, fscore_thresh, stats, workspace=None):
+    """Voxel-face surface metrics (include/s3d.h, s3d_voxel_surface_eval).  fused fp32 [B,n,n,n] or [B,n^3], gt8 uint8 of the
+    same shape (nonzero = occupied), 1 <= n <= 64.  stats int64 [B,T,2,3+F] (T = len(voxel_thresh), F = len(fscore_thresh))
+    += per sample, threshold and direction (0: predicted -> GT, 1: GT -> predicted) [n_pts, sum s, sum q(sqrt s),
+    count(s < voxel_kbound(tau)) per tau], s the squared distance in doubled lattice units.  workspace: optional uint8
+    buffer of at least voxel_surface_workspace_bytes(B, T, n) bytes.  Two kernel launches."""
+    _chk(fused, gt8, stats, workspace)
+    if fused.dtype != torch.float32 or gt8.dtype != torch.uint8:
+        raise ValueError('voxel_surface_eval: fused must be float32 and gt8 uint8, got %s / %s' % (fused.dtype, gt8.dtype))
+    if fused.shape != gt8.shape or fused.dim() not in (2, 4):
+        raise ValueError('voxel_surface_eval: expected fused and gt8 of one shape [B,n,n,n] or [B,n^3], got %s / %s'
+                         % (tuple(fused.shape), tuple(gt8.shape)))
+    B = fused.shape[0]
+    nvox = fused[0].numel()
+    n = round(nvox ** (1.0 / 3.0))
+    if n ** 3 != nvox or (fused.dim() == 4 and tuple(fused.shape[1:]) != (n, n, n)) or not 1 <= n <= 64:
+        raise ValueError('voxel_surface_eval: a sample must be an n^3 grid with 1 <= n <= 64, got %s' % (tuple(fused.shape),))
+    T, F = len(voxel_thresh), len(fscore_thresh)
+    if T > 8 or F > 8:
+        raise ValueError('voxel_surface_eval: at most 8 voxel and 8 F-score thresholds, got %d / %d' % (T, F))
+    if stats.dtype != torch.int64 or tuple(stats.shape) != (B, T, 2, 3 + F):
+        raise ValueError('voxel_surface_eval: stats must be int64 [%d, %d, 2, %d]' % (B, T, 3 + F))
+    for t in (gt8, stats, workspace):
+        if t is not None and t.device != fused.device:
+            raise ValueError('voxel_surface_eval: every tensor must be on %s' % fused.device)
+    need = voxel_surface_workspace_bytes(B, T, n)
+    if workspace is None:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=fused.device)
+    elif workspace.numel() * workspace.element_size() < need:
+        raise ValueError('voxel_surface_eval: workspace of %d bytes, need %d' % (workspace.numel() * workspace.element_size(), need))
+    th = (ctypes.c_float * max(T, 1))(*[float(t) for t in voxel_thresh])
+    kb = (ctypes.c_int * max(F, 1))(*[voxel_kbound(t, n) for t in fscore_thresh])
+    rc = _lib.load().s3d_voxel_surface_eval(fused.data_ptr(), gt8.data_ptr(), B, n, th, T, kb, F, stats.data_ptr(),
+                                            workspace.data_ptr(), need, _stream())
+    _lib.check(rc, 's3d_voxel_surface_eval')
+    if B and T:
+        _lib.count_launch(2)                   # surface_plane_kernel + surface_count_kernel
+    return stats
