@@ -202,16 +202,26 @@ int s3d_cost_volume_concat(const void* feat, void* vol, int B, int h, int w, int
 /* cost: fp32 [N,D,h,w] -> disp fp32 [N,h,w] = sum_d d*softmax_d(sign*cost).  sign=-1: soft-argmin. */
 int s3d_soft_argmin(const float* cost, float* disp, int N, int D, int h, int w, float sign,
                     void* stream);
+
+/* --- disparity uncertainty ------------------------------------------------------------------------------------------------
+ * The four soft-argmin calls below (tap_gather, cls, conv_cls, corr) take disp_std_q fp32 [N,h,w] right after disp; NULL means
+ * "do not compute it".  When it is set they write the same disp bit for bit, and into disp_std_q the standard deviation of
+ * each pixel's soft-argmin distribution, in planes: with p_d = softmax_d(sign * cost_d) the weights whose mean is disp_q,
+ *   sigma_q = sqrt(sum_d p_d (d - disp_q)^2)     (fp32, >= 0; NaN where disp_q is not finite).
+ * The corr kernels include the cost-0 planes outside the image, as for the mean.  Accuracy: |sigma_q - sigma_ref| <= 1e-4 *
+ * (1 + sigma_ref) against sigma_ref computed in fp64 from the same costs, also for sharp peaks at large d (the online kernels
+ * accumulate the moments about the running arg-max plane, the corr kernels take a second pass about the mean). */
+
 /* Cout=1 3x3x3 classifier conv + soft-argmin from per-tap planes.  taps: fp32, line-planar [N,D,h,tap_stride,w] with
  * taps[n,z,y,(kz*3+ky)*3+kx,x] = W[kz,ky,kx,:] . in[n,z,y,x,:] (a pointwise GEMM done by s3d_conv_igemm with osC=w);
  * cost[z,y,x] = sum_t taps[z+kz-1, y+ky-1, x+kx-1, t] (zero outside), disp = sum_z z*softmax_z(sign*cost).
  * cost_out may be NULL (debug: fp32 [N,D,h,w]). */
-int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* cost_out, int N, int D, int h, int w,
+int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* disp_std_q, float* cost_out, int N, int D, int h, int w,
                                int tap_stride, float sign, void* stream);
 /* The same classifier + soft-argmin in ONE pass over the aggregated volume, no per-tap tensor (csrc/cls_fused.cu):
  * x: bf16 channels-last [N,D,h,w,C], C in {16,32,64}; w_taps: bf16 [32][C], row t = (kz*3+ky)*3+kx holds W[kz,ky,kx,:]
  * (rows 27..31 zero) -- the weight tensor of the pointwise layer above; disp: fp32 [N,h,w]. */
-int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, int N, int D, int h, int w, int C,
+int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, float* disp_std_q, int N, int D, int h, int w, int C,
                         float sign, void* stream);
 /* Last aggregation layer + classifier + soft-argmin WITHOUT the layer's output volume (csrc/conv_scatter_cls.cu): `p` is the
  * bf16 stride-1 3x3x3 64 -> 64 ReLU layer (w_nstack set) over in [N,D,h,w,64]; its output Y is projected on the 27 classifier
@@ -221,70 +231,51 @@ int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, int N, i
  * the stored tensor would be) up to the fp32 summation order of the 27 taps.  Needs N * ceil(h/32) * ceil(w/8) >= 2. */
 int64_t s3d_conv_cls_workspace_bytes(int N, int D, int h, int w);
 int s3d_conv_cls_soft_argmin(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps, void* workspace,
-                             float* disp, float sign, void* stream);
+                             float* disp, float* disp_std_q, float sign, void* stream);
 /* Fused correlation + soft-argmax; the [2B,D,h,w] cost is never materialised.
  * feat: [2B,1,h,w,C] with C the PADDED channel count (row pitch); cost = (1/c_real) * sum_c ref*tgt over the real
  * channels (padded channels must be zero; c_real = 0 means C).
  * disp: fp32 [2B,h,w]; cost_out may be NULL (debug: fp32 [2B,D,h,w]). */
-int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_out, int B, int h, int w,
+int s3d_corr_soft_argmin(const void* feat, float* disp, float* disp_std_q, float* cost_out, int B, int h, int w,
                          int C, int c_real, int D, int dtype, void* stream);
 /* disp_q fp32 [N,h,w] (1/4-res units) -> fp32 [N,H,W] = bilinear(scale*disp_q), align_corners=False. */
 int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h, int w, int H, int W,
                       float scale, void* stream);
-/* s3d_upsample_disp + evaluation against GT disparity.  disp_q fp32 [2B,h,w] (left-referenced first), disp fp32 [2B,H,W]
- * (written bit-identically to s3d_upsample_disp), gt fp32 [B,2,H,W] (view 0 = left-referenced, 1 = right-referenced),
- * thresholds: T <= 8 fp32 HOST values, stats int64 [B,2,2+T], ACCUMULATED (the caller zeroes it):
+/* s3d_upsample_disp + per-pixel evaluation, in one launch.  disp_q fp32 [2B,h,w] (left-referenced first), disp fp32 [2B,H,W]
+ * (written bit-identically to s3d_upsample_disp).  Three optional groups, each on when its lead pointer is set: gt comes with
+ * disp_stats, lr_mask with lr_stats, disp_std_q with disp_std (both or neither).  A call with no group on is rejected: the
+ * plain upsampling is s3d_upsample_disp.  Every stats tensor is ACCUMULATED (the caller zeroes it).  thresholds: T <= 8 fp32
+ * HOST values; T sets the row length of every stats tensor, also when gt == NULL (then lr_stats and unc_stats get column 0
+ * only).
+ *
+ * GT (gt, disp_stats): gt fp32 [B,2,H,W] (view 0 = left-referenced, 1 = right-referenced), disp_stats int64 [B,2,2+T]:
  *   [n_valid, sum_valid q(|disp - gt|), count_valid(|disp - gt| > thresholds[t]) for t < T]
  * valid: gt finite and 0 <= gt < max_gt.  q(e) = round-half-even(e * 65536) of the fp32 error (fixed point, 2^-16 px).
  * Range: q < 2^26 per pixel while disparities are below 1024 px, so one image's sum stays below 2^50 for H*W <= 2^24 and
  * int64 holds the sums of more than 2^12 such images.  Integer counters, one atomic per counter per block and no block
- * spans two images: the stats do not depend on the launch order, batch split or number of GPUs. */
-int s3d_upsample_disp_eval(const float* disp_q, float* disp, const float* gt, const float* thresholds, int T,
-                           float max_gt, long long* stats, int B, int h, int w, int H, int W, float scale, void* stream);
-/* s3d_upsample_disp (+ s3d_upsample_disp_eval when gt is set) + the left-right consistency check of the two views, in one
- * launch.  disp is bit-identical to s3d_upsample_disp, disp_stats to what s3d_upsample_disp_eval adds.  With D0 / D1 the
+ * spans two images: the stats do not depend on the launch order, batch split or number of GPUs.
+ *
+ * LR check (lr_mask, lr_stats): the left-right consistency check of the two views.  With D0 / D1 the
  * left- / right-referenced maps of a sample and d = Dv[y,x] finite, k = round-half-even(d), xo = x - k (view 0) or x + k
  * (view 1): the pixel is KEPT iff 0 <= xo < W and |d - D(1-v)[y,xo]| <= lr_thresh (fp32 subtraction, one rounding; a NaN
  * on the other side is not kept).  A non-finite d is not kept; |d| >= W + 1 is out of range.  lr_mask uint8 [B,2,H,W]
- * (1 = kept).  lr_stats int64 [B,2,3+T], ACCUMULATED:
+ * (1 = kept).  lr_stats int64 [B,2,3+T]:
  *   [n_kept, n_valid_kept, sum_{valid & kept} q(|disp - gt|), count_{valid & kept}(|disp - gt| > thresholds[t]) for t < T]
- * (valid and q as for s3d_upsample_disp_eval).  gt == NULL needs disp_stats == NULL and adds column 0 only; T still sets the
- * row length.  lr_thresh must be >= 0. */
-int s3d_upsample_disp_lr(const float* disp_q, float* disp, uint8_t* lr_mask, float lr_thresh, const float* gt,
-                         const float* thresholds, int T, float max_gt, long long* disp_stats, long long* lr_stats,
-                         int B, int h, int w, int H, int W, float scale, void* stream);
-
-/* --- disparity uncertainty ------------------------------------------------------------------------------------------------
- * The *_std entry points below take the arguments of their siblings plus disp_std_q fp32 [N,h,w] (non-NULL).  They write the
- * same disp bit for bit, and into disp_std_q the standard deviation of each pixel's soft-argmin distribution, in planes:
- * with p_d = softmax_d(sign * cost_d) the weights whose mean is disp_q,
- *   sigma_q = sqrt(sum_d p_d (d - disp_q)^2)     (fp32, >= 0; NaN where disp_q is not finite).
- * The corr kernels include the cost-0 planes outside the image, as for the mean.  Accuracy: |sigma_q - sigma_ref| <= 1e-4 *
- * (1 + sigma_ref) against sigma_ref computed in fp64 from the same costs, also for sharp peaks at large d (the online kernels
- * accumulate the moments about the running arg-max plane, the corr kernels take a second pass about the mean). */
-int s3d_tap_gather_soft_argmin_std(const float* taps, float* disp, float* disp_std_q, float* cost_out, int N, int D, int h, int w,
-                                   int tap_stride, float sign, void* stream);
-int s3d_cls_soft_argmin_std(const void* x, const void* w_taps, float* disp, float* disp_std_q, int N, int D, int h, int w, int C,
-                            float sign, void* stream);
-int s3d_conv_cls_soft_argmin_std(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps, void* workspace,
-                                 float* disp, float* disp_std_q, float sign, void* stream);
-int s3d_corr_soft_argmin_std(const void* feat, float* disp, float* disp_std_q, float* cost_out, int B, int h, int w,
-                             int C, int c_real, int D, int dtype, void* stream);
-/* s3d_upsample_disp (+ s3d_upsample_disp_eval when gt is set, + s3d_upsample_disp_lr when lr_mask is set) + the upsampled
- * standard deviation and confidence-filtered counters, in one launch.  disp, disp_stats, lr_mask and lr_stats are what the
- * siblings write / add, bit for bit.  disp_std_q fp32 [2B,h,w] (from a *_std entry point) -> disp_std fp32 [B,2,H,W] (view 0
- * = left-referenced) = bilinear(scale * disp_std_q), bit-identical to s3d_upsample_disp(disp_std_q, scale) of the image.
- * unc_thresh: K <= 4 HOST values in input pixels, finite and >= 0.  unc_stats int64 [B,2,K,3+T], ACCUMULATED: per view and
- * threshold k, over the CONFIDENT pixels (disp_std <= unc_thresh[k] in fp32; a non-finite disp_std never is)
+ * lr_thresh must be >= 0.
+ *
+ * Uncertainty (disp_std_q, disp_std; unc_thresh, K, unc_stats): disp_std_q fp32 [2B,h,w] (from a soft-argmin call) ->
+ * disp_std fp32 [B,2,H,W] (view 0 = left-referenced) = bilinear(scale * disp_std_q), bit-identical to
+ * s3d_upsample_disp(disp_std_q, scale) of the image where both take the same (16-byte or scalar) path: W % 4 == 0 and 16-byte
+ * aligned outputs, or neither.  unc_thresh: K <= 4 HOST values in input pixels, finite and >= 0 (K > 0 needs disp_std_q).
+ * unc_stats int64 [B,2,K,3+T]: per view and threshold k, over the CONFIDENT pixels (disp_std <= unc_thresh[k] in fp32; a
+ * non-finite disp_std never is)
  *   [n_conf, n_valid_conf, sum_{valid & conf} q(|disp - gt|), count_{valid & conf}(|disp - gt| > thresholds[t]) for t < T]
- * (valid and q as for s3d_upsample_disp_eval; the range argument there holds for these sums, which run over fewer pixels).
- * gt == NULL needs disp_stats == NULL and adds column 0 only; T still sets the row length.  lr_mask and lr_stats come together
- * (NULL: no LR check), lr_thresh as for s3d_upsample_disp_lr.  disp_std is bit-identical to s3d_upsample_disp where both take the
- * same (16-byte or scalar) path: W % 4 == 0 and 16-byte aligned outputs, or neither. */
-int s3d_upsample_disp_std(const float* disp_q, float* disp, const float* disp_std_q, float* disp_std, const float* unc_thresh,
-                          int K, long long* unc_stats, const float* gt, const float* thresholds, int T, float max_gt,
-                          long long* disp_stats, uint8_t* lr_mask, float lr_thresh, long long* lr_stats, int B, int h, int w,
-                          int H, int W, float scale, void* stream);
+ * (the range argument above holds for these sums, which run over fewer pixels). */
+int s3d_upsample_disp_eval(const float* disp_q, float* disp, int B, int h, int w, int H, int W, float scale,
+                           const float* gt, const float* thresholds, int T, float max_gt, long long* disp_stats,
+                           uint8_t* lr_mask, float lr_thresh, long long* lr_stats,
+                           const float* disp_std_q, float* disp_std, const float* unc_thresh, int K, long long* unc_stats,
+                           void* stream);
 
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)

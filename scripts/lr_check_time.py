@@ -1,9 +1,10 @@
 #!/usr/bin/env python3
-"""Cost of the left-right consistency check (s3d_upsample_disp_lr, forward(..., lr_check=True)), in one run, CUDA events,
-the arms alternating:
+"""Cost of the left-right consistency check (s3d_upsample_disp_eval with lr_mask, forward(..., lr_check=True)), in one run,
+CUDA events, the arms alternating:
 
-  1. the upsample kernel alone in its four forms -- plain (s3d_upsample_disp), eval (s3d_upsample_disp_eval), lr and
-     lr + eval (s3d_upsample_disp_lr without / with GT) -- at B = 64, 256 x 256, D = 32 (1/4-res input 64 x 64).  Four
+  1. the upsample kernel alone in its four forms -- plain (s3d_upsample_disp), eval (s3d_upsample_disp_eval with GT), lr and
+     lr + eval (s3d_upsample_disp_eval with lr_mask, without / with GT) -- at B = 64, 256 x 256, D = 32 (1/4-res input
+     64 x 64).  Four
      buffer sets are rotated (more than the 126 MB L2), so every launch writes its 33.5 MB of disparity (+ 8.4 MB of mask)
      to HBM and the GT arms read their 33.5 MB of GT from there;
   2. the default Stereo2Voxel forward replayed from its CUDA graph, model.graphed(left, right, gt) against the same call
@@ -63,10 +64,10 @@ def main():
     arms = {
         'plain': lambda k: ops.upsample_disp(S(k)['q'], H, W, 4.0, out=S(k)['out']),
         'eval': lambda k: ops.upsample_disp_eval(S(k)['q'], H, W, 4.0, S(k)['gt'], th, max_gt, S(k)['st'], out=S(k)['out']),
-        'lr': lambda k: ops.upsample_disp_lr(S(k)['q'], H, W, 4.0, tau, S(k)['mask'], S(k)['ls'], thresholds=th,
-                                             out=S(k)['out']),
-        'lr_eval': lambda k: ops.upsample_disp_lr(S(k)['q'], H, W, 4.0, tau, S(k)['mask'], S(k)['ls'], gt=S(k)['gt'],
-                                                  thresholds=th, max_gt=max_gt, stats=S(k)['st'], out=S(k)['out']),
+        'lr': lambda k: ops.upsample_disp_eval(S(k)['q'], H, W, 4.0, thresholds=th, lr_thresh=tau, mask=S(k)['mask'],
+                                               lr_stats=S(k)['ls'], out=S(k)['out']),
+        'lr_eval': lambda k: ops.upsample_disp_eval(S(k)['q'], H, W, 4.0, S(k)['gt'], th, max_gt, S(k)['st'], lr_thresh=tau,
+                                                    mask=S(k)['mask'], lr_stats=S(k)['ls'], out=S(k)['out']),
     }
     time_alternating(arms, 8, 3)                                    # warm-up
     k = time_alternating(arms, 200, args.reps)

@@ -1,12 +1,12 @@
 #!/usr/bin/env python3
-"""Cost of the disparity uncertainty (the *_std entry points, forward(..., uncertainty=True)), in one run, CUDA events, the
+"""Cost of the disparity uncertainty (disp_std_q set, forward(..., uncertainty=True)), in one run, CUDA events, the
 arms alternating, at B = 64, 256 x 256, D = 32 (1/4-res 64 x 64, 2B = 128 images):
 
   1. each soft-argmin kernel without and with the standard deviation: the bf16 chain (s3d_conv_cls_soft_argmin: cls_a +
      classifier + partials_soft_argmin_kernel), cls_fused_kernel, tap_gather_soft_argmin_kernel, corr_tc_kernel and the SIMT
      corr_soft_argmin_kernel (fp32 features).  Their inputs are 2.1 GB volumes, or four rotated feature sets of more than the
      126 MB L2 for the corr kernels;
-  2. the upsample kernel plain (s3d_upsample_disp), with the standard deviation (s3d_upsample_disp_std) and with it plus GT
+  2. the upsample kernel plain (s3d_upsample_disp), with the standard deviation (s3d_upsample_disp_eval) and with it plus GT
      evaluation and the LR check, four rotated buffer sets;
   3. the default Stereo2Voxel forward replayed from its CUDA graph, with and without uncertainty=True.
 
@@ -113,12 +113,12 @@ def main():
         return sets[k % 4]
     arms = {
         'plain': lambda k: ops.upsample_disp(S(k)['q'], H, W, 4.0, out=S(k)['out']),
-        'std': lambda k: ops.upsample_disp_std(S(k)['q'], S(k)['s'], H, W, 4.0, ut, S(k)['us0'], out=S(k)['out'],
-                                               std_out=S(k)['sd']),
-        'std_eval_lr': lambda k: ops.upsample_disp_std(S(k)['q'], S(k)['s'], H, W, 4.0, ut, S(k)['us'], gt=S(k)['gt'], thresholds=th,
-                                                       max_gt=4.0 * D, stats=S(k)['st'], lr_thresh=cfg.TEST.LR_THRESH,
-                                                       mask=S(k)['mask'], lr_stats=S(k)['ls'], out=S(k)['out'],
-                                                       std_out=S(k)['sd']),
+        'std': lambda k: ops.upsample_disp_eval(S(k)['q'], H, W, 4.0, std_q=S(k)['s'], unc_thresh=ut, unc_stats=S(k)['us0'],
+                                                std_out=S(k)['sd'], out=S(k)['out']),
+        'std_eval_lr': lambda k: ops.upsample_disp_eval(S(k)['q'], H, W, 4.0, S(k)['gt'], th, 4.0 * D, S(k)['st'],
+                                                        lr_thresh=cfg.TEST.LR_THRESH, mask=S(k)['mask'], lr_stats=S(k)['ls'],
+                                                        std_q=S(k)['s'], unc_thresh=ut, unc_stats=S(k)['us'],
+                                                        std_out=S(k)['sd'], out=S(k)['out']),
     }
     time_alternating(arms, 8, 3)
     t = time_alternating(arms, 200, args.reps)

@@ -236,9 +236,8 @@ cls_fused_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
 }  // namespace
 }  // namespace s3d
 
-// s3d_cls_soft_argmin (std_q == NULL) and s3d_cls_soft_argmin_std
-static int cls_soft_argmin(const void* x, const void* w_taps, float* disp, float* std_q, int N, int D, int h, int w, int C,
-                           float sign, void* stream) {
+extern "C" int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, float* std_q, int N, int D, int h, int w,
+                                   int C, float sign, void* stream) {
   using namespace s3d;
   if (!x || !w_taps || !disp) { set_error("cls_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(N > 0 && D > 0 && h > 0 && w > 0, "cls_soft_argmin: bad shape");
@@ -279,15 +278,4 @@ static int cls_soft_argmin(const void* x, const void* w_taps, float* disp, float
   kern<<<grid, kThreads, smem_bytes, static_cast<cudaStream_t>(stream)>>>(map_x, map_w, a);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
-}
-
-extern "C" int s3d_cls_soft_argmin(const void* x, const void* w_taps, float* disp, int N, int D, int h, int w, int C,
-                                   float sign, void* stream) {
-  return cls_soft_argmin(x, w_taps, disp, nullptr, N, D, h, w, C, sign, stream);
-}
-
-extern "C" int s3d_cls_soft_argmin_std(const void* x, const void* w_taps, float* disp, float* disp_std_q, int N, int D, int h,
-                                       int w, int C, float sign, void* stream) {
-  if (!disp_std_q) { s3d::set_error("cls_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
-  return cls_soft_argmin(x, w_taps, disp, disp_std_q, N, D, h, w, C, sign, stream);
 }

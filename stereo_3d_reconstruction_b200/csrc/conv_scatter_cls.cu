@@ -388,9 +388,8 @@ extern "C" int64_t s3d_conv_cls_workspace_bytes(int N, int D, int h, int w) {
   return (int64_t)N * ((h + kTY - 1) / kTY) * ((w + kTX - 1) / kTX) * D * kCells * 4;
 }
 
-// s3d_conv_cls_soft_argmin (std_q == NULL) and s3d_conv_cls_soft_argmin_std
-static int conv_cls_soft_argmin(const S3dConvParams* p_in, const void* in, const float* bias, const void* w_taps, void* workspace,
-                                float* disp, float* std_q, float sign, void* stream) {
+extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p_in, const void* in, const float* bias, const void* w_taps,
+                                        void* workspace, float* disp, float* std_q, float sign, void* stream) {
   using namespace s3d;
   using namespace s3d::scatter;
   if (!p_in || !in || !bias || !w_taps || !workspace || !disp) { set_error("conv_cls_soft_argmin: null argument"); return S3D_ERR_INVALID; }
@@ -446,15 +445,4 @@ static int conv_cls_soft_argmin(const S3dConvParams* p_in, const void* in, const
                                                                nullptr);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
-}
-
-extern "C" int s3d_conv_cls_soft_argmin(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps,
-                                        void* workspace, float* disp, float sign, void* stream) {
-  return conv_cls_soft_argmin(p, in, bias, w_taps, workspace, disp, nullptr, sign, stream);
-}
-
-extern "C" int s3d_conv_cls_soft_argmin_std(const S3dConvParams* p, const void* in, const float* bias, const void* w_taps,
-                                            void* workspace, float* disp, float* disp_std_q, float sign, void* stream) {
-  if (!disp_std_q) { s3d::set_error("conv_cls_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
-  return conv_cls_soft_argmin(p, in, bias, w_taps, workspace, disp, disp_std_q, sign, stream);
 }

@@ -480,7 +480,7 @@ struct UncCounters {
 // [B,2,2+nT], lr_stats [B,2,3+nT], unc_stats [B,2,nU,3+nT]
 __device__ __forceinline__ int64_t eval_image_index(int n, int B) { return (int64_t)(n % B) * 2 + n / B; }
 
-// Left-right consistency of the pixel at column X whose stored disparity is d (include/s3d.h, s3d_upsample_disp_lr).  `ro`:
+// Left-right consistency of the pixel at column X whose stored disparity is d (include/s3d.h, s3d_upsample_disp_eval).  `ro`:
 // the OTHER view's source rows of the same output row, so up_px gives the value the other image's blocks store at xo.
 // dir = -1 for view 0 (xo = X - k), +1 for view 1 (xo = X + k).
 __device__ __forceinline__ bool lr_kept(float d, int X, const UpRow& ro, int w, int W, float rx, float scale, int dir,
@@ -599,39 +599,48 @@ upsample_disp_eval_kernel(const float* __restrict__ q, float* __restrict__ out, 
   if (kStd) uc.flush<kEval>(unc_stats + eval_image_index(n, B) * nU * (3 + nT), nU, nT);
 }
 
-// The standard-deviation arguments of launch_upsample_eval (kStd)
-struct UncArgs {
-  const float* std_q = nullptr;
+// The arguments of one s3d_upsample_disp_eval call, checked there.  The pointers of a group that is off are NULL.
+struct UpsampleEvalArgs {
+  const float* disp_q = nullptr;
+  float* disp = nullptr;
+  int B = 0, h = 0, w = 0, H = 0, W = 0;
+  float scale = 0.f;
+  const float* gt = nullptr;                     // kEval
+  Thresh th = {};
+  int T = 0;
+  float max_gt = 0.f;
+  long long* disp_stats = nullptr;
+  uint8_t* lr_mask = nullptr;                    // kLR
+  float lr_thresh = 0.f;
+  long long* lr_stats = nullptr;
+  const float* std_q = nullptr;                  // kStd
   float* std_out = nullptr;
   Thresh ut = {};
-  int nU = 0;
-  long long* stats = nullptr;
+  int K = 0;
+  long long* unc_stats = nullptr;
 };
 
-// Shared launcher of s3d_upsample_disp_eval (kEval), s3d_upsample_disp_lr (kLR, kEval when it has GT) and
-// s3d_upsample_disp_std (kStd, with kEval / kLR when it has GT / a mask); arguments checked.
-template <bool kEval, bool kLR, bool kStd = false>
-int launch_upsample_eval(const float* disp_q, float* disp, const float* gt, const Thresh& th, int T, float max_gt,
-                         long long* stats, uint8_t* lr_mask, float lr_thresh, long long* lr_stats, int B, int h, int w, int H,
-                         int W, float scale, cudaStream_t s, const UncArgs& u = UncArgs()) {
-  const int64_t img = (int64_t)H * W;
-  auto* st = reinterpret_cast<unsigned long long*>(stats);
-  auto* lst = reinterpret_cast<unsigned long long*>(lr_stats);
-  auto* ust = reinterpret_cast<unsigned long long*>(u.stats);
-  if (W % 4 == 0 && ((reinterpret_cast<uintptr_t>(disp) | reinterpret_cast<uintptr_t>(gt) | reinterpret_cast<uintptr_t>(u.std_out)) &
-                     15) == 0 &&
-      (reinterpret_cast<uintptr_t>(lr_mask) & 3) == 0) {
+template <bool kEval, bool kLR, bool kStd>
+int launch_upsample_eval(const UpsampleEvalArgs& a, cudaStream_t s) {
+  const int64_t img = (int64_t)a.H * a.W;
+  auto* st = reinterpret_cast<unsigned long long*>(a.disp_stats);
+  auto* lst = reinterpret_cast<unsigned long long*>(a.lr_stats);
+  auto* ust = reinterpret_cast<unsigned long long*>(a.unc_stats);
+  if (a.W % 4 == 0 &&
+      ((reinterpret_cast<uintptr_t>(a.disp) | reinterpret_cast<uintptr_t>(a.gt) | reinterpret_cast<uintptr_t>(a.std_out)) & 15) == 0 &&
+      (reinterpret_cast<uintptr_t>(a.lr_mask) & 3) == 0) {
     // 16 outputs per thread: 4x fewer blocks (and counter atomics) than one vector per thread
-    const dim3 grid((unsigned)ceil_div64(img / 4, 256 * 4), 2 * B);
+    const dim3 grid((unsigned)ceil_div64(img / 4, 256 * 4), 2 * a.B);
     upsample_disp_eval_v4_kernel<kEval, kLR, kStd><<<grid, 256, 0, s>>>(
-        disp_q, reinterpret_cast<float4*>(disp), reinterpret_cast<const float4*>(gt), B, h, w, H, W / 4, (float)h / (float)H,
-        (float)w / (float)W, scale, th, T, max_gt, st, reinterpret_cast<uint32_t*>(lr_mask), lr_thresh, lst, u.std_q,
-        reinterpret_cast<float4*>(u.std_out), u.ut, u.nU, ust);
+        a.disp_q, reinterpret_cast<float4*>(a.disp), reinterpret_cast<const float4*>(a.gt), a.B, a.h, a.w, a.H, a.W / 4,
+        (float)a.h / (float)a.H, (float)a.w / (float)a.W, a.scale, a.th, a.T, a.max_gt, st, reinterpret_cast<uint32_t*>(a.lr_mask),
+        a.lr_thresh, lst, a.std_q, reinterpret_cast<float4*>(a.std_out), a.ut, a.K, ust);
     S3D_LAUNCH_CHECK();
     return S3D_OK;
   }
-  upsample_disp_eval_kernel<kEval, kLR, kStd><<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * B), 256, 0, s>>>(
-      disp_q, disp, gt, B, h, w, H, W, scale, th, T, max_gt, st, lr_mask, lr_thresh, lst, u.std_q, u.std_out, u.ut, u.nU, ust);
+  upsample_disp_eval_kernel<kEval, kLR, kStd><<<dim3((unsigned)ceil_div64(img, 256 * 4), 2 * a.B), 256, 0, s>>>(
+      a.disp_q, a.disp, a.gt, a.B, a.h, a.w, a.H, a.W, a.scale, a.th, a.T, a.max_gt, st, a.lr_mask, a.lr_thresh, lst, a.std_q,
+      a.std_out, a.ut, a.K, ust);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
 }
@@ -687,9 +696,8 @@ extern "C" int s3d_soft_argmin(const float* cost, float* disp, int N, int D, int
   return S3D_OK;
 }
 
-// s3d_corr_soft_argmin (std_q == NULL) and s3d_corr_soft_argmin_std
-static int corr_soft_argmin(const void* feat, float* disp, float* std_q, float* cost_out, int B, int h, int w, int C, int c_real,
-                            int D, int dtype, void* stream) {
+extern "C" int s3d_corr_soft_argmin(const void* feat, float* disp, float* std_q, float* cost_out, int B, int h, int w, int C,
+                                    int c_real, int D, int dtype, void* stream) {
   if (!feat || !disp) { set_error("corr_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(dtype == S3D_DTYPE_F32 || dtype == S3D_DTYPE_BF16, "corr_soft_argmin: bad dtype");
   S3D_CHECK_ARG(B > 0 && h > 0 && w > 0 && C > 0 && D > 0, "corr_soft_argmin: bad shape");
@@ -723,17 +731,6 @@ static int corr_soft_argmin(const void* feat, float* disp, float* std_q, float* 
   return std_q ? launch(corr_soft_argmin_kernel<float, true>, f) : launch(corr_soft_argmin_kernel<float, false>, f);
 }
 
-extern "C" int s3d_corr_soft_argmin(const void* feat, float* disp, float* cost_out, int B, int h, int w, int C, int c_real,
-                                    int D, int dtype, void* stream) {
-  return corr_soft_argmin(feat, disp, nullptr, cost_out, B, h, w, C, c_real, D, dtype, stream);
-}
-
-extern "C" int s3d_corr_soft_argmin_std(const void* feat, float* disp, float* disp_std_q, float* cost_out, int B, int h, int w,
-                                        int C, int c_real, int D, int dtype, void* stream) {
-  if (!disp_std_q) { set_error("corr_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
-  return corr_soft_argmin(feat, disp, disp_std_q, cost_out, B, h, w, C, c_real, D, dtype, stream);
-}
-
 extern "C" int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h, int w, int H, int W, float scale,
                                  void* stream) {
   if (!disp_q || !disp) { set_error("upsample_disp: null argument"); return S3D_ERR_INVALID; }
@@ -753,87 +750,50 @@ extern "C" int s3d_upsample_disp(const float* disp_q, float* disp, int N, int h,
   return S3D_OK;
 }
 
-extern "C" int s3d_upsample_disp_eval(const float* disp_q, float* disp, const float* gt, const float* thresholds, int T,
-                                      float max_gt, long long* stats, int B, int h, int w, int H, int W, float scale,
-                                      void* stream) {
-  if (!disp_q || !disp || !gt || !stats || (T > 0 && !thresholds)) {
+extern "C" int s3d_upsample_disp_eval(const float* disp_q, float* disp, int B, int h, int w, int H, int W, float scale,
+                                      const float* gt, const float* thresholds, int T, float max_gt, long long* disp_stats,
+                                      uint8_t* lr_mask, float lr_thresh, long long* lr_stats, const float* disp_std_q,
+                                      float* disp_std, const float* unc_thresh, int K, long long* unc_stats, void* stream) {
+  if (!disp_q || !disp || (gt && T > 0 && !thresholds) || (K > 0 && (!unc_thresh || !unc_stats))) {
     set_error("upsample_disp_eval: null argument");
     return S3D_ERR_INVALID;
   }
+  S3D_CHECK_ARG(gt || lr_mask || disp_std_q,
+                "upsample_disp_eval: gt, lr_mask and disp_std_q are all NULL (the plain upsampling is s3d_upsample_disp)");
+  S3D_CHECK_ARG(!gt == !disp_stats, "upsample_disp_eval: gt and disp_stats must be both set or both NULL");
+  S3D_CHECK_ARG(!lr_mask == !lr_stats, "upsample_disp_eval: lr_mask and lr_stats must be both set or both NULL");
+  S3D_CHECK_ARG(!disp_std_q == !disp_std, "upsample_disp_eval: disp_std_q and disp_std must be both set or both NULL");
   S3D_CHECK_ARG(B > 0 && 2 * B < 65536 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31),
                 "upsample_disp_eval: bad shape");
   S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "upsample_disp_eval: T must be in [0, 8]");
-  S3D_CHECK_ARG(max_gt > 0.f, "upsample_disp_eval: max_gt must be > 0");
-  Thresh th;
-  for (int t = 0; t < kMaxThresh; ++t) th.t[t] = t < T ? thresholds[t] : 0.f;
-  return launch_upsample_eval<true, false>(disp_q, disp, gt, th, T, max_gt, stats, nullptr, 0.f, nullptr, B, h, w, H, W, scale,
-                                           static_cast<cudaStream_t>(stream));
-}
-
-extern "C" int s3d_upsample_disp_lr(const float* disp_q, float* disp, uint8_t* lr_mask, float lr_thresh, const float* gt,
-                                    const float* thresholds, int T, float max_gt, long long* disp_stats, long long* lr_stats,
-                                    int B, int h, int w, int H, int W, float scale, void* stream) {
-  if (!disp_q || !disp || !lr_mask || !lr_stats || (gt && T > 0 && !thresholds)) {
-    set_error("upsample_disp_lr: null argument");
-    return S3D_ERR_INVALID;
-  }
-  S3D_CHECK_ARG(!gt == !disp_stats, "upsample_disp_lr: gt and disp_stats must be both set or both NULL");
-  S3D_CHECK_ARG(B > 0 && 2 * B < 65536 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31),
-                "upsample_disp_lr: bad shape");
-  S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "upsample_disp_lr: T must be in [0, 8]");
-  S3D_CHECK_ARG(lr_thresh >= 0.f, "upsample_disp_lr: lr_thresh must be >= 0 (and not NaN)");
-  S3D_CHECK_ARG(!gt || max_gt > 0.f, "upsample_disp_lr: max_gt must be > 0");
-  Thresh th;
-  for (int t = 0; t < kMaxThresh; ++t) th.t[t] = gt && t < T ? thresholds[t] : 0.f;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (gt)
-    return launch_upsample_eval<true, true>(disp_q, disp, gt, th, T, max_gt, disp_stats, lr_mask, lr_thresh, lr_stats, B, h, w,
-                                            H, W, scale, s);
-  return launch_upsample_eval<false, true>(disp_q, disp, nullptr, th, T, 0.f, nullptr, lr_mask, lr_thresh, lr_stats, B, h, w, H,
-                                           W, scale, s);
-}
-
-extern "C" int s3d_upsample_disp_std(const float* disp_q, float* disp, const float* disp_std_q, float* disp_std,
-                                     const float* unc_thresh, int K, long long* unc_stats, const float* gt, const float* thresholds,
-                                     int T, float max_gt, long long* disp_stats, uint8_t* lr_mask, float lr_thresh,
-                                     long long* lr_stats, int B, int h, int w, int H, int W, float scale, void* stream) {
-  if (!disp_q || !disp || !disp_std_q || !disp_std || (K > 0 && (!unc_thresh || !unc_stats)) || (gt && T > 0 && !thresholds)) {
-    set_error("upsample_disp_std: null argument");
-    return S3D_ERR_INVALID;
-  }
-  S3D_CHECK_ARG(!gt == !disp_stats, "upsample_disp_std: gt and disp_stats must be both set or both NULL");
-  S3D_CHECK_ARG(!lr_mask == !lr_stats, "upsample_disp_std: lr_mask and lr_stats must be both set or both NULL");
-  S3D_CHECK_ARG(B > 0 && 2 * B < 65536 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31),
-                "upsample_disp_std: bad shape");
-  S3D_CHECK_ARG(K >= 0 && K <= kMaxUnc, "upsample_disp_std: K must be in [0, 4]");
-  S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "upsample_disp_std: T must be in [0, 8]");
-  S3D_CHECK_ARG(!lr_mask || lr_thresh >= 0.f, "upsample_disp_std: lr_thresh must be >= 0 (and not NaN)");
-  S3D_CHECK_ARG(!gt || max_gt > 0.f, "upsample_disp_std: max_gt must be > 0");
-  UncArgs u;
-  u.std_q = disp_std_q;  u.std_out = disp_std;  u.nU = K;  u.stats = unc_stats;
+  S3D_CHECK_ARG(K >= 0 && K <= kMaxUnc, "upsample_disp_eval: K must be in [0, 4]");
+  S3D_CHECK_ARG(disp_std_q || K == 0, "upsample_disp_eval: unc_thresh needs disp_std_q");
+  S3D_CHECK_ARG(!lr_mask || lr_thresh >= 0.f, "upsample_disp_eval: lr_thresh must be >= 0 (and not NaN)");
+  S3D_CHECK_ARG(!gt || max_gt > 0.f, "upsample_disp_eval: max_gt must be > 0");
+  UpsampleEvalArgs a;
+  a.disp_q = disp_q;  a.disp = disp;  a.B = B;  a.h = h;  a.w = w;  a.H = H;  a.W = W;  a.scale = scale;
+  a.gt = gt;  a.T = T;  a.max_gt = max_gt;  a.disp_stats = disp_stats;
+  for (int t = 0; t < kMaxThresh; ++t) a.th.t[t] = gt && t < T ? thresholds[t] : 0.f;
+  a.lr_mask = lr_mask;  a.lr_thresh = lr_thresh;  a.lr_stats = lr_stats;
+  a.std_q = disp_std_q;  a.std_out = disp_std;  a.K = K;  a.unc_stats = unc_stats;
   for (int k = 0; k < K; ++k) {
-    S3D_CHECK_ARG(unc_thresh[k] >= 0.f && unc_thresh[k] < INFINITY, "upsample_disp_std: unc_thresh must be finite and >= 0");
-    u.ut.t[k] = unc_thresh[k];
+    S3D_CHECK_ARG(unc_thresh[k] >= 0.f && unc_thresh[k] < INFINITY, "upsample_disp_eval: unc_thresh must be finite and >= 0");
+    a.ut.t[k] = unc_thresh[k];
   }
-  Thresh th;
-  for (int t = 0; t < kMaxThresh; ++t) th.t[t] = gt && t < T ? thresholds[t] : 0.f;
+  // one instantiation per combination of groups that are on
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (gt && lr_mask)
-    return launch_upsample_eval<true, true, true>(disp_q, disp, gt, th, T, max_gt, disp_stats, lr_mask, lr_thresh, lr_stats, B, h,
-                                                  w, H, W, scale, s, u);
-  if (gt)
-    return launch_upsample_eval<true, false, true>(disp_q, disp, gt, th, T, max_gt, disp_stats, nullptr, 0.f, nullptr, B, h, w, H,
-                                                   W, scale, s, u);
-  if (lr_mask)
-    return launch_upsample_eval<false, true, true>(disp_q, disp, nullptr, th, T, 0.f, nullptr, lr_mask, lr_thresh, lr_stats, B, h,
-                                                   w, H, W, scale, s, u);
-  return launch_upsample_eval<false, false, true>(disp_q, disp, nullptr, th, T, 0.f, nullptr, nullptr, 0.f, nullptr, B, h, w, H, W,
-                                                  scale, s, u);
+  if (!disp_std_q) {
+    if (!lr_mask) return launch_upsample_eval<true, false, false>(a, s);
+    return gt ? launch_upsample_eval<true, true, false>(a, s) : launch_upsample_eval<false, true, false>(a, s);
+  }
+  if (gt && lr_mask) return launch_upsample_eval<true, true, true>(a, s);
+  if (gt) return launch_upsample_eval<true, false, true>(a, s);
+  if (lr_mask) return launch_upsample_eval<false, true, true>(a, s);
+  return launch_upsample_eval<false, false, true>(a, s);
 }
 
-// s3d_tap_gather_soft_argmin (std_q == NULL) and s3d_tap_gather_soft_argmin_std
-static int tap_gather_soft_argmin(const float* taps, float* disp, float* std_q, float* cost_out, int N, int D, int h, int w,
-                                  int tap_stride, float sign, void* stream) {
+extern "C" int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* std_q, float* cost_out, int N, int D, int h,
+                                          int w, int tap_stride, float sign, void* stream) {
   if (!taps || !disp) { set_error("tap_gather_soft_argmin: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(N > 0 && D > 0 && h > 0 && w > 0 && tap_stride >= 27 && h < 65536 && N < 65536,
                 "tap_gather_soft_argmin: bad shape");
@@ -846,15 +806,4 @@ static int tap_gather_soft_argmin(const float* taps, float* disp, float* std_q, 
     tap_gather_soft_argmin_kernel<false><<<grid, threads, 0, st>>>(taps, disp, cost_out, N, D, h, w, tap_stride, sign, nullptr);
   S3D_LAUNCH_CHECK();
   return S3D_OK;
-}
-
-extern "C" int s3d_tap_gather_soft_argmin(const float* taps, float* disp, float* cost_out, int N, int D, int h, int w,
-                                          int tap_stride, float sign, void* stream) {
-  return tap_gather_soft_argmin(taps, disp, nullptr, cost_out, N, D, h, w, tap_stride, sign, stream);
-}
-
-extern "C" int s3d_tap_gather_soft_argmin_std(const float* taps, float* disp, float* disp_std_q, float* cost_out, int N, int D,
-                                              int h, int w, int tap_stride, float sign, void* stream) {
-  if (!disp_std_q) { set_error("tap_gather_soft_argmin_std: null argument"); return S3D_ERR_INVALID; }
-  return tap_gather_soft_argmin(taps, disp, disp_std_q, cost_out, N, D, h, w, tap_stride, sign, stream);
 }

@@ -60,24 +60,20 @@ SIGNATURES = {
     's3d_conv_concat_volume': ([ctypes.POINTER(S3dConvParams), _vp, _i, _i, _vp, _vp, _vp], _i),
     's3d_conv_concat_volume_ro': ([ctypes.POINTER(S3dConvParams), _vp, _i, _i, _vp, _vp, _vp, _vp], _i),
     's3d_conv_cls_workspace_bytes': ([_i, _i, _i, _i], ctypes.c_int64),
-    's3d_conv_cls_soft_argmin': ([ctypes.POINTER(S3dConvParams), _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp], _i),
+    's3d_conv_cls_soft_argmin': ([ctypes.POINTER(S3dConvParams), _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp], _i),
     's3d_conv2d_halo': ([_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i, _vp], _i),
     's3d_map_conv': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_concat_gonce_assemble': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_cost_volume_concat': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_soft_argmin': ([_vp, _vp, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_tap_gather_soft_argmin': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_cls_soft_argmin': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_corr_soft_argmin': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),
+    's3d_tap_gather_soft_argmin': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
+    's3d_cls_soft_argmin': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
+    's3d_corr_soft_argmin': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_upsample_disp': ([_vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_upsample_disp_eval': ([_vp, _vp, _vp, ctypes.POINTER(_f), _i, _f, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_upsample_disp_lr': ([_vp, _vp, _vp, _f, _vp, ctypes.POINTER(_f), _i, _f, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_tap_gather_soft_argmin_std': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_cls_soft_argmin_std': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp], _i),
-    's3d_conv_cls_soft_argmin_std': ([ctypes.POINTER(S3dConvParams), _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp], _i),
-    's3d_corr_soft_argmin_std': ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),
-    's3d_upsample_disp_std': ([_vp, _vp, _vp, _vp, ctypes.POINTER(_f), _i, _vp, _vp, ctypes.POINTER(_f), _i, _f, _vp, _vp, _f, _vp,
-                               _i, _i, _i, _i, _i, _f, _vp], _i),
+    's3d_upsample_disp_eval': ([_vp, _vp, _i, _i, _i, _i, _i, _f,
+                                _vp, ctypes.POINTER(_f), _i, _f, _vp,
+                                _vp, _f, _vp,
+                                _vp, _vp, ctypes.POINTER(_f), _i, _vp, _vp], _i),
     's3d_latent_to_vox': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_avg_pool': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_depth_to_space': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),

@@ -389,23 +389,24 @@ class _StereoBase(nn.Module):
         """Last kernel of the disparity stage: 1/4-res disparity -> input pixels [2B,H,W].  With disp_gt [B,2,H,W] the same
         kernel also counts, per sample and view, [n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) for t in
         TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> stats int64 [B,2,2+T] (else None).  With lr_check it
-        also runs the left-right consistency check (include/s3d.h, s3d_upsample_disp_lr; tolerance TEST.LR_THRESH px) ->
+        also runs the left-right consistency check (include/s3d.h, s3d_upsample_disp_eval; tolerance TEST.LR_THRESH px) ->
         lr = (lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T]: [n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and
         count(|disp - gt| > t) over the kept valid pixels]; GT columns zero without disp_gt) (else None).  With std_q (the
-        1/4-res standard deviation) the same kernel also upsamples it and counts the confident pixels (include/s3d.h,
-        s3d_upsample_disp_std; thresholds TEST.UNC_THRESH px) -> unc = (disp_std fp32 [B,2,H,W], unc_stats int64
-        [B,2,K,3+T]: per threshold [n_conf, n_valid_conf, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the
+        1/4-res standard deviation) the same kernel also upsamples it and counts the confident pixels (thresholds
+        TEST.UNC_THRESH px) -> unc = (disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T]: per threshold [n_conf, n_valid_conf, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the
         confident valid pixels]; GT columns zero without disp_gt) (else None).
         -> (disp, stats, lr, unc)."""
         B = disp_q.shape[0] // 2
         out = self._buf('disp', (2 * B, H, W), torch.float32)
+        if disp_gt is None and not lr_check and std_q is None:
+            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None, None, None
         th = list(self.cfg.TEST.DISP_THRESH)
         stats = None
         if disp_gt is not None:
             stats = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64)
             stats.zero_()
         max_gt = 4.0 * self.cfg.NETWORK.MAX_DISP
-        lr = None
+        tau, mask, lr_stats = 0.0, None, None
         if lr_check:
             tau = float(self.cfg.TEST.LR_THRESH)
             if not (math.isfinite(tau) and tau >= 0):
@@ -413,24 +414,16 @@ class _StereoBase(nn.Module):
             mask = self._buf('lr_mask', (B, 2, H, W), torch.uint8)
             lr_stats = self._buf('lr_stats', (B, 2, 3 + len(th)), torch.int64)
             lr_stats.zero_()
-            lr = (mask, lr_stats)
+        ut, unc_stats, disp_std = (), None, None
         if std_q is not None:
             ut = unc_thresholds(self.cfg)
             unc_stats = self._buf('unc_stats', (B, 2, len(ut), 3 + len(th)), torch.int64)
             unc_stats.zero_()
-            _, disp_std = ops.upsample_disp_std(disp_q, std_q, H, W, 4.0, ut, unc_stats, gt=disp_gt, thresholds=th, max_gt=max_gt,
-                                                stats=stats, lr_thresh=tau if lr_check else 0.0, mask=None if lr is None else lr[0],
-                                                lr_stats=None if lr is None else lr[1], out=out,
-                                                std_out=self._buf('disp_std', (B, 2, H, W), torch.float32))
-            return out, stats, lr, (disp_std, unc_stats)
-        if lr_check:
-            ops.upsample_disp_lr(disp_q, H, W, 4.0, tau, lr[0], lr[1], gt=disp_gt, thresholds=th, max_gt=max_gt, stats=stats,
-                                 out=out)
-            return out, stats, lr, None
-        if disp_gt is None:
-            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None, None, None
-        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, max_gt, stats, out=out)
-        return out, stats, None, None
+            disp_std = self._buf('disp_std', (B, 2, H, W), torch.float32)
+        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, max_gt, stats, lr_thresh=tau, mask=mask, lr_stats=lr_stats,
+                               std_q=std_q, unc_thresh=ut, unc_stats=unc_stats, std_out=disp_std, out=out)
+        return (out, stats, None if mask is None else (mask, lr_stats),
+                None if disp_std is None else (disp_std, unc_stats))
 
     def _bufo(self, name, layer, x):
         """Output buffer of `layer` for input x (channels-last, padded channels)."""

@@ -96,7 +96,7 @@ def soft_argmin(cost, sign=-1.0, out=None):
 
 
 def _std_buf(std_out, like):
-    """std_out (the *_std entry points' disp_std_q) must be an fp32 tensor shaped like the disparity `like`."""
+    """std_out (the soft-argmin calls' disp_std_q) must be an fp32 tensor shaped like the disparity `like`."""
     _chk(std_out)
     if std_out.dtype != torch.float32 or std_out.shape != like.shape:
         raise ValueError('std_out must be float32 %s, got %s %s' % (tuple(like.shape), std_out.dtype, tuple(std_out.shape)))
@@ -105,22 +105,17 @@ def _std_buf(std_out, like):
 
 def tap_gather_soft_argmin(taps, sign=-1.0, out=None, want_cost=False, std_out=None):
     """taps fp32, line-planar [N,D,h,S>=27,w] (per-tap projections) -> disp fp32 [N,h,w]; see include/s3d.h.
-    std_out: fp32 [N,h,w] that receives the standard deviation of each pixel's distribution (s3d_tap_gather_soft_argmin_std)."""
+    std_out: fp32 [N,h,w] that receives the standard deviation of each pixel's distribution (disp_std_q)."""
     _chk(taps, out)
     assert taps.dtype == torch.float32 and taps.dim() == 5
     N, D, h, S, w = taps.shape
     if out is None:
         out = torch.empty((N, h, w), dtype=torch.float32, device=taps.device)
     cost = torch.empty((N, D, h, w), dtype=torch.float32, device=taps.device) if want_cost else None
-    if std_out is not None:
-        rc = _lib.load().s3d_tap_gather_soft_argmin_std(taps.data_ptr(), out.data_ptr(), _std_buf(std_out, out).data_ptr(),
-                                                        cost.data_ptr() if want_cost else None, N, D, h, w, S, float(sign),
-                                                        _stream())
-        _lib.check(rc, 's3d_tap_gather_soft_argmin_std')
-    else:
-        rc = _lib.load().s3d_tap_gather_soft_argmin(taps.data_ptr(), out.data_ptr(), cost.data_ptr() if want_cost else None,
-                                                    N, D, h, w, S, float(sign), _stream())
-        _lib.check(rc, 's3d_tap_gather_soft_argmin')
+    std = None if std_out is None else _std_buf(std_out, out).data_ptr()
+    rc = _lib.load().s3d_tap_gather_soft_argmin(taps.data_ptr(), out.data_ptr(), std, cost.data_ptr() if want_cost else None,
+                                                N, D, h, w, S, float(sign), _stream())
+    _lib.check(rc, 's3d_tap_gather_soft_argmin')
     _lib.count_launch()
     return (out, cost) if want_cost else out
 
@@ -293,21 +288,17 @@ def conv_concat_volume_sheared(pc, featp, B, D, pad, out=None, bufs=None):
 def cls_soft_argmin(x, w_taps, sign=-1.0, out=None, std_out=None):
     """x bf16 [N,D,h,w,C] (aggregated volume), w_taps bf16 [32,C] (27 classifier taps) -> disp fp32 [N,h,w]: the Cout=1
     3x3x3 classifier and the soft-argmin in one pass (include/s3d.h, s3d_cls_soft_argmin).  std_out: as for
-    tap_gather_soft_argmin (s3d_cls_soft_argmin_std)."""
+    tap_gather_soft_argmin."""
     _chk(x, w_taps, out)
     assert x.dtype == torch.bfloat16 and w_taps.dtype == torch.bfloat16 and x.dim() == 5 and x.is_contiguous()
     N, D, h, w, C = x.shape
     assert w_taps.numel() == 32 * C and w_taps.is_contiguous()
     if out is None:
         out = torch.empty((N, h, w), dtype=torch.float32, device=x.device)
-    if std_out is not None:
-        rc = _lib.load().s3d_cls_soft_argmin_std(x.data_ptr(), w_taps.data_ptr(), out.data_ptr(), _std_buf(std_out, out).data_ptr(),
-                                                 N, D, h, w, C, float(sign), _stream())
-        _lib.check(rc, 's3d_cls_soft_argmin_std')
-    else:
-        rc = _lib.load().s3d_cls_soft_argmin(x.data_ptr(), w_taps.data_ptr(), out.data_ptr(), N, D, h, w, C, float(sign),
-                                             _stream())
-        _lib.check(rc, 's3d_cls_soft_argmin')
+    std = None if std_out is None else _std_buf(std_out, out).data_ptr()
+    rc = _lib.load().s3d_cls_soft_argmin(x.data_ptr(), w_taps.data_ptr(), out.data_ptr(), std, N, D, h, w, C, float(sign),
+                                         _stream())
+    _lib.check(rc, 's3d_cls_soft_argmin')
     _lib.count_launch()
     return out
 
@@ -320,7 +311,7 @@ def conv_cls_soft_argmin(pc, x, w_taps, sign=-1.0, out=None, workspace=None, std
     """The last aggregation layer `pc` (PackedConv, bf16 3x3x3 64 -> 64 + ReLU) over x [N,D,h,w,64], the Cout = 1 classifier
     (w_taps bf16 [32,64]) and the soft-argmin, the layer's output volume never written (include/s3d.h,
     s3d_conv_cls_soft_argmin; csrc/conv_scatter_cls.cu).  workspace: >= conv_cls_workspace_bytes(N, D, h, w) bytes.
-    std_out: as for tap_gather_soft_argmin (s3d_conv_cls_soft_argmin_std).  -> disp fp32 [N,h,w]."""
+    std_out: as for tap_gather_soft_argmin.  -> disp fp32 [N,h,w]."""
     import ctypes
     _chk(x, w_taps, out, workspace)
     assert x.dtype == torch.bfloat16 and w_taps.dtype == torch.bfloat16 and x.dim() == 5 and x.is_contiguous()
@@ -333,15 +324,10 @@ def conv_cls_soft_argmin(pc, x, w_taps, sign=-1.0, out=None, workspace=None, std
     if out is None:
         out = torch.empty((N, h, w), dtype=torch.float32, device=x.device)
     p = pc.params(N, D, h, w, (D * h * w * 64, h * w * 64, w * 64, 64), _lib.DTYPE_BF16, 64)
-    if std_out is not None:
-        rc = _lib.load().s3d_conv_cls_soft_argmin_std(ctypes.byref(p), x.data_ptr(), pc.bias.data_ptr(), w_taps.data_ptr(),
-                                                      workspace.data_ptr(), out.data_ptr(), _std_buf(std_out, out).data_ptr(),
-                                                      float(sign), _stream())
-        _lib.check(rc, 's3d_conv_cls_soft_argmin_std')
-    else:
-        rc = _lib.load().s3d_conv_cls_soft_argmin(ctypes.byref(p), x.data_ptr(), pc.bias.data_ptr(), w_taps.data_ptr(),
-                                                  workspace.data_ptr(), out.data_ptr(), float(sign), _stream())
-        _lib.check(rc, 's3d_conv_cls_soft_argmin')
+    std = None if std_out is None else _std_buf(std_out, out).data_ptr()
+    rc = _lib.load().s3d_conv_cls_soft_argmin(ctypes.byref(p), x.data_ptr(), pc.bias.data_ptr(), w_taps.data_ptr(),
+                                              workspace.data_ptr(), out.data_ptr(), std, float(sign), _stream())
+    _lib.check(rc, 's3d_conv_cls_soft_argmin')
     _lib.count_launch(2)
     return out
 
@@ -349,22 +335,17 @@ def conv_cls_soft_argmin(pc, x, w_taps, sign=-1.0, out=None, workspace=None, std
 def corr_soft_argmin(feat, B, D, out=None, want_cost=False, c_real=None, std_out=None):
     """feat [2B,1,h,w,C] -> disp fp32 [2B,h,w] (fused correlation + soft-argmax).  c_real: number of REAL feature
     channels when C is a padded pitch (the correlation is a mean over the real channels; padded ones are zero).
-    std_out: as for tap_gather_soft_argmin (s3d_corr_soft_argmin_std)."""
+    std_out: as for tap_gather_soft_argmin."""
     _chk(feat, out)
     n2, one, h, w, C = feat.shape
     assert n2 == 2 * B and one == 1
     if out is None:
         out = torch.empty((2 * B, h, w), dtype=torch.float32, device=feat.device)
     cost = torch.empty((2 * B, D, h, w), dtype=torch.float32, device=feat.device) if want_cost else None
-    if std_out is not None:
-        rc = _lib.load().s3d_corr_soft_argmin_std(feat.data_ptr(), out.data_ptr(), _std_buf(std_out, out).data_ptr(),
-                                                  cost.data_ptr() if want_cost else None, B, h, w, C, int(c_real or 0), D,
-                                                  _code(feat), _stream())
-        _lib.check(rc, 's3d_corr_soft_argmin_std')
-    else:
-        rc = _lib.load().s3d_corr_soft_argmin(feat.data_ptr(), out.data_ptr(), cost.data_ptr() if want_cost else None,
-                                              B, h, w, C, int(c_real or 0), D, _code(feat), _stream())
-        _lib.check(rc, 's3d_corr_soft_argmin')
+    std = None if std_out is None else _std_buf(std_out, out).data_ptr()
+    rc = _lib.load().s3d_corr_soft_argmin(feat.data_ptr(), out.data_ptr(), std, cost.data_ptr() if want_cost else None,
+                                          B, h, w, C, int(c_real or 0), D, _code(feat), _stream())
+    _lib.check(rc, 's3d_corr_soft_argmin')
     _lib.count_launch()
     return (out, cost) if want_cost else out
 
@@ -381,89 +362,48 @@ def upsample_disp(disp_q, H, W, scale, out=None):
     return out
 
 
-def upsample_disp_eval(disp_q, H, W, scale, gt, thresholds, max_gt, stats, out=None):
-    """upsample_disp + evaluation against GT disparity (include/s3d.h, s3d_upsample_disp_eval).  disp_q fp32 [2B,h,w] (left-
-    referenced first) -> disp fp32 [2B,H,W], bit-identical to upsample_disp.  gt fp32 [B,2,H,W] (NaN = no GT).  The per-image
-    counters [n_valid, sum of |disp - gt| in 2^-16 px, count(|disp - gt| > t) per threshold] are ADDED to stats int64
-    [B,2,2+T]."""
-    _chk(disp_q, gt, stats, out)
-    assert disp_q.dtype == torch.float32 and gt.dtype == torch.float32 and stats.dtype == torch.int64
+def upsample_disp_eval(disp_q, H, W, scale, gt=None, thresholds=(), max_gt=0.0, stats=None, *, lr_thresh=0.0, mask=None,
+                       lr_stats=None, std_q=None, unc_thresh=(), unc_stats=None, std_out=None, out=None):
+    """upsample_disp + per-pixel evaluation in one launch (include/s3d.h, s3d_upsample_disp_eval).  disp_q fp32 [2B,h,w] (left-
+    referenced first) -> disp fp32 [2B,H,W], bit-identical to upsample_disp.  At least one of three groups is on; every stats
+    tensor is ADDED to, and T = len(thresholds) sets the row length of each (without gt only column 0 of lr_stats / unc_stats):
+      gt fp32 [B,2,H,W] (NaN = no GT), stats int64 [B,2,2+T]: per image [n_valid, sum of |disp - gt| in 2^-16 px,
+        count(|disp - gt| > t) per threshold];
+      mask uint8 [B,2,H,W] <- 1 where the left-right consistency check keeps the pixel (tolerance lr_thresh px), lr_stats int64
+        [B,2,3+T] += [n_kept, n_valid_kept, sum of |disp - gt| in 2^-16 px over valid & kept, count(|disp - gt| > t) over
+        valid & kept];
+      std_q fp32 [2B,h,w] (from a soft-argmin wrapper's std_out) -> std_out fp32 [B,2,H,W] (view 0 = left-referenced, allocated
+        by the caller), unc_stats int64 [B,2,K,3+T] (K = len(unc_thresh) <= 4) += per view and threshold k, over the pixels with
+        disp_std <= unc_thresh[k]: [n_conf, n_valid_conf, sum of |disp - gt| in 2^-16 px over valid & confident,
+        count(|disp - gt| > t) over valid & confident]."""
+    _chk(disp_q, gt, stats, mask, lr_stats, std_q, unc_stats, std_out, out)
+    assert disp_q.dtype == torch.float32
     N, h, w = disp_q.shape
-    B, T = N // 2, len(thresholds)
-    assert N == 2 * B and tuple(gt.shape) == (B, 2, H, W) and tuple(stats.shape) == (B, 2, 2 + T)
-    if out is None:
-        out = torch.empty((N, H, W), dtype=torch.float32, device=disp_q.device)
-    th = (ctypes.c_float * max(T, 1))(*[float(t) for t in thresholds])
-    rc = _lib.load().s3d_upsample_disp_eval(disp_q.data_ptr(), out.data_ptr(), gt.data_ptr(), th, T, float(max_gt),
-                                            stats.data_ptr(), B, h, w, H, W, float(scale), _stream())
-    _lib.check(rc, 's3d_upsample_disp_eval')
-    _lib.count_launch()
-    return out
-
-
-def upsample_disp_lr(disp_q, H, W, scale, lr_thresh, mask, lr_stats, gt=None, thresholds=(), max_gt=0.0, stats=None, out=None):
-    """upsample_disp + the left-right consistency check of the two views (include/s3d.h, s3d_upsample_disp_lr), and with gt
-    the evaluation of upsample_disp_eval, in one launch.  disp_q fp32 [2B,h,w] (left-referenced first) -> disp fp32 [2B,H,W],
-    bit-identical to upsample_disp.  mask uint8 [B,2,H,W] <- 1 where the pixel is kept.  lr_stats int64 [B,2,3+T] (T =
-    len(thresholds)) += [n_kept, n_valid_kept, sum of |disp - gt| in 2^-16 px over valid & kept, count(|disp - gt| > t) over
-    valid & kept]; without gt only column 0.  gt fp32 [B,2,H,W] and stats int64 [B,2,2+T] come together (stats += what
-    upsample_disp_eval adds)."""
-    _chk(disp_q, mask, lr_stats, gt, stats, out)
-    assert disp_q.dtype == torch.float32 and mask.dtype == torch.uint8 and lr_stats.dtype == torch.int64
-    assert (gt is None) == (stats is None)
-    N, h, w = disp_q.shape
-    B, T = N // 2, len(thresholds)
-    assert N == 2 * B and tuple(mask.shape) == (B, 2, H, W) and tuple(lr_stats.shape) == (B, 2, 3 + T)
-    if gt is not None:
-        assert gt.dtype == torch.float32 and stats.dtype == torch.int64
-        assert tuple(gt.shape) == (B, 2, H, W) and tuple(stats.shape) == (B, 2, 2 + T)
-    if out is None:
-        out = torch.empty((N, H, W), dtype=torch.float32, device=disp_q.device)
-    th = (ctypes.c_float * max(T, 1))(*[float(t) for t in thresholds])
-    rc = _lib.load().s3d_upsample_disp_lr(disp_q.data_ptr(), out.data_ptr(), mask.data_ptr(), float(lr_thresh),
-                                          None if gt is None else gt.data_ptr(), th, T, float(max_gt),
-                                          None if stats is None else stats.data_ptr(), lr_stats.data_ptr(), B, h, w, H, W,
-                                          float(scale), _stream())
-    _lib.check(rc, 's3d_upsample_disp_lr')
-    _lib.count_launch()
-    return out
-
-
-def upsample_disp_std(disp_q, std_q, H, W, scale, unc_thresh, unc_stats, gt=None, thresholds=(), max_gt=0.0, stats=None,
-                      lr_thresh=0.0, mask=None, lr_stats=None, out=None, std_out=None):
-    """upsample_disp of the disparity AND of its standard deviation std_q fp32 [2B,h,w] (from a soft-argmin wrapper's std_out),
-    with the confidence-filtered counters, in one launch (include/s3d.h, s3d_upsample_disp_std).  With gt / stats it adds what
-    upsample_disp_eval adds, with mask / lr_stats it runs the check of upsample_disp_lr, in the same launch.
-    -> (disp fp32 [2B,H,W], bit-identical to upsample_disp; disp_std fp32 [B,2,H,W], view 0 = left-referenced).
-    unc_stats int64 [B,2,K,3+T] (K = len(unc_thresh) <= 4, T = len(thresholds)) += per view and threshold k, over the pixels
-    with disp_std <= unc_thresh[k]: [n_conf, n_valid_conf, sum of |disp - gt| in 2^-16 px over valid & confident,
-    count(|disp - gt| > t) over valid & confident]; without gt only column 0."""
-    _chk(disp_q, std_q, unc_stats, gt, stats, mask, lr_stats, out, std_out)
-    N, h, w = disp_q.shape
-    B, K, T = N // 2, len(unc_thresh), len(thresholds)
-    assert N == 2 * B and disp_q.dtype == torch.float32 and std_q.dtype == torch.float32 and std_q.shape == disp_q.shape
-    assert unc_stats.dtype == torch.int64 and tuple(unc_stats.shape) == (B, 2, K, 3 + T)
-    assert (gt is None) == (stats is None) and (mask is None) == (lr_stats is None)
+    B, T, K = N // 2, len(thresholds), len(unc_thresh)
+    assert N == 2 * B
+    assert (gt is None) == (stats is None) and (mask is None) == (lr_stats is None) and (std_q is None) == (std_out is None)
     if gt is not None:
         assert gt.dtype == torch.float32 and stats.dtype == torch.int64
         assert tuple(gt.shape) == (B, 2, H, W) and tuple(stats.shape) == (B, 2, 2 + T)
     if mask is not None:
         assert mask.dtype == torch.uint8 and lr_stats.dtype == torch.int64
         assert tuple(mask.shape) == (B, 2, H, W) and tuple(lr_stats.shape) == (B, 2, 3 + T)
+    if std_q is not None:
+        assert std_q.dtype == torch.float32 and std_q.shape == disp_q.shape
+        assert unc_stats.dtype == torch.int64 and tuple(unc_stats.shape) == (B, 2, K, 3 + T)
+        assert std_out.dtype == torch.float32 and tuple(std_out.shape) == (B, 2, H, W)
     if out is None:
         out = torch.empty((N, H, W), dtype=torch.float32, device=disp_q.device)
-    if std_out is None:
-        std_out = torch.empty((B, 2, H, W), dtype=torch.float32, device=disp_q.device)
-    assert std_out.dtype == torch.float32 and tuple(std_out.shape) == (B, 2, H, W)
-    ut = (ctypes.c_float * max(K, 1))(*[float(t) for t in unc_thresh])
     th = (ctypes.c_float * max(T, 1))(*[float(t) for t in thresholds])
+    ut = (ctypes.c_float * max(K, 1))(*[float(t) for t in unc_thresh])
     ptr = lambda t: None if t is None else t.data_ptr()
-    rc = _lib.load().s3d_upsample_disp_std(disp_q.data_ptr(), out.data_ptr(), std_q.data_ptr(), std_out.data_ptr(), ut, K,
-                                           unc_stats.data_ptr(), ptr(gt), th, T, float(max_gt), ptr(stats), ptr(mask),
-                                           float(lr_thresh), ptr(lr_stats), B, h, w, H, W, float(scale), _stream())
-    _lib.check(rc, 's3d_upsample_disp_std')
+    rc = _lib.load().s3d_upsample_disp_eval(disp_q.data_ptr(), out.data_ptr(), B, h, w, H, W, float(scale),
+                                            ptr(gt), th, T, float(max_gt), ptr(stats),
+                                            ptr(mask), float(lr_thresh), ptr(lr_stats),
+                                            ptr(std_q), ptr(std_out), ut, K, ptr(unc_stats), _stream())
+    _lib.check(rc, 's3d_upsample_disp_eval')
     _lib.count_launch()
-    return out, std_out
+    return out
 
 
 def latent_to_vox(x, L, out=None, split=False):

@@ -1,5 +1,5 @@
 """Reference statement of the left-right consistency check (test infrastructure): plain numpy fp32, the rule of
-s3d_upsample_disp_lr (include/s3d.h).  The kernel's mask and integers must equal it exactly when both see the same disparity
+s3d_upsample_disp_eval (include/s3d.h).  The kernel's mask and integers must equal it exactly when both see the same disparity
 maps."""
 import numpy as np
 import torch

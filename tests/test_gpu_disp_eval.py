@@ -73,7 +73,7 @@ def test_kernel_matches_upsample_and_oracle(N, h, w, H, W):
     assert torch.equal(s0.cpu(), want[..., :2])
 
 
-def test_kernel_bad_arguments():
+def test_gt_group_bad_arguments():
     L = lib.load()
     B, h, w, H, W = 1, 8, 8, 32, 32
     q = torch.rand(2 * B, h, w, device='cuda')
@@ -86,10 +86,12 @@ def test_kernel_bad_arguments():
 
     def call(T_=2, max_gt=32.0, th_=th, B_=B, **kw):
         p = dict(ptr, **kw)
-        return L.s3d_upsample_disp_eval(p['q'], p['out'], p['gt'], th_, T_, max_gt, p['st'], B_, h, w, H, W, 4.0, s)
+        return L.s3d_upsample_disp_eval(p['q'], p['out'], B_, h, w, H, W, 4.0, p['gt'], th_, T_, max_gt, p['st'],
+                                        None, 0.0, None, None, None, None, 0, None, s)
     assert call() == 0
     for bad in (dict(q=None), dict(out=None), dict(gt=None), dict(st=None), dict(th_=None), dict(T_=9), dict(T_=-1),
-                dict(max_gt=0.0), dict(max_gt=-1.0), dict(max_gt=float('nan')), dict(B_=0)):
+                dict(max_gt=0.0), dict(max_gt=-1.0), dict(max_gt=float('nan')), dict(B_=0),
+                dict(gt=None, st=None)):                                     # no group on: the plain call is s3d_upsample_disp
         rc = call(**bad)
         assert rc == -1, bad
         with pytest.raises(lib.S3dError):

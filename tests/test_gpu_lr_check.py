@@ -1,5 +1,6 @@
-"""Left-right consistency check inside the forward (s3d_upsample_disp_lr): the disparity and the disparity stats are
-bit-identical to s3d_upsample_disp / s3d_upsample_disp_eval, and the mask and integer counters equal the reference
+"""Left-right consistency check inside the forward (s3d_upsample_disp_eval with lr_mask): the disparity and the disparity
+stats are bit-identical to s3d_upsample_disp / s3d_upsample_disp_eval with GT only, and the mask and integer counters equal
+the reference
 statement (tests/lr_oracle.py) on the very disparities the kernel returns."""
 import ctypes
 
@@ -25,7 +26,7 @@ def _lr(q, H, W, scale, tau, gt=None, th=TH, max_gt=32.0, out=None):
     mask = torch.full((B, 2, H, W), 7, dtype=torch.uint8, device='cuda')      # every byte must be written
     ls = torch.zeros(B, 2, 3 + len(th), dtype=torch.int64, device='cuda')
     st = None if gt is None else torch.zeros(B, 2, 2 + len(th), dtype=torch.int64, device='cuda')
-    out = ops.upsample_disp_lr(q, H, W, scale, tau, mask, ls, gt=gt, thresholds=th, max_gt=max_gt, stats=st, out=out)
+    out = ops.upsample_disp_eval(q, H, W, scale, gt, th, max_gt, st, lr_thresh=tau, mask=mask, lr_stats=ls, out=out)
     return out, mask, ls, st
 
 
@@ -36,7 +37,7 @@ def _lr(q, H, W, scale, tau, gt=None, th=TH, max_gt=32.0, out=None):
     (6, 13, 13, 50, 50),        # W = 50: scalar path
     (2, 9, 25, 37, 101),
 ])
-def test_kernel_matches_upsample_eval_and_oracle(N, h, w, H, W):
+def test_lr_group_matches_upsample_eval_and_oracle(N, h, w, H, W):
     B = N // 2
     g = torch.Generator().manual_seed(N * 1000 + W + 1)
     # both views near one smooth per-row level: about half the pixels agree within tau after the x4 scale
@@ -57,7 +58,7 @@ def test_kernel_matches_upsample_eval_and_oracle(N, h, w, H, W):
     assert 0.1 * n_img < want[..., 0].min() and want[..., 0].max() < 0.95 * n_img          # neither vacuous nor trivial
     assert (want[..., 1] > 0).all() and (want[..., 1] < want[..., 0]).all() and (want[..., 3] > 0).all()
     # accumulate contract
-    ops.upsample_disp_lr(q, H, W, 4.0, tau, mask, ls, gt=gt, thresholds=TH, max_gt=max_gt, stats=st, out=out)
+    ops.upsample_disp_eval(q, H, W, 4.0, gt, TH, max_gt, st, lr_thresh=tau, mask=mask, lr_stats=ls, out=out)
     assert torch.equal(ls.cpu(), 2 * want) and torch.equal(st, 2 * st_ref) and torch.equal(out, ref)
     # no GT: same mask, column 0 only, the rest of the row untouched
     out0, mask0, ls0, _ = _lr(q, H, W, 4.0, tau)
@@ -77,7 +78,7 @@ def test_kernel_matches_upsample_eval_and_oracle(N, h, w, H, W):
 
 
 @pytest.mark.parametrize('W', [64, 61])                                # 16-byte and scalar path
-def test_kernel_hand_built_cases(W):
+def test_lr_group_hand_built_cases(W):
     """Identity scale (H = h, W = w, scale 1): a pixel stores q itself while its right and lower neighbours are finite.
     Row y of sample 0 carries one planted case; each is checked in the returned disparity, and the kernel's mask equals the
     oracle everywhere."""
@@ -129,7 +130,7 @@ def test_kernel_hand_built_cases(W):
     assert disp[1, 0, 4, 10] == 1.0 and disp[1, 1, 4, 9] != disp[1, 1, 4, 9] and want_mask[1, 0, 4, 10] == 0
 
 
-def test_kernel_bad_arguments():
+def test_lr_group_bad_arguments():
     L = lib.load()
     B, h, w, H, W = 1, 8, 8, 32, 32
     q = torch.rand(2 * B, h, w, device='cuda')
@@ -145,8 +146,8 @@ def test_kernel_bad_arguments():
 
     def call(T_=2, max_gt=32.0, th_=th, B_=B, tau=1.0, H_=H, **kw):
         p = dict(ptr, **kw)
-        return L.s3d_upsample_disp_lr(p['q'], p['out'], p['mask'], tau, p['gt'], th_, T_, max_gt, p['st'], p['ls'], B_, h, w,
-                                      H_, W, 4.0, s)
+        return L.s3d_upsample_disp_eval(p['q'], p['out'], B_, h, w, H_, W, 4.0, p['gt'], th_, T_, max_gt, p['st'],
+                                        p['mask'], tau, p['ls'], None, None, None, 0, None, s)
     assert call() == 0
     assert call(gt=None, st=None) == 0
     assert call(tau=0.0) == 0 and call(tau=INF) == 0
@@ -158,7 +159,7 @@ def test_kernel_bad_arguments():
         rc = call(**bad)
         assert rc == -1, bad
         with pytest.raises(lib.S3dError):
-            lib.check(rc, 's3d_upsample_disp_lr')
+            lib.check(rc, 's3d_upsample_disp_eval')
     torch.cuda.synchronize()
 
 

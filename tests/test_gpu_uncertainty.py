@@ -194,16 +194,6 @@ def test_corr_tc_std(B, C, h, w, D):
     _close(sd, sd2.cpu().double().numpy(), 1e-3 * (1 + ref.max()))
 
 
-def test_std_entry_points_reject_null():
-    L = lib.load()
-    s = torch.cuda.current_stream().cuda_stream
-    t = torch.zeros(1, 8, 4, 32, 4, device='cuda')
-    d = torch.zeros(1, 4, 4, device='cuda')
-    assert L.s3d_tap_gather_soft_argmin_std(t.data_ptr(), d.data_ptr(), None, None, 1, 8, 4, 4, 32, -1.0, s) == -1
-    assert L.s3d_corr_soft_argmin_std(t.data_ptr(), d.data_ptr(), None, None, 1, 4, 4, 16, 0, 8, 0, s) == -1
-    assert L.s3d_cls_soft_argmin_std(t.data_ptr(), t.data_ptr(), d.data_ptr(), None, 1, 8, 4, 4, 16, -1.0, s) == -1
-
-
 # ---- upsampling ---------------------------------------------------------------------------------------------------------
 def _std_up(q, sq, H, W, scale, ut=UT, gt=None, th=TH, max_gt=32.0, lr=None):
     B = q.shape[0] // 2
@@ -213,9 +203,9 @@ def _std_up(q, sq, H, W, scale, ut=UT, gt=None, th=TH, max_gt=32.0, lr=None):
     if lr is not None:
         mask = torch.full((B, 2, H, W), 7, dtype=torch.uint8, device='cuda')
         ls = torch.zeros(B, 2, 3 + len(th), dtype=torch.int64, device='cuda')
-    std_out = torch.full((B, 2, H, W), 7.0, device='cuda')                 # every element must be written
-    out, sd = ops.upsample_disp_std(q, sq, H, W, scale, ut, us, gt=gt, thresholds=th, max_gt=max_gt, stats=st,
-                                    lr_thresh=lr or 0.0, mask=mask, lr_stats=ls, std_out=std_out)
+    sd = torch.full((B, 2, H, W), 7.0, device='cuda')                      # every element must be written
+    out = ops.upsample_disp_eval(q, H, W, scale, gt, th, max_gt, st, lr_thresh=lr or 0.0, mask=mask, lr_stats=ls, std_q=sq,
+                                 unc_thresh=ut, unc_stats=us, std_out=sd)
     return out, sd, us, st, mask, ls
 
 
@@ -225,7 +215,7 @@ def _std_up(q, sq, H, W, scale, ut=UT, gt=None, th=TH, max_gt=32.0, lr=None):
     (4, 17, 26, 70, 101),       # scalar path
     (2, 9, 25, 37, 101),
 ])
-def test_upsample_std_kernel_matches_siblings_and_oracle(N, h, w, H, W):
+def test_std_group_matches_upsample_and_oracle(N, h, w, H, W):
     B = N // 2
     g = torch.Generator().manual_seed(N * 100 + W)
     base = torch.rand(B, h, 1, generator=g) * 4 + 1
@@ -257,7 +247,7 @@ def test_upsample_std_kernel_matches_siblings_and_oracle(N, h, w, H, W):
     assert 0 < want[..., 0, 0].min() and want[..., 0, 0].max() < n_img and (want[..., 3, 0] > want[..., 0, 0]).all()
     # accumulate contract, fewer thresholds, none
     out, sd, us, st, _, _ = _std_up(q, sq, H, W, 4.0, gt=gt)
-    ops.upsample_disp_std(q, sq, H, W, 4.0, UT, us, gt=gt, thresholds=TH, max_gt=32.0, stats=st, std_out=sd)
+    ops.upsample_disp_eval(q, H, W, 4.0, gt, TH, 32.0, st, std_q=sq, unc_thresh=UT, unc_stats=us, std_out=sd)
     assert torch.equal(us.cpu(), 2 * want) and torch.equal(st, 2 * st_ref)
     _, _, u1, _, _, _ = _std_up(q, sq, H, W, 4.0, ut=[1.0], gt=gt)
     assert torch.equal(u1.cpu(), want[:, :, 1:2])
@@ -265,7 +255,7 @@ def test_upsample_std_kernel_matches_siblings_and_oracle(N, h, w, H, W):
     assert u0.numel() == 0 and torch.equal(sd0.view(torch.int32), ref_sd.contiguous().view(torch.int32))
 
 
-def test_upsample_std_bad_arguments():
+def test_std_group_bad_arguments():
     L = lib.load()
     B, h, w, H, W = 1, 8, 8, 32, 32
     q = torch.rand(2 * B, h, w, device='cuda')
@@ -278,8 +268,8 @@ def test_upsample_std_bad_arguments():
     s = torch.cuda.current_stream().cuda_stream
 
     def call(K=2, ut_=ut, sq=q.data_ptr(), so=sd.data_ptr(), u=us.data_ptr(), B_=B):
-        return L.s3d_upsample_disp_std(q.data_ptr(), out.data_ptr(), sq, so, ut_, K, u, None, th, 2, 0.0, None, None, 0.0,
-                                       None, B_, h, w, H, W, 4.0, s)
+        return L.s3d_upsample_disp_eval(q.data_ptr(), out.data_ptr(), B_, h, w, H, W, 4.0, None, th, 2, 0.0, None,
+                                        None, 0.0, None, sq, so, ut_, K, u, s)
     assert call() == 0 and call(K=0, u=None) == 0 and call(K=4) == 0
     for bad in (dict(K=5), dict(K=-1), dict(sq=None), dict(so=None), dict(u=None), dict(B_=0),
                 dict(ut_=(ctypes.c_float * 2)(1, NAN)), dict(ut_=(ctypes.c_float * 2)(-1, 2)), dict(ut_=(ctypes.c_float * 2)(1, INF))):

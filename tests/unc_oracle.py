@@ -1,5 +1,5 @@
 """Reference statement of the disparity uncertainty (test infrastructure): the soft-argmin mean and standard deviation in fp64
-from a cost tensor, and the confidence-filtered counters of s3d_upsample_disp_std (include/s3d.h) in plain numpy fp32, whose
+from a cost tensor, and the confidence-filtered counters of s3d_upsample_disp_eval (include/s3d.h) in plain numpy fp32, whose
 integers the kernel must equal exactly when both see the same disparity and standard-deviation maps."""
 import numpy as np
 import torch
