@@ -97,3 +97,6 @@ __C.TEST.UNC_THRESH = [1.0, 2.0, 4.0]
 # in the other cloud is closer than t, a Euclidean distance in the points' units (0.01 = F-Score@1% on unit-scale shapes);
 # at most 8, each finite and > 0
 __C.TEST.FSCORE_THRESH = [0.01]
+# iso-level of the exported mesh (forward(..., mesh=True), runner.py --test --save-meshes): marching cubes over the predicted
+# occupancy, a voxel is inside when its value is >= this; finite and in (0, 1]
+__C.TEST.MESH_THRESH = 0.5

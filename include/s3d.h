@@ -325,6 +325,21 @@ int s3d_fuse_views(const void* score, int64_t score_stride, const void* vol, int
 int64_t s3d_voxel_surface_workspace_bytes(int B, int T, int n);
 int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
                            const int* kbound, int F, long long* stats, void* workspace, int64_t workspace_bytes, void* stream);
+/* Triangle mesh of an occupancy grid: marching cubes at iso-level t, closed and consistently oriented.
+ * vol fp32 [B,n,n,n] (sample b is vol[b,k,j,i], x along i), 1 <= n <= 64, padded with one layer of 0 on every side; the
+ * padded field is clamped (NaN -> 0, then min(max(v, 0), 1)) and a corner is inside when v >= t; t finite, 0 < t <= 1, so
+ * the padding is outside and every mesh is closed.  Cells: the (n+1)^3 cubes of the padded lattice, case table
+ * csrc/mc_table.cuh (generated with its rule by stereo_3d_reconstruction_b200/mc_table.py; faces with inside corners on a
+ * diagonal separate them).  One vertex per crossing lattice edge, id = its rank in (padded corner linear index, axis x < y
+ * < z) order; with a, b the values at its lower corner p and at p + e_axis, s = (t - a) / (b - a) and the coordinate along
+ * the axis is ((float)p + 0.5f + s) / n, the other two (q + 0.5f) / n (fp32, round to nearest, left to right): the grid
+ * spans the unit cube.  Faces: 0-based per-sample vertex ids, in cell linear order then table order, each oriented so that
+ * (v1 - v0) x (v2 - v0) points from occupied to empty.  verts fp32 [B,max_verts,3], faces int32 [B,max_faces,3], counts
+ * int32 [B,2] = (n_verts, n_faces); rows past the counts are not written.  max_verts / max_faces must be at least the
+ * worst case of s3d_voxel_mesh_bounds.  One kernel, one block per sample, no atomics: the output is deterministic. */
+int s3d_voxel_mesh_bounds(int n, int* max_verts, int* max_faces);    /* 3 (n+1)(n+2)^2 and 5 (n+1)^3 */
+int s3d_voxel_mesh(const float* vol, int B, int n, float t, float* verts, int max_verts, int* faces, int max_faces,
+                   int* counts, void* stream);
 
 /* --- Chamfer distance (row C; replaces extensions/chamfer_dist, README.md:62-65) ------- */
 /* xyz1 fp32 [B,N,3], xyz2 fp32 [B,M,3] -> dist1 fp32 [B,N], idx1 int32 [B,N] (nearest in

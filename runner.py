@@ -33,6 +33,9 @@ def get_args():
     p.add_argument('--surface', action='store_true',
                    help='Stereo2Voxel: also evaluate the voxel-face surfaces against GT and report Chamfer L2 / L1 and '
                         'F-score as surface')
+    p.add_argument('--save-meshes', metavar='DIR', default=None,
+                   help='Stereo2Voxel: also write the marching-cubes mesh of each prediction (at TEST.MESH_THRESH) and of its '
+                        'GT occupancy as DIR/%%06d.obj and DIR/%%06d_gt.obj, numbered by sample')
     return p.parse_args()
 
 
@@ -83,6 +86,8 @@ def main():
         sys.exit('Only `runner.py --test` is implemented: this is the inference-tier build (training is out of scope).')
     if args.surface and args.model != 'Stereo2Voxel':
         sys.exit('--surface evaluates voxel surfaces: Stereo2Voxel only')
+    if args.save_meshes is not None and args.model != 'Stereo2Voxel':
+        sys.exit('--save-meshes meshes the voxel occupancy: Stereo2Voxel only')
     if not torch.cuda.is_available():
         sys.exit('runner.py --test needs a CUDA device (sm_100a); there is no CPU fallback.')
     from stereo_3d_reconstruction_b200 import models
@@ -104,7 +109,7 @@ def main():
     # one stats vector: the head's statistics, then the disparity counters of the same forwards
     if args.model == 'Stereo2Voxel':
         stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check,
-                             eval_unc=args.uncertainty, eval_surface=args.surface).cpu()
+                             eval_unc=args.uncertainty, eval_surface=args.surface, mesh_dir=args.save_meshes).cpu()
         nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
         res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
     else:

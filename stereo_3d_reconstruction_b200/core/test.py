@@ -25,11 +25,18 @@ Stereo2Voxel._surface_stats), per t in TEST.VOXEL_THRESH (surface_block):
     n_both, sum_b q(CD_L2_b), sum_b q(CD_L1_b), then per tau in TEST.FSCORE_THRESH sum_b q(P_b), sum_b q(R_b), sum_b q(F_b)
                                                                                                (int64)
 again computed per batch in fp64 on the device.
+With mesh_dir (test_voxel) the same forwards also return the marching-cubes mesh of the prediction (models.py,
+Stereo2Voxel._mesh), and each sample of the rank's shard is written as mesh_dir/%06d.obj (predicted) and %06d_gt.obj (the GT
+occupancy, meshed by the same kernel at t = 0.5), numbered by global sample id; the stats vector does not change.
 """
+import os
+
+import numpy as np
 import torch
 import torch.distributed as dist
 
-from ..models import fscore_thresholds, unc_thresholds
+from .. import ops
+from ..models import fscore_thresholds, mesh_thresh, unc_thresholds
 from ..utils import synthetic
 
 _FX = float(1 << 40)
@@ -212,6 +219,25 @@ def _surface_len(cfg, eval_surface):
     return len(cfg.TEST.VOXEL_THRESH) * (3 + 3 * F)
 
 
+def write_obj(path, verts, faces):
+    """Plain OBJ of verts fp32 [V,3] and 0-based faces int [F,3]: `v x y z` with %.9g (an fp32 value reads back exactly),
+    then `f a b c` with 1-based ids."""
+    with open(path, 'w') as fh:
+        np.savetxt(fh, np.asarray(verts, np.float32).reshape(-1, 3), fmt='v %.9g %.9g %.9g')
+        np.savetxt(fh, np.asarray(faces, np.int64).reshape(-1, 3) + 1, fmt='f %d %d %d')
+
+
+def save_meshes(mesh_dir, ids, mesh, gt):
+    """Writes the predicted meshes mesh = (verts, faces, counts) of samples `ids` (global ids) and the meshes of their GT
+    occupancy gt [B,n,n,n] (nonzero = occupied, meshed at t = 0.5) as mesh_dir/%06d.obj and %06d_gt.obj."""
+    gmesh = ops.voxel_mesh((gt != 0).to(torch.float32).contiguous(), 0.5)
+    for name, (v, f, c) in (('%06d.obj', mesh), ('%06d_gt.obj', gmesh)):
+        c = c.cpu()
+        for b, i in enumerate(ids):
+            nv, nf = int(c[b, 0]), int(c[b, 1])
+            write_obj(os.path.join(mesh_dir, name % i), v[b, :nv].cpu().numpy(), f[b, :nf].cpu().numpy())
+
+
 def _point_len(cfg, eval_points):
     if not eval_points:
         return 0
@@ -237,13 +263,14 @@ def _unc_len(cfg, eval_disp, eval_unc):
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_unc=False, eval_surface=False):
+               eval_unc=False, eval_surface=False, mesh_dir=None):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
     eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
     eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones.
-    eval_surface: the same forward also evaluates the voxel surfaces; their block comes last."""
+    eval_surface: the same forward also evaluates the voxel surfaces; their block comes last.
+    mesh_dir: the same forward also meshes the prediction; the meshes and the GT's are written there (module docstring)."""
     th = list(cfg.TEST.VOXEL_THRESH)
     T = len(th)
     nl = _lr_len(cfg, eval_disp, eval_lr)
@@ -252,6 +279,11 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
     ns = _surface_len(cfg, eval_surface)
     stats = torch.zeros(2 * T + 1 + nd + nl + nu + ns, dtype=torch.int64, device=device)
     sk = {'surface': True} if eval_surface else {}
+    if mesh_dir is not None:
+        mesh_thresh(cfg)                                # ValueError on a bad TEST.MESH_THRESH, before any forward
+        os.makedirs(mesh_dir, exist_ok=True)
+        sk['mesh'] = True
+    tail = 3 * ('mesh' in sk)                           # mesh_verts, mesh_faces, mesh_counts come last
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -267,7 +299,7 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
                 stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
                 if eval_lr:
                     stats[2 * T + 1 + nd:2 * T + 1 + nd + nl] += out[6].sum(0).flatten()
-                stats[2 * T + 1 + nd + nl:2 * T + 1 + nd + nl + nu] += out[-1 - bool(sk)].sum(0).flatten()   # before surf_stats
+                stats[2 * T + 1 + nd + nl:2 * T + 1 + nd + nl + nu] += out[-1 - eval_surface - tail].sum(0).flatten()
             elif eval_lr:
                 out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True, **sk)
                 iou, ds, ls = out[3], out[4], out[6]
@@ -281,7 +313,9 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
                 out = model(left, right, gt, **sk)
                 iou = out[3]
             if eval_surface:
-                stats[2 * T + 1 + nd + nl + nu:] += surface_block(out[-1], cfg.CONST.N_VOX)
+                stats[2 * T + 1 + nd + nl + nu:] += surface_block(out[-1 - tail], cfg.CONST.N_VOX)
+            if tail:
+                save_meshes(mesh_dir, ids, out[-3:], gt)
             stats[:T] += iou[:, :, 0].sum(0)
             stats[T:2 * T] += iou[:, :, 1].sum(0)
             stats[2 * T] += len(ids)

@@ -11,6 +11,7 @@ The torch.nn layers below are PARAMETER CONTAINERS only -- their forward is neve
 folds BatchNorm and re-lays every weight for the tcgen05 implicit-GEMM engine once; `forward()` is a
 sequence of C-ABI calls (include/s3d.h) on the current CUDA stream, with no torch math on the path.
 """
+import ctypes
 import math
 import os
 
@@ -135,7 +136,7 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
+    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
         self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
@@ -148,6 +149,8 @@ class _GraphedForward:
             kw['uncertainty'] = True
         if surface:
             kw['surface'] = True
+        if mesh:
+            kw['mesh'] = True
 
         def run():                                    # zeroes its IoU / disparity / LR / uncertainty / surface counters itself: inside the graph
             return model._forward_impl(*args, **kw)
@@ -464,7 +467,7 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -474,6 +477,7 @@ class _StereoBase(nn.Module):
         if uncertainty:
             unc_thresholds(self.cfg)
         self._check_surface(surface, gt)
+        self._check_mesh(mesh)
         left, right = self._check_inputs(left, right)
         gt = self._check_gt(gt, left)
         disp_gt = self._check_disp_gt(disp_gt, left)
@@ -482,10 +486,10 @@ class _StereoBase(nn.Module):
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
         key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
                None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check), bool(uncertainty),
-               bool(surface))
+               bool(surface), bool(mesh))
         g = self._graphs.get(key)
         if g is None:
-            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check), bool(uncertainty), bool(surface))
+            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh))
             self._graphs[key] = g
         return g(left, right, gt, disp_gt)
 
@@ -512,6 +516,11 @@ class _StereoBase(nn.Module):
         if surface:
             raise ValueError('surface=True evaluates voxel surfaces: Stereo2Voxel only')
 
+    def _check_mesh(self, mesh):
+        """mesh=True (the marching-cubes mesh of the occupancy) is a Stereo2Voxel option."""
+        if mesh:
+            raise ValueError('mesh=True meshes the voxel occupancy: Stereo2Voxel only')
+
     def _check_disp_gt(self, disp_gt, left):
         """GT disparity of (checked) inputs `left`: fp32 [B,2,H,W] on their device, in input pixels, view 0 = left-referenced
         (as disp_left), 1 = right-referenced; NaN marks pixels without GT."""
@@ -532,7 +541,8 @@ class _StereoBase(nn.Module):
 class Stereo2Voxel(_StereoBase):
     """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W],
     voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64
-    [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, surf_stats int64 [B,T,2,3+F]]).
+    [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, surf_stats int64 [B,T,2,3+F]][, mesh_verts fp32
+    [B,max_verts,3], mesh_faces int32 [B,max_faces,3], mesh_counts int32 [B,2]]).
     Outputs are views of the module's workspace: clone to keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views
     (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; uncertainty=True: the standard
     deviation of each pixel's soft-argmin distribution in input pixels, and counters over the pixels it marks as confident
@@ -540,7 +550,11 @@ class Stereo2Voxel(_StereoBase):
     surface=True (needs gt): the voxel-face surfaces of the prediction at each t in TEST.VOXEL_THRESH and of gt, evaluated
     against each other; surf_stats per sample, t and direction (0: predicted -> GT, 1: GT -> predicted) = [n_pts, sum s,
     sum q(sqrt s), count(s < k) per tau in TEST.FSCORE_THRESH] with s the exact squared distance to the other surface in
-    doubled lattice units (include/s3d.h, s3d_voxel_surface_eval; two more launches)."""
+    doubled lattice units (include/s3d.h, s3d_voxel_surface_eval; two more launches).
+    mesh=True (with or without gt): the marching-cubes mesh of voxels at the iso-level TEST.MESH_THRESH, a closed,
+    outward-oriented triangle mesh in the unit cube the grid spans; per sample mesh_counts = (n_verts, n_faces) and only the
+    first rows of mesh_verts / mesh_faces (0-based ids) are written; (max_verts, max_faces) = ops.voxel_mesh_bounds(N_VOX)
+    (include/s3d.h, s3d_voxel_mesh; one more launch)."""
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -586,10 +600,16 @@ class Stereo2Voxel(_StereoBase):
                 raise ValueError('surface=True needs the GT occupancy gt')
             fscore_thresholds(self.cfg)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
+    def _check_mesh(self, mesh):
+        """mesh=True needs a valid TEST.MESH_THRESH: checked before anything is launched."""
+        if mesh:
+            mesh_thresh(self.cfg)
+
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
         if uncertainty:
             unc_thresholds(self.cfg)                   # a bad TEST.UNC_THRESH fails before anything is launched
         self._check_surface(surface, gt)
+        self._check_mesh(mesh)
         left, right = self._check_inputs(left, right)
         disp_gt = self._check_disp_gt(disp_gt, left)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
@@ -598,15 +618,15 @@ class Stereo2Voxel(_StereoBase):
             outs = []
             for s in range(0, B, mb):
                 o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
-                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check, uncertainty, surface)
+                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check, uncertainty, surface, mesh)
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface)
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface)
+    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
+        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
 
-    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False):
+    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
@@ -657,7 +677,18 @@ class Stereo2Voxel(_StereoBase):
         out += (lr or ()) + (unc or ())
         if surface:
             out += (self._surface_stats(fused, gt8),)
+        if mesh:
+            out += self._mesh(fused)
         return out
+
+    def _mesh(self, fused):
+        """Marching-cubes mesh of fused [B,n^3] at TEST.MESH_THRESH -> (mesh_verts, mesh_faces, mesh_counts).  Every buffer
+        comes from the workspace: no allocation on this path."""
+        B, nv = fused.shape[0], self.cfg.CONST.N_VOX
+        mv, mf = ops.voxel_mesh_bounds(nv)
+        return ops.voxel_mesh(fused, mesh_thresh(self.cfg), out=(self._buf('mesh_verts', (B, mv, 3), torch.float32),
+                                                                  self._buf('mesh_faces', (B, mf, 3), torch.int32),
+                                                                  self._buf('mesh_counts', (B, 2), torch.int32)))
 
     def _surface_stats(self, fused, gt8):
         """Voxel-surface counters of fused [B,n^3] against gt8 [B,n^3] -> surf_stats int64 [B,T,2,3+F], zeroed here (so a
@@ -681,6 +712,19 @@ def unc_thresholds(cfg):
     if len(th) > 4 or not all(math.isfinite(t) and t >= 0 for t in th):
         raise ValueError('TEST.UNC_THRESH must hold at most 4 finite values >= 0, got %r' % (cfg.TEST.UNC_THRESH,))
     return th
+
+
+def mesh_thresh(cfg):
+    """TEST.MESH_THRESH as a float: the iso-level of the exported mesh, finite and in (0, 1] (a voxel is inside when its
+    occupancy is >= it, as for the IoU); anything else is a ValueError."""
+    t = cfg.TEST.get('MESH_THRESH')
+    try:
+        t = float(t)
+    except (TypeError, ValueError):
+        raise ValueError('TEST.MESH_THRESH must be a number, got %r' % (t,)) from None
+    if not (math.isfinite(t) and 0.0 < t <= 1.0) or float(ctypes.c_float(t).value) <= 0.0:
+        raise ValueError('TEST.MESH_THRESH must be finite and in (0, 1], got %r' % (cfg.TEST.MESH_THRESH,))
+    return t
 
 
 def fscore_thresholds(cfg):
@@ -731,7 +775,8 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False):
+        self._check_mesh(mesh)                         # ValueError: the mesh is a Stereo2Voxel output
         if uncertainty:
             unc_thresholds(self.cfg)
         left, right = self._check_inputs(left, right)

@@ -577,3 +577,54 @@ def voxel_surface_eval(fused, gt8, voxel_thresh, fscore_thresh, stats, workspace
     if B and T:
         _lib.count_launch(2)                   # surface_plane_kernel + surface_count_kernel
     return stats
+
+
+def voxel_mesh_bounds(n):
+    """-> (max_verts, max_faces) of an n^3 grid: 3 (n+1)(n+2)^2 and 5 (n+1)^3, the worst case (include/s3d.h)."""
+    mv, mf = ctypes.c_int(), ctypes.c_int()
+    _lib.check(_lib.load().s3d_voxel_mesh_bounds(int(n), ctypes.byref(mv), ctypes.byref(mf)), 's3d_voxel_mesh_bounds')
+    return mv.value, mf.value
+
+
+def voxel_mesh(vol, t, out=None):
+    """Marching-cubes mesh of each sample of vol fp32 [B,n,n,n] or [B,n^3] (1 <= n <= 64) at iso-level t (finite, 0 < t <= 1)
+    -> (verts fp32 [B,max_verts,3], faces int32 [B,max_faces,3], counts int32 [B,2] = (n_verts, n_faces)) with
+    (max_verts, max_faces) = voxel_mesh_bounds(n); only the first counts rows of each sample are written.  Vertices are xyz in
+    the unit cube the grid spans, faces 0-based per-sample ids oriented outwards (include/s3d.h, s3d_voxel_mesh).  out: the
+    three output tensors.  One kernel launch."""
+    _chk(vol)
+    if vol.dtype != torch.float32 or vol.dim() not in (2, 4):
+        raise ValueError('voxel_mesh: expected vol float32 [B,n,n,n] or [B,n^3], got %s %s' % (vol.dtype, tuple(vol.shape)))
+    B = vol.shape[0]
+    nvox = vol[0].numel() if B else (vol.shape[1] if vol.dim() == 2 else vol.shape[1] * vol.shape[2] * vol.shape[3])
+    n = round(nvox ** (1.0 / 3.0))
+    if n ** 3 != nvox or (vol.dim() == 4 and tuple(vol.shape[1:]) != (n, n, n)) or not 1 <= n <= 64:
+        raise ValueError('voxel_mesh: a sample must be an n^3 grid with 1 <= n <= 64, got %s' % (tuple(vol.shape),))
+    try:
+        t = float(t)
+    except (TypeError, ValueError):
+        raise ValueError('voxel_mesh: t must be a number, got %r' % (t,)) from None
+    if not (math.isfinite(t) and 0.0 < t <= 1.0):
+        raise ValueError('voxel_mesh: t must be finite and in (0, 1], got %r' % t)
+    if float(ctypes.c_float(t).value) <= 0.0:
+        raise ValueError('voxel_mesh: t = %r rounds to 0 in fp32' % t)
+    mv, mf = voxel_mesh_bounds(n)
+    want = ((torch.float32, (B, mv, 3)), (torch.int32, (B, mf, 3)), (torch.int32, (B, 2)))
+    if out is None:
+        out = tuple(torch.empty(s, dtype=d, device=vol.device) for d, s in want)
+    else:
+        out = tuple(out)
+        if len(out) != 3:
+            raise ValueError('voxel_mesh: out must hold (verts, faces, counts)')
+        _chk(*out)
+        for o, (d, s) in zip(out, want):
+            if o.dtype != d or tuple(o.shape) != s or o.device != vol.device:
+                raise ValueError('voxel_mesh: out tensors must be %s on %s, got %s'
+                                 % ([(str(d), s) for d, s in want], vol.device, [(str(o.dtype), tuple(o.shape)) for o in out]))
+    verts, faces, counts = out
+    rc = _lib.load().s3d_voxel_mesh(vol.data_ptr(), B, n, t, verts.data_ptr(), mv, faces.data_ptr(), mf, counts.data_ptr(),
+                                    _stream())
+    _lib.check(rc, 's3d_voxel_mesh')
+    if B:
+        _lib.count_launch(1)                   # voxel_mesh_kernel
+    return verts, faces, counts
