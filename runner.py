@@ -106,34 +106,27 @@ def main():
     if args.weights:
         load_checkpoint(model, args.weights)
     model.cuda().pack()
-    # one stats vector: the head's statistics, then the disparity counters of the same forwards
+    # one stats vector: the head's statistics, then the disparity counters of the same forwards (core/test.py::stats_layout)
+    ev = dict(eval_disp=True, eval_lr=args.lr_check, eval_unc=args.uncertainty)
     if args.model == 'Stereo2Voxel':
-        stats = T.test_voxel(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check,
-                             eval_unc=args.uncertainty, eval_surface=args.surface, mesh_dir=args.save_meshes).cpu()
-        nh = 2 * len(cfg.TEST.VOXEL_THRESH) + 1
-        res = T.iou_summary(stats[:nh], cfg.TEST.VOXEL_THRESH)
+        ev.update(eval_surface=args.surface)
+        stats = T.test_voxel(cfg, model, n, bs, rank, world, mesh_dir=args.save_meshes, **ev).cpu()
     else:
-        # + the point-cloud counters (Chamfer L2 / L1, precision, recall, F-score) of the same forwards, at the very end
-        stats = T.test_point(cfg, model, n, bs, rank, world, eval_disp=True, eval_lr=args.lr_check, eval_points=True,
-                             eval_unc=args.uncertainty).cpu()
-        nh = 2
-        res = T.chamfer_summary(stats[:nh])
-    nd = 2 * (2 + len(cfg.TEST.DISP_THRESH))
-    nl = 2 * (3 + len(cfg.TEST.DISP_THRESH)) if args.lr_check else 0
-    nu = 2 * len(cfg.TEST.UNC_THRESH) * (3 + len(cfg.TEST.DISP_THRESH)) if args.uncertainty else 0
-    res['disparity'] = T.disp_summary(stats[nh:nh + nd], cfg.TEST.DISP_THRESH)
-    if args.lr_check:
-        res['lr_consistency'] = T.lr_summary(stats[nh + nd:nh + nd + nl], cfg.TEST.DISP_THRESH,
-                                             res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
+        ev.update(eval_points=True)
+        stats = T.test_point(cfg, model, n, bs, rank, world, **ev).cpu()
+    b = T.split_stats(stats, T.stats_layout(cfg, args.model, **ev))
+    res = T.iou_summary(b['iou'], cfg.TEST.VOXEL_THRESH) if 'iou' in b else T.chamfer_summary(b['chamfer'])
+    npix = res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W
+    res['disparity'] = T.disp_summary(b['disparity'], cfg.TEST.DISP_THRESH)
+    if 'lr_consistency' in b:
+        res['lr_consistency'] = T.lr_summary(b['lr_consistency'], cfg.TEST.DISP_THRESH, npix, b['disparity'])
         res['lr_consistency']['lr_thresh'] = float(cfg.TEST.LR_THRESH)
-    if args.uncertainty:
-        res['uncertainty'] = T.unc_summary(stats[nh + nd + nl:nh + nd + nl + nu], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH,
-                                           res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W, stats[nh:nh + nd])
-    if args.surface:
-        res['surface'] = T.surface_summary(stats[nh + nd + nl + nu:], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH,
-                                           res['n_samples'])
-    if args.model == 'Stereo2Point':
-        res['points'] = T.points_summary(stats[nh + nd + nl + nu:], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
+    if 'uncertainty' in b:
+        res['uncertainty'] = T.unc_summary(b['uncertainty'], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH, npix, b['disparity'])
+    if 'surface' in b:
+        res['surface'] = T.surface_summary(b['surface'], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH, res['n_samples'])
+    if 'points' in b:
+        res['points'] = T.points_summary(b['points'], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
                                          cfg.CONST.N_GT_POINTS)
     if rank == 0:
         res.update(model=args.model, precision=cfg.NETWORK.PRECISION, world_size=world, data='synthetic')

@@ -24,7 +24,8 @@ With eval_surface=True (test_voxel) the voxel-surface counters of the same forwa
 Stereo2Voxel._surface_stats), per t in TEST.VOXEL_THRESH (surface_block):
     n_both, sum_b q(CD_L2_b), sum_b q(CD_L1_b), then per tau in TEST.FSCORE_THRESH sum_b q(P_b), sum_b q(R_b), sum_b q(F_b)
                                                                                                (int64)
-again computed per batch in fp64 on the device.
+again computed per batch in fp64 on the device.  stats_layout() declares these blocks and their order, split_stats() cuts a
+vector into them.
 With mesh_dir (test_voxel) the same forwards also return the marching-cubes mesh of the prediction (models.py,
 Stereo2Voxel._mesh), and each sample of the rank's shard is written as mesh_dir/%06d.obj (predicted) and %06d_gt.obj (the GT
 occupancy, meshed by the same kernel at t = 0.5), numbered by global sample id; the stats vector does not change.
@@ -36,7 +37,7 @@ import torch
 import torch.distributed as dist
 
 from .. import ops
-from ..models import fscore_thresholds, mesh_thresh, unc_thresholds
+from ..models import Stereo2Point, Stereo2Voxel, fscore_thresholds, mesh_thresh, unc_thresholds
 from ..utils import synthetic
 
 _FX = float(1 << 40)
@@ -212,13 +213,6 @@ def surface_summary(block, voxel_thresh, fscore_thresh, n_samples):
             'by_thresh': per}
 
 
-def _surface_len(cfg, eval_surface):
-    if not eval_surface:
-        return 0
-    F = len(fscore_thresholds(cfg))                     # ValueError on a bad TEST.FSCORE_THRESH, before any forward
-    return len(cfg.TEST.VOXEL_THRESH) * (3 + 3 * F)
-
-
 def write_obj(path, verts, faces):
     """Plain OBJ of verts fp32 [V,3] and 0-based faces int [F,3]: `v x y z` with %.9g (an fp32 value reads back exactly),
     then `f a b c` with 1-based ids."""
@@ -238,28 +232,49 @@ def save_meshes(mesh_dir, ids, mesh, gt):
             write_obj(os.path.join(mesh_dir, name % i), v[b, :nv].cpu().numpy(), f[b, :nf].cpu().numpy())
 
 
-def _point_len(cfg, eval_points):
-    if not eval_points:
-        return 0
-    T = len(fscore_thresholds(cfg))                     # ValueError on a bad TEST.FSCORE_THRESH, before any forward
-    return 2 * (3 + T) + T
-
-
 def _disp_gt(pairs, H, W, device):
     return torch.cat([synthetic.disparity_gt(p[2], H, W) for p in pairs]).to(device)
 
 
-def _lr_len(cfg, eval_disp, eval_lr):
+def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eval_surface=False, eval_points=False):
+    """The driver's int64 stats vector for `model` ('Stereo2Voxel' / 'Stereo2Point') as ordered blocks [(name, length)]: the
+    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', then 'surface'
+    (Stereo2Voxel) / 'points' (Stereo2Point), each present when its evaluation is on (module docstring).  ValueError on an
+    evaluation without the disparity counters it needs or on a bad cfg.TEST threshold: raised before any forward."""
     if eval_lr and not eval_disp:
         raise ValueError('eval_lr=True needs eval_disp=True')
-    return 2 * (3 + len(cfg.TEST.DISP_THRESH)) if eval_lr else 0
-
-
-def _unc_len(cfg, eval_disp, eval_unc):
     if eval_unc and not eval_disp:
         raise ValueError('eval_unc=True needs eval_disp=True')
-    # ValueError on a bad TEST.UNC_THRESH, before any forward
-    return 2 * len(unc_thresholds(cfg)) * (3 + len(cfg.TEST.DISP_THRESH)) if eval_unc else 0
+    T = len(cfg.TEST.DISP_THRESH)
+    blocks = [('iou', 2 * len(cfg.TEST.VOXEL_THRESH) + 1) if model == 'Stereo2Voxel' else ('chamfer', 2)]
+    if eval_disp:
+        blocks.append(('disparity', 2 * (2 + T)))
+    if eval_lr:
+        blocks.append(('lr_consistency', 2 * (3 + T)))
+    if eval_unc:
+        blocks.append(('uncertainty', 2 * len(unc_thresholds(cfg)) * (3 + T)))
+    if eval_surface:
+        blocks.append(('surface', len(cfg.TEST.VOXEL_THRESH) * (3 + 3 * len(fscore_thresholds(cfg)))))
+    if eval_points:
+        F = len(fscore_thresholds(cfg))
+        blocks.append(('points', 2 * (3 + F) + F))
+    return blocks
+
+
+def split_stats(stats, layout):
+    """{name: slice of the 1-D stats vector} for the blocks of `layout` (stats_layout); the slices are views."""
+    out, lo = {}, 0
+    for name, n in layout:
+        out[name] = stats[lo:lo + n]
+        lo += n
+    return out
+
+
+def _add_disp_blocks(blocks, out):
+    """Adds the batch's disparity, LR-check and uncertainty counters of the named forward outputs `out` to their blocks."""
+    for block, name in (('disparity', 'disp_stats'), ('lr_consistency', 'lr_stats'), ('uncertainty', 'unc_stats')):
+        if block in blocks:
+            blocks[block] += out[name].sum(0).flatten()
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
@@ -270,20 +285,18 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
     eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
     eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones.
     eval_surface: the same forward also evaluates the voxel surfaces; their block comes last.
-    mesh_dir: the same forward also meshes the prediction; the meshes and the GT's are written there (module docstring)."""
-    th = list(cfg.TEST.VOXEL_THRESH)
-    T = len(th)
-    nl = _lr_len(cfg, eval_disp, eval_lr)
-    nu = _unc_len(cfg, eval_disp, eval_unc)
-    nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    ns = _surface_len(cfg, eval_surface)
-    stats = torch.zeros(2 * T + 1 + nd + nl + nu + ns, dtype=torch.int64, device=device)
-    sk = {'surface': True} if eval_surface else {}
+    mesh_dir: the same forward also meshes the prediction; the meshes and the GT's are written there (module docstring).
+    The vector's blocks: stats_layout(cfg, 'Stereo2Voxel', ...)."""
+    layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface)
     if mesh_dir is not None:
         mesh_thresh(cfg)                                # ValueError on a bad TEST.MESH_THRESH, before any forward
         os.makedirs(mesh_dir, exist_ok=True)
-        sk['mesh'] = True
-    tail = 3 * ('mesh' in sk)                           # mesh_verts, mesh_faces, mesh_counts come last
+    kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc), ('surface', eval_surface),
+                                ('mesh', mesh_dir is not None)) if on}    # the options that are on, and only those
+    names = Stereo2Voxel.output_names(gt=True, disp_gt=eval_disp, **kw)
+    stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
+    blocks = split_stats(stats, layout)
+    T = len(cfg.TEST.VOXEL_THRESH)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -293,45 +306,32 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.gt_volume(1, cfg.CONST.N_VOX, seed=100000 + i) for i in ids]).to(device)
-            if eval_unc:
-                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=eval_lr, uncertainty=True, **sk)
-                iou, ds = out[3], out[4]
-                stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
-                if eval_lr:
-                    stats[2 * T + 1 + nd:2 * T + 1 + nd + nl] += out[6].sum(0).flatten()
-                stats[2 * T + 1 + nd + nl:2 * T + 1 + nd + nl + nu] += out[-1 - eval_surface - tail].sum(0).flatten()
-            elif eval_lr:
-                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True, **sk)
-                iou, ds, ls = out[3], out[4], out[6]
-                stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
-                stats[2 * T + 1 + nd:2 * T + 1 + nd + nl] += ls.sum(0).flatten()
-            elif eval_disp:
-                out = model(left, right, gt, disp_gt=_disp_gt(pairs, H, W, device), **sk)
-                iou, ds = out[3], out[4]
-                stats[2 * T + 1:2 * T + 1 + nd] += ds.sum(0).flatten()
-            else:
-                out = model(left, right, gt, **sk)
-                iou = out[3]
+            if eval_disp:
+                kw['disp_gt'] = _disp_gt(pairs, H, W, device)
+            out = dict(zip(names, model(left, right, gt, **kw)))
+            _add_disp_blocks(blocks, out)
             if eval_surface:
-                stats[2 * T + 1 + nd + nl + nu:] += surface_block(out[-1 - tail], cfg.CONST.N_VOX)
-            if tail:
-                save_meshes(mesh_dir, ids, out[-3:], gt)
-            stats[:T] += iou[:, :, 0].sum(0)
-            stats[T:2 * T] += iou[:, :, 1].sum(0)
-            stats[2 * T] += len(ids)
+                blocks['surface'] += surface_block(out['surf_stats'], cfg.CONST.N_VOX)
+            if mesh_dir is not None:
+                save_meshes(mesh_dir, ids, (out['mesh_verts'], out['mesh_faces'], out['mesh_counts']), gt)
+            iou = out['iou_counts']
+            blocks['iou'][:T] += iou[:, :, 0].sum(0)
+            blocks['iou'][T:2 * T] += iou[:, :, 1].sum(0)
+            blocks['iou'][2 * T] += len(ids)
     return reduce_stats(stats)
 
 
 def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
                eval_points=False, eval_unc=False):
     """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, the
-    uncertainty counters with eval_unc, as for test_voxel, + the point-cloud counters with eval_points: module docstring)."""
+    uncertainty counters with eval_unc, as for test_voxel, + the point-cloud counters with eval_points: module docstring).
+    The vector's blocks: stats_layout(cfg, 'Stereo2Point', ...)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
-    nl = _lr_len(cfg, eval_disp, eval_lr)
-    nu = _unc_len(cfg, eval_disp, eval_unc)
-    nd = 2 * (2 + len(cfg.TEST.DISP_THRESH)) if eval_disp else 0
-    npt = _point_len(cfg, eval_points)
-    stats = torch.zeros(2 + nd + nl + nu + npt, dtype=torch.int64, device=device)
+    layout = stats_layout(cfg, 'Stereo2Point', eval_disp, eval_lr, eval_unc, eval_points=eval_points)
+    kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc)) if on}
+    names = Stereo2Point.output_names(gt=eval_points, disp_gt=eval_disp, **kw)
+    stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
+    blocks = split_stats(stats, layout)
     lo, hi = shard_range(n_samples, rank, world)
     H, W = cfg.CONST.IMG_H, cfg.CONST.IMG_W
     with torch.no_grad():
@@ -342,29 +342,16 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.point_clouds(1, 1, cfg.CONST.N_GT_POINTS, seed=200000 + i)[1] for i in ids]).to(device)
             head = (gt,) if eval_points else ()
-            if eval_unc:
-                out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device), lr_check=eval_lr, uncertainty=True)
-                k = 3 + len(head)                                  # disp_stats, then [lr_mask, lr_stats], disp_std, unc_stats
-                stats[2:2 + nd] += out[k].sum(0).flatten()
-                if eval_lr:
-                    stats[2 + nd:2 + nd + nl] += out[k + 2].sum(0).flatten()
-                stats[2 + nd + nl:2 + nd + nl + nu] += out[-1].sum(0).flatten()
-            elif eval_lr:
-                out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device), lr_check=True)
-                ds, ls = out[-3], out[-1]
-                stats[2:2 + nd] += ds.sum(0).flatten()
-                stats[2 + nd:2 + nd + nl] += ls.sum(0).flatten()
-            elif eval_disp:
-                out = model(left, right, *head, disp_gt=_disp_gt(pairs, H, W, device))
-                stats[2:2 + nd] += out[-1].sum(0).flatten()
-            else:
-                out = model(left, right, *head)
-            pts = out[2]
+            if eval_disp:
+                kw['disp_gt'] = _disp_gt(pairs, H, W, device)
+            out = dict(zip(names, model(left, right, *head, **kw)))
+            _add_disp_blocks(blocks, out)
+            pts = out['points']
             if eval_points:
-                stats[2 + nd + nl + nu:] += point_block(out[3], pts.shape[1], gt.shape[1])
+                blocks['points'] += point_block(out['point_stats'], pts.shape[1], gt.shape[1])
             cd = chamfer_per_sample(pts.contiguous(), gt)
-            stats[0] += torch.round(cd.sum() * _FX).to(torch.int64)
-            stats[1] += len(ids)
+            blocks['chamfer'][0] += torch.round(cd.sum() * _FX).to(torch.int64)
+            blocks['chamfer'][1] += len(ids)
     return reduce_stats(stats)
 
 

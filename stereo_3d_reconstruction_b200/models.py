@@ -11,6 +11,7 @@ The torch.nn layers below are PARAMETER CONTAINERS only -- their forward is neve
 folds BatchNorm and re-lays every weight for the tcgen05 implicit-GEMM engine once; `forward()` is a
 sequence of C-ABI calls (include/s3d.h) on the current CUDA stream, with no torch math on the path.
 """
+import collections
 import ctypes
 import math
 import os
@@ -28,6 +29,19 @@ A = _lib  # activation / dtype codes
 # hi*hi + lo*hi + hi*lo on kind::f16 MMAs into one fp32 accumulator (include/s3d.h, S3D_DTYPE_BF16X2): the FAST mode that
 # meets the north_star's 1e-3 fp32 tolerance.  'tf32x3' does the same with three kind::tf32 passes per layer through HBM.
 PRECISIONS = ('bf16', 'bf16x3', 'tf32', 'tf32x3', 'fp32')
+
+# The forward's optional output groups, in tuple order after the head's outputs and the gt output (iou_counts /
+# point_stats): (keyword that turns the group on, its outputs).  output_names() derives every tuple layout from this.
+OPTIONAL_OUTPUTS = (('disp_gt', ('disp_stats',)),
+                    ('lr_check', ('lr_mask', 'lr_stats')),
+                    ('uncertainty', ('disp_std', 'unc_stats')),
+                    ('surface', ('surf_stats',)),
+                    ('mesh', ('mesh_verts', 'mesh_faces', 'mesh_counts')))
+_VOXEL_ONLY = {'surface': 'surface=True evaluates voxel surfaces: Stereo2Voxel only',
+               'mesh': 'mesh=True meshes the voxel occupancy: Stereo2Voxel only'}
+
+# The options of one forward, checked (_StereoBase._check_args): what the stages branch on and part of the graph key.
+Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty surface mesh')
 
 
 def _conv_bn2d(cin, cout, k, s, p):
@@ -136,24 +150,14 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
+    def __init__(self, model, left, right, gt, disp_gt, opts):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
         self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
         self._copy_in(left, right, gt, disp_gt)
-        args = (self.left, self.right) if gt is None else (self.left, self.right, self.gt)
-        kw = {} if disp_gt is None else {'disp_gt': self.disp_gt}
-        if lr_check:
-            kw['lr_check'] = True
-        if uncertainty:
-            kw['uncertainty'] = True
-        if surface:
-            kw['surface'] = True
-        if mesh:
-            kw['mesh'] = True
 
         def run():                                    # zeroes its IoU / disparity / LR / uncertainty / surface counters itself: inside the graph
-            return model._forward_impl(*args, **kw)
+            return model._forward_impl(self.left, self.right, self.gt, self.disp_gt, opts)
         side = torch.cuda.Stream(device=left.device)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):                 # warm-up: workspace buffers and tensor maps exist before capture
@@ -284,9 +288,8 @@ class _StereoBase(nn.Module):
         return (img.shape[0], img.shape[1], img.shape[2]) if img.dtype == torch.uint8 else (img.shape[0], img.shape[2], img.shape[3])
 
     def _disparity(self, left, right, disp_gt=None, lr_check=False, uncertainty=False):
-        """-> disp fp32 [2B,H,W] (left-referenced first), in input pixels, disp_q, the disparity stats int64 [B,2,2+T]
-        against disp_gt (None without it), the LR check's (lr_mask, lr_stats) (None without lr_check) and with uncertainty
-        (disp_std, unc_stats) (else None; see _upsample_disp)."""
+        """-> (disp fp32 [2B,H,W] (left-referenced first) in input pixels, the dict of named evaluation outputs of
+        _upsample_disp)."""
         cfg = self.cfg
         B, H, W = self._bhw(left)
         D = cfg.NETWORK.MAX_DISP
@@ -371,8 +374,7 @@ class _StereoBase(nn.Module):
                 nb = ops.conv_cls_workspace_bytes(2 * B, D, h, w)
                 ops.conv_cls_soft_argmin(pa, a, self._packed['cls_b'].weight, -1.0, out=disp_q,
                                          workspace=self._buf('cls_ws', (nb,), torch.uint8), **std_kw)
-                disp, stats, lr, unc = self._upsample_disp(disp_q, H, W, disp_gt, lr_check, std_q)
-                return disp, disp_q, stats, lr, unc
+                return self._upsample_disp(disp_q, H, W, disp_gt, lr_check, std_q)
             c = self._conv('cls_a', a, out=self._bufo('a0', 'cls_a', a))
             if self.precision == 'bf16' and c.shape[-1] in (16, 32, 64) and S == 32 and not _lib.KNOBS['no_cls_fused']:
                 # classifier + soft-argmin in one pass over the volume (csrc/cls_fused.cu)
@@ -385,48 +387,42 @@ class _StereoBase(nn.Module):
             if self._split:                                               # exact fp32 correlation on hi + lo
                 feat = ops.unsplit_bf16(feat, out=self._buf('feat32', feat.shape[:-1] + (feat.shape[-1] // 2,), torch.float32))
             ops.corr_soft_argmin(feat, B, D, out=disp_q, c_real=C, **std_kw)        # mean over the REAL channels (feat is padded)
-        disp, stats, lr, unc = self._upsample_disp(disp_q, H, W, disp_gt, lr_check, std_q)
-        return disp, disp_q, stats, lr, unc
+        return self._upsample_disp(disp_q, H, W, disp_gt, lr_check, std_q)
 
     def _upsample_disp(self, disp_q, H, W, disp_gt, lr_check=False, std_q=None):
         """Last kernel of the disparity stage: 1/4-res disparity -> input pixels [2B,H,W].  With disp_gt [B,2,H,W] the same
         kernel also counts, per sample and view, [n_valid, sum |disp - gt| in 2^-16 px, count(|disp - gt| > t) for t in
-        TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> stats int64 [B,2,2+T] (else None).  With lr_check it
+        TEST.DISP_THRESH] over the pixels with 0 <= gt < 4 * MAX_DISP -> disp_stats int64 [B,2,2+T].  With lr_check it
         also runs the left-right consistency check (include/s3d.h, s3d_upsample_disp_eval; tolerance TEST.LR_THRESH px) ->
-        lr = (lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T]: [n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and
-        count(|disp - gt| > t) over the kept valid pixels]; GT columns zero without disp_gt) (else None).  With std_q (the
-        1/4-res standard deviation) the same kernel also upsamples it and counts the confident pixels (thresholds
-        TEST.UNC_THRESH px) -> unc = (disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T]: per threshold [n_conf, n_valid_conf, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the
-        confident valid pixels]; GT columns zero without disp_gt) (else None).
-        -> (disp, stats, lr, unc)."""
+        lr_mask uint8 [B,2,H,W], lr_stats int64 [B,2,3+T]: [n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and
+        count(|disp - gt| > t) over the kept valid pixels]; GT columns zero without disp_gt.  With std_q (the 1/4-res
+        standard deviation) the same kernel also upsamples it and counts the confident pixels (thresholds TEST.UNC_THRESH
+        px) -> disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T]: per threshold [n_conf, n_valid_conf, sum |disp - gt| in
+        2^-16 px and count(|disp - gt| > t) over the confident valid pixels]; GT columns zero without disp_gt.
+        -> (disp, {name: tensor} of the outputs above that were computed)."""
         B = disp_q.shape[0] // 2
         out = self._buf('disp', (2 * B, H, W), torch.float32)
         if disp_gt is None and not lr_check and std_q is None:
-            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), None, None, None
+            return ops.upsample_disp(disp_q, H, W, 4.0, out=out), {}
         th = list(self.cfg.TEST.DISP_THRESH)
-        stats = None
+        ev = {}
         if disp_gt is not None:
-            stats = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64)
-            stats.zero_()
+            ev['disp_stats'] = self._buf('disp_stats', (B, 2, 2 + len(th)), torch.int64).zero_()
         max_gt = 4.0 * self.cfg.NETWORK.MAX_DISP
-        tau, mask, lr_stats = 0.0, None, None
+        tau = 0.0
         if lr_check:
-            tau = float(self.cfg.TEST.LR_THRESH)
-            if not (math.isfinite(tau) and tau >= 0):
-                raise ValueError('TEST.LR_THRESH must be finite and >= 0, got %r' % self.cfg.TEST.LR_THRESH)
-            mask = self._buf('lr_mask', (B, 2, H, W), torch.uint8)
-            lr_stats = self._buf('lr_stats', (B, 2, 3 + len(th)), torch.int64)
-            lr_stats.zero_()
-        ut, unc_stats, disp_std = (), None, None
+            tau = lr_thresh(self.cfg)
+            ev['lr_mask'] = self._buf('lr_mask', (B, 2, H, W), torch.uint8)
+            ev['lr_stats'] = self._buf('lr_stats', (B, 2, 3 + len(th)), torch.int64).zero_()
+        ut = ()
         if std_q is not None:
             ut = unc_thresholds(self.cfg)
-            unc_stats = self._buf('unc_stats', (B, 2, len(ut), 3 + len(th)), torch.int64)
-            unc_stats.zero_()
-            disp_std = self._buf('disp_std', (B, 2, H, W), torch.float32)
-        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, max_gt, stats, lr_thresh=tau, mask=mask, lr_stats=lr_stats,
-                               std_q=std_q, unc_thresh=ut, unc_stats=unc_stats, std_out=disp_std, out=out)
-        return (out, stats, None if mask is None else (mask, lr_stats),
-                None if disp_std is None else (disp_std, unc_stats))
+            ev['unc_stats'] = self._buf('unc_stats', (B, 2, len(ut), 3 + len(th)), torch.int64).zero_()
+            ev['disp_std'] = self._buf('disp_std', (B, 2, H, W), torch.float32)
+        ops.upsample_disp_eval(disp_q, H, W, 4.0, disp_gt, th, max_gt, ev.get('disp_stats'), lr_thresh=tau,
+                               mask=ev.get('lr_mask'), lr_stats=ev.get('lr_stats'), std_q=std_q, unc_thresh=ut,
+                               unc_stats=ev.get('unc_stats'), std_out=ev.get('disp_std'), out=out)
+        return out, ev
 
     def _bufo(self, name, layer, x):
         """Output buffer of `layer` for input x (channels-last, padded channels)."""
@@ -474,24 +470,58 @@ class _StereoBase(nn.Module):
         ~0.12 ms per aggregation layer), so the graph only removes the launch gaps.
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
-        if uncertainty:
-            unc_thresholds(self.cfg)
-        self._check_surface(surface, gt)
-        self._check_mesh(mesh)
-        left, right = self._check_inputs(left, right)
-        gt = self._check_gt(gt, left)
-        disp_gt = self._check_disp_gt(disp_gt, left)
+        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
         key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
-               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), bool(lr_check), bool(uncertainty),
-               bool(surface), bool(mesh))
+               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), opts)
         g = self._graphs.get(key)
         if g is None:
-            g = _GraphedForward(self, left, right, gt, disp_gt, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh))
-            self._graphs[key] = g
+            g = self._graphs[key] = _GraphedForward(self, left, right, gt, disp_gt, opts)
         return g(left, right, gt, disp_gt)
+
+    # ---- outputs and their checks --------------------------------------------------------------
+    @classmethod
+    def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False):
+        """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt: whether the tensor is given):
+        the head's outputs, the gt output, then the groups of OPTIONAL_OUTPUTS that are on.  ValueError on an option the
+        class does not have."""
+        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'surface': surface, 'mesh': mesh}
+        names = cls.HEAD_OUTPUTS + ((cls.GT_OUTPUT,) if gt else ())
+        for opt, outs in OPTIONAL_OUTPUTS:
+            if on[opt]:
+                if opt not in cls.OPTIONS:
+                    raise ValueError(_VOXEL_ONLY[opt])
+                names += outs
+        return names
+
+    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh):
+        """The one check of forward() / graphed()'s arguments, before anything is launched: first the options (which the
+        class has, what they need), then the cfg.TEST thresholds of the enabled outputs, then the tensors.
+        -> (left, right, gt, disp_gt) as the forward takes them and the options value: an Options of bools."""
+        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh))
+        self.output_names(**opts._asdict())                   # ValueError on an option this class does not have
+        if opts.surface and not opts.gt:
+            raise ValueError('surface=True needs the GT occupancy gt')
+        if opts.uncertainty:
+            unc_thresholds(self.cfg)
+        if opts.surface or (opts.gt and self.GT_OUTPUT == 'point_stats'):     # the surface and point-cloud F-scores
+            fscore_thresholds(self.cfg)
+        if opts.mesh:
+            mesh_thresh(self.cfg)
+        if opts.lr_check:
+            lr_thresh(self.cfg)
+        left, right = self._check_inputs(left, right)
+        return left, right, self._check_gt(gt, left), self._check_disp_gt(disp_gt, left), opts
+
+    def _forward_impl(self, left, right, gt, disp_gt, opts):
+        """The forward of checked arguments: the stages fill one dict of named outputs, returned in output_names order."""
+        B = left.shape[0]
+        disp, out = self._disparity(left, right, disp_gt, opts.lr_check, opts.uncertainty)
+        out.update(disp_left=disp[:B].unsqueeze(1), disp_right=disp[B:].unsqueeze(1))
+        self._head(left, right, gt, disp, opts, out)
+        return tuple(out[n] for n in self.output_names(**opts._asdict()))
 
     def _check_inputs(self, left, right):
         if self._packed is None or self._packed_prec != self.precision:
@@ -510,16 +540,6 @@ class _StereoBase(nn.Module):
     def _check_gt(self, gt, left):
         """The head's GT as the head takes it (Stereo2Point validates its point cloud)."""
         return gt
-
-    def _check_surface(self, surface, gt):
-        """surface=True (the voxel-surface metrics) is a Stereo2Voxel option."""
-        if surface:
-            raise ValueError('surface=True evaluates voxel surfaces: Stereo2Voxel only')
-
-    def _check_mesh(self, mesh):
-        """mesh=True (the marching-cubes mesh of the occupancy) is a Stereo2Voxel option."""
-        if mesh:
-            raise ValueError('mesh=True meshes the voxel occupancy: Stereo2Voxel only')
 
     def _check_disp_gt(self, disp_gt, left):
         """GT disparity of (checked) inputs `left`: fp32 [B,2,H,W] on their device, in input pixels, view 0 = left-referenced
@@ -555,6 +575,10 @@ class Stereo2Voxel(_StereoBase):
     outward-oriented triangle mesh in the unit cube the grid spans; per sample mesh_counts = (n_verts, n_faces) and only the
     first rows of mesh_verts / mesh_faces (0-based ids) are written; (max_verts, max_faces) = ops.voxel_mesh_bounds(N_VOX)
     (include/s3d.h, s3d_voxel_mesh; one more launch)."""
+
+    HEAD_OUTPUTS = ('disp_left', 'disp_right', 'voxels')
+    GT_OUTPUT = 'iou_counts'
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'surface', 'mesh')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -593,44 +617,24 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def _check_surface(self, surface, gt):
-        """surface=True needs the GT occupancy and a valid TEST.FSCORE_THRESH: checked before anything is launched."""
-        if surface:
-            if gt is None:
-                raise ValueError('surface=True needs the GT occupancy gt')
-            fscore_thresholds(self.cfg)
-
-    def _check_mesh(self, mesh):
-        """mesh=True needs a valid TEST.MESH_THRESH: checked before anything is launched."""
-        if mesh:
-            mesh_thresh(self.cfg)
-
     def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
-        if uncertainty:
-            unc_thresholds(self.cfg)                   # a bad TEST.UNC_THRESH fails before anything is launched
-        self._check_surface(surface, gt)
-        self._check_mesh(mesh)
-        left, right = self._check_inputs(left, right)
-        disp_gt = self._check_disp_gt(disp_gt, left)
+        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
             outs = []
             for s in range(0, B, mb):
-                o = self._forward_chunk(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
-                                        None if disp_gt is None else disp_gt[s:s + mb], lr_check, uncertainty, surface, mesh)
+                o = self._forward_impl(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
+                                       None if disp_gt is None else disp_gt[s:s + mb], opts)
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
+        return self._forward_impl(left, right, gt, disp_gt, opts)
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
-        return self._forward_chunk(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
-
-    def _forward_chunk(self, left, right, gt, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
+    def _head(self, left, right, gt, disp, opts, out):
+        """The voxel head: adds voxels, iou_counts (with gt), surf_stats (surface) and the mesh (mesh) to `out`."""
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
-        disp, _, dstats, lr, unc = self._disparity(left, right, disp_gt, lr_check, uncertainty)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         k0 = cfg.NETWORK.DEC_CHANNELS[0]
@@ -669,17 +673,13 @@ class Stereo2Voxel(_StereoBase):
         ops.fuse_views(s, 0, s.shape[-1], m_in, craw, cm, B, 2, nv ** 3, gt=gt8,
                        thresholds=list(cfg.TEST.VOXEL_THRESH) if gt is not None else None, iou=iou, out=fused,
                        score_lo=s.shape[-1] // 2 if self._split else 0, vol_lo=split_lo)
-        out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), fused.view(B, nv, nv, nv))
+        out['voxels'] = fused.view(B, nv, nv, nv)
         if gt is not None:
-            out += (iou,)
-        if disp_gt is not None:
-            out += (dstats,)
-        out += (lr or ()) + (unc or ())
-        if surface:
-            out += (self._surface_stats(fused, gt8),)
-        if mesh:
-            out += self._mesh(fused)
-        return out
+            out['iou_counts'] = iou
+        if opts.surface:
+            out['surf_stats'] = self._surface_stats(fused, gt8)
+        if opts.mesh:
+            out['mesh_verts'], out['mesh_faces'], out['mesh_counts'] = self._mesh(fused)
 
     def _mesh(self, fused):
         """Marching-cubes mesh of fused [B,n^3] at TEST.MESH_THRESH -> (mesh_verts, mesh_faces, mesh_counts).  Every buffer
@@ -712,6 +712,15 @@ def unc_thresholds(cfg):
     if len(th) > 4 or not all(math.isfinite(t) and t >= 0 for t in th):
         raise ValueError('TEST.UNC_THRESH must hold at most 4 finite values >= 0, got %r' % (cfg.TEST.UNC_THRESH,))
     return th
+
+
+def lr_thresh(cfg):
+    """TEST.LR_THRESH as a float: the left-right consistency tolerance in input pixels, finite and >= 0; anything else is a
+    ValueError."""
+    tau = float(cfg.TEST.LR_THRESH)
+    if not (math.isfinite(tau) and tau >= 0):
+        raise ValueError('TEST.LR_THRESH must be finite and >= 0, got %r' % cfg.TEST.LR_THRESH)
+    return tau
 
 
 def mesh_thresh(cfg):
@@ -748,6 +757,10 @@ class Stereo2Point(_StereoBase):
     distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
     (include/s3d.h, s3d_chamfer_eval)."""
 
+    HEAD_OUTPUTS = ('disp_left', 'disp_right', 'points')
+    GT_OUTPUT = 'point_stats'
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty')
+
     def __init__(self, cfg):
         super().__init__(cfg)
         self.point_decoder = _PointDecoder(cfg)
@@ -765,7 +778,6 @@ class Stereo2Point(_StereoBase):
             raise ValueError('gt must be float32, got %s' % gt.dtype)
         if gt.device != left.device:
             raise ValueError('gt must be on %s (the images\' device), got %s' % (left.device, gt.device))
-        fscore_thresholds(self.cfg)                    # a bad TEST.FSCORE_THRESH fails before anything is launched
         return gt.contiguous()
 
     def _pack_head(self, P, dc, dev):
@@ -776,17 +788,12 @@ class Stereo2Point(_StereoBase):
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
     def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False):
-        self._check_mesh(mesh)                         # ValueError: the mesh is a Stereo2Voxel output
-        if uncertainty:
-            unc_thresholds(self.cfg)
-        left, right = self._check_inputs(left, right)
-        return self._forward_impl(left, right, self._check_gt(gt, left), disp_gt=self._check_disp_gt(disp_gt, left),
-                                  lr_check=lr_check, uncertainty=uncertainty)
+        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, False, mesh))
 
-    def _forward_impl(self, left, right, gt=None, disp_gt=None, lr_check=False, uncertainty=False):
+    def _head(self, left, right, gt, disp, opts, out):
+        """The point head: adds points and point_stats (with gt) to `out`."""
         cfg = self.cfg
         B = left.shape[0]
-        disp, _, dstats, lr, unc = self._disparity(left, right, disp_gt, lr_check, uncertainty)
         x = self._latent(left, right, disp)
         L = cfg.NETWORK.LATENT_HW
         if x.shape[2] != L or x.shape[3] != L:
@@ -806,12 +813,9 @@ class Stereo2Point(_StereoBase):
         pts = self._buf('pts', (B, 1, 1, 1, pad_to(npts * 3)), torch.float32)
         self._conv('pt_fc2', y, out=pts)
         points = pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3)
-        out = (disp[:B].unsqueeze(1), disp[B:].unsqueeze(1), points)
+        out['points'] = points
         if gt is not None:
-            out += (self._point_stats(points, gt),)
-        if disp_gt is not None:
-            out += (dstats,)
-        return out + (lr or ()) + (unc or ())
+            out['point_stats'] = self._point_stats(points, gt)
 
     def _point_stats(self, points, gt):
         """Chamfer search of points [B,N,3] against gt [B,M,3] + the metric counters -> point_stats int64 [B,2,3+T], zeroed

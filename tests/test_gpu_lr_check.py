@@ -257,10 +257,14 @@ def test_micro_batched_lr_matches_unsplit():
 def test_lr_thresh_validation():
     cfg, model = _model('Stereo2Voxel', 'concat', 'bf16')
     args, _ = _inputs(cfg, 'Stereo2Voxel', 1, seed=0)
+    n0 = lib.launches()
     for bad in (-0.5, NAN, INF):
         cfg.TEST.LR_THRESH = bad
         with pytest.raises(ValueError):
             model(*args, lr_check=True)
+        with pytest.raises(ValueError):
+            model.graphed(*args, lr_check=True)
+    assert lib.launches() == n0                                     # rejected before anything is launched
 
 
 @pytest.mark.parametrize('name', ['Stereo2Voxel', 'Stereo2Point'])

@@ -185,16 +185,19 @@ _NS = _TV * (3 + 3 * _F)
 
 
 class _FakeVoxel:
-    """Stands in for Stereo2Voxel in test_voxel: seeded per-sample outputs in the forward's tuple layout."""
+    """Stands in for Stereo2Voxel in test_voxel: seeded per-sample outputs in the forward's tuple layout for the keywords
+    it is given (disp_stats when disp_gt= is passed at all: the driver's synthetic GT disparity is stubbed out)."""
 
-    def __call__(self, left, right, gt, disp_gt=None, lr_check=False, surface=False):
+    def __call__(self, left, right, gt, lr_check=False, surface=False, **kw):
+        assert set(kw) <= {'disp_gt'}
         B = left.shape[0]
         ids = [int(v) for v in left[:, 0, 0, 0].tolist()]
         g = [torch.Generator().manual_seed(9000 + i) for i in ids]
         iou = torch.stack([torch.randint(0, 1 << 15, (_TV, 2), generator=x) for x in g])
         ds = torch.stack([torch.randint(0, 1 << 20, (2, 2 + _TD), generator=x) for x in g])
         ls = torch.stack([torch.randint(0, 1 << 20, (2, 3 + _TD), generator=x) for x in g])
-        out = (None, None, None, iou, ds, None, ls)
+        out = (None, None, None) + ((iou,) if gt is not None else ()) + ((ds,) if 'disp_gt' in kw else ())
+        out += (None, ls) if lr_check else ()
         if surface:
             ss = []
             for i, x in zip(ids, g):
@@ -225,7 +228,7 @@ def _patch_inputs(monkeypatch):
     monkeypatch.setattr(T, '_disp_gt', lambda pairs, H, W, device: None)
 
 
-def test_driver_vector_layout(monkeypatch):
+def test_driver_vector_layout_in_forward_order(monkeypatch):
     _patch_inputs(monkeypatch)
     cfg, model = _cfg(), _FakeVoxel()
     base = T.test_voxel(cfg, model, 7, 3, device='cpu', eval_disp=True, eval_lr=True)
