@@ -100,3 +100,7 @@ __C.TEST.FSCORE_THRESH = [0.01]
 # iso-level of the exported mesh (forward(..., mesh=True), runner.py --test --save-meshes): marching cubes over the predicted
 # occupancy, a voxel is inside when its value is >= this; finite and in (0, 1]
 __C.TEST.MESH_THRESH = 0.5
+# bins of the threshold-free occupancy evaluation (forward(..., curves=True), runner.py --test --curves): the IoU and precision-
+# recall curves are exact at the thresholds k / CURVE_BINS, and the calibration merges them into min(CURVE_BINS, 16) bins;
+# an int, a power of two in [2, 1024]
+__C.TEST.CURVE_BINS = 256

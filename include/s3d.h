@@ -340,6 +340,19 @@ int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int B, int n, 
 int s3d_voxel_mesh_bounds(int n, int* max_verts, int* max_faces);    /* 3 (n+1)(n+2)^2 and 5 (n+1)^3 */
 int s3d_voxel_mesh(const float* vol, int B, int n, float t, float* verts, int max_verts, int* faces, int max_faces,
                    int* counts, void* stream);
+/* Threshold-free occupancy evaluation: per-sample probability histograms split by GT label, and BCE / Brier sums, from which
+ * the IoU at every threshold k / K, the precision-recall curve and the calibration follow.  fused fp32 [B,nvox], gt uint8
+ * [B,nvox], 1 <= nvox <= 2^24, 0 <= B; K a power of two in [2, 1024].  Per voxel: v = fused clamped as for s3d_voxel_mesh
+ * (NaN -> 0, then min(max(v, 0), 1)), g = (gt != 0), bin k = min(floor(v * K), K - 1) in fp32 (v * K is exact, so bin >= k
+ * exactly when v >= k / K), q(x) = round-half-even(x * 2^20) in fp64.  Per sample b (written, not added; no zeroing needed):
+ *   hist int64 [B,3,K]: row 0 the voxels with g = 0 in bin k, row 1 those with g = 1, row 2 sum q(v) over bin k (both);
+ *   loss int64 [B,2]:   sum q(bce), bce = -max(log(v), -100) if g else -max(log(1 - v), -100) (PyTorch's BCELoss clamp;
+ *                       1 - v and log in fp64 on the fp32 v), then sum q((v - g)^2) (fp64).
+ * Overflow: a voxel adds at most 100 * 2^20 to a counter, so at n = 32 (32768 voxels) a sample's counters stay below 2^42
+ * and an int64 sum over samples holds more than 2M samples even if every voxel hits the BCE clamp.  One kernel, one cluster
+ * of blocks per sample reducing through distributed shared memory: integer sums, no global atomics, deterministic. */
+int s3d_occupancy_curves(const float* fused, const uint8_t* gt, int B, int nvox, int K, int64_t* hist, int64_t* loss,
+                         void* stream);
 
 /* --- Chamfer distance (row C; replaces extensions/chamfer_dist, README.md:62-65) ------- */
 /* xyz1 fp32 [B,N,3], xyz2 fp32 [B,M,3] -> dist1 fp32 [B,N], idx1 int32 [B,N] (nearest in

@@ -36,6 +36,9 @@ def get_args():
     p.add_argument('--save-meshes', metavar='DIR', default=None,
                    help='Stereo2Voxel: also write the marching-cubes mesh of each prediction (at TEST.MESH_THRESH) and of its '
                         'GT occupancy as DIR/%%06d.obj and DIR/%%06d_gt.obj, numbered by sample')
+    p.add_argument('--curves', action='store_true',
+                   help='Stereo2Voxel: also evaluate the occupancy probabilities in TEST.CURVE_BINS bins and report the IoU '
+                        'and precision-recall curves over every bin threshold, BCE, Brier and calibration as occupancy_curves')
     return p.parse_args()
 
 
@@ -88,6 +91,8 @@ def main():
         sys.exit('--surface evaluates voxel surfaces: Stereo2Voxel only')
     if args.save_meshes is not None and args.model != 'Stereo2Voxel':
         sys.exit('--save-meshes meshes the voxel occupancy: Stereo2Voxel only')
+    if args.curves and args.model != 'Stereo2Voxel':
+        sys.exit('--curves evaluates the voxel occupancy: Stereo2Voxel only')
     if not torch.cuda.is_available():
         sys.exit('runner.py --test needs a CUDA device (sm_100a); there is no CPU fallback.')
     from stereo_3d_reconstruction_b200 import models
@@ -109,7 +114,7 @@ def main():
     # one stats vector: the head's statistics, then the disparity counters of the same forwards (core/test.py::stats_layout)
     ev = dict(eval_disp=True, eval_lr=args.lr_check, eval_unc=args.uncertainty)
     if args.model == 'Stereo2Voxel':
-        ev.update(eval_surface=args.surface)
+        ev.update(eval_surface=args.surface, eval_curves=args.curves)
         stats = T.test_voxel(cfg, model, n, bs, rank, world, mesh_dir=args.save_meshes, **ev).cpu()
     else:
         ev.update(eval_points=True)
@@ -125,6 +130,8 @@ def main():
         res['uncertainty'] = T.unc_summary(b['uncertainty'], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH, npix, b['disparity'])
     if 'surface' in b:
         res['surface'] = T.surface_summary(b['surface'], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH, res['n_samples'])
+    if 'curves' in b:
+        res['occupancy_curves'] = T.curves_summary(b['curves'], cfg.TEST.CURVE_BINS, res['n_samples'])
     if 'points' in b:
         res['points'] = T.points_summary(b['points'], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
                                          cfg.CONST.N_GT_POINTS)

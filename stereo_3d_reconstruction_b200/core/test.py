@@ -20,12 +20,18 @@ TEST.FSCORE_THRESH:
     sum q(d), sum q(sqrt d), n_out, count(sqrt d < t) per t                                    (int64)
     sum_b q(F_b(t)),  F_b = 2 P R / (P + R) (0 when both are 0), P = count_pred / N, R = count_gt / M   (int64)
 with q(x) = round-half-even(x * 2^32); F_b is computed elementwise in fp64 on the device, so the vector stays integer.
-With eval_surface=True (test_voxel) the voxel-surface counters of the same forwards come last (models.py,
+With eval_surface=True (test_voxel) the voxel-surface counters of the same forwards follow (models.py,
 Stereo2Voxel._surface_stats), per t in TEST.VOXEL_THRESH (surface_block):
     n_both, sum_b q(CD_L2_b), sum_b q(CD_L1_b), then per tau in TEST.FSCORE_THRESH sum_b q(P_b), sum_b q(R_b), sum_b q(F_b)
                                                                                                (int64)
-again computed per batch in fp64 on the device.  stats_layout() declares these blocks and their order, split_stats() cuts a
-vector into them.
+again computed per batch in fp64 on the device.
+With eval_curves=True (test_voxel) the threshold-free occupancy counters of the same forwards follow (models.py,
+Stereo2Voxel._occupancy_curves; K = TEST.CURVE_BINS, curves_block):
+    n_empty per bin (K), n_occ per bin (K), sum q20(v) per bin (K), sum q20(BCE), sum q20(Brier),
+    sum_b q(IoU_b(k / K)) per k (K)                                                           (int64)
+with q20(x) = round-half-even(x * 2^20) (include/s3d.h, s3d_occupancy_curves) and the per-sample IoU at every bin threshold
+computed per batch in fp64 on the device; a sample whose GT and prediction are both empty at t has IoU 1 there.
+stats_layout() declares these blocks and their order, split_stats() cuts a vector into them.
 With mesh_dir (test_voxel) the same forwards also return the marching-cubes mesh of the prediction (models.py,
 Stereo2Voxel._mesh), and each sample of the rank's shard is written as mesh_dir/%06d.obj (predicted) and %06d_gt.obj (the GT
 occupancy, meshed by the same kernel at t = 0.5), numbered by global sample id; the stats vector does not change.
@@ -37,12 +43,13 @@ import torch
 import torch.distributed as dist
 
 from .. import ops
-from ..models import Stereo2Point, Stereo2Voxel, fscore_thresholds, mesh_thresh, unc_thresholds
+from ..models import Stereo2Point, Stereo2Voxel, curve_bins, fscore_thresholds, mesh_thresh, unc_thresholds
 from ..utils import synthetic
 
 _FX = float(1 << 40)
 _DISP_FX = float(1 << 16)
 _PT_FX = float(1 << 32)
+_OCC_FX = float(1 << 20)
 
 
 def shard_range(n_total, rank, world):
@@ -213,6 +220,54 @@ def surface_summary(block, voxel_thresh, fscore_thresh, n_samples):
             'by_thresh': per}
 
 
+def curves_block(occ_hist, occ_loss):
+    """Per-batch increment of the curves block from the forward's occ_hist int64 [B,3,K] and occ_loss int64 [B,2] -> int64
+    [4K + 2]: the histogram rows and the loss sums summed over the batch, then per k sum_b q(IoU_b(k / K)), q(x) =
+    round-half-even(x * 2^32), in fp64.  IoU_b(t_k) = I / U with I = sum_{j >= k} n_occ_j, U = sum_{j >= k} (n_empty_j +
+    n_occ_j) + G_b - I, G_b the sample's occupied voxels; U = 0 (GT and prediction both empty) counts as IoU 1."""
+    empty, occ = occ_hist[:, 0], occ_hist[:, 1]
+    inter = occ.flip(1).cumsum(1).flip(1)
+    union = (empty + occ).flip(1).cumsum(1).flip(1) + occ.sum(1, keepdim=True) - inter
+    iou = torch.where(union > 0, inter.double() / union.clamp(min=1).double(), torch.ones_like(inter, dtype=torch.float64))
+    return torch.cat([occ_hist.sum(0).flatten(), occ_loss.sum(0), torch.round(iou * _PT_FX).to(torch.int64).sum(0)])
+
+
+def curves_summary(block, K, n_samples):
+    """Curves counters (int64 [4K + 2], as curves_block sums them) -> dict.  thresholds t_k = k / K; iou: the pooled IoU
+    sum I_k / sum U_k at every t_k (1 where U = 0, as per sample) and mean_iou: the mean of the per-sample IoUs; best /
+    best_mean: the first t_k of the largest iou / mean_iou; ap = sum_k (R_k - R_{k+1}) P_k with R_k = I_k / G, P_k = I_k /
+    Pred_k, R_K = 0 (average precision over the voxels' scores quantised to the bins; None when the GT is empty); bce and
+    brier: means per voxel; ece = sum_m |S_m - O_m| / N over M = min(K, 16) equal-width bins merging K / M histogram bins
+    (S_m the summed predictions, O_m the occupied voxels, N all voxels) and reliability: per merged bin {count, confidence
+    S_m / count, frequency O_m / count} (None for an empty bin)."""
+    v = [int(x) for x in block.tolist()]
+    assert len(v) == 4 * K + 2
+    empty, occ, sq, (bce, brier), miou = v[:K], v[K:2 * K], v[2 * K:3 * K], v[3 * K:3 * K + 2], v[3 * K + 2:]
+    inter, pred = [0] * (K + 1), [0] * (K + 1)
+    for k in range(K - 1, -1, -1):
+        inter[k], pred[k] = inter[k + 1] + occ[k], pred[k + 1] + empty[k] + occ[k]
+    G, N, n = inter[0], pred[0], n_samples
+    thresholds = [k / K for k in range(K)]
+    iou = [inter[k] / (pred[k] + G - inter[k]) if pred[k] + G - inter[k] else 1.0 for k in range(K)]
+    mean_iou = [m / _PT_FX / n if n else 0.0 for m in miou]
+    kb, km = max(range(K), key=iou.__getitem__), max(range(K), key=mean_iou.__getitem__)
+    ap = sum(occ[k] / G * (inter[k] / pred[k]) for k in range(K) if occ[k]) if G else None
+    M = min(K, 16)
+    w = K // M
+    ece, rel = 0.0, []
+    for m in range(M):
+        bins = range(m * w, (m + 1) * w)
+        cnt = sum(empty[k] + occ[k] for k in bins)
+        conf, obs = sum(sq[k] for k in bins) / _OCC_FX, sum(occ[k] for k in bins)
+        ece += abs(conf - obs)
+        rel.append({'count': cnt, 'confidence': conf / cnt if cnt else None, 'frequency': obs / cnt if cnt else None})
+    return {'n_samples': n, 'n_voxels': N, 'bins': K, 'thresholds': thresholds, 'iou': iou, 'mean_iou': mean_iou,
+            'best': {'threshold': thresholds[kb], 'iou': iou[kb]},
+            'best_mean': {'threshold': thresholds[km], 'mean_iou': mean_iou[km]}, 'ap': ap,
+            'bce': bce / _OCC_FX / N if N else 0.0, 'brier': brier / _OCC_FX / N if N else 0.0,
+            'ece': ece / N if N else 0.0, 'reliability': rel}
+
+
 def write_obj(path, verts, faces):
     """Plain OBJ of verts fp32 [V,3] and 0-based faces int [F,3]: `v x y z` with %.9g (an fp32 value reads back exactly),
     then `f a b c` with 1-based ids."""
@@ -236,10 +291,11 @@ def _disp_gt(pairs, H, W, device):
     return torch.cat([synthetic.disparity_gt(p[2], H, W) for p in pairs]).to(device)
 
 
-def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eval_surface=False, eval_points=False):
+def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eval_surface=False, eval_points=False,
+                 eval_curves=False):
     """The driver's int64 stats vector for `model` ('Stereo2Voxel' / 'Stereo2Point') as ordered blocks [(name, length)]: the
-    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', then 'surface'
-    (Stereo2Voxel) / 'points' (Stereo2Point), each present when its evaluation is on (module docstring).  ValueError on an
+    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', then 'surface' and
+    'curves' (Stereo2Voxel) / 'points' (Stereo2Point), each present when its evaluation is on (module docstring).  ValueError on an
     evaluation without the disparity counters it needs or on a bad cfg.TEST threshold: raised before any forward."""
     if eval_lr and not eval_disp:
         raise ValueError('eval_lr=True needs eval_disp=True')
@@ -255,6 +311,8 @@ def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eva
         blocks.append(('uncertainty', 2 * len(unc_thresholds(cfg)) * (3 + T)))
     if eval_surface:
         blocks.append(('surface', len(cfg.TEST.VOXEL_THRESH) * (3 + 3 * len(fscore_thresholds(cfg)))))
+    if eval_curves:
+        blocks.append(('curves', 4 * curve_bins(cfg) + 2))
     if eval_points:
         F = len(fscore_thresholds(cfg))
         blocks.append(('points', 2 * (3 + F) + F))
@@ -278,21 +336,22 @@ def _add_disp_blocks(blocks, out):
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_unc=False, eval_surface=False, mesh_dir=None):
+               eval_unc=False, eval_surface=False, mesh_dir=None, eval_curves=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
     eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
     eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones.
-    eval_surface: the same forward also evaluates the voxel surfaces; their block comes last.
+    eval_surface: the same forward also evaluates the voxel surfaces; their block follows the uncertainty one.
+    eval_curves: the same forward also returns the occupancy histograms and loss sums; their block comes last.
     mesh_dir: the same forward also meshes the prediction; the meshes and the GT's are written there (module docstring).
     The vector's blocks: stats_layout(cfg, 'Stereo2Voxel', ...)."""
-    layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface)
+    layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface, eval_curves=eval_curves)
     if mesh_dir is not None:
         mesh_thresh(cfg)                                # ValueError on a bad TEST.MESH_THRESH, before any forward
         os.makedirs(mesh_dir, exist_ok=True)
     kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc), ('surface', eval_surface),
-                                ('mesh', mesh_dir is not None)) if on}    # the options that are on, and only those
+                                ('mesh', mesh_dir is not None), ('curves', eval_curves)) if on}    # the options that are on
     names = Stereo2Voxel.output_names(gt=True, disp_gt=eval_disp, **kw)
     stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
     blocks = split_stats(stats, layout)
@@ -312,6 +371,8 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             _add_disp_blocks(blocks, out)
             if eval_surface:
                 blocks['surface'] += surface_block(out['surf_stats'], cfg.CONST.N_VOX)
+            if eval_curves:
+                blocks['curves'] += curves_block(out['occ_hist'], out['occ_loss'])
             if mesh_dir is not None:
                 save_meshes(mesh_dir, ids, (out['mesh_verts'], out['mesh_faces'], out['mesh_counts']), gt)
             iou = out['iou_counts']

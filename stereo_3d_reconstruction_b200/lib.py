@@ -85,6 +85,7 @@ SIGNATURES = {
     's3d_voxel_surface_eval': ([_vp, _vp, _i, _i, ctypes.POINTER(_f), _i, ctypes.POINTER(_i), _i, _vp, _vp, _i64, _vp], _i),
     's3d_voxel_mesh_bounds': ([_i, ctypes.POINTER(_i), ctypes.POINTER(_i)], _i),
     's3d_voxel_mesh': ([_vp, _i, _i, _f, _vp, _i, _vp, _i, _vp, _vp], _i),
+    's3d_occupancy_curves': ([_vp, _vp, _i, _i, _i, _vp, _vp, _vp], _i),
     's3d_chamfer_forward': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp], _i),
     's3d_chamfer_workspace_bytes': ([_i, _i, _i], ctypes.c_int64),
     's3d_chamfer_forward_ws': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _i64, _vp], _i),

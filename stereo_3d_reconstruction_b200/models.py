@@ -36,12 +36,14 @@ OPTIONAL_OUTPUTS = (('disp_gt', ('disp_stats',)),
                     ('lr_check', ('lr_mask', 'lr_stats')),
                     ('uncertainty', ('disp_std', 'unc_stats')),
                     ('surface', ('surf_stats',)),
-                    ('mesh', ('mesh_verts', 'mesh_faces', 'mesh_counts')))
+                    ('mesh', ('mesh_verts', 'mesh_faces', 'mesh_counts')),
+                    ('curves', ('occ_hist', 'occ_loss')))
 _VOXEL_ONLY = {'surface': 'surface=True evaluates voxel surfaces: Stereo2Voxel only',
-               'mesh': 'mesh=True meshes the voxel occupancy: Stereo2Voxel only'}
+               'mesh': 'mesh=True meshes the voxel occupancy: Stereo2Voxel only',
+               'curves': 'curves=True evaluates the voxel occupancy: Stereo2Voxel only'}
 
 # The options of one forward, checked (_StereoBase._check_args): what the stages branch on and part of the graph key.
-Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty surface mesh')
+Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty surface mesh curves')
 
 
 def _conv_bn2d(cin, cout, k, s, p):
@@ -463,14 +465,16 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False,
+                curves=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
         ~0.12 ms per aggregation layer), so the graph only removes the launch gaps.
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
-        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
+        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh,
+                                                          curves)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
@@ -483,11 +487,13 @@ class _StereoBase(nn.Module):
 
     # ---- outputs and their checks --------------------------------------------------------------
     @classmethod
-    def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False):
+    def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False,
+                     curves=False):
         """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt: whether the tensor is given):
         the head's outputs, the gt output, then the groups of OPTIONAL_OUTPUTS that are on.  ValueError on an option the
         class does not have."""
-        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'surface': surface, 'mesh': mesh}
+        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'surface': surface, 'mesh': mesh,
+              'curves': curves}
         names = cls.HEAD_OUTPUTS + ((cls.GT_OUTPUT,) if gt else ())
         for opt, outs in OPTIONAL_OUTPUTS:
             if on[opt]:
@@ -496,20 +502,25 @@ class _StereoBase(nn.Module):
                 names += outs
         return names
 
-    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh):
+    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh, curves):
         """The one check of forward() / graphed()'s arguments, before anything is launched: first the options (which the
         class has, what they need), then the cfg.TEST thresholds of the enabled outputs, then the tensors.
         -> (left, right, gt, disp_gt) as the forward takes them and the options value: an Options of bools."""
-        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh))
+        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh),
+                       bool(curves))
         self.output_names(**opts._asdict())                   # ValueError on an option this class does not have
         if opts.surface and not opts.gt:
             raise ValueError('surface=True needs the GT occupancy gt')
+        if opts.curves and not opts.gt:
+            raise ValueError('curves=True needs the GT occupancy gt')
         if opts.uncertainty:
             unc_thresholds(self.cfg)
         if opts.surface or (opts.gt and self.GT_OUTPUT == 'point_stats'):     # the surface and point-cloud F-scores
             fscore_thresholds(self.cfg)
         if opts.mesh:
             mesh_thresh(self.cfg)
+        if opts.curves:
+            curve_bins(self.cfg)
         if opts.lr_check:
             lr_thresh(self.cfg)
         left, right = self._check_inputs(left, right)
@@ -562,7 +573,8 @@ class Stereo2Voxel(_StereoBase):
     """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W],
     voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64
     [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, surf_stats int64 [B,T,2,3+F]][, mesh_verts fp32
-    [B,max_verts,3], mesh_faces int32 [B,max_faces,3], mesh_counts int32 [B,2]]).
+    [B,max_verts,3], mesh_faces int32 [B,max_faces,3], mesh_counts int32 [B,2]][, occ_hist int64 [B,3,K], occ_loss int64
+    [B,2]]).
     Outputs are views of the module's workspace: clone to keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views
     (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; uncertainty=True: the standard
     deviation of each pixel's soft-argmin distribution in input pixels, and counters over the pixels it marks as confident
@@ -574,11 +586,15 @@ class Stereo2Voxel(_StereoBase):
     mesh=True (with or without gt): the marching-cubes mesh of voxels at the iso-level TEST.MESH_THRESH, a closed,
     outward-oriented triangle mesh in the unit cube the grid spans; per sample mesh_counts = (n_verts, n_faces) and only the
     first rows of mesh_verts / mesh_faces (0-based ids) are written; (max_verts, max_faces) = ops.voxel_mesh_bounds(N_VOX)
-    (include/s3d.h, s3d_voxel_mesh; one more launch)."""
+    (include/s3d.h, s3d_voxel_mesh; one more launch).
+    curves=True (needs gt): the threshold-free evaluation of voxels against gt in K = TEST.CURVE_BINS probability bins; per
+    sample occ_hist = [voxels with gt = 0 per bin, voxels with gt != 0 per bin, sum q(v) per bin] and occ_loss = [sum q(BCE),
+    sum q(Brier)], q(x) = round-half-even(x * 2^20): the IoU and precision-recall curves at the thresholds k / K, the
+    calibration and the test losses follow from them (include/s3d.h, s3d_occupancy_curves; one more launch)."""
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'voxels')
     GT_OUTPUT = 'iou_counts'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'surface', 'mesh')
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'surface', 'mesh', 'curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -617,8 +633,10 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False):
-        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh)
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False,
+                curves=False):
+        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh,
+                                                          curves)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
@@ -631,7 +649,8 @@ class Stereo2Voxel(_StereoBase):
         return self._forward_impl(left, right, gt, disp_gt, opts)
 
     def _head(self, left, right, gt, disp, opts, out):
-        """The voxel head: adds voxels, iou_counts (with gt), surf_stats (surface) and the mesh (mesh) to `out`."""
+        """The voxel head: adds voxels, iou_counts (with gt), surf_stats (surface), the mesh (mesh) and occ_hist / occ_loss
+        (curves) to `out`."""
         cfg = self.cfg
         B, H, W = self._bhw(left)
         nv = cfg.CONST.N_VOX
@@ -680,6 +699,16 @@ class Stereo2Voxel(_StereoBase):
             out['surf_stats'] = self._surface_stats(fused, gt8)
         if opts.mesh:
             out['mesh_verts'], out['mesh_faces'], out['mesh_counts'] = self._mesh(fused)
+        if opts.curves:
+            out['occ_hist'], out['occ_loss'] = self._occupancy_curves(fused, gt8)
+
+    def _occupancy_curves(self, fused, gt8):
+        """Probability histograms and loss sums of fused [B,n^3] against gt8 [B,n^3] -> (occ_hist int64 [B,3,K], occ_loss int64
+        [B,2]), K = TEST.CURVE_BINS.  The kernel writes every counter (nothing to zero) into workspace buffers: no allocation on
+        this path."""
+        K, B = curve_bins(self.cfg), fused.shape[0]
+        return ops.occupancy_curves(fused, gt8, K, out=(self._buf('occ_hist', (B, 3, K), torch.int64),
+                                                        self._buf('occ_loss', (B, 2), torch.int64)))
 
     def _mesh(self, fused):
         """Marching-cubes mesh of fused [B,n^3] at TEST.MESH_THRESH -> (mesh_verts, mesh_faces, mesh_counts).  Every buffer
@@ -736,6 +765,15 @@ def mesh_thresh(cfg):
     return t
 
 
+def curve_bins(cfg):
+    """TEST.CURVE_BINS: the bins of the threshold-free occupancy evaluation, an int (not a bool) that is a power of two in
+    [2, 1024] (the curves are exact at the thresholds k / CURVE_BINS); anything else is a ValueError."""
+    k = cfg.TEST.get('CURVE_BINS')
+    if not (isinstance(k, int) and not isinstance(k, bool) and 2 <= k <= 1024 and k & (k - 1) == 0):
+        raise ValueError('TEST.CURVE_BINS must be an int, a power of two in [2, 1024], got %r' % (k,))
+    return k
+
+
 def fscore_thresholds(cfg):
     """TEST.FSCORE_THRESH as floats: at most 8 (the kernel's limit) Euclidean distances in the points' units, each finite
     and > 0; anything else is a ValueError."""
@@ -787,8 +825,8 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False):
-        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, False, mesh))
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False, curves=False):
+        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, False, mesh, curves))
 
     def _head(self, left, right, gt, disp, opts, out):
         """The point head: adds points and point_stats (with gt) to `out`."""

@@ -628,3 +628,44 @@ def voxel_mesh(vol, t, out=None):
     if B:
         _lib.count_launch(1)                   # voxel_mesh_kernel
     return verts, faces, counts
+
+
+def occupancy_curves(fused, gt8, K, out=None):
+    """Threshold-free occupancy evaluation (include/s3d.h, s3d_occupancy_curves).  fused fp32 and gt8 uint8 (nonzero =
+    occupied) of one shape [B, ...], a sample holding 1 to 2^24 voxels; K a power of two in [2, 1024].  -> (hist int64
+    [B,3,K], loss int64 [B,2]): per sample the voxels with gt = 0 / gt = 1 in each bin k = min(floor(v * K), K - 1) of the
+    clamped fused value v and sum q(v) per bin, then sum q(bce) and sum q((v - g)^2), q(x) = round-half-even(x * 2^20).  out:
+    the two output tensors, written (not added to).  One kernel launch."""
+    _chk(fused, gt8)
+    if fused.dtype != torch.float32 or gt8.dtype != torch.uint8:
+        raise ValueError('occupancy_curves: fused must be float32 and gt8 uint8, got %s / %s' % (fused.dtype, gt8.dtype))
+    if fused.shape != gt8.shape or fused.dim() < 2:
+        raise ValueError('occupancy_curves: expected fused and gt8 of one shape [B, ...], got %s / %s'
+                         % (tuple(fused.shape), tuple(gt8.shape)))
+    if gt8.device != fused.device:
+        raise ValueError('occupancy_curves: gt8 must be on %s, got %s' % (fused.device, gt8.device))
+    B = fused.shape[0]
+    nvox = math.prod(fused.shape[1:])
+    if not 1 <= nvox <= 1 << 24:
+        raise ValueError('occupancy_curves: a sample must hold 1 to 2^24 voxels, got %d' % nvox)
+    if not (isinstance(K, int) and not isinstance(K, bool) and 2 <= K <= 1024 and K & (K - 1) == 0):
+        raise ValueError('occupancy_curves: K must be a power of two in [2, 1024], got %r' % (K,))
+    want = ((B, 3, K), (B, 2))
+    if out is None:
+        out = tuple(torch.empty(s, dtype=torch.int64, device=fused.device) for s in want)
+    else:
+        out = tuple(out)
+        if len(out) != 2:
+            raise ValueError('occupancy_curves: out must hold (hist, loss)')
+        _chk(*out)
+        for o, s in zip(out, want):
+            if o.dtype != torch.int64 or tuple(o.shape) != s or o.device != fused.device:
+                raise ValueError('occupancy_curves: out tensors must be int64 %s on %s, got %s'
+                                 % (list(want), fused.device, [(str(o.dtype), tuple(o.shape), str(o.device)) for o in out]))
+    hist, loss = out
+    rc = _lib.load().s3d_occupancy_curves(fused.data_ptr(), gt8.data_ptr(), B, nvox, K, hist.data_ptr(), loss.data_ptr(),
+                                          _stream())
+    _lib.check(rc, 's3d_occupancy_curves')
+    if B:
+        _lib.count_launch(1)                   # occupancy_curves_kernel
+    return hist, loss
