@@ -104,3 +104,10 @@ __C.TEST.MESH_THRESH = 0.5
 # recall curves are exact at the thresholds k / CURVE_BINS, and the calibration merges them into min(CURVE_BINS, 16) bins;
 # an int, a power of two in [2, 1024]
 __C.TEST.CURVE_BINS = 256
+# nearest-neighbour distance histograms (forward(..., fscore_curves=True), runner.py --test --fscore-curves): edges
+# e_k = DIST_MAX * k / DIST_BINS, k = 1..DIST_BINS (computed in fp64, rounded once to fp32), in the points' units (the unit
+# cube for voxel surfaces); the F-score, accuracy and completeness follow at every e_k.  The defaults give 1e-3 bins, and
+# e_10 is exactly fp32(0.01), the default FSCORE_THRESH.  DIST_BINS: an int in [1, 1024]; DIST_MAX: finite and > 0, with
+# strictly increasing rounded edges
+__C.TEST.DIST_BINS = 128
+__C.TEST.DIST_MAX = 0.128

@@ -325,6 +325,16 @@ int s3d_fuse_views(const void* score, int64_t score_stride, const void* vol, int
 int64_t s3d_voxel_surface_workspace_bytes(int B, int T, int n);
 int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
                            const int* kbound, int F, long long* stats, void* workspace, int64_t workspace_bytes, void* stream);
+/* s3d_voxel_surface_eval (the same stats, bit for bit; s3d_voxel_surface_eval is this call with K = 0) + the distance
+ * histogram of every surface point, from the same pass.  hist_kbound: K HOST ints, 0 <= K <= 1024, non-decreasing, each in
+ * [0, 3 (2n)^2 + 1] (repeats give empty bins); from Euclidean edges e_k in unit-cube units, kb_k = voxel_kbound(e_k, n) as
+ * for the F-score.  hist int64 [B,T,2,K+1] is ADDED to (caller zeroes; may be NULL when K = 0): per sample, t and direction,
+ * bin = the number of kb_j <= s, so bin 0 holds s < kb_0 and the cumulative count over bins < k equals count(s < kb_k), the
+ * F-score counter at that bound.  When the other surface is empty its points all go to bin K (the stats count them in n_pts
+ * only), so every row sums to n_pts.  No extra launch; the counts are integers and do not depend on the launch order. */
+int s3d_voxel_surface_eval_hist(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
+                                const int* kbound, int F, long long* stats, void* workspace, int64_t workspace_bytes,
+                                void* stream, const int* hist_kbound, int K, long long* hist);
 /* Triangle mesh of an occupancy grid: marching cubes at iso-level t, closed and consistently oriented.
  * vol fp32 [B,n,n,n] (sample b is vol[b,k,j,i], x along i), 1 <= n <= 64, padded with one layer of 0 on every side; the
  * padded field is clamped (NaN -> 0, then min(max(v, 0), 1)) and a corner is inside when v >= t; t finite, 0 < t <= 1, so
@@ -384,6 +394,17 @@ int s3d_chamfer_forward_ws(const float* xyz1, const float* xyz2, float* dist1, i
 int s3d_chamfer_eval(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2, int32_t* idx2,
                      int B, int N, int M, const float* tau, int T, long long* stats,
                      void* workspace, int64_t workspace_bytes, void* stream);
+/* s3d_chamfer_eval (the same dist / idx / stats, bit for bit; s3d_chamfer_eval is this call with K = 0) + the distance
+ * histogram of every point, from the same kernel.  edges: K HOST values e_0 < ... < e_{K-1}, 0 <= K <= 1024, each finite
+ * and > 0, in the points' units.  hist int64 [B,2,K+1] is ADDED to (caller zeroes; may be NULL when K = 0): per sample and
+ * direction, a point with d in range goes to bin = the number of edges e_j <= sqrt_rn(d) (the fp32 value the tau counters
+ * compare), so bin 0 holds sqrt_rn(d) < e_0; bin K also takes every out-of-range point.  Each row sums to N (direction 0)
+ * or M (direction 1), and the cumulative count over bins < k equals count(sqrt_rn(d) < e_k), the tau counter at tau = e_k.
+ * The edges go to the kernel by value (4 KB of parameters); no extra launch, integer counts that do not depend on the
+ * launch order. */
+int s3d_chamfer_eval_hist(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2, int32_t* idx2,
+                          int B, int N, int M, const float* tau, int T, long long* stats,
+                          void* workspace, int64_t workspace_bytes, void* stream, const float* edges, int K, long long* hist);
 
 /* Measurement aid (bench.py): a launch of independent fp32 FMA chains that is bound by the FMA issue rate only;
  * *fma_count (HOST) receives the number of thread-level FMAs the launch executes.  Timed with CUDA events it gives the

@@ -39,6 +39,10 @@ def get_args():
     p.add_argument('--curves', action='store_true',
                    help='Stereo2Voxel: also evaluate the occupancy probabilities in TEST.CURVE_BINS bins and report the IoU '
                         'and precision-recall curves over every bin threshold, BCE, Brier and calibration as occupancy_curves')
+    p.add_argument('--fscore-curves', action='store_true',
+                   help='also histogram the nearest-neighbour distances over TEST.DIST_BINS edges up to TEST.DIST_MAX and '
+                        'report precision, recall and F-score at every edge, accuracy and completeness as point_curves '
+                        '(Stereo2Point) or surface_curves (Stereo2Voxel, with --surface)')
     return p.parse_args()
 
 
@@ -93,6 +97,8 @@ def main():
         sys.exit('--save-meshes meshes the voxel occupancy: Stereo2Voxel only')
     if args.curves and args.model != 'Stereo2Voxel':
         sys.exit('--curves evaluates the voxel occupancy: Stereo2Voxel only')
+    if args.fscore_curves and args.model == 'Stereo2Voxel' and not args.surface:
+        sys.exit('--fscore-curves evaluates the voxel surfaces for Stereo2Voxel: add --surface')
     if not torch.cuda.is_available():
         sys.exit('runner.py --test needs a CUDA device (sm_100a); there is no CPU fallback.')
     from stereo_3d_reconstruction_b200 import models
@@ -113,6 +119,8 @@ def main():
     model.cuda().pack()
     # one stats vector: the head's statistics, then the disparity counters of the same forwards (core/test.py::stats_layout)
     ev = dict(eval_disp=True, eval_lr=args.lr_check, eval_unc=args.uncertainty)
+    if args.fscore_curves:
+        ev.update(eval_fscore_curves=True)
     if args.model == 'Stereo2Voxel':
         ev.update(eval_surface=args.surface, eval_curves=args.curves)
         stats = T.test_voxel(cfg, model, n, bs, rank, world, mesh_dir=args.save_meshes, **ev).cpu()
@@ -135,6 +143,11 @@ def main():
     if 'points' in b:
         res['points'] = T.points_summary(b['points'], cfg.TEST.FSCORE_THRESH, res['n_samples'], cfg.CONST.N_POINTS,
                                          cfg.CONST.N_GT_POINTS)
+    if 'surface_curves' in b:
+        res['surface_curves'] = T.surface_curves_summary(b['surface_curves'], cfg.TEST.VOXEL_THRESH, models.dist_edges(cfg),
+                                                         res['n_samples'])
+    if 'point_curves' in b:
+        res['point_curves'] = T.point_curves_summary(b['point_curves'], models.dist_edges(cfg), res['n_samples'])
     if rank == 0:
         res.update(model=args.model, precision=cfg.NETWORK.PRECISION, world_size=world, data='synthetic')
         print(json.dumps(res))

@@ -31,6 +31,12 @@ Stereo2Voxel._occupancy_curves; K = TEST.CURVE_BINS, curves_block):
     sum_b q(IoU_b(k / K)) per k (K)                                                           (int64)
 with q20(x) = round-half-even(x * 2^20) (include/s3d.h, s3d_occupancy_curves) and the per-sample IoU at every bin threshold
 computed per batch in fp64 on the device; a sample whose GT and prediction are both empty at t has IoU 1 there.
+With eval_fscore_curves=True (test_voxel with eval_surface, test_point with eval_points) the nearest-neighbour distance
+histograms of the same forwards come last (models.py, _surface_stats / _point_stats; K = TEST.DIST_BINS edges e_k of
+models.dist_edges, surface_curves_block per t in TEST.VOXEL_THRESH / point_curves_block):
+    the histogram per direction (2 (K+1)), then per k sum_b q(P_b(e_k)), sum_b q(R_b(e_k)), sum_b q(F_b(e_k))   (int64)
+with P_b, R_b the fractions of the predicted / GT points closer than e_k (the denominators of the surface / points blocks),
+computed per batch in fp64 on the device.
 stats_layout() declares these blocks and their order, split_stats() cuts a vector into them.
 With mesh_dir (test_voxel) the same forwards also return the marching-cubes mesh of the prediction (models.py,
 Stereo2Voxel._mesh), and each sample of the rank's shard is written as mesh_dir/%06d.obj (predicted) and %06d_gt.obj (the GT
@@ -43,7 +49,7 @@ import torch
 import torch.distributed as dist
 
 from .. import ops
-from ..models import Stereo2Point, Stereo2Voxel, curve_bins, fscore_thresholds, mesh_thresh, unc_thresholds
+from ..models import Stereo2Point, Stereo2Voxel, curve_bins, dist_edges, fscore_thresholds, mesh_thresh, unc_thresholds
 from ..utils import synthetic
 
 _FX = float(1 << 40)
@@ -268,6 +274,110 @@ def curves_summary(block, K, n_samples):
             'ece': ece / N if N else 0.0, 'reliability': rel}
 
 
+def _prf_curves(hist, n0, n1):
+    """hist int64 [..., 2, K+1] (direction 0: predicted -> GT, 1: GT -> predicted), n0 / n1 the denominators broadcastable to
+    [...] -> int64 [K, 3]: per edge e_k (k = 1..K) sum over the leading dims of q(P), q(R), q(F) in fp64, P = (points of
+    direction 0 in bins < k) / n0, R likewise for direction 1 over n1 (0 when the denominator is 0), F = 2 P R / (P + R)
+    (0 when P + R = 0), q(x) = round-half-even(x * 2^32)."""
+    K = hist.shape[-1] - 1
+    cum = hist[..., :K].double().cumsum(-1)                   # [..., 2, K]: points closer than e_1 .. e_K
+    n0 = torch.as_tensor(n0, dtype=torch.float64, device=hist.device)[..., None].expand_as(cum[..., 0, :])
+    n1 = torch.as_tensor(n1, dtype=torch.float64, device=hist.device)[..., None].expand_as(cum[..., 1, :])
+    z = torch.zeros_like(cum[..., 0, :])
+    p = torch.where(n0 > 0, cum[..., 0, :] / n0.clamp(min=1), z)
+    r = torch.where(n1 > 0, cum[..., 1, :] / n1.clamp(min=1), z)
+    f = torch.where(p + r > 0, 2 * p * r / (p + r), z)
+    q = torch.stack([p, r, f], -1)                            # [..., K, 3]
+    return torch.round(q * _PT_FX).to(torch.int64).reshape(-1, K, 3).sum(0)
+
+
+def point_curves_block(dist_hist, N, M):
+    """Per-batch increment of the point_curves block from the forward's dist_hist int64 [B,2,K+1] (N predicted, M GT points
+    per sample) -> int64 [2 (K+1) + 3K]: the histograms summed over the batch, then per edge e_k sum_b q(P_b), q(R_b),
+    q(F_b) with P_b = (predicted points closer than e_k) / N and R_b = (GT points closer than e_k) / M, as point_block."""
+    return torch.cat([dist_hist.sum(0).flatten(), _prf_curves(dist_hist, N, M).flatten()])
+
+
+def surface_curves_block(dist_hist):
+    """Per-batch increment of the surface_curves block from the forward's dist_hist int64 [B,T,2,K+1] -> int64
+    [T * (2 (K+1) + 3K)]: per t the histograms summed over the batch, then per edge e_k sum_b q(P_b), q(R_b), q(F_b) with
+    P_b = count_0(< e_k) / n_0 and R_b = count_1(< e_k) / n_1, n_d the row sums (the surface block's n_pts; 0 when empty)."""
+    n = dist_hist.sum(-1).double()                            # [B,T,2]
+    T = dist_hist.shape[1]
+    per_t = [torch.cat([dist_hist[:, t].sum(0).flatten(), _prf_curves(dist_hist[:, t], n[:, t, 0], n[:, t, 1]).flatten()])
+             for t in range(T)]
+    return torch.cat(per_t) if per_t else torch.zeros(0, dtype=torch.int64, device=dist_hist.device)
+
+
+def _first_reaching(cum, total, num, den):
+    """The smallest k (0-based) with cum[k] / total >= num / den, in integers; None if none (or total = 0)."""
+    if total <= 0:
+        return None
+    return next((k for k, c in enumerate(cum) if den * c >= num * total), None)
+
+
+def _curves_summary(hist0, hist1, prf, edges, n_samples):
+    """Summed histograms hist0 / hist1 (K+1 ints each) and the per-edge sums prf [K][3] -> the curves dict of one block."""
+    K, n = len(edges), n_samples
+    cum0, cum1, c0, c1 = [], [], 0, 0
+    for k in range(K):
+        c0 += hist0[k]
+        c1 += hist1[k]
+        cum0.append(c0)
+        cum1.append(c1)
+    t0, t1 = sum(hist0), sum(hist1)
+    fscore = [prf[k][2] / _PT_FX / n if n else 0.0 for k in range(K)]
+
+    def at(cum, total, num, den):
+        k = _first_reaching(cum, total, num, den)
+        return None if k is None else edges[k]
+    return {'precision': [prf[k][0] / _PT_FX / n if n else 0.0 for k in range(K)],
+            'recall': [prf[k][1] / _PT_FX / n if n else 0.0 for k in range(K)],
+            'fscore': fscore,
+            'pooled_precision': [c / t0 if t0 else 0.0 for c in cum0],
+            'pooled_recall': [c / t1 if t1 else 0.0 for c in cum1],
+            'fscore_auc': sum(fscore) / K,
+            'accuracy': {'p50': at(cum0, t0, 1, 2), 'p90': at(cum0, t0, 9, 10)},
+            'completeness': {'p50': at(cum1, t1, 1, 2), 'p90': at(cum1, t1, 9, 10)},
+            'hist_pred': hist0, 'hist_gt': hist1}
+
+
+def point_curves_summary(block, edges, n_samples):
+    """point_curves counters (int64 [2 (K+1) + 3K], as point_curves_block sums them) -> dict over the K edges e_k
+    (`thresholds`): precision / recall / fscore, the means of the per-sample values at every e_k; pooled_precision /
+    pooled_recall, the fractions of all predicted / GT points closer than e_k; fscore_auc, the mean of the F-score curve over
+    the K edges; accuracy / completeness {p50, p90}, the smallest e_k at which the pooled fraction of predicted / GT points
+    closer than e_k reaches 0.5 / 0.9 (None if e_K does not); hist_pred / hist_gt, the summed histograms (bin K: beyond e_K
+    or out of range)."""
+    edges = [float(e) for e in edges]
+    K = len(edges)
+    v = [int(x) for x in block.tolist()]
+    assert len(v) == 2 * (K + 1) + 3 * K
+    prf = [v[2 * (K + 1) + 3 * k:2 * (K + 1) + 3 * k + 3] for k in range(K)]
+    out = {'n_samples': n_samples, 'thresholds': edges}
+    out.update(_curves_summary(v[:K + 1], v[K + 1:2 * (K + 1)], prf, edges, n_samples))
+    return out
+
+
+def surface_curves_summary(block, voxel_thresh, edges, n_samples):
+    """surface_curves counters (int64 [T * (2 (K+1) + 3K)], as surface_curves_block sums them) -> dict with one entry per t
+    in voxel_thresh holding the curves of point_curves_summary over the surface points (unit-cube units); a direction whose
+    other surface is empty counts its points in bin K."""
+    edges = [float(e) for e in edges]
+    K, T = len(edges), len(voxel_thresh)
+    v = [int(x) for x in block.tolist()]
+    w = 2 * (K + 1) + 3 * K
+    assert len(v) == T * w
+    per = []
+    for t in range(T):
+        r = v[t * w:(t + 1) * w]
+        prf = [r[2 * (K + 1) + 3 * k:2 * (K + 1) + 3 * k + 3] for k in range(K)]
+        e = {'voxel_thresh': float(voxel_thresh[t])}
+        e.update(_curves_summary(r[:K + 1], r[K + 1:2 * (K + 1)], prf, edges, n_samples))
+        per.append(e)
+    return {'n_samples': n_samples, 'thresholds': edges, 'by_thresh': per}
+
+
 def write_obj(path, verts, faces):
     """Plain OBJ of verts fp32 [V,3] and 0-based faces int [F,3]: `v x y z` with %.9g (an fp32 value reads back exactly),
     then `f a b c` with 1-based ids."""
@@ -292,15 +402,20 @@ def _disp_gt(pairs, H, W, device):
 
 
 def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eval_surface=False, eval_points=False,
-                 eval_curves=False):
+                 eval_curves=False, eval_fscore_curves=False):
     """The driver's int64 stats vector for `model` ('Stereo2Voxel' / 'Stereo2Point') as ordered blocks [(name, length)]: the
-    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', then 'surface' and
-    'curves' (Stereo2Voxel) / 'points' (Stereo2Point), each present when its evaluation is on (module docstring).  ValueError on an
-    evaluation without the disparity counters it needs or on a bad cfg.TEST threshold: raised before any forward."""
+    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', then 'surface',
+    'curves' and 'surface_curves' (Stereo2Voxel) / 'points' and 'point_curves' (Stereo2Point), each present when its
+    evaluation is on (module docstring).  ValueError on an evaluation without the counters it needs or on a bad cfg.TEST
+    threshold: raised before any forward."""
     if eval_lr and not eval_disp:
         raise ValueError('eval_lr=True needs eval_disp=True')
     if eval_unc and not eval_disp:
         raise ValueError('eval_unc=True needs eval_disp=True')
+    if eval_fscore_curves and model == 'Stereo2Voxel' and not eval_surface:
+        raise ValueError('eval_fscore_curves=True for Stereo2Voxel needs eval_surface=True')
+    if eval_fscore_curves and model != 'Stereo2Voxel' and not eval_points:
+        raise ValueError('eval_fscore_curves=True for Stereo2Point needs eval_points=True')
     T = len(cfg.TEST.DISP_THRESH)
     blocks = [('iou', 2 * len(cfg.TEST.VOXEL_THRESH) + 1) if model == 'Stereo2Voxel' else ('chamfer', 2)]
     if eval_disp:
@@ -316,6 +431,12 @@ def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eva
     if eval_points:
         F = len(fscore_thresholds(cfg))
         blocks.append(('points', 2 * (3 + F) + F))
+    if eval_fscore_curves:
+        K = len(dist_edges(cfg))
+        if model == 'Stereo2Voxel':
+            blocks.append(('surface_curves', len(cfg.TEST.VOXEL_THRESH) * (2 * (K + 1) + 3 * K)))
+        else:
+            blocks.append(('point_curves', 2 * (K + 1) + 3 * K))
     return blocks
 
 
@@ -336,22 +457,26 @@ def _add_disp_blocks(blocks, out):
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_unc=False, eval_surface=False, mesh_dir=None, eval_curves=False):
+               eval_unc=False, eval_surface=False, mesh_dir=None, eval_curves=False, eval_fscore_curves=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
     eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
     eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones.
     eval_surface: the same forward also evaluates the voxel surfaces; their block follows the uncertainty one.
-    eval_curves: the same forward also returns the occupancy histograms and loss sums; their block comes last.
+    eval_curves: the same forward also returns the occupancy histograms and loss sums; their block follows the surface one.
+    eval_fscore_curves (needs eval_surface): the same call that counts the surface metrics also returns the surface distance
+    histograms; their block comes last.
     mesh_dir: the same forward also meshes the prediction; the meshes and the GT's are written there (module docstring).
     The vector's blocks: stats_layout(cfg, 'Stereo2Voxel', ...)."""
-    layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface, eval_curves=eval_curves)
+    layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface, eval_curves=eval_curves,
+                          eval_fscore_curves=eval_fscore_curves)
     if mesh_dir is not None:
         mesh_thresh(cfg)                                # ValueError on a bad TEST.MESH_THRESH, before any forward
         os.makedirs(mesh_dir, exist_ok=True)
     kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc), ('surface', eval_surface),
-                                ('mesh', mesh_dir is not None), ('curves', eval_curves)) if on}    # the options that are on
+                                ('mesh', mesh_dir is not None), ('curves', eval_curves),
+                                ('fscore_curves', eval_fscore_curves)) if on}    # the options that are on
     names = Stereo2Voxel.output_names(gt=True, disp_gt=eval_disp, **kw)
     stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
     blocks = split_stats(stats, layout)
@@ -373,6 +498,8 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
                 blocks['surface'] += surface_block(out['surf_stats'], cfg.CONST.N_VOX)
             if eval_curves:
                 blocks['curves'] += curves_block(out['occ_hist'], out['occ_loss'])
+            if eval_fscore_curves:
+                blocks['surface_curves'] += surface_curves_block(out['dist_hist'])
             if mesh_dir is not None:
                 save_meshes(mesh_dir, ids, (out['mesh_verts'], out['mesh_faces'], out['mesh_counts']), gt)
             iou = out['iou_counts']
@@ -383,13 +510,16 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
 
 
 def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_points=False, eval_unc=False):
+               eval_points=False, eval_unc=False, eval_fscore_curves=False):
     """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, the
-    uncertainty counters with eval_unc, as for test_voxel, + the point-cloud counters with eval_points: module docstring).
+    uncertainty counters with eval_unc, as for test_voxel, + the point-cloud counters with eval_points, + the distance
+    histograms of the same call with eval_fscore_curves (needs eval_points): module docstring).
     The vector's blocks: stats_layout(cfg, 'Stereo2Point', ...)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
-    layout = stats_layout(cfg, 'Stereo2Point', eval_disp, eval_lr, eval_unc, eval_points=eval_points)
-    kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc)) if on}
+    layout = stats_layout(cfg, 'Stereo2Point', eval_disp, eval_lr, eval_unc, eval_points=eval_points,
+                          eval_fscore_curves=eval_fscore_curves)
+    kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc), ('fscore_curves', eval_fscore_curves))
+          if on}
     names = Stereo2Point.output_names(gt=eval_points, disp_gt=eval_disp, **kw)
     stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
     blocks = split_stats(stats, layout)
@@ -410,6 +540,8 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             pts = out['points']
             if eval_points:
                 blocks['points'] += point_block(out['point_stats'], pts.shape[1], gt.shape[1])
+            if eval_fscore_curves:
+                blocks['point_curves'] += point_curves_block(out['dist_hist'], pts.shape[1], gt.shape[1])
             cd = chamfer_per_sample(pts.contiguous(), gt)
             blocks['chamfer'][0] += torch.round(cd.sum() * _FX).to(torch.int64)
             blocks['chamfer'][1] += len(ids)

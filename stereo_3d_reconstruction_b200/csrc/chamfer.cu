@@ -29,6 +29,7 @@
 //     the minimum distance at the lowest block; chamfer_sym_finish_kernel rescans that one block for the lowest index.
 // About 9.6 issued instructions per pair for BOTH directions against 2 x 11, and 8 of them are the exact arithmetic.
 #include <cmath>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -328,19 +329,36 @@ int launch_dir(const float* q, const float* r, float* dist, int32_t* idx, int B,
   return S3D_OK;
 }
 
-// ---- point-cloud metrics over the search's distances (s3d_chamfer_eval) ------------------------------------------------
+// ---- point-cloud metrics over the search's distances (s3d_chamfer_eval_hist) -------------------------------------------
 // A separate pass over dist1 / dist2 (just written, read from L2), so the search kernels above stay as they are.  Blocks
 // [0, B * c0) cover direction 0 (dist1, c0 blocks per sample), the rest direction 1 (dist2, c1 per sample); a block never
 // spans two (sample, direction) slices.  Integer counters: warp shuffle -> shared memory -> one 64-bit atomic per counter
 // per block, so the sums do not depend on the launch order.
+//
+// With a PointHist argument the same pass also bins every point's sqrt_rn(d) against the K edges: the block copies the
+// edges from the parameter bank into shared memory (a binary search with divergent indices would serialise on the
+// constant bank), keeps an int32 histogram there and flushes its non-zero bins with one 64-bit atomic each.  Untrained
+// predictions put most points into one or two bins (the overflow bin in particular), so the updates are warp-aggregated
+// with __match_any_sync: one shared atomic per distinct bin per warp.  NoHist compiles to the counters-only kernel.
 constexpr int kEvalThreads = 256;
 constexpr int kEvalPts = 4 * kEvalThreads;   // distances per block
 constexpr float kEvalMaxD = 256.f;           // in range: d finite and d < 2^8, so q(d) < 2^40
 constexpr float kFx = 4294967296.f;          // 2^32: q(x) = round-half-even(x * 2^32), the product exact in fp32
 
+struct NoHist {};
+struct Edges { float e[kMaxBins]; };
+struct PointHist {
+  Edges e;                                   // e[0..K) strictly increasing, finite, > 0
+  unsigned long long* hist;                  // [B,2,K+1]
+  int K;
+};
+
+template <class H>
 __global__ void __launch_bounds__(kEvalThreads)
 chamfer_eval_kernel(const float* __restrict__ dist1, const float* __restrict__ dist2, int N, int M, int c0, int c1, int B,
-                    Thresh th, int nT, unsigned long long* __restrict__ stats) {
+                    Thresh th, int nT, unsigned long long* __restrict__ stats, H h) {
+  constexpr bool kHist = std::is_same<H, PointHist>::value;
+  constexpr int kPer = kEvalPts / kEvalThreads;
   const int64_t blk0 = (int64_t)B * c0;
   const bool d1 = blockIdx.x < blk0;
   const int64_t k = d1 ? blockIdx.x : blockIdx.x - blk0;
@@ -349,18 +367,47 @@ chamfer_eval_kernel(const float* __restrict__ dist1, const float* __restrict__ d
   const float* d = (d1 ? dist1 : dist2) + (int64_t)b * n;
   unsigned long long sum_d = 0, sum_s = 0;
   unsigned n_out = 0, cnt[kMaxThresh] = {};
+  int bin[kPer];                                                 // histogram bin per point, -1: no point
+  float* se = nullptr;
+  unsigned* hs = nullptr;
+  if constexpr (kHist) {
+    extern __shared__ uint32_t smem_hist[];
+    se = reinterpret_cast<float*>(smem_hist);                    // [K] edges
+    hs = smem_hist + h.K;                                        // [K+1] counts
+    for (int i = threadIdx.x; i < h.K; i += kEvalThreads) se[i] = h.e.e[i];
+    for (int i = threadIdx.x; i <= h.K; i += kEvalThreads) hs[i] = 0;
 #pragma unroll
-  for (int j = 0; j < kEvalPts / kEvalThreads; ++j) {
+    for (int j = 0; j < kPer; ++j) bin[j] = -1;
+    __syncthreads();
+  }
+#pragma unroll
+  for (int j = 0; j < kPer; ++j) {
     const int i = chunk * kEvalPts + j * kEvalThreads + threadIdx.x;
     if (i >= n) break;
     const float v = d[i];
-    if (!(v < kEvalMaxD)) { ++n_out; continue; }                 // +inf (NaN point or nothing compared less), NaN, >= 2^8
+    if (!(v < kEvalMaxD)) {                                      // +inf (NaN point or nothing compared less), NaN, >= 2^8
+      ++n_out;
+      if constexpr (kHist) bin[j] = h.K;
+      continue;
+    }
     const float s = __fsqrt_rn(v);
     sum_d += (unsigned long long)__float2ll_rn(v * kFx);
     sum_s += (unsigned long long)__float2ll_rn(s * kFx);
 #pragma unroll
     for (int t = 0; t < kMaxThresh; ++t)
       if (t < nT) cnt[t] += s < th.t[t];
+    if constexpr (kHist) {                                       // the number of edges <= s
+      int lo = 0, hi = h.K;
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (se[mid] <= s) lo = mid + 1; else hi = mid; }
+      bin[j] = lo;
+    }
+  }
+  if constexpr (kHist) {
+#pragma unroll
+    for (int j = 0; j < kPer; ++j) {
+      const unsigned grp = __match_any_sync(0xffffffffu, bin[j]);
+      if (bin[j] >= 0 && (int)(threadIdx.x & 31) == __ffs(grp) - 1) atomicAdd(hs + bin[j], (unsigned)__popc(grp));
+    }
   }
   constexpr int kN = 3 + kMaxThresh;
   __shared__ unsigned long long acc[kN];
@@ -381,6 +428,11 @@ chamfer_eval_kernel(const float* __restrict__ dist1, const float* __restrict__ d
   __syncthreads();
   if ((int)threadIdx.x < nc && acc[threadIdx.x])
     atomicAdd(stats + ((int64_t)b * 2 + (d1 ? 0 : 1)) * nc + threadIdx.x, acc[threadIdx.x]);
+  if constexpr (kHist) {
+    unsigned long long* row = h.hist + ((int64_t)b * 2 + (d1 ? 0 : 1)) * (h.K + 1);
+    for (int i = threadIdx.x; i <= h.K; i += kEvalThreads)
+      if (hs[i]) atomicAdd(row + i, (unsigned long long)hs[i]);
+  }
 }
 
 }  // namespace
@@ -449,9 +501,10 @@ extern "C" int s3d_chamfer_forward_ws(const float* xyz1, const float* xyz2, floa
   return launch_dir(xyz2, xyz1, dist2, idx2, B, M, N, st);
 }
 
-extern "C" int s3d_chamfer_eval(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2, int32_t* idx2,
-                                int B, int N, int M, const float* tau, int T, long long* stats, void* workspace,
-                                int64_t workspace_bytes, void* stream) {
+extern "C" int s3d_chamfer_eval_hist(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2,
+                                     int32_t* idx2, int B, int N, int M, const float* tau, int T, long long* stats,
+                                     void* workspace, int64_t workspace_bytes, void* stream, const float* edges, int K,
+                                     long long* hist) {
   using namespace s3d;
   if (!stats || (T > 0 && !tau)) { set_error("chamfer_eval: null argument"); return S3D_ERR_INVALID; }
   S3D_CHECK_ARG(T >= 0 && T <= kMaxThresh, "chamfer_eval: T must be in [0, %d], got %d", kMaxThresh, T);
@@ -463,12 +516,36 @@ extern "C" int s3d_chamfer_eval(const float* xyz1, const float* xyz2, float* dis
   S3D_CHECK_ARG(N < (1 << 22) && M < (1 << 22), "chamfer_eval: N and M must be below 2^22 (N=%d, M=%d)", N, M);
   const int c0 = N > 0 ? ceil_div(N, kEvalPts) : 0, c1 = M > 0 ? ceil_div(M, kEvalPts) : 0;
   S3D_CHECK_ARG((int64_t)B * (c0 + c1) < (1ll << 31), "chamfer_eval: grid too large");
+  S3D_CHECK_ARG(K >= 0 && K <= kMaxBins, "chamfer_eval: K must be in [0, %d], got %d", kMaxBins, K);
+  PointHist ph;
+  if (K > 0) {
+    if (!edges || !hist) { set_error("chamfer_eval: null edges or hist"); return S3D_ERR_INVALID; }
+    for (int i = 0; i < K; ++i) {
+      ph.e.e[i] = edges[i];
+      S3D_CHECK_ARG(std::isfinite(edges[i]) && edges[i] > 0.f && (i == 0 || edges[i] > edges[i - 1]),
+                    "chamfer_eval: edges must be finite, > 0 and strictly increasing (edge %d = %g)", i, (double)edges[i]);
+    }
+    ph.hist = reinterpret_cast<unsigned long long*>(hist);
+    ph.K = K;
+  }
   const int rc = s3d_chamfer_forward_ws(xyz1, xyz2, dist1, idx1, dist2, idx2, B, N, M, workspace, workspace_bytes, stream);
   if (rc != S3D_OK || B == 0) return rc;
-  chamfer_eval_kernel<<<(unsigned)((int64_t)B * (c0 + c1)), kEvalThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      dist1, dist2, N, M, c0, c1, B, th, T, reinterpret_cast<unsigned long long*>(stats));
+  const unsigned grid = (unsigned)((int64_t)B * (c0 + c1));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  auto* stats_u = reinterpret_cast<unsigned long long*>(stats);
+  if (K > 0)
+    chamfer_eval_kernel<<<grid, kEvalThreads, (2 * K + 1) * sizeof(uint32_t), st>>>(dist1, dist2, N, M, c0, c1, B, th, T, stats_u, ph);
+  else
+    chamfer_eval_kernel<<<grid, kEvalThreads, 0, st>>>(dist1, dist2, N, M, c0, c1, B, th, T, stats_u, NoHist{});
   S3D_LAUNCH_CHECK();
   return S3D_OK;
+}
+
+extern "C" int s3d_chamfer_eval(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2, int32_t* idx2,
+                                int B, int N, int M, const float* tau, int T, long long* stats, void* workspace,
+                                int64_t workspace_bytes, void* stream) {
+  return s3d_chamfer_eval_hist(xyz1, xyz2, dist1, idx1, dist2, idx2, B, N, M, tau, T, stats, workspace, workspace_bytes, stream,
+                               nullptr, 0, nullptr);
 }
 
 extern "C" int s3d_chamfer_forward(const float* xyz1, const float* xyz2, float* dist1, int32_t* idx1, float* dist2,

@@ -61,6 +61,9 @@ static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b;
 namespace {
 constexpr int kMaxThresh = 8;
 struct Thresh { float t[kMaxThresh]; };
+// Distance-histogram edges of the point / surface evaluations (s3d_chamfer_eval_hist, s3d_voxel_surface_eval_hist), passed
+// by value: 4 KB of kernel parameters, copied to shared memory by each block.
+constexpr int kMaxBins = 1024;
 }  // namespace
 
 template <typename T> __device__ __forceinline__ float to_f32(T v);

@@ -11,8 +11,14 @@
 //   surface_count_kernel   pass 3 along z, only on the lattice columns holding query sites of the other surface, fused with
 //                          the counters: registers -> warp shuffle -> shared memory -> one 64-bit atomic per counter per
 //                          block; no block spans two (sample, t, direction) slices, so the sums do not depend on launch order.
+//                          With a SurfHist argument it also bins every s against the K integer bounds: the bounds are copied
+//                          to shared memory after the envelope stacks, next to an int32 histogram whose updates are
+//                          warp-aggregated (__match_any_sync over the lanes active at that site) and whose non-zero bins
+//                          are flushed with one 64-bit atomic each.  NoHist compiles to the counters-only kernel.
 // Grid 0 of a sample is the GT surface, grid 1 + t the prediction at threshold t.  Both lower envelopes are the integer
 // form of Felzenszwalb & Huttenlocher's (Meijster et al.'s separation): exact, O(2n+1) per line.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace s3d {
@@ -23,6 +29,13 @@ constexpr int kSurfMaxN = 64;
 constexpr unsigned kNoSite = 0xFFFFu;     // workspace value: no site on this line / plane
 
 struct KBound { int k[kMaxThresh]; };
+struct NoHist {};
+struct Bounds { int k[kMaxBins]; };
+struct SurfHist {
+  Bounds kb;                                 // kb[0..K) non-decreasing, in [0, 3 (2n)^2 + 1]
+  unsigned long long* hist;                  // [B,T,2,K+1]
+  int K;
+};
 
 // Lower envelope of the parabolas (x - u)^2 + f(u) over u in [0, m) with f(u) != kNoSite.  Stack entry e (in st[e * stride])
 // = f << 16 | start << 8 | u: parabola u is the lowest for integer x in [start, next entry's start).  -> entries.
@@ -141,9 +154,11 @@ __device__ __forceinline__ int column_sites(const unsigned long long* P, int n, 
   return 1;
 }
 
+template <class H>
 __global__ void __launch_bounds__(kSurfThreads)
 surface_count_kernel(const unsigned long long* __restrict__ pack, const uint16_t* __restrict__ dt, int n, int T, int nchunk,
-                     KBound kb, int F, unsigned long long* __restrict__ stats) {
+                     KBound kb, int F, unsigned long long* __restrict__ stats, H h) {
+  constexpr bool kHist = std::is_same<H, SurfHist>::value;
   extern __shared__ uint32_t smem[];
   const int m = 2 * n + 1, G = T + 1;
   const int chunk = blockIdx.x % nchunk;
@@ -152,6 +167,16 @@ surface_count_kernel(const unsigned long long* __restrict__ pack, const uint16_t
   const int qg = dir == 0 ? 1 + t : 0, sg = dir == 0 ? 0 : 1 + t;        // query surface, searched surface
   unsigned long long sum_s = 0, sum_q = 0;
   unsigned npts = 0, cnt[kMaxThresh] = {};
+  int* hb = nullptr;                                                     // [K] bounds
+  unsigned* hs = nullptr;                                                // [K+1] counts
+  unsigned n_far = 0;                                                    // points of this thread that go to bin K
+  if constexpr (kHist) {
+    hb = reinterpret_cast<int*>(smem + m * blockDim.x);
+    hs = reinterpret_cast<unsigned*>(hb + h.K);
+    for (int i = threadIdx.x; i < h.K; i += blockDim.x) hb[i] = h.kb.k[i];
+    for (int i = threadIdx.x; i <= h.K; i += blockDim.x) hs[i] = 0;
+    __syncthreads();
+  }
   const int c = chunk * blockDim.x + threadIdx.x;
   if (c < m * m) {
     const int y = c / m, x = c % m;
@@ -178,9 +203,21 @@ surface_count_kernel(const unsigned long long* __restrict__ pack, const uint16_t
 #pragma unroll
           for (int f = 0; f < kMaxThresh; ++f)
             if (f < F) cnt[f] += (int)d < kb.k[f];
+          if constexpr (kHist) {                                         // the number of bounds <= d
+            int lo = 0, hi = h.K;
+            while (lo < hi) { const int mid = (lo + hi) >> 1; if (hb[mid] <= (int)d) lo = mid + 1; else hi = mid; }
+            const unsigned grp = __match_any_sync(__activemask(), lo);
+            if ((int)(threadIdx.x & 31) == __ffs(grp) - 1) atomicAdd(hs + lo, (unsigned)__popc(grp));
+          }
         }
+      } else if constexpr (kHist) {
+        n_far = npts;
       }
     }
+  }
+  if constexpr (kHist) {
+    for (int o = 16; o > 0; o >>= 1) n_far += __shfl_xor_sync(0xffffffffu, n_far, o);
+    if ((threadIdx.x & 31) == 0 && n_far) atomicAdd(hs + h.K, n_far);
   }
   constexpr int kN = 3 + kMaxThresh;
   __shared__ unsigned long long acc[kN];
@@ -200,6 +237,11 @@ surface_count_kernel(const unsigned long long* __restrict__ pack, const uint16_t
   }
   __syncthreads();
   if ((int)threadIdx.x < nc && acc[threadIdx.x]) atomicAdd(stats + (int64_t)slice * nc + threadIdx.x, acc[threadIdx.x]);
+  if constexpr (kHist) {
+    unsigned long long* row = h.hist + (int64_t)slice * (h.K + 1);
+    for (int i = threadIdx.x; i <= h.K; i += blockDim.x)
+      if (hs[i]) atomicAdd(row + i, (unsigned long long)hs[i]);
+  }
 }
 
 int64_t pack_bytes(int B, int T, int n) { return (int64_t)B * (T + 1) * n * n * 8; }
@@ -215,9 +257,10 @@ extern "C" int64_t s3d_voxel_surface_workspace_bytes(int B, int T, int n) {
   return pack_bytes(B, T, n) + grid_bytes(B, T, n);
 }
 
-extern "C" int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
-                                      const int* kbound, int F, long long* stats, void* workspace, int64_t workspace_bytes,
-                                      void* stream) {
+extern "C" int s3d_voxel_surface_eval_hist(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
+                                           const int* kbound, int F, long long* stats, void* workspace,
+                                           int64_t workspace_bytes, void* stream, const int* hist_kbound, int K,
+                                           long long* hist) {
   if (!fused || !gt || !stats || (T > 0 && !thresholds) || (F > 0 && !kbound)) {
     set_error("voxel_surface_eval: null argument");
     return S3D_ERR_INVALID;
@@ -234,6 +277,19 @@ extern "C" int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int
     kb.k[i] = i < F ? kbound[i] : 0;
     S3D_CHECK_ARG(i >= F || (kb.k[i] >= 0 && kb.k[i] <= kmax), "voxel_surface_eval: kbound[%d] must be in [0, %d], got %d",
                   i, kmax, kb.k[i]);
+  }
+  S3D_CHECK_ARG(K >= 0 && K <= kMaxBins, "voxel_surface_eval: K must be in [0, %d], got %d", kMaxBins, K);
+  SurfHist sh;
+  if (K > 0) {
+    if (!hist_kbound || !hist) { set_error("voxel_surface_eval: null hist_kbound or hist"); return S3D_ERR_INVALID; }
+    for (int i = 0; i < K; ++i) {
+      sh.kb.k[i] = hist_kbound[i];
+      S3D_CHECK_ARG(hist_kbound[i] >= 0 && hist_kbound[i] <= kmax && (i == 0 || hist_kbound[i] >= hist_kbound[i - 1]),
+                    "voxel_surface_eval: hist_kbound must be non-decreasing in [0, %d] (bound %d = %d)", kmax, i,
+                    hist_kbound[i]);
+    }
+    sh.hist = reinterpret_cast<unsigned long long*>(hist);
+    sh.K = K;
   }
   const int64_t need = s3d_voxel_surface_workspace_bytes(B, T, n);
   if (B == 0 || T == 0) return S3D_OK;
@@ -252,9 +308,23 @@ extern "C" int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int
   S3D_LAUNCH_CHECK();
   const int nchunk = ceil_div(m * m, kSurfThreads);
   S3D_CHECK_ARG((int64_t)B * T * 2 * nchunk < (1ll << 31), "voxel_surface_eval: grid too large");
-  S3D_CUDA(cudaFuncSetAttribute(surface_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, stack_bytes));
-  surface_count_kernel<<<(unsigned)((int64_t)B * T * 2 * nchunk), kSurfThreads, stack_bytes, st>>>(
-      pack, dt, n, T, nchunk, kb, F, reinterpret_cast<unsigned long long*>(stats));
+  const unsigned grid = (unsigned)((int64_t)B * T * 2 * nchunk);
+  auto* stats_u = reinterpret_cast<unsigned long long*>(stats);
+  if (K > 0) {
+    const int smem2 = stack_bytes + (2 * K + 1) * 4;                    // + the bounds and the histogram
+    S3D_CUDA(cudaFuncSetAttribute(surface_count_kernel<SurfHist>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    surface_count_kernel<<<grid, kSurfThreads, smem2, st>>>(pack, dt, n, T, nchunk, kb, F, stats_u, sh);
+  } else {
+    S3D_CUDA(cudaFuncSetAttribute(surface_count_kernel<NoHist>, cudaFuncAttributeMaxDynamicSharedMemorySize, stack_bytes));
+    surface_count_kernel<<<grid, kSurfThreads, stack_bytes, st>>>(pack, dt, n, T, nchunk, kb, F, stats_u, NoHist{});
+  }
   S3D_LAUNCH_CHECK();
   return S3D_OK;
+}
+
+extern "C" int s3d_voxel_surface_eval(const float* fused, const uint8_t* gt, int B, int n, const float* thresholds, int T,
+                                      const int* kbound, int F, long long* stats, void* workspace, int64_t workspace_bytes,
+                                      void* stream) {
+  return s3d_voxel_surface_eval_hist(fused, gt, B, n, thresholds, T, kbound, F, stats, workspace, workspace_bytes, stream,
+                                     nullptr, 0, nullptr);
 }

@@ -83,6 +83,8 @@ SIGNATURES = {
     's3d_fuse_views': ([_vp, _i64, _vp, _i64, _i, _vp, _i, _i, _i, _vp, ctypes.POINTER(_f), _i, _vp, _i64, _i64, _vp], _i),
     's3d_voxel_surface_workspace_bytes': ([_i, _i, _i], ctypes.c_int64),
     's3d_voxel_surface_eval': ([_vp, _vp, _i, _i, ctypes.POINTER(_f), _i, ctypes.POINTER(_i), _i, _vp, _vp, _i64, _vp], _i),
+    's3d_voxel_surface_eval_hist': ([_vp, _vp, _i, _i, ctypes.POINTER(_f), _i, ctypes.POINTER(_i), _i, _vp, _vp, _i64, _vp,
+                                     ctypes.POINTER(_i), _i, _vp], _i),
     's3d_voxel_mesh_bounds': ([_i, ctypes.POINTER(_i), ctypes.POINTER(_i)], _i),
     's3d_voxel_mesh': ([_vp, _i, _i, _f, _vp, _i, _vp, _i, _vp, _vp], _i),
     's3d_occupancy_curves': ([_vp, _vp, _i, _i, _i, _vp, _vp, _vp], _i),
@@ -90,6 +92,8 @@ SIGNATURES = {
     's3d_chamfer_workspace_bytes': ([_i, _i, _i], ctypes.c_int64),
     's3d_chamfer_forward_ws': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _i64, _vp], _i),
     's3d_chamfer_eval': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, ctypes.POINTER(_f), _i, _vp, _vp, _i64, _vp], _i),
+    's3d_chamfer_eval_hist': ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, ctypes.POINTER(_f), _i, _vp, _vp, _i64, _vp,
+                               ctypes.POINTER(_f), _i, _vp], _i),
     's3d_fma_probe': ([_vp, _i, ctypes.POINTER(ctypes.c_int64), _vp], _i),
 }
 

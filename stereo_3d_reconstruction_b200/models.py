@@ -16,6 +16,7 @@ import ctypes
 import math
 import os
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -37,13 +38,14 @@ OPTIONAL_OUTPUTS = (('disp_gt', ('disp_stats',)),
                     ('uncertainty', ('disp_std', 'unc_stats')),
                     ('surface', ('surf_stats',)),
                     ('mesh', ('mesh_verts', 'mesh_faces', 'mesh_counts')),
-                    ('curves', ('occ_hist', 'occ_loss')))
+                    ('curves', ('occ_hist', 'occ_loss')),
+                    ('fscore_curves', ('dist_hist',)))
 _VOXEL_ONLY = {'surface': 'surface=True evaluates voxel surfaces: Stereo2Voxel only',
                'mesh': 'mesh=True meshes the voxel occupancy: Stereo2Voxel only',
                'curves': 'curves=True evaluates the voxel occupancy: Stereo2Voxel only'}
 
 # The options of one forward, checked (_StereoBase._check_args): what the stages branch on and part of the graph key.
-Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty surface mesh curves')
+Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty surface mesh curves fscore_curves')
 
 
 def _conv_bn2d(cin, cout, k, s, p):
@@ -466,7 +468,7 @@ class _StereoBase(nn.Module):
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
     def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                curves=False):
+                curves=False, fscore_curves=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -474,7 +476,7 @@ class _StereoBase(nn.Module):
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
         left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh,
-                                                          curves)
+                                                          curves, fscore_curves)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
@@ -488,12 +490,12 @@ class _StereoBase(nn.Module):
     # ---- outputs and their checks --------------------------------------------------------------
     @classmethod
     def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                     curves=False):
+                     curves=False, fscore_curves=False):
         """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt: whether the tensor is given):
         the head's outputs, the gt output, then the groups of OPTIONAL_OUTPUTS that are on.  ValueError on an option the
         class does not have."""
         on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'surface': surface, 'mesh': mesh,
-              'curves': curves}
+              'curves': curves, 'fscore_curves': fscore_curves}
         names = cls.HEAD_OUTPUTS + ((cls.GT_OUTPUT,) if gt else ())
         for opt, outs in OPTIONAL_OUTPUTS:
             if on[opt]:
@@ -502,17 +504,22 @@ class _StereoBase(nn.Module):
                 names += outs
         return names
 
-    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh, curves):
+    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh, curves, fscore_curves):
         """The one check of forward() / graphed()'s arguments, before anything is launched: first the options (which the
         class has, what they need), then the cfg.TEST thresholds of the enabled outputs, then the tensors.
         -> (left, right, gt, disp_gt) as the forward takes them and the options value: an Options of bools."""
         opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh),
-                       bool(curves))
+                       bool(curves), bool(fscore_curves))
         self.output_names(**opts._asdict())                   # ValueError on an option this class does not have
         if opts.surface and not opts.gt:
             raise ValueError('surface=True needs the GT occupancy gt')
         if opts.curves and not opts.gt:
             raise ValueError('curves=True needs the GT occupancy gt')
+        if opts.fscore_curves and not opts.gt:
+            raise ValueError('fscore_curves=True needs the GT %s gt' % ('point cloud' if self.GT_OUTPUT == 'point_stats'
+                                                                          else 'occupancy'))
+        if opts.fscore_curves and 'surface' in self.OPTIONS and not opts.surface:
+            raise ValueError('fscore_curves=True evaluates the voxel surfaces: it needs surface=True')
         if opts.uncertainty:
             unc_thresholds(self.cfg)
         if opts.surface or (opts.gt and self.GT_OUTPUT == 'point_stats'):     # the surface and point-cloud F-scores
@@ -523,6 +530,8 @@ class _StereoBase(nn.Module):
             curve_bins(self.cfg)
         if opts.lr_check:
             lr_thresh(self.cfg)
+        if opts.fscore_curves:
+            dist_edges(self.cfg)
         left, right = self._check_inputs(left, right)
         return left, right, self._check_gt(gt, left), self._check_disp_gt(disp_gt, left), opts
 
@@ -590,11 +599,14 @@ class Stereo2Voxel(_StereoBase):
     curves=True (needs gt): the threshold-free evaluation of voxels against gt in K = TEST.CURVE_BINS probability bins; per
     sample occ_hist = [voxels with gt = 0 per bin, voxels with gt != 0 per bin, sum q(v) per bin] and occ_loss = [sum q(BCE),
     sum q(Brier)], q(x) = round-half-even(x * 2^20): the IoU and precision-recall curves at the thresholds k / K, the
-    calibration and the test losses follow from them (include/s3d.h, s3d_occupancy_curves; one more launch)."""
+    calibration and the test losses follow from them (include/s3d.h, s3d_occupancy_curves; one more launch).
+    fscore_curves=True (needs gt and surface=True): dist_hist int64 [B,T,2,K+1], the histogram of the surface points'
+    distances over the K = TEST.DIST_BINS edges of dist_edges (unit-cube units) per sample, t and direction, from the same
+    kernel that counts surf_stats (include/s3d.h, s3d_voxel_surface_eval_hist; no more launches)."""
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'voxels')
     GT_OUTPUT = 'iou_counts'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'surface', 'mesh', 'curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'surface', 'mesh', 'curves', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -634,9 +646,9 @@ class Stereo2Voxel(_StereoBase):
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
     def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                curves=False):
+                curves=False, fscore_curves=False):
         left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh,
-                                                          curves)
+                                                          curves, fscore_curves)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
@@ -696,7 +708,9 @@ class Stereo2Voxel(_StereoBase):
         if gt is not None:
             out['iou_counts'] = iou
         if opts.surface:
-            out['surf_stats'] = self._surface_stats(fused, gt8)
+            out['surf_stats'], hist = self._surface_stats(fused, gt8, opts.fscore_curves)
+            if opts.fscore_curves:
+                out['dist_hist'] = hist
         if opts.mesh:
             out['mesh_verts'], out['mesh_faces'], out['mesh_counts'] = self._mesh(fused)
         if opts.curves:
@@ -719,15 +733,22 @@ class Stereo2Voxel(_StereoBase):
                                                                   self._buf('mesh_faces', (B, mf, 3), torch.int32),
                                                                   self._buf('mesh_counts', (B, 2), torch.int32)))
 
-    def _surface_stats(self, fused, gt8):
-        """Voxel-surface counters of fused [B,n^3] against gt8 [B,n^3] -> surf_stats int64 [B,T,2,3+F], zeroed here (so a
-        graph replay starts from zero).  Every buffer comes from the workspace: no allocation on this path."""
+    def _surface_stats(self, fused, gt8, want_hist=False):
+        """Voxel-surface counters of fused [B,n^3] against gt8 [B,n^3] -> (surf_stats int64 [B,T,2,3+F], dist_hist int64
+        [B,T,2,K+1] if want_hist else None), both zeroed here (so a graph replay starts from zero) and filled by one call.
+        Every buffer comes from the workspace: no allocation on this path."""
         th, fth = list(self.cfg.TEST.VOXEL_THRESH), fscore_thresholds(self.cfg)
         B, nv = fused.shape[0], self.cfg.CONST.N_VOX
         stats = self._buf('surf_stats', (B, len(th), 2, 3 + len(fth)), torch.int64)
         stats.zero_()
+        e, hist = None, None
+        if want_hist:
+            e = dist_edges(self.cfg)
+            hist = self._buf('dist_hist', (B, len(th), 2, len(e) + 1), torch.int64).zero_()
         nb = ops.voxel_surface_workspace_bytes(B, len(th), nv)
-        return ops.voxel_surface_eval(fused, gt8, th, fth, stats, workspace=self._buf('surf_ws', (max(nb, 1),), torch.uint8))
+        ops.voxel_surface_eval(fused, gt8, th, fth, stats, workspace=self._buf('surf_ws', (max(nb, 1),), torch.uint8),
+                               edges=e, hist=hist)
+        return stats, hist
 
 
 def unc_thresholds(cfg):
@@ -774,6 +795,28 @@ def curve_bins(cfg):
     return k
 
 
+def dist_edges(cfg):
+    """The edges of the nearest-neighbour distance histograms (fscore_curves=True): e_k = fp32(TEST.DIST_MAX * k /
+    TEST.DIST_BINS) for k = 1..DIST_BINS, computed in fp64 and rounded once -> float32 numpy array.  DIST_BINS must be an int
+    (not a bool) in [1, 1024] and DIST_MAX finite and > 0, and the rounded edges must be finite, > 0 and strictly
+    increasing; anything else is a ValueError."""
+    K, dmax = cfg.TEST.get('DIST_BINS'), cfg.TEST.get('DIST_MAX')
+    if not (isinstance(K, int) and not isinstance(K, bool) and 1 <= K <= 1024):
+        raise ValueError('TEST.DIST_BINS must be an int in [1, 1024], got %r' % (K,))
+    try:
+        dmax = float(dmax)
+    except (TypeError, ValueError):
+        raise ValueError('TEST.DIST_MAX must be a number, got %r' % (dmax,)) from None
+    if not (math.isfinite(dmax) and dmax > 0):
+        raise ValueError('TEST.DIST_MAX must be finite and > 0, got %r' % (cfg.TEST.DIST_MAX,))
+    with np.errstate(over='ignore'):                          # an edge beyond fp32 becomes inf: rejected below
+        e = np.array([dmax * k / K for k in range(1, K + 1)], dtype=np.float64).astype(np.float32)
+    if not (np.isfinite(e).all() and (e > 0).all() and (np.diff(e) > 0).all()):
+        raise ValueError('TEST.DIST_MAX = %r over TEST.DIST_BINS = %d gives edges that are not finite, > 0 and strictly '
+                         'increasing in fp32' % (cfg.TEST.DIST_MAX, K))
+    return e
+
+
 def fscore_thresholds(cfg):
     """TEST.FSCORE_THRESH as floats: at most 8 (the kernel's limit) Euclidean distances in the points' units, each finite
     and > 0; anything else is a ValueError."""
@@ -793,11 +836,13 @@ class Stereo2Point(_StereoBase):
     lr_check, uncertainty and their outputs as for Stereo2Voxel).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
     `points` against it and counts, per sample and direction (0: predicted -> GT, 1: GT -> predicted), [sum of squared
     distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
-    (include/s3d.h, s3d_chamfer_eval)."""
+    (include/s3d.h, s3d_chamfer_eval).  fscore_curves=True (needs gt): dist_hist int64 [B,2,K+1], the histogram of the
+    points' nearest-neighbour distances over the K = TEST.DIST_BINS edges of dist_edges per sample and direction, from the
+    same kernel that counts point_stats (include/s3d.h, s3d_chamfer_eval_hist; no more launches)."""
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'points')
     GT_OUTPUT = 'point_stats'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty')
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -825,8 +870,10 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False, curves=False):
-        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, False, mesh, curves))
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False, curves=False,
+                fscore_curves=False):
+        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, False, mesh, curves,
+                                                    fscore_curves))
 
     def _head(self, left, right, gt, disp, opts, out):
         """The point head: adds points and point_stats (with gt) to `out`."""
@@ -853,22 +900,30 @@ class Stereo2Point(_StereoBase):
         points = pts.view(B, -1)[:, :npts * 3].reshape(B, npts, 3)
         out['points'] = points
         if gt is not None:
-            out['point_stats'] = self._point_stats(points, gt)
+            out['point_stats'], hist = self._point_stats(points, gt, opts.fscore_curves)
+            if opts.fscore_curves:
+                out['dist_hist'] = hist
 
-    def _point_stats(self, points, gt):
-        """Chamfer search of points [B,N,3] against gt [B,M,3] + the metric counters -> point_stats int64 [B,2,3+T], zeroed
-        here (so a graph replay starts from zero).  Every buffer comes from the workspace: no allocation on this path."""
+    def _point_stats(self, points, gt, want_hist=False):
+        """Chamfer search of points [B,N,3] against gt [B,M,3] + the metric counters -> (point_stats int64 [B,2,3+T],
+        dist_hist int64 [B,2,K+1] if want_hist else None), both zeroed here (so a graph replay starts from zero) and filled
+        by one call.  Every buffer comes from the workspace: no allocation on this path."""
         th = fscore_thresholds(self.cfg)
         B, N, M = points.shape[0], points.shape[1], gt.shape[1]
         if not points.is_contiguous():                 # the fc2 output row is padded: copy the points out of it
             points = self._buf('pts_xyz', (B, N, 3), torch.float32).copy_(points)
         stats = self._buf('point_stats', (B, 2, 3 + len(th)), torch.int64)
         stats.zero_()
+        e, hist = None, None
+        if want_hist:
+            e = dist_edges(self.cfg)
+            hist = self._buf('dist_hist', (B, 2, len(e) + 1), torch.int64).zero_()
         nb = ops.chamfer_workspace_bytes(B, N, M)
         ops.chamfer_eval(points, gt, th, stats, workspace=self._buf('cd_ws', (nb,), torch.uint8) if nb else None,
                          out=(self._buf('cd_d1', (B, N), torch.float32), self._buf('cd_d2', (B, M), torch.float32),
-                              self._buf('cd_i1', (B, N), torch.int32), self._buf('cd_i2', (B, M), torch.int32)))
-        return stats
+                              self._buf('cd_i1', (B, N), torch.int32), self._buf('cd_i2', (B, M), torch.int32)),
+                         edges=e, hist=hist)
+        return stats, hist
 
 
 def build_model(name, cfg, seed=None):

@@ -490,12 +490,37 @@ def chamfer_workspace_bytes(B, N, M):
     return int(_lib.load().s3d_chamfer_workspace_bytes(B, N, M)) if min(B, N, M) > 0 else 0
 
 
-def chamfer_eval(xyz1, xyz2, tau, stats, workspace=None, out=None):
+def _dist_hist_args(what, edges, hist, shape, dev):
+    """Validate the optional distance-histogram arguments -> (edges as fp32 Python floats, K).  edges: a sequence of 1 to
+    1024 values that are finite, > 0 and strictly increasing once rounded to fp32; hist: int64 `shape` + (K + 1,) on dev."""
+    if edges is None and hist is None:
+        return [], 0
+    if edges is None or hist is None:
+        raise ValueError('%s: edges and hist go together' % what)
+    try:
+        e = [float(ctypes.c_float(float(x)).value) for x in edges]
+    except (TypeError, ValueError):
+        raise ValueError('%s: edges must be a sequence of numbers, got %r' % (what, edges)) from None
+    K = len(e)
+    if not 1 <= K <= 1024:
+        raise ValueError('%s: 1 to 1024 edges, got %d' % (what, K))
+    if not all(math.isfinite(x) and x > 0.0 for x in e) or any(b <= a for a, b in zip(e, e[1:])):
+        raise ValueError('%s: edges must be finite, > 0 and strictly increasing in fp32, got %r' % (what, e))
+    want = tuple(shape) + (K + 1,)
+    if not isinstance(hist, torch.Tensor) or hist.dtype != torch.int64 or tuple(hist.shape) != want or hist.device != dev:
+        raise ValueError('%s: hist must be int64 %s on %s' % (what, want, dev))
+    _chk(hist)
+    return e, K
+
+
+def chamfer_eval(xyz1, xyz2, tau, stats, workspace=None, out=None, edges=None, hist=None):
     """chamfer_forward + per-sample point-cloud metrics (include/s3d.h, s3d_chamfer_eval).  xyz1 = predicted [B,N,3], xyz2 =
     GT [B,M,3], fp32.  stats int64 [B,2,3+T] (T = len(tau)) += per direction (0: xyz1 -> xyz2, 1: xyz2 -> xyz1)
     [sum q(d), sum q(sqrt d), n_out, count(sqrt d < tau_t) per t], q(x) = round-half-even(x * 2^32), over the points with
     finite d < 2^8 (the others are n_out).  out: optional (dist1 [B,N], dist2 [B,M], idx1 [B,N], idx2 [B,M]) buffers (fp32,
-    fp32, int32, int32) to write into.  -> (dist1, dist2, idx1, idx2), bit-identical to chamfer_forward."""
+    fp32, int32, int32) to write into.  -> (dist1, dist2, idx1, idx2), bit-identical to chamfer_forward.
+    edges (K fp32 distances, strictly increasing) with hist int64 [B,2,K+1]: hist += per direction the number of points in
+    each bin = the number of edges <= sqrt(d), out-of-range points in bin K (s3d_chamfer_eval_hist; same launches)."""
     _chk(xyz1, xyz2, stats, workspace)
     if xyz1.dtype != torch.float32 or xyz2.dtype != torch.float32:
         raise ValueError('chamfer_eval: point clouds must be float32')
@@ -507,6 +532,7 @@ def chamfer_eval(xyz1, xyz2, tau, stats, workspace=None, out=None):
     if stats.dtype != torch.int64 or tuple(stats.shape) != (B, 2, 3 + T):
         raise ValueError('chamfer_eval: stats must be int64 [%d, 2, %d]' % (B, 3 + T))
     dev = xyz1.device
+    e, K = _dist_hist_args('chamfer_eval', edges, hist, (B, 2), dev)
     if out is None:
         out = (torch.empty((B, N), dtype=torch.float32, device=dev), torch.empty((B, M), dtype=torch.float32, device=dev),
                torch.empty((B, N), dtype=torch.int32, device=dev), torch.empty((B, M), dtype=torch.int32, device=dev))
@@ -520,10 +546,12 @@ def chamfer_eval(xyz1, xyz2, tau, stats, workspace=None, out=None):
     if need and (workspace is None or workspace.numel() * workspace.element_size() < need):
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
     th = (ctypes.c_float * max(T, 1))(*[float(t) for t in tau])
-    rc = _lib.load().s3d_chamfer_eval(xyz1.data_ptr(), xyz2.data_ptr(), dist1.data_ptr(), idx1.data_ptr(), dist2.data_ptr(),
-                                      idx2.data_ptr(), B, N, M, th, T, stats.data_ptr(),
-                                      workspace.data_ptr() if need else None, need, _stream())
-    _lib.check(rc, 's3d_chamfer_eval')
+    ed = (ctypes.c_float * max(K, 1))(*e)
+    rc = _lib.load().s3d_chamfer_eval_hist(xyz1.data_ptr(), xyz2.data_ptr(), dist1.data_ptr(), idx1.data_ptr(),
+                                           dist2.data_ptr(), idx2.data_ptr(), B, N, M, th, T, stats.data_ptr(),
+                                           workspace.data_ptr() if need else None, need, _stream(), ed, K,
+                                           hist.data_ptr() if K else None)
+    _lib.check(rc, 's3d_chamfer_eval_hist')
     _lib.count_launch(3)                       # the two search kernels + chamfer_eval_kernel
     return dist1, dist2, idx1, idx2
 
@@ -539,12 +567,15 @@ def voxel_surface_workspace_bytes(B, T, n):
     return int(_lib.load().s3d_voxel_surface_workspace_bytes(B, T, n))
 
 
-def voxel_surface_eval(fused, gt8, voxel_thresh, fscore_thresh, stats, workspace=None):
+def voxel_surface_eval(fused, gt8, voxel_thresh, fscore_thresh, stats, workspace=None, edges=None, hist=None):
     """Voxel-face surface metrics (include/s3d.h, s3d_voxel_surface_eval).  fused fp32 [B,n,n,n] or [B,n^3], gt8 uint8 of the
     same shape (nonzero = occupied), 1 <= n <= 64.  stats int64 [B,T,2,3+F] (T = len(voxel_thresh), F = len(fscore_thresh))
     += per sample, threshold and direction (0: predicted -> GT, 1: GT -> predicted) [n_pts, sum s, sum q(sqrt s),
     count(s < voxel_kbound(tau)) per tau], s the squared distance in doubled lattice units.  workspace: optional uint8
-    buffer of at least voxel_surface_workspace_bytes(B, T, n) bytes.  Two kernel launches."""
+    buffer of at least voxel_surface_workspace_bytes(B, T, n) bytes.  Two kernel launches.
+    edges (K fp32 distances in unit-cube units, strictly increasing) with hist int64 [B,T,2,K+1]: hist += per sample,
+    threshold and direction the number of surface points in each bin = the number of voxel_kbound(e_j, n) <= s; the points
+    of a direction whose other surface is empty go to bin K (s3d_voxel_surface_eval_hist; same launches)."""
     _chk(fused, gt8, stats, workspace)
     if fused.dtype != torch.float32 or gt8.dtype != torch.uint8:
         raise ValueError('voxel_surface_eval: fused must be float32 and gt8 uint8, got %s / %s' % (fused.dtype, gt8.dtype))
@@ -564,6 +595,7 @@ def voxel_surface_eval(fused, gt8, voxel_thresh, fscore_thresh, stats, workspace
     for t in (gt8, stats, workspace):
         if t is not None and t.device != fused.device:
             raise ValueError('voxel_surface_eval: every tensor must be on %s' % fused.device)
+    e, K = _dist_hist_args('voxel_surface_eval', edges, hist, (B, T, 2), fused.device)
     need = voxel_surface_workspace_bytes(B, T, n)
     if workspace is None:
         workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=fused.device)
@@ -571,9 +603,11 @@ def voxel_surface_eval(fused, gt8, voxel_thresh, fscore_thresh, stats, workspace
         raise ValueError('voxel_surface_eval: workspace of %d bytes, need %d' % (workspace.numel() * workspace.element_size(), need))
     th = (ctypes.c_float * max(T, 1))(*[float(t) for t in voxel_thresh])
     kb = (ctypes.c_int * max(F, 1))(*[voxel_kbound(t, n) for t in fscore_thresh])
-    rc = _lib.load().s3d_voxel_surface_eval(fused.data_ptr(), gt8.data_ptr(), B, n, th, T, kb, F, stats.data_ptr(),
-                                            workspace.data_ptr(), need, _stream())
-    _lib.check(rc, 's3d_voxel_surface_eval')
+    hkb = (ctypes.c_int * max(K, 1))(*[voxel_kbound(x, n) for x in e])
+    rc = _lib.load().s3d_voxel_surface_eval_hist(fused.data_ptr(), gt8.data_ptr(), B, n, th, T, kb, F, stats.data_ptr(),
+                                                 workspace.data_ptr(), need, _stream(), hkb, K,
+                                                 hist.data_ptr() if K else None)
+    _lib.check(rc, 's3d_voxel_surface_eval_hist')
     if B and T:
         _lib.count_launch(2)                   # surface_plane_kernel + surface_count_kernel
     return stats
