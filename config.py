@@ -60,6 +60,10 @@ __C.CONST.N_GT_POINTS = 16384
 __C.CONST.BATCH_SIZE = 64
 __C.CONST.SEED = 0
 __C.CONST.MICRO_BATCH = 64          # forward() splits larger batches into chunks of this many pairs
+# [SPEC] camera of the synthetic 256 x 256 pairs, (f, cx, cy, baseline, doffs): f in px, principal point (cx, cy) in px,
+# baseline in the clouds' units, doffs the principal-point offset between the views in px.  runner.py --save-clouds /
+# --camera only: a forward takes its camera as the camera= tensor
+__C.CONST.CAMERA = [256.0, 127.5, 127.5, 0.1, 0.0]
 
 #
 # Network  [SPEC]
@@ -111,3 +115,8 @@ __C.TEST.CURVE_BINS = 256
 # strictly increasing rounded edges
 __C.TEST.DIST_BINS = 128
 __C.TEST.DIST_MAX = 0.128
+# stereo point clouds (forward(..., camera=...), runner.py --test --save-clouds): a pixel is back-projected when its disparity
+# plus doffs is >= CLOUD_MIN_DISP px (this bounds the depth at f * baseline / CLOUD_MIN_DISP), finite and > 0; with
+# uncertainty=True also only when its disparity standard deviation is <= CLOUD_MAX_STD px, finite and >= 0
+__C.TEST.CLOUD_MIN_DISP = 1.0
+__C.TEST.CLOUD_MAX_STD = 2.0

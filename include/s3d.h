@@ -276,6 +276,33 @@ int s3d_upsample_disp_eval(const float* disp_q, float* disp, int B, int h, int w
                            uint8_t* lr_mask, float lr_thresh, long long* lr_stats,
                            const float* disp_std_q, float* disp_std, const float* unc_thresh, int K, long long* unc_stats,
                            void* stream);
+/* Coloured point clouds of the two disparity maps: every kept pixel back-projected with the camera, one cloud per sample.
+ * For each sample b and view v (0 = left-referenced, 1 = right-referenced) the kernel visits the pixels (x, y) with
+ * disparity d = disp[v*B + b, y, x]; disp fp32 [2B,H,W] is view-major, as the forward's disparity buffer.
+ * camera fp32 [B,5] = (f, cx, cy, baseline, doffs), on the device: f in pixels (square pixels), (cx, cy) the principal point
+ * shared by the two rectified views, doffs the principal-point offset between the views (0 for most rectified data;
+ * Middlebury-style data needs it), baseline in the output's units.  The camera is not checked on the host (that would need
+ * a device sync): a non-finite or non-positive f or baseline gives non-finite points.
+ * A pixel is KEPT when all of these hold:
+ *   d is finite;  den = d + doffs >= min_disp (fp32 add; this bounds the depth);
+ *   if lr_mask is given (uint8 [B,2,H,W]): lr_mask[b,v,y,x] == 1;
+ *   if disp_std is given (fp32 [B,2,H,W]): disp_std[b,v,y,x] <= max_std (a NaN spread is never kept).
+ * Point, every operation a single fp32 round-to-nearest (__fmul_rn / __fdiv_rn / __fadd_rn, no FMA contraction):
+ *   fb = f * baseline, z = fb / den, s = z / f;  X = ((float)x - cx) * s, then X = X + baseline for view 1;
+ *   Y = ((float)y - cy) * s, Z = z.
+ * The result is in the left camera's frame (x right, y down, z forward); for view 1 this is exact algebra, the right camera
+ * sits at +baseline on x.  Colour: view 0 from `left`, view 1 from `right`, at (x, y); img_u8 = 1: uint8 HWC [B,H,W,3], the
+ * bytes themselves; img_u8 = 0: fp32 NCHW [B,3,H,W], rint(clamp(v, 0, 1) * 255) with NaN -> 0 (fp32 product, round half to
+ * even).
+ * Outputs: xyz fp32 [B,2HW,3] and rgb uint8 [B,2HW,3]: per sample the kept points of view 0 in raster order (y, then x), then
+ * those of view 1; rows past counts[b,0] + counts[b,1] are not written.  counts int32 [B,2] = kept points per view, written
+ * (not accumulated).  workspace: s3d_disp_cloud_workspace_bytes(B, H) bytes (int32 [B,2H] row counts), 4-byte aligned.
+ * min_disp finite and > 0; max_std finite and >= 0 when disp_std is given; 2HW < 2^31.  Two kernels (a count pass and a
+ * write pass), no atomics: the output is deterministic and does not depend on the batch split. */
+int64_t s3d_disp_cloud_workspace_bytes(int B, int H);
+int s3d_disp_cloud(const float* disp, int B, int H, int W, const void* left, const void* right, int img_u8,
+                   const uint8_t* lr_mask, const float* disp_std, float max_std, const float* camera, float min_disp,
+                   float* xyz, uint8_t* rgb, int* counts, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)

@@ -12,10 +12,23 @@ IoU / Chamfer statistics are reduced with one NCCL all-reduce.
 """
 import argparse
 import json
+import math
 import os
 import sys
 
 import torch
+
+
+def camera_arg(text):
+    """--camera f,cx,cy,baseline[,doffs] -> [5 floats]: finite, f > 0, baseline > 0 (doffs defaults to 0)."""
+    try:
+        c = [float(v) for v in text.split(',')]
+    except ValueError:
+        raise argparse.ArgumentTypeError('expected f,cx,cy,baseline[,doffs] as numbers, got %r' % text) from None
+    if len(c) not in (4, 5) or not all(math.isfinite(v) for v in c) or not (c[0] > 0 and c[3] > 0):
+        raise argparse.ArgumentTypeError('expected 4 or 5 finite numbers f,cx,cy,baseline[,doffs] with f > 0 and baseline > 0, '
+                                         'got %r' % text)
+    return c + [0.0] * (5 - len(c))
 
 
 def get_args():
@@ -43,6 +56,13 @@ def get_args():
                    help='also histogram the nearest-neighbour distances over TEST.DIST_BINS edges up to TEST.DIST_MAX and '
                         'report precision, recall and F-score at every edge, accuracy and completeness as point_curves '
                         '(Stereo2Point) or surface_curves (Stereo2Voxel, with --surface)')
+    p.add_argument('--save-clouds', metavar='DIR', default=None,
+                   help='also back-project both disparity maps of each pair into one coloured point cloud (filtered by '
+                        '--lr-check / --uncertainty when given) and write it, with the cloud of its GT disparity, as '
+                        'DIR/%%06d.ply and DIR/%%06d_gt.ply (binary PLY), numbered by sample; reports the points as cloud')
+    p.add_argument('--camera', metavar='F,CX,CY,BASELINE[,DOFFS]', type=camera_arg, default=None,
+                   help='camera of --save-clouds (default CONST.CAMERA): focal length and principal point in px, baseline in '
+                        'the clouds\' units, principal-point offset between the views in px')
     return p.parse_args()
 
 
@@ -99,6 +119,10 @@ def main():
         sys.exit('--curves evaluates the voxel occupancy: Stereo2Voxel only')
     if args.fscore_curves and args.model == 'Stereo2Voxel' and not args.surface:
         sys.exit('--fscore-curves evaluates the voxel surfaces for Stereo2Voxel: add --surface')
+    if args.camera is not None and args.save_clouds is None:
+        sys.exit('--camera sets the camera of --save-clouds: add --save-clouds DIR')
+    if args.camera is not None:
+        cfg.CONST.CAMERA = args.camera
     if not torch.cuda.is_available():
         sys.exit('runner.py --test needs a CUDA device (sm_100a); there is no CPU fallback.')
     from stereo_3d_reconstruction_b200 import models
@@ -119,14 +143,16 @@ def main():
     model.cuda().pack()
     # one stats vector: the head's statistics, then the disparity counters of the same forwards (core/test.py::stats_layout)
     ev = dict(eval_disp=True, eval_lr=args.lr_check, eval_unc=args.uncertainty)
+    if args.save_clouds is not None:
+        ev.update(eval_cloud=True)
     if args.fscore_curves:
         ev.update(eval_fscore_curves=True)
     if args.model == 'Stereo2Voxel':
         ev.update(eval_surface=args.surface, eval_curves=args.curves)
-        stats = T.test_voxel(cfg, model, n, bs, rank, world, mesh_dir=args.save_meshes, **ev).cpu()
+        stats = T.test_voxel(cfg, model, n, bs, rank, world, mesh_dir=args.save_meshes, cloud_dir=args.save_clouds, **ev).cpu()
     else:
         ev.update(eval_points=True)
-        stats = T.test_point(cfg, model, n, bs, rank, world, **ev).cpu()
+        stats = T.test_point(cfg, model, n, bs, rank, world, cloud_dir=args.save_clouds, **ev).cpu()
     b = T.split_stats(stats, T.stats_layout(cfg, args.model, **ev))
     res = T.iou_summary(b['iou'], cfg.TEST.VOXEL_THRESH) if 'iou' in b else T.chamfer_summary(b['chamfer'])
     npix = res['n_samples'] * cfg.CONST.IMG_H * cfg.CONST.IMG_W
@@ -136,6 +162,10 @@ def main():
         res['lr_consistency']['lr_thresh'] = float(cfg.TEST.LR_THRESH)
     if 'uncertainty' in b:
         res['uncertainty'] = T.unc_summary(b['uncertainty'], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH, npix, b['disparity'])
+    if 'cloud' in b:
+        res['cloud'] = T.cloud_summary(b['cloud'], res['n_samples'], cfg.CONST.IMG_H, cfg.CONST.IMG_W)
+        res['cloud'].update(camera=models.camera_values(cfg), min_disp=models.cloud_min_disp(cfg),
+                            max_std=models.cloud_max_std(cfg) if args.uncertainty else None)
     if 'surface' in b:
         res['surface'] = T.surface_summary(b['surface'], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH, res['n_samples'])
     if 'curves' in b:

@@ -38,6 +38,11 @@ models.dist_edges, surface_curves_block per t in TEST.VOXEL_THRESH / point_curve
 with P_b, R_b the fractions of the predicted / GT points closer than e_k (the denominators of the surface / points blocks),
 computed per batch in fp64 on the device.
 stats_layout() declares these blocks and their order, split_stats() cuts a vector into them.
+With eval_cloud=True (test_voxel / test_point) the same forwards also return the stereo point clouds (models.py,
+_StereoBase._cloud, with the camera CONST.CAMERA), and their block follows the uncertainty one:
+    kept points of view 0 (left-referenced), kept points of view 1, summed over the samples        (int64)
+With cloud_dir (needs eval_cloud) each sample's cloud is also written as cloud_dir/%06d.ply and the GT disparity's cloud
+(the same op without filters) as %06d_gt.ply, numbered by global sample id (save_clouds).
 With mesh_dir (test_voxel) the same forwards also return the marching-cubes mesh of the prediction (models.py,
 Stereo2Voxel._mesh), and each sample of the rank's shard is written as mesh_dir/%06d.obj (predicted) and %06d_gt.obj (the GT
 occupancy, meshed by the same kernel at t = 0.5), numbered by global sample id; the stats vector does not change.
@@ -49,7 +54,8 @@ import torch
 import torch.distributed as dist
 
 from .. import ops
-from ..models import Stereo2Point, Stereo2Voxel, curve_bins, dist_edges, fscore_thresholds, mesh_thresh, unc_thresholds
+from ..models import (Stereo2Point, Stereo2Voxel, camera_values, cloud_max_std, cloud_min_disp, curve_bins, dist_edges,
+                      fscore_thresholds, mesh_thresh, unc_thresholds)
 from ..utils import synthetic
 
 _FX = float(1 << 40)
@@ -397,14 +403,77 @@ def save_meshes(mesh_dir, ids, mesh, gt):
             write_obj(os.path.join(mesh_dir, name % i), v[b, :nv].cpu().numpy(), f[b, :nf].cpu().numpy())
 
 
+def cloud_summary(block, n_samples, H, W):
+    """Cloud counters [kept points of view 0, of view 1] (int64 [2], summed over n_samples samples of H x W pairs) -> dict:
+    per view and over both views the kept points, their mean per sample and the kept fraction of the view's pixels."""
+    v = [int(x) for x in block.tolist()]
+    assert len(v) == 2
+    n, pix = n_samples, H * W
+
+    def one(k, views):
+        return {'n_points': k, 'per_sample': k / n if n else 0.0, 'kept_fraction': k / (views * n * pix) if n * pix else 0.0}
+    return {'n_samples': n, 'left': one(v[0], 1), 'right': one(v[1], 1), 'all': one(v[0] + v[1], 2)}
+
+
+_PLY_DTYPE = np.dtype([('x', '<f4'), ('y', '<f4'), ('z', '<f4'), ('red', 'u1'), ('green', 'u1'), ('blue', 'u1')])
+
+
+def write_ply(path, xyz, rgb):
+    """Binary little-endian PLY of points xyz fp32 [N,3] with colours rgb uint8 [N,3]: one vertex element with float x, y, z
+    and uchar red, green, blue, 15 bytes per point."""
+    xyz = np.asarray(xyz, np.float32).reshape(-1, 3)
+    rgb = np.asarray(rgb, np.uint8).reshape(-1, 3)
+    assert len(xyz) == len(rgb)
+    rec = np.empty(len(xyz), _PLY_DTYPE)
+    for i, k in enumerate(('x', 'y', 'z')):
+        rec[k] = xyz[:, i]
+    for i, k in enumerate(('red', 'green', 'blue')):
+        rec[k] = rgb[:, i]
+    head = ('ply\nformat binary_little_endian 1.0\nelement vertex %d\nproperty float x\nproperty float y\nproperty float z\n'
+            'property uchar red\nproperty uchar green\nproperty uchar blue\nend_header\n' % len(rec))
+    with open(path, 'wb') as fh:
+        fh.write(head.encode('ascii'))
+        fh.write(rec.tobytes())
+
+
+def save_clouds(cloud_dir, ids, cloud, left, right, camera, disp_gt, min_disp):
+    """Writes the forward's clouds cloud = (xyz, rgb, counts) of samples `ids` (global ids) as cloud_dir/%06d.ply, and the
+    clouds of their GT disparity disp_gt fp32 [B,2,H,W] (NaN = none), back-projected by the same op with the same camera and
+    min_disp and no other filter, as %06d_gt.ply."""
+    B = disp_gt.shape[0]
+    gcloud = ops.disp_cloud(disp_gt.transpose(0, 1).reshape(2 * B, disp_gt.shape[2], disp_gt.shape[3]).contiguous(), B,
+                            left, right, camera, min_disp)
+    for name, (xyz, rgb, c) in (('%06d.ply', cloud), ('%06d_gt.ply', gcloud)):
+        n = c.to(torch.int64).sum(1).cpu()
+        for b, i in enumerate(ids):
+            write_ply(os.path.join(cloud_dir, name % i), xyz[b, :int(n[b])].cpu().numpy(), rgb[b, :int(n[b])].cpu().numpy())
+
+
+def _camera(cfg, B, device):
+    return torch.tensor([camera_values(cfg)], dtype=torch.float32).repeat(B, 1).to(device)
+
+
+def _check_cloud(cfg, eval_cloud, eval_unc, cloud_dir):
+    """ValueError on a bad cloud configuration, before any forward; creates cloud_dir."""
+    if cloud_dir is not None and not eval_cloud:
+        raise ValueError('cloud_dir needs eval_cloud=True')
+    if eval_cloud:
+        camera_values(cfg)
+        cloud_min_disp(cfg)
+        if eval_unc:
+            cloud_max_std(cfg)
+    if cloud_dir is not None:
+        os.makedirs(cloud_dir, exist_ok=True)
+
+
 def _disp_gt(pairs, H, W, device):
     return torch.cat([synthetic.disparity_gt(p[2], H, W) for p in pairs]).to(device)
 
 
 def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eval_surface=False, eval_points=False,
-                 eval_curves=False, eval_fscore_curves=False):
+                 eval_curves=False, eval_fscore_curves=False, eval_cloud=False):
     """The driver's int64 stats vector for `model` ('Stereo2Voxel' / 'Stereo2Point') as ordered blocks [(name, length)]: the
-    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', then 'surface',
+    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'uncertainty', 'cloud' [2], then 'surface',
     'curves' and 'surface_curves' (Stereo2Voxel) / 'points' and 'point_curves' (Stereo2Point), each present when its
     evaluation is on (module docstring).  ValueError on an evaluation without the counters it needs or on a bad cfg.TEST
     threshold: raised before any forward."""
@@ -424,6 +493,8 @@ def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eva
         blocks.append(('lr_consistency', 2 * (3 + T)))
     if eval_unc:
         blocks.append(('uncertainty', 2 * len(unc_thresholds(cfg)) * (3 + T)))
+    if eval_cloud:
+        blocks.append(('cloud', 2))
     if eval_surface:
         blocks.append(('surface', len(cfg.TEST.VOXEL_THRESH) * (3 + 3 * len(fscore_thresholds(cfg)))))
     if eval_curves:
@@ -450,14 +521,17 @@ def split_stats(stats, layout):
 
 
 def _add_disp_blocks(blocks, out):
-    """Adds the batch's disparity, LR-check and uncertainty counters of the named forward outputs `out` to their blocks."""
-    for block, name in (('disparity', 'disp_stats'), ('lr_consistency', 'lr_stats'), ('uncertainty', 'unc_stats')):
+    """Adds the batch's disparity, LR-check, uncertainty and cloud counters of the named forward outputs `out` to their
+    blocks."""
+    for block, name in (('disparity', 'disp_stats'), ('lr_consistency', 'lr_stats'), ('uncertainty', 'unc_stats'),
+                        ('cloud', 'cloud_counts')):
         if block in blocks:
             blocks[block] += out[name].sum(0).flatten()
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_unc=False, eval_surface=False, mesh_dir=None, eval_curves=False, eval_fscore_curves=False):
+               eval_unc=False, eval_surface=False, mesh_dir=None, eval_curves=False, eval_fscore_curves=False, cloud_dir=None,
+               eval_cloud=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
@@ -468,16 +542,19 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
     eval_fscore_curves (needs eval_surface): the same call that counts the surface metrics also returns the surface distance
     histograms; their block comes last.
     mesh_dir: the same forward also meshes the prediction; the meshes and the GT's are written there (module docstring).
+    eval_cloud: the same forward also returns the stereo point clouds (camera CONST.CAMERA); their counters follow the
+    uncertainty ones.  cloud_dir (needs eval_cloud): the clouds and the GT disparity's are written there as PLY.
     The vector's blocks: stats_layout(cfg, 'Stereo2Voxel', ...)."""
     layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface, eval_curves=eval_curves,
-                          eval_fscore_curves=eval_fscore_curves)
+                          eval_fscore_curves=eval_fscore_curves, eval_cloud=eval_cloud)
+    _check_cloud(cfg, eval_cloud, eval_unc, cloud_dir)
     if mesh_dir is not None:
         mesh_thresh(cfg)                                # ValueError on a bad TEST.MESH_THRESH, before any forward
         os.makedirs(mesh_dir, exist_ok=True)
     kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc), ('surface', eval_surface),
                                 ('mesh', mesh_dir is not None), ('curves', eval_curves),
                                 ('fscore_curves', eval_fscore_curves)) if on}    # the options that are on
-    names = Stereo2Voxel.output_names(gt=True, disp_gt=eval_disp, **kw)
+    names = Stereo2Voxel.output_names(gt=True, disp_gt=eval_disp, camera=eval_cloud, **kw)
     stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
     blocks = split_stats(stats, layout)
     T = len(cfg.TEST.VOXEL_THRESH)
@@ -490,10 +567,16 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             left = torch.cat([p[0] for p in pairs]).to(device)
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.gt_volume(1, cfg.CONST.N_VOX, seed=100000 + i) for i in ids]).to(device)
+            dgt = _disp_gt(pairs, H, W, device) if eval_disp or cloud_dir is not None else None
             if eval_disp:
-                kw['disp_gt'] = _disp_gt(pairs, H, W, device)
+                kw['disp_gt'] = dgt
+            if eval_cloud:
+                kw['camera'] = _camera(cfg, len(ids), device)
             out = dict(zip(names, model(left, right, gt, **kw)))
             _add_disp_blocks(blocks, out)
+            if cloud_dir is not None:
+                save_clouds(cloud_dir, ids, (out['cloud_xyz'], out['cloud_rgb'], out['cloud_counts']), left, right,
+                            kw['camera'], dgt, cloud_min_disp(cfg))
             if eval_surface:
                 blocks['surface'] += surface_block(out['surf_stats'], cfg.CONST.N_VOX)
             if eval_curves:
@@ -510,17 +593,19 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
 
 
 def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
-               eval_points=False, eval_unc=False, eval_fscore_curves=False):
+               eval_points=False, eval_unc=False, eval_fscore_curves=False, cloud_dir=None, eval_cloud=False):
     """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, the
-    uncertainty counters with eval_unc, as for test_voxel, + the point-cloud counters with eval_points, + the distance
-    histograms of the same call with eval_fscore_curves (needs eval_points): module docstring).
+    uncertainty counters with eval_unc, the stereo-cloud counters with eval_cloud (and the PLY files with cloud_dir), as for
+    test_voxel, + the point-cloud counters with eval_points, + the distance histograms of the same call with
+    eval_fscore_curves (needs eval_points): module docstring).
     The vector's blocks: stats_layout(cfg, 'Stereo2Point', ...)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
     layout = stats_layout(cfg, 'Stereo2Point', eval_disp, eval_lr, eval_unc, eval_points=eval_points,
-                          eval_fscore_curves=eval_fscore_curves)
+                          eval_fscore_curves=eval_fscore_curves, eval_cloud=eval_cloud)
+    _check_cloud(cfg, eval_cloud, eval_unc, cloud_dir)
     kw = {k: True for k, on in (('lr_check', eval_lr), ('uncertainty', eval_unc), ('fscore_curves', eval_fscore_curves))
           if on}
-    names = Stereo2Point.output_names(gt=eval_points, disp_gt=eval_disp, **kw)
+    names = Stereo2Point.output_names(gt=eval_points, disp_gt=eval_disp, camera=eval_cloud, **kw)
     stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)
     blocks = split_stats(stats, layout)
     lo, hi = shard_range(n_samples, rank, world)
@@ -533,10 +618,16 @@ def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
             right = torch.cat([p[1] for p in pairs]).to(device)
             gt = torch.cat([synthetic.point_clouds(1, 1, cfg.CONST.N_GT_POINTS, seed=200000 + i)[1] for i in ids]).to(device)
             head = (gt,) if eval_points else ()
+            dgt = _disp_gt(pairs, H, W, device) if eval_disp or cloud_dir is not None else None
             if eval_disp:
-                kw['disp_gt'] = _disp_gt(pairs, H, W, device)
+                kw['disp_gt'] = dgt
+            if eval_cloud:
+                kw['camera'] = _camera(cfg, len(ids), device)
             out = dict(zip(names, model(left, right, *head, **kw)))
             _add_disp_blocks(blocks, out)
+            if cloud_dir is not None:
+                save_clouds(cloud_dir, ids, (out['cloud_xyz'], out['cloud_rgb'], out['cloud_counts']), left, right,
+                            kw['camera'], dgt, cloud_min_disp(cfg))
             pts = out['points']
             if eval_points:
                 blocks['points'] += point_block(out['point_stats'], pts.shape[1], gt.shape[1])

@@ -36,6 +36,7 @@ PRECISIONS = ('bf16', 'bf16x3', 'tf32', 'tf32x3', 'fp32')
 OPTIONAL_OUTPUTS = (('disp_gt', ('disp_stats',)),
                     ('lr_check', ('lr_mask', 'lr_stats')),
                     ('uncertainty', ('disp_std', 'unc_stats')),
+                    ('camera', ('cloud_xyz', 'cloud_rgb', 'cloud_counts')),
                     ('surface', ('surf_stats',)),
                     ('mesh', ('mesh_verts', 'mesh_faces', 'mesh_counts')),
                     ('curves', ('occ_hist', 'occ_loss')),
@@ -45,7 +46,7 @@ _VOXEL_ONLY = {'surface': 'surface=True evaluates voxel surfaces: Stereo2Voxel o
                'curves': 'curves=True evaluates the voxel occupancy: Stereo2Voxel only'}
 
 # The options of one forward, checked (_StereoBase._check_args): what the stages branch on and part of the graph key.
-Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty surface mesh curves fscore_curves')
+Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty camera surface mesh curves fscore_curves')
 
 
 def _conv_bn2d(cin, cout, k, s, p):
@@ -154,14 +155,15 @@ def init_synthetic_weights(model, seed=0):
 class _GraphedForward:
     """One captured forward: static input buffers, a torch.cuda.CUDAGraph of the model's launch sequence, static outputs."""
 
-    def __init__(self, model, left, right, gt, disp_gt, opts):
+    def __init__(self, model, left, right, gt, disp_gt, camera, opts):
         self.left, self.right = torch.empty_like(left), torch.empty_like(right)
         self.gt = None if gt is None else torch.empty_like(gt)
         self.disp_gt = None if disp_gt is None else torch.empty_like(disp_gt)
-        self._copy_in(left, right, gt, disp_gt)
+        self.camera = None if camera is None else torch.empty_like(camera)
+        self._copy_in(left, right, gt, disp_gt, camera)
 
         def run():                                    # zeroes its IoU / disparity / LR / uncertainty / surface counters itself: inside the graph
-            return model._forward_impl(self.left, self.right, self.gt, self.disp_gt, opts)
+            return model._forward_impl(self.left, self.right, self.gt, self.disp_gt, self.camera, opts)
         side = torch.cuda.Stream(device=left.device)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):                 # warm-up: workspace buffers and tensor maps exist before capture
@@ -172,16 +174,18 @@ class _GraphedForward:
         with torch.cuda.graph(self.graph):
             self.out = run()
 
-    def _copy_in(self, left, right, gt, disp_gt):
+    def _copy_in(self, left, right, gt, disp_gt, camera):
         self.left.copy_(left, non_blocking=True)
         self.right.copy_(right, non_blocking=True)
         if self.gt is not None:
             self.gt.copy_(gt, non_blocking=True)
         if self.disp_gt is not None:
             self.disp_gt.copy_(disp_gt, non_blocking=True)
+        if self.camera is not None:
+            self.camera.copy_(camera, non_blocking=True)
 
-    def __call__(self, left, right, gt, disp_gt=None):
-        self._copy_in(left, right, gt, disp_gt)
+    def __call__(self, left, right, gt, disp_gt=None, camera=None):
+        self._copy_in(left, right, gt, disp_gt, camera)
         self.graph.replay()
         return self.out
 
@@ -467,35 +471,36 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                curves=False, fscore_curves=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, camera=None, surface=False,
+                mesh=False, curves=False, fscore_curves=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
         ~0.12 ms per aggregation layer), so the graph only removes the launch gaps.
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
-        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh,
-                                                          curves, fscore_curves)
+        left, right, gt, disp_gt, camera, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera,
+                                                                  surface, mesh, curves, fscore_curves)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
         key = (tuple(left.shape), left.dtype, None if gt is None else (tuple(gt.shape), gt.dtype),
-               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype), opts)
+               None if disp_gt is None else (tuple(disp_gt.shape), disp_gt.dtype),
+               None if camera is None else (tuple(camera.shape), camera.dtype), opts)
         g = self._graphs.get(key)
         if g is None:
-            g = self._graphs[key] = _GraphedForward(self, left, right, gt, disp_gt, opts)
-        return g(left, right, gt, disp_gt)
+            g = self._graphs[key] = _GraphedForward(self, left, right, gt, disp_gt, camera, opts)
+        return g(left, right, gt, disp_gt, camera)
 
     # ---- outputs and their checks --------------------------------------------------------------
     @classmethod
     def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                     curves=False, fscore_curves=False):
-        """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt: whether the tensor is given):
+                     curves=False, fscore_curves=False, camera=False):
+        """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt / camera: whether the tensor is given):
         the head's outputs, the gt output, then the groups of OPTIONAL_OUTPUTS that are on.  ValueError on an option the
         class does not have."""
-        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'surface': surface, 'mesh': mesh,
-              'curves': curves, 'fscore_curves': fscore_curves}
+        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'camera': camera, 'surface': surface,
+              'mesh': mesh, 'curves': curves, 'fscore_curves': fscore_curves}
         names = cls.HEAD_OUTPUTS + ((cls.GT_OUTPUT,) if gt else ())
         for opt, outs in OPTIONAL_OUTPUTS:
             if on[opt]:
@@ -504,12 +509,12 @@ class _StereoBase(nn.Module):
                 names += outs
         return names
 
-    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh, curves, fscore_curves):
+    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, camera, surface, mesh, curves, fscore_curves):
         """The one check of forward() / graphed()'s arguments, before anything is launched: first the options (which the
         class has, what they need), then the cfg.TEST thresholds of the enabled outputs, then the tensors.
-        -> (left, right, gt, disp_gt) as the forward takes them and the options value: an Options of bools."""
-        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), bool(surface), bool(mesh),
-                       bool(curves), bool(fscore_curves))
+        -> (left, right, gt, disp_gt, camera) as the forward takes them and the options value: an Options of bools."""
+        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), camera is not None,
+                       bool(surface), bool(mesh), bool(curves), bool(fscore_curves))
         self.output_names(**opts._asdict())                   # ValueError on an option this class does not have
         if opts.surface and not opts.gt:
             raise ValueError('surface=True needs the GT occupancy gt')
@@ -532,14 +537,21 @@ class _StereoBase(nn.Module):
             lr_thresh(self.cfg)
         if opts.fscore_curves:
             dist_edges(self.cfg)
+        if opts.camera:
+            cloud_min_disp(self.cfg)
+            if opts.uncertainty:
+                cloud_max_std(self.cfg)
         left, right = self._check_inputs(left, right)
-        return left, right, self._check_gt(gt, left), self._check_disp_gt(disp_gt, left), opts
+        return (left, right, self._check_gt(gt, left), self._check_disp_gt(disp_gt, left), self._check_camera(camera, left),
+                opts)
 
-    def _forward_impl(self, left, right, gt, disp_gt, opts):
+    def _forward_impl(self, left, right, gt, disp_gt, camera, opts):
         """The forward of checked arguments: the stages fill one dict of named outputs, returned in output_names order."""
         B = left.shape[0]
         disp, out = self._disparity(left, right, disp_gt, opts.lr_check, opts.uncertainty)
         out.update(disp_left=disp[:B].unsqueeze(1), disp_right=disp[B:].unsqueeze(1))
+        if camera is not None:
+            out['cloud_xyz'], out['cloud_rgb'], out['cloud_counts'] = self._cloud(left, right, disp, camera, out)
         self._head(left, right, gt, disp, opts, out)
         return tuple(out[n] for n in self.output_names(**opts._asdict()))
 
@@ -577,17 +589,55 @@ class _StereoBase(nn.Module):
             raise ValueError('disp_gt must be on %s (the images\' device), got %s' % (left.device, disp_gt.device))
         return disp_gt.contiguous()
 
+    def _check_camera(self, camera, left):
+        """Camera of (checked) inputs `left`: fp32 [B,5] = (f, cx, cy, baseline, doffs) per sample on their device (include/s3d.h,
+        s3d_disp_cloud).  Its values stay on the device and are not checked."""
+        if camera is None:
+            return None
+        B = left.shape[0]
+        if not isinstance(camera, torch.Tensor):
+            raise ValueError('camera must be a tensor, got %s' % type(camera).__name__)
+        if tuple(camera.shape) != (B, 5):
+            raise ValueError('expected camera of shape %s, got %s' % ((B, 5), tuple(camera.shape)))
+        if camera.dtype != torch.float32:
+            raise ValueError('camera must be float32, got %s' % camera.dtype)
+        if camera.device != left.device:
+            raise ValueError('camera must be on %s (the images\' device), got %s' % (left.device, camera.device))
+        return camera.contiguous()
+
+    def _cloud(self, left, right, disp, camera, ev):
+        """Coloured point clouds of disp [2B,H,W] with the camera -> (cloud_xyz fp32 [B,2HW,3], cloud_rgb uint8 [B,2HW,3],
+        cloud_counts int32 [B,2]), filtered by the LR mask and the disparity spread (TEST.CLOUD_MAX_STD) when the forward
+        computed them in `ev` (include/s3d.h, s3d_disp_cloud; TEST.CLOUD_MIN_DISP).  The kernels write every output (nothing
+        to zero) into workspace buffers: no allocation on this path."""
+        B, H, W = disp.shape[0] // 2, disp.shape[1], disp.shape[2]
+        std = ev.get('disp_std')
+        nb = ops.disp_cloud_workspace_bytes(B, H)
+        return ops.disp_cloud(disp, B, left, right, camera, cloud_min_disp(self.cfg), lr_mask=ev.get('lr_mask'), disp_std=std,
+                              max_std=None if std is None else cloud_max_std(self.cfg),
+                              out=(self._buf('cloud_xyz', (B, 2 * H * W, 3), torch.float32),
+                                   self._buf('cloud_rgb', (B, 2 * H * W, 3), torch.uint8),
+                                   self._buf('cloud_counts', (B, 2), torch.int32)),
+                              workspace=self._buf('cloud_ws', (max(nb, 1),), torch.uint8))
+
 
 class Stereo2Voxel(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left [B,1,H,W], disp_right [B,1,H,W],
-    voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W], lr_stats int64
-    [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, surf_stats int64 [B,T,2,3+F]][, mesh_verts fp32
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=][, camera=]) -> (disp_left [B,1,H,W], disp_right
+    [B,1,H,W], voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W],
+    lr_stats int64 [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, cloud_xyz fp32 [B,2HW,3], cloud_rgb
+    uint8 [B,2HW,3], cloud_counts int32 [B,2]][, surf_stats int64 [B,T,2,3+F]][, mesh_verts fp32
     [B,max_verts,3], mesh_faces int32 [B,max_faces,3], mesh_counts int32 [B,2]][, occ_hist int64 [B,3,K], occ_loss int64
     [B,2]]).
     Outputs are views of the module's workspace: clone to keep them.  disp_gt: fp32 [B,2,H,W] GT disparity of the two views
     (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; uncertainty=True: the standard
     deviation of each pixel's soft-argmin distribution in input pixels, and counters over the pixels it marks as confident
     (K = len(TEST.UNC_THRESH)); disp_stats, lr_mask, lr_stats, disp_std, unc_stats: _StereoBase._upsample_disp.
+    camera= (fp32 [B,5] = (f, cx, cy, baseline, doffs) per sample on the images' device, with or without gt): the coloured
+    point clouds of the two disparity maps in the left camera's frame, one per sample: the kept pixels of disp_left in raster
+    order, then those of disp_right, each at depth f * baseline / (d + doffs) and coloured from its own image; a pixel is kept
+    when d is finite and d + doffs >= TEST.CLOUD_MIN_DISP, with lr_check=True only where lr_mask is 1 and with
+    uncertainty=True only where disp_std <= TEST.CLOUD_MAX_STD; cloud_counts = kept points per view and only the first
+    cloud_counts[b,0] + cloud_counts[b,1] rows are written (include/s3d.h, s3d_disp_cloud; two more launches).
     surface=True (needs gt): the voxel-face surfaces of the prediction at each t in TEST.VOXEL_THRESH and of gt, evaluated
     against each other; surf_stats per sample, t and direction (0: predicted -> GT, 1: GT -> predicted) = [n_pts, sum s,
     sum q(sqrt s), count(s < k) per tau in TEST.FSCORE_THRESH] with s the exact squared distance to the other surface in
@@ -606,7 +656,7 @@ class Stereo2Voxel(_StereoBase):
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'voxels')
     GT_OUTPUT = 'iou_counts'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'surface', 'mesh', 'curves', 'fscore_curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'camera', 'surface', 'mesh', 'curves', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -645,20 +695,21 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                curves=False, fscore_curves=False):
-        left, right, gt, disp_gt, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, surface, mesh,
-                                                          curves, fscore_curves)
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, camera=None, surface=False,
+                mesh=False, curves=False, fscore_curves=False):
+        left, right, gt, disp_gt, camera, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera,
+                                                                  surface, mesh, curves, fscore_curves)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
             outs = []
             for s in range(0, B, mb):
                 o = self._forward_impl(left[s:s + mb], right[s:s + mb], None if gt is None else gt[s:s + mb],
-                                       None if disp_gt is None else disp_gt[s:s + mb], opts)
+                                       None if disp_gt is None else disp_gt[s:s + mb],
+                                       None if camera is None else camera[s:s + mb], opts)
                 outs.append(tuple(t.clone() for t in o))
             return tuple(torch.cat(ts, 0) for ts in zip(*outs))
-        return self._forward_impl(left, right, gt, disp_gt, opts)
+        return self._forward_impl(left, right, gt, disp_gt, camera, opts)
 
     def _head(self, left, right, gt, disp, opts, out):
         """The voxel head: adds voxels, iou_counts (with gt), surf_stats (surface), the mesh (mesh) and occ_hist / occ_loss
@@ -786,6 +837,46 @@ def mesh_thresh(cfg):
     return t
 
 
+def cloud_min_disp(cfg):
+    """TEST.CLOUD_MIN_DISP as a float: the smallest disparity + doffs (input px) a stereo cloud back-projects, which bounds
+    the depth at f * baseline / CLOUD_MIN_DISP; finite and > 0 (also in fp32); anything else is a ValueError."""
+    t = cfg.TEST.get('CLOUD_MIN_DISP')
+    try:
+        t = float(t)
+    except (TypeError, ValueError):
+        raise ValueError('TEST.CLOUD_MIN_DISP must be a number, got %r' % (t,)) from None
+    if not (math.isfinite(t) and t > 0) or float(ctypes.c_float(t).value) <= 0.0:
+        raise ValueError('TEST.CLOUD_MIN_DISP must be finite and > 0, got %r' % (cfg.TEST.CLOUD_MIN_DISP,))
+    return t
+
+
+def cloud_max_std(cfg):
+    """TEST.CLOUD_MAX_STD as a float: with uncertainty=True a stereo cloud keeps only the pixels whose disparity standard
+    deviation is <= it (input px); finite and >= 0; anything else is a ValueError."""
+    t = cfg.TEST.get('CLOUD_MAX_STD')
+    try:
+        t = float(t)
+    except (TypeError, ValueError):
+        raise ValueError('TEST.CLOUD_MAX_STD must be a number, got %r' % (t,)) from None
+    if not (math.isfinite(t) and t >= 0):
+        raise ValueError('TEST.CLOUD_MAX_STD must be finite and >= 0, got %r' % (cfg.TEST.CLOUD_MAX_STD,))
+    return t
+
+
+def camera_values(cfg):
+    """CONST.CAMERA as 5 floats (f, cx, cy, baseline, doffs): 4 or 5 finite numbers (doffs defaults to 0) with f > 0 and
+    baseline > 0, the camera the test driver and runner.py hand to forward(..., camera=); anything else is a ValueError."""
+    c = cfg.CONST.get('CAMERA')
+    try:
+        c = [float(v) for v in c]
+    except (TypeError, ValueError):
+        raise ValueError('CONST.CAMERA must be a list of numbers (f, cx, cy, baseline[, doffs]), got %r' % (c,)) from None
+    if len(c) not in (4, 5) or not all(math.isfinite(v) for v in c) or not (c[0] > 0 and c[3] > 0):
+        raise ValueError('CONST.CAMERA must hold 4 or 5 finite numbers (f, cx, cy, baseline[, doffs]) with f > 0 and '
+                         'baseline > 0, got %r' % (cfg.CONST.CAMERA,))
+    return c + [0.0] * (5 - len(c))
+
+
 def curve_bins(cfg):
     """TEST.CURVE_BINS: the bins of the threshold-free occupancy evaluation, an int (not a bool) that is a power of two in
     [2, 1024] (the curves are exact at the thresholds k / CURVE_BINS); anything else is a ValueError."""
@@ -831,9 +922,10 @@ def fscore_thresholds(cfg):
 
 
 class Stereo2Point(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=]) -> (disp_left, disp_right, points [B,N_POINTS,3]
-    [, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats][, disp_std, unc_stats]) (disp_gt,
-    lr_check, uncertainty and their outputs as for Stereo2Voxel).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=][, camera=]) -> (disp_left, disp_right, points
+    [B,N_POINTS,3][, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats][, disp_std, unc_stats]
+    [, cloud_xyz, cloud_rgb, cloud_counts][, dist_hist]) (disp_gt, lr_check, uncertainty, camera and their outputs as for
+    Stereo2Voxel: the stereo clouds are the dense counterpart of the decoder's points).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
     `points` against it and counts, per sample and direction (0: predicted -> GT, 1: GT -> predicted), [sum of squared
     distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
     (include/s3d.h, s3d_chamfer_eval).  fscore_curves=True (needs gt): dist_hist int64 [B,2,K+1], the histogram of the
@@ -842,7 +934,7 @@ class Stereo2Point(_StereoBase):
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'points')
     GT_OUTPUT = 'point_stats'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'fscore_curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'camera', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -870,10 +962,10 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, mesh=False, curves=False,
-                fscore_curves=False):
-        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, False, mesh, curves,
-                                                    fscore_curves))
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, camera=None, mesh=False,
+                curves=False, fscore_curves=False):
+        return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera, False, mesh,
+                                                    curves, fscore_curves))
 
     def _head(self, left, right, gt, disp, opts, out):
         """The point head: adds points and point_stats (with gt) to `out`."""

@@ -703,3 +703,75 @@ def occupancy_curves(fused, gt8, K, out=None):
     if B:
         _lib.count_launch(1)                   # occupancy_curves_kernel
     return hist, loss
+
+
+def disp_cloud_workspace_bytes(B, H):
+    """Bytes of the workspace of disp_cloud: the int32 row counts [B, 2H]."""
+    return int(_lib.load().s3d_disp_cloud_workspace_bytes(int(B), int(H)))
+
+
+def disp_cloud(disp, B, left, right, camera, min_disp, lr_mask=None, disp_std=None, max_std=None, out=None, workspace=None):
+    """Coloured point clouds of the two disparity maps (include/s3d.h, s3d_disp_cloud).  disp fp32 [2B,H,W], view-major (the
+    forward's buffer: left-referenced maps first); left / right the images, both fp32 NCHW [B,3,H,W] or both uint8 HWC
+    [B,H,W,3]; camera fp32 [B,5] = (f, cx, cy, baseline, doffs) on the same device; min_disp finite and > 0.  Filters:
+    lr_mask uint8 [B,2,H,W] (kept where 1) and disp_std fp32 [B,2,H,W] (kept where <= max_std, finite and >= 0; needed with
+    disp_std, ignored without it).
+    -> (xyz fp32 [B,2HW,3], rgb uint8 [B,2HW,3], counts int32 [B,2]): per sample the kept points of view 0 in raster order,
+    then those of view 1, in the left camera's frame; only the first counts[b,0] + counts[b,1] rows are written.  out: the
+    three output tensors; workspace: uint8 of at least disp_cloud_workspace_bytes(B, H) bytes.  Two kernel launches."""
+    _chk(disp, left, right, camera, lr_mask, disp_std, workspace)
+    if disp.dtype != torch.float32 or disp.dim() != 3:
+        raise ValueError('disp_cloud: expected disp float32 [2B,H,W], got %s %s' % (disp.dtype, tuple(disp.shape)))
+    if not isinstance(B, int) or B < 0 or disp.shape[0] != 2 * B:
+        raise ValueError('disp_cloud: disp must hold 2B = %r maps, got %s' % (2 * B if isinstance(B, int) else B,
+                                                                             tuple(disp.shape)))
+    H, W = disp.shape[1], disp.shape[2]
+    dev = disp.device
+    if left.dtype == torch.uint8 and right.dtype == torch.uint8:
+        u8, want = 1, (B, H, W, 3)
+    elif left.dtype == torch.float32 and right.dtype == torch.float32:
+        u8, want = 0, (B, 3, H, W)
+    else:
+        raise ValueError('disp_cloud: left / right must be both float32 or both uint8, got %s / %s' % (left.dtype, right.dtype))
+    for name, t, d, s in (('left', left, None, want), ('right', right, None, want), ('camera', camera, torch.float32, (B, 5)),
+                          ('lr_mask', lr_mask, torch.uint8, (B, 2, H, W)), ('disp_std', disp_std, torch.float32, (B, 2, H, W))):
+        if t is None:
+            continue
+        if (d is not None and t.dtype != d) or tuple(t.shape) != s or t.device != dev:
+            raise ValueError('disp_cloud: expected %s %s %s on %s, got %s %s on %s'
+                             % (name, '' if d is None else d, s, dev, t.dtype, tuple(t.shape), t.device))
+    try:
+        min_disp = float(min_disp)
+        max_std = 0.0 if disp_std is None else float(max_std)
+    except (TypeError, ValueError):
+        raise ValueError('disp_cloud: min_disp and max_std must be numbers, got %r / %r' % (min_disp, max_std)) from None
+    if not (math.isfinite(min_disp) and min_disp > 0) or float(ctypes.c_float(min_disp).value) <= 0.0:
+        raise ValueError('disp_cloud: min_disp must be finite and > 0, got %r' % min_disp)
+    if not (math.isfinite(max_std) and max_std >= 0):
+        raise ValueError('disp_cloud: max_std must be finite and >= 0, got %r' % max_std)
+    shapes = ((torch.float32, (B, 2 * H * W, 3)), (torch.uint8, (B, 2 * H * W, 3)), (torch.int32, (B, 2)))
+    if out is None:
+        out = tuple(torch.empty(s, dtype=d, device=dev) for d, s in shapes)
+    else:
+        out = tuple(out)
+        if len(out) != 3:
+            raise ValueError('disp_cloud: out must hold (xyz, rgb, counts)')
+        _chk(*out)
+        for o, (d, s) in zip(out, shapes):
+            if o.dtype != d or tuple(o.shape) != s or o.device != dev:
+                raise ValueError('disp_cloud: out tensors must be %s on %s, got %s'
+                                 % ([(str(d), s) for d, s in shapes], dev, [(str(o.dtype), tuple(o.shape)) for o in out]))
+    nb = disp_cloud_workspace_bytes(B, H)
+    if workspace is None:
+        workspace = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
+    elif workspace.dtype != torch.uint8 or workspace.numel() < nb or workspace.device != dev:
+        raise ValueError('disp_cloud: workspace must be uint8 of at least %d bytes on %s' % (nb, dev))
+    xyz, rgb, counts = out
+    ptr = lambda t: None if t is None else t.data_ptr()
+    rc = _lib.load().s3d_disp_cloud(disp.data_ptr(), B, H, W, left.data_ptr(), right.data_ptr(), u8, ptr(lr_mask),
+                                    ptr(disp_std), max_std, camera.data_ptr(), min_disp, xyz.data_ptr(), rgb.data_ptr(),
+                                    counts.data_ptr(), workspace.data_ptr(), workspace.numel(), _stream())
+    _lib.check(rc, 's3d_disp_cloud')
+    if B:
+        _lib.count_launch(2)                   # cloud_count_kernel + cloud_write_kernel
+    return xyz, rgb, counts
