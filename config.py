@@ -120,3 +120,10 @@ __C.TEST.DIST_MAX = 0.128
 # uncertainty=True also only when its disparity standard deviation is <= CLOUD_MAX_STD px, finite and >= 0
 __C.TEST.CLOUD_MIN_DISP = 1.0
 __C.TEST.CLOUD_MAX_STD = 2.0
+# [SPEC] speckle filter (forward(..., speckle=True), runner.py --test --speckle), OpenCV's filterSpeckles: a connected region
+# of finite disparities (and, with lr_check=True, of pixels the LR check keeps) whose 4-neighbours differ by at most
+# SPECKLE_MAX_DIFF input px is removed when it has at most SPECKLE_MAX_SIZE pixels.  SPECKLE_MAX_SIZE is OpenCV's
+# maxSpeckleSize / StereoSGBM's speckleWindowSize (50-200 recommended), an int >= 0 (not a bool); SPECKLE_MAX_DIFF is
+# StereoSGBM's speckleRange in px (filterSpeckles' maxDiff on 1/16-px maps is 16 times it; 1 or 2 recommended), finite and >= 0
+__C.TEST.SPECKLE_MAX_SIZE = 100
+__C.TEST.SPECKLE_MAX_DIFF = 1.0

@@ -303,6 +303,32 @@ int64_t s3d_disp_cloud_workspace_bytes(int B, int H);
 int s3d_disp_cloud(const float* disp, int B, int H, int W, const void* left, const void* right, int img_u8,
                    const uint8_t* lr_mask, const float* disp_std, float max_std, const float* camera, float min_disp,
                    float* xyz, uint8_t* rgb, int* counts, void* workspace, int64_t workspace_bytes, void* stream);
+/* Speckle filter of the two disparity maps: the small connected regions of each map are removed, as OpenCV's filterSpeckles
+ * (and StereoSGBM's speckleWindowSize / speckleRange, which run it after the left-right check) does on the host.
+ * disp fp32 [2B,H,W] is view-major (map v*B + b, as for s3d_disp_cloud); lr_mask, gt, mask are [B,2,H,W].
+ *   CANDIDATE: d = disp[v*B + b, y, x] is finite and, when lr_mask (uint8) is given, lr_mask[b,v,y,x] == 1 (the left-right
+ *     check runs first, so the pixels it rejects break regions).
+ *   ADJACENT: two candidates of the same map that are 4-neighbours with fabsf(d_p - d_q) <= max_diff (fp32 subtraction, one
+ *     rounding, no FMA).
+ *   REGION: a connected component of candidates; its size is its pixel count.
+ * mask uint8 [B,2,H,W]: 1 exactly when the pixel is a candidate and its region's size is > max_size; every pixel is written.
+ * stats int64 [B,2,5+T], ACCUMULATED (the caller zeroes it), per (sample, view):
+ *   [n_kept, n_valid_kept, sum_{valid & kept} q(|disp - gt|), count_{valid & kept}(|disp - gt| > thresholds[t]) for t < T,
+ *    n_speckles (regions of size <= max_size), n_speckle_px (the pixels in them)]
+ * valid and q as for s3d_upsample_disp_eval: gt fp32 finite and 0 <= gt < max_gt, q(e) = round-half-even(e * 65536) of the
+ * fp32 error; with gt == NULL the GT columns are zero.  The first 3+T columns have the layout of lr_stats.  thresholds: T <= 8
+ * fp32 HOST values; T sets the row length.  max_size >= 0; max_diff finite and >= 0; max_gt > 0 with gt; H*W < 2^31;
+ * 2B < 65536.  workspace: s3d_speckle_filter_workspace_bytes(B, H, W) bytes (int32 labels and region sizes, 8 bytes per
+ * pixel), 4-byte aligned.
+ * The partition into regions is unique and the counters are integers: mask and stats do not depend on launch order,
+ * scheduling or batch split.  For a map whose finite values are multiples of 1/16 in the int16 range and a max_diff that is a
+ * multiple of 1/16, mask equals cv2.filterSpeckles(int16(16 d), newVal, max_size, 16 max_diff) != newVal with the
+ * non-candidates set to a newVal no candidate holds.  Four kernels (block-based union-find: tile-local unions in shared
+ * memory, unions across tile borders, region sizes, mask and counters). */
+int64_t s3d_speckle_filter_workspace_bytes(int B, int H, int W);
+int s3d_speckle_filter(const float* disp, int B, int H, int W, const uint8_t* lr_mask, int max_size, float max_diff,
+                       const float* gt, const float* thresholds, int T, float max_gt,
+                       uint8_t* mask, long long* stats, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)

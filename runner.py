@@ -41,6 +41,10 @@ def get_args():
     p.add_argument('--n-samples', type=int, default=None, help='synthetic test-set size (default: one batch per rank)')
     p.add_argument('--lr-check', action='store_true',
                    help='also run the left-right disparity consistency check and report it as lr_consistency')
+    p.add_argument('--speckle', action='store_true',
+                   help='also remove the small connected regions of each disparity map (OpenCV\'s filterSpeckles with '
+                        'TEST.SPECKLE_MAX_SIZE / SPECKLE_MAX_DIFF, after the LR check with --lr-check) and report the kept '
+                        'pixels as speckle; with --save-clouds the clouds keep only those pixels')
     p.add_argument('--uncertainty', action='store_true',
                    help='also compute the per-pixel disparity uncertainty and report the confidence-filtered metrics as uncertainty')
     p.add_argument('--surface', action='store_true',
@@ -145,6 +149,8 @@ def main():
     ev = dict(eval_disp=True, eval_lr=args.lr_check, eval_unc=args.uncertainty)
     if args.save_clouds is not None:
         ev.update(eval_cloud=True)
+    if args.speckle:
+        ev.update(eval_speckle=True)
     if args.fscore_curves:
         ev.update(eval_fscore_curves=True)
     if args.model == 'Stereo2Voxel':
@@ -160,12 +166,18 @@ def main():
     if 'lr_consistency' in b:
         res['lr_consistency'] = T.lr_summary(b['lr_consistency'], cfg.TEST.DISP_THRESH, npix, b['disparity'])
         res['lr_consistency']['lr_thresh'] = float(cfg.TEST.LR_THRESH)
+    if 'speckle' in b:
+        res['speckle'] = T.speckle_summary(b['speckle'], cfg.TEST.DISP_THRESH, npix, b['disparity'])
+        max_size, max_diff = models.speckle_params(cfg)
+        res['speckle'].update(max_size=max_size, max_diff=max_diff, after_lr_check=args.lr_check)
     if 'uncertainty' in b:
         res['uncertainty'] = T.unc_summary(b['uncertainty'], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH, npix, b['disparity'])
     if 'cloud' in b:
         res['cloud'] = T.cloud_summary(b['cloud'], res['n_samples'], cfg.CONST.IMG_H, cfg.CONST.IMG_W)
         res['cloud'].update(camera=models.camera_values(cfg), min_disp=models.cloud_min_disp(cfg),
                             max_std=models.cloud_max_std(cfg) if args.uncertainty else None)
+        if args.speckle:
+            res['cloud'].update(speckle=dict(max_size=max_size, max_diff=max_diff))
     if 'surface' in b:
         res['surface'] = T.surface_summary(b['surface'], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH, res['n_samples'])
     if 'curves' in b:

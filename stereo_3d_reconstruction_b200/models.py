@@ -35,6 +35,7 @@ PRECISIONS = ('bf16', 'bf16x3', 'tf32', 'tf32x3', 'fp32')
 # point_stats): (keyword that turns the group on, its outputs).  output_names() derives every tuple layout from this.
 OPTIONAL_OUTPUTS = (('disp_gt', ('disp_stats',)),
                     ('lr_check', ('lr_mask', 'lr_stats')),
+                    ('speckle', ('speckle_mask', 'speckle_stats')),
                     ('uncertainty', ('disp_std', 'unc_stats')),
                     ('camera', ('cloud_xyz', 'cloud_rgb', 'cloud_counts')),
                     ('surface', ('surf_stats',)),
@@ -46,7 +47,7 @@ _VOXEL_ONLY = {'surface': 'surface=True evaluates voxel surfaces: Stereo2Voxel o
                'curves': 'curves=True evaluates the voxel occupancy: Stereo2Voxel only'}
 
 # The options of one forward, checked (_StereoBase._check_args): what the stages branch on and part of the graph key.
-Options = collections.namedtuple('Options', 'gt disp_gt lr_check uncertainty camera surface mesh curves fscore_curves')
+Options = collections.namedtuple('Options', 'gt disp_gt lr_check speckle uncertainty camera surface mesh curves fscore_curves')
 
 
 def _conv_bn2d(cin, cout, k, s, p):
@@ -471,8 +472,8 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, camera=None, surface=False,
-                mesh=False, curves=False, fscore_curves=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, uncertainty=False, camera=None,
+                surface=False, mesh=False, curves=False, fscore_curves=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -480,7 +481,7 @@ class _StereoBase(nn.Module):
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
         left, right, gt, disp_gt, camera, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera,
-                                                                  surface, mesh, curves, fscore_curves)
+                                                                  surface, mesh, curves, fscore_curves, speckle)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
@@ -495,12 +496,12 @@ class _StereoBase(nn.Module):
     # ---- outputs and their checks --------------------------------------------------------------
     @classmethod
     def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                     curves=False, fscore_curves=False, camera=False):
+                     curves=False, fscore_curves=False, camera=False, speckle=False):
         """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt / camera: whether the tensor is given):
         the head's outputs, the gt output, then the groups of OPTIONAL_OUTPUTS that are on.  ValueError on an option the
         class does not have."""
-        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'uncertainty': uncertainty, 'camera': camera, 'surface': surface,
-              'mesh': mesh, 'curves': curves, 'fscore_curves': fscore_curves}
+        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'speckle': speckle, 'uncertainty': uncertainty, 'camera': camera,
+              'surface': surface, 'mesh': mesh, 'curves': curves, 'fscore_curves': fscore_curves}
         names = cls.HEAD_OUTPUTS + ((cls.GT_OUTPUT,) if gt else ())
         for opt, outs in OPTIONAL_OUTPUTS:
             if on[opt]:
@@ -509,11 +510,12 @@ class _StereoBase(nn.Module):
                 names += outs
         return names
 
-    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, camera, surface, mesh, curves, fscore_curves):
+    def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, camera, surface, mesh, curves, fscore_curves,
+                    speckle=False):
         """The one check of forward() / graphed()'s arguments, before anything is launched: first the options (which the
         class has, what they need), then the cfg.TEST thresholds of the enabled outputs, then the tensors.
         -> (left, right, gt, disp_gt, camera) as the forward takes them and the options value: an Options of bools."""
-        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(uncertainty), camera is not None,
+        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(speckle), bool(uncertainty), camera is not None,
                        bool(surface), bool(mesh), bool(curves), bool(fscore_curves))
         self.output_names(**opts._asdict())                   # ValueError on an option this class does not have
         if opts.surface and not opts.gt:
@@ -535,6 +537,8 @@ class _StereoBase(nn.Module):
             curve_bins(self.cfg)
         if opts.lr_check:
             lr_thresh(self.cfg)
+        if opts.speckle:
+            speckle_params(self.cfg)
         if opts.fscore_curves:
             dist_edges(self.cfg)
         if opts.camera:
@@ -550,6 +554,8 @@ class _StereoBase(nn.Module):
         B = left.shape[0]
         disp, out = self._disparity(left, right, disp_gt, opts.lr_check, opts.uncertainty)
         out.update(disp_left=disp[:B].unsqueeze(1), disp_right=disp[B:].unsqueeze(1))
+        if opts.speckle:
+            out['speckle_mask'], out['speckle_stats'] = self._speckle(disp, disp_gt, out.get('lr_mask'))
         if camera is not None:
             out['cloud_xyz'], out['cloud_rgb'], out['cloud_counts'] = self._cloud(left, right, disp, camera, out)
         self._head(left, right, gt, disp, opts, out)
@@ -605,15 +611,33 @@ class _StereoBase(nn.Module):
             raise ValueError('camera must be on %s (the images\' device), got %s' % (left.device, camera.device))
         return camera.contiguous()
 
+    def _speckle(self, disp, disp_gt, lr_mask):
+        """Speckle filter of disp [2B,H,W] (include/s3d.h, s3d_speckle_filter; TEST.SPECKLE_MAX_SIZE / SPECKLE_MAX_DIFF), after
+        the LR check when lr_mask is given -> (speckle_mask uint8 [B,2,H,W], speckle_stats int64 [B,2,5+T]): the counters of
+        lr_stats over the kept pixels against disp_gt (TEST.DISP_THRESH, valid below 4 * MAX_DISP; zero without it), then
+        n_speckles, n_speckle_px.  The stats are zeroed here, so a graph replay starts from zero; every buffer comes from the
+        workspace: no allocation on this path."""
+        B, H, W = disp.shape[0] // 2, disp.shape[1], disp.shape[2]
+        max_size, max_diff = speckle_params(self.cfg)
+        th = list(self.cfg.TEST.DISP_THRESH)
+        nb = ops.speckle_filter_workspace_bytes(B, H, W)
+        return ops.speckle_filter(disp, B, max_size, max_diff, lr_mask=lr_mask, disp_gt=disp_gt, thresholds=th,
+                                  max_gt=4.0 * self.cfg.NETWORK.MAX_DISP,
+                                  out=(self._buf('speckle_mask', (B, 2, H, W), torch.uint8),
+                                       self._buf('speckle_stats', (B, 2, 5 + len(th)), torch.int64).zero_()),
+                                  workspace=self._buf('speckle_ws', (max(nb, 1),), torch.uint8))
+
     def _cloud(self, left, right, disp, camera, ev):
         """Coloured point clouds of disp [2B,H,W] with the camera -> (cloud_xyz fp32 [B,2HW,3], cloud_rgb uint8 [B,2HW,3],
-        cloud_counts int32 [B,2]), filtered by the LR mask and the disparity spread (TEST.CLOUD_MAX_STD) when the forward
-        computed them in `ev` (include/s3d.h, s3d_disp_cloud; TEST.CLOUD_MIN_DISP).  The kernels write every output (nothing
-        to zero) into workspace buffers: no allocation on this path."""
+        cloud_counts int32 [B,2]), filtered by the speckle mask (which includes the LR check) or else the LR mask, and by the
+        disparity spread (TEST.CLOUD_MAX_STD), when the forward computed them in `ev` (include/s3d.h, s3d_disp_cloud;
+        TEST.CLOUD_MIN_DISP).  The kernels write every output (nothing to zero) into workspace buffers: no allocation on this
+        path."""
         B, H, W = disp.shape[0] // 2, disp.shape[1], disp.shape[2]
         std = ev.get('disp_std')
         nb = ops.disp_cloud_workspace_bytes(B, H)
-        return ops.disp_cloud(disp, B, left, right, camera, cloud_min_disp(self.cfg), lr_mask=ev.get('lr_mask'), disp_std=std,
+        mask = ev['speckle_mask'] if 'speckle_mask' in ev else ev.get('lr_mask')
+        return ops.disp_cloud(disp, B, left, right, camera, cloud_min_disp(self.cfg), lr_mask=mask, disp_std=std,
                               max_std=None if std is None else cloud_max_std(self.cfg),
                               out=(self._buf('cloud_xyz', (B, 2 * H * W, 3), torch.float32),
                                    self._buf('cloud_rgb', (B, 2 * H * W, 3), torch.uint8),
@@ -622,9 +646,10 @@ class _StereoBase(nn.Module):
 
 
 class Stereo2Voxel(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=][, camera=]) -> (disp_left [B,1,H,W], disp_right
-    [B,1,H,W], voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8 [B,2,H,W],
-    lr_stats int64 [B,2,3+T']][, disp_std fp32 [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, cloud_xyz fp32 [B,2HW,3], cloud_rgb
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, speckle=][, uncertainty=][, camera=]) -> (disp_left [B,1,H,W],
+    disp_right [B,1,H,W], voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8
+    [B,2,H,W], lr_stats int64 [B,2,3+T']][, speckle_mask uint8 [B,2,H,W], speckle_stats int64 [B,2,5+T']][, disp_std fp32
+    [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, cloud_xyz fp32 [B,2HW,3], cloud_rgb
     uint8 [B,2HW,3], cloud_counts int32 [B,2]][, surf_stats int64 [B,T,2,3+F]][, mesh_verts fp32
     [B,max_verts,3], mesh_faces int32 [B,max_faces,3], mesh_counts int32 [B,2]][, occ_hist int64 [B,3,K], occ_loss int64
     [B,2]]).
@@ -632,7 +657,12 @@ class Stereo2Voxel(_StereoBase):
     (NaN = none); lr_check=True: left-right consistency check of the two disparity maps; uncertainty=True: the standard
     deviation of each pixel's soft-argmin distribution in input pixels, and counters over the pixels it marks as confident
     (K = len(TEST.UNC_THRESH)); disp_stats, lr_mask, lr_stats, disp_std, unc_stats: _StereoBase._upsample_disp.
-    camera= (fp32 [B,5] = (f, cx, cy, baseline, doffs) per sample on the images' device, with or without gt): the coloured
+    speckle=True: OpenCV's speckle filter of the two disparity maps (after the LR check with lr_check=True): speckle_mask is 1
+    where a pixel's region of finite disparities whose 4-neighbours differ by at most TEST.SPECKLE_MAX_DIFF px has more than
+    TEST.SPECKLE_MAX_SIZE pixels; speckle_stats = the lr_stats counters over those pixels, then the number of removed regions
+    and their pixels (_StereoBase._speckle; include/s3d.h, s3d_speckle_filter; four more launches).  With camera= as well the
+    cloud keeps only the pixels of speckle_mask.
+    camera=(fp32 [B,5] = (f, cx, cy, baseline, doffs) per sample on the images' device, with or without gt): the coloured
     point clouds of the two disparity maps in the left camera's frame, one per sample: the kept pixels of disp_left in raster
     order, then those of disp_right, each at depth f * baseline / (d + doffs) and coloured from its own image; a pixel is kept
     when d is finite and d + doffs >= TEST.CLOUD_MIN_DISP, with lr_check=True only where lr_mask is 1 and with
@@ -656,7 +686,7 @@ class Stereo2Voxel(_StereoBase):
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'voxels')
     GT_OUTPUT = 'iou_counts'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'camera', 'surface', 'mesh', 'curves', 'fscore_curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'speckle', 'uncertainty', 'camera', 'surface', 'mesh', 'curves', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -695,10 +725,10 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, camera=None, surface=False,
-                mesh=False, curves=False, fscore_curves=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, uncertainty=False, camera=None,
+                surface=False, mesh=False, curves=False, fscore_curves=False):
         left, right, gt, disp_gt, camera, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera,
-                                                                  surface, mesh, curves, fscore_curves)
+                                                                  surface, mesh, curves, fscore_curves, speckle)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
@@ -837,6 +867,23 @@ def mesh_thresh(cfg):
     return t
 
 
+def speckle_params(cfg):
+    """(TEST.SPECKLE_MAX_SIZE, TEST.SPECKLE_MAX_DIFF) of the speckle filter: the largest region (px) that is removed, an int
+    >= 0 and not a bool (OpenCV's maxSpeckleSize), and the largest disparity step (input px) inside a region, finite and >= 0
+    also in fp32 (StereoSGBM's speckleRange); anything else is a ValueError."""
+    n, t = cfg.TEST.get('SPECKLE_MAX_SIZE'), cfg.TEST.get('SPECKLE_MAX_DIFF')
+    if not (isinstance(n, int) and not isinstance(n, bool) and 0 <= n < 2 ** 31):
+        raise ValueError('TEST.SPECKLE_MAX_SIZE must be an int >= 0, got %r' % (n,))
+    try:
+        t = float(t)
+    except (TypeError, ValueError):
+        raise ValueError('TEST.SPECKLE_MAX_DIFF must be a number, got %r' % (t,)) from None
+    if isinstance(cfg.TEST.SPECKLE_MAX_DIFF, bool) or not (math.isfinite(t) and t >= 0) or \
+            not math.isfinite(ctypes.c_float(t).value):
+        raise ValueError('TEST.SPECKLE_MAX_DIFF must be finite and >= 0, got %r' % (cfg.TEST.SPECKLE_MAX_DIFF,))
+    return n, t
+
+
 def cloud_min_disp(cfg):
     """TEST.CLOUD_MIN_DISP as a float: the smallest disparity + doffs (input px) a stereo cloud back-projects, which bounds
     the depth at f * baseline / CLOUD_MIN_DISP; finite and > 0 (also in fp32); anything else is a ValueError."""
@@ -922,9 +969,10 @@ def fscore_thresholds(cfg):
 
 
 class Stereo2Point(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=][, uncertainty=][, camera=]) -> (disp_left, disp_right, points
-    [B,N_POINTS,3][, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats][, disp_std, unc_stats]
-    [, cloud_xyz, cloud_rgb, cloud_counts][, dist_hist]) (disp_gt, lr_check, uncertainty, camera and their outputs as for
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, speckle=][, uncertainty=][, camera=]) -> (disp_left, disp_right,
+    points [B,N_POINTS,3][, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats][, speckle_mask,
+    speckle_stats][, disp_std, unc_stats][, cloud_xyz, cloud_rgb, cloud_counts][, dist_hist]) (disp_gt, lr_check, speckle,
+    uncertainty, camera and their outputs as for
     Stereo2Voxel: the stereo clouds are the dense counterpart of the decoder's points).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
     `points` against it and counts, per sample and direction (0: predicted -> GT, 1: GT -> predicted), [sum of squared
     distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
@@ -934,7 +982,7 @@ class Stereo2Point(_StereoBase):
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'points')
     GT_OUTPUT = 'point_stats'
-    OPTIONS = ('disp_gt', 'lr_check', 'uncertainty', 'camera', 'fscore_curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'speckle', 'uncertainty', 'camera', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -962,10 +1010,10 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, uncertainty=False, camera=None, mesh=False,
-                curves=False, fscore_curves=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, uncertainty=False, camera=None,
+                mesh=False, curves=False, fscore_curves=False):
         return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera, False, mesh,
-                                                    curves, fscore_curves))
+                                                    curves, fscore_curves, speckle))
 
     def _head(self, left, right, gt, disp, opts, out):
         """The point head: adds points and point_stats (with gt) to `out`."""

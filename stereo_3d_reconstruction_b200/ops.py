@@ -775,3 +775,78 @@ def disp_cloud(disp, B, left, right, camera, min_disp, lr_mask=None, disp_std=No
     if B:
         _lib.count_launch(2)                   # cloud_count_kernel + cloud_write_kernel
     return xyz, rgb, counts
+
+
+def speckle_filter_workspace_bytes(B, H, W):
+    """Bytes of the workspace of speckle_filter: int32 labels and region sizes, 8 bytes per pixel of the 2B maps."""
+    return int(_lib.load().s3d_speckle_filter_workspace_bytes(int(B), int(H), int(W)))
+
+
+def speckle_filter(disp, B, max_size, max_diff, lr_mask=None, disp_gt=None, thresholds=(), max_gt=None, out=None,
+                   workspace=None):
+    """Speckle filter of the two disparity maps (include/s3d.h, s3d_speckle_filter), OpenCV's filterSpeckles on the GPU.  disp
+    fp32 [2B,H,W], view-major (the forward's buffer: left-referenced maps first).  A pixel is a candidate where d is finite
+    and, with lr_mask uint8 [B,2,H,W], lr_mask is 1; two 4-neighbour candidates are adjacent when |d_p - d_q| <= max_diff
+    (finite, >= 0, input px); a region (connected component) of at most max_size pixels (an int >= 0) is a speckle.
+    -> (mask uint8 [B,2,H,W]: 1 where a candidate's region is larger than max_size, stats int64 [B,2,5+T] ADDED to:
+    [n_kept, n_valid_kept, sum of |disp - gt| in 2^-16 px and count(|disp - gt| > t) per threshold over the kept pixels with
+    valid GT (disp_gt fp32 [B,2,H,W], valid where finite and 0 <= gt < max_gt; zero without it), n_speckles,
+    n_speckle_px]).  T = len(thresholds) <= 8.  out: (mask, stats), else a new mask and zeroed stats; workspace: uint8 of
+    at least speckle_filter_workspace_bytes(B, H, W) bytes.  Four kernel launches."""
+    _chk(disp, lr_mask, disp_gt, workspace)
+    if disp.dtype != torch.float32 or disp.dim() != 3:
+        raise ValueError('speckle_filter: expected disp float32 [2B,H,W], got %s %s' % (disp.dtype, tuple(disp.shape)))
+    if not isinstance(B, int) or isinstance(B, bool) or B < 0 or disp.shape[0] != 2 * B:
+        raise ValueError('speckle_filter: disp must hold 2B maps for an int B >= 0, got B = %r and %s' % (B, tuple(disp.shape)))
+    H, W = disp.shape[1], disp.shape[2]
+    dev = disp.device
+    for name, t, d in (('lr_mask', lr_mask, torch.uint8), ('disp_gt', disp_gt, torch.float32)):
+        if t is not None and (t.dtype != d or tuple(t.shape) != (B, 2, H, W) or t.device != dev):
+            raise ValueError('speckle_filter: expected %s %s %s on %s, got %s %s on %s'
+                             % (name, d, (B, 2, H, W), dev, t.dtype, tuple(t.shape), t.device))
+    if not isinstance(max_size, int) or isinstance(max_size, bool) or not 0 <= max_size < 2 ** 31:
+        raise ValueError('speckle_filter: max_size must be an int in [0, 2^31), got %r' % (max_size,))
+    try:
+        max_diff = float(max_diff)
+        th = [float(t) for t in thresholds]
+        max_gt = None if max_gt is None else float(max_gt)
+    except (TypeError, ValueError):
+        raise ValueError('speckle_filter: max_diff, thresholds and max_gt must be numbers, got %r / %r / %r'
+                         % (max_diff, thresholds, max_gt)) from None
+    if not (math.isfinite(max_diff) and max_diff >= 0 and math.isfinite(ctypes.c_float(max_diff).value)):
+        raise ValueError('speckle_filter: max_diff must be finite and >= 0 (also in fp32), got %r' % max_diff)
+    if len(th) > 8:
+        raise ValueError('speckle_filter: at most 8 thresholds, got %d' % len(th))
+    if disp_gt is not None and not (max_gt is not None and max_gt > 0 and ctypes.c_float(max_gt).value > 0):
+        raise ValueError('speckle_filter: disp_gt needs max_gt > 0, got %r' % (max_gt,))
+    T = len(th)
+    shapes = ((torch.uint8, (B, 2, H, W)), (torch.int64, (B, 2, 5 + T)))
+    if out is None:
+        out = (torch.empty(shapes[0][1], dtype=torch.uint8, device=dev), torch.zeros(shapes[1][1], dtype=torch.int64, device=dev))
+    else:
+        out = tuple(out)
+        if len(out) != 2:
+            raise ValueError('speckle_filter: out must hold (mask, stats)')
+        _chk(*out)
+        for o, (d, s) in zip(out, shapes):
+            if o.dtype != d or tuple(o.shape) != s or o.device != dev:
+                raise ValueError('speckle_filter: out tensors must be %s on %s, got %s'
+                                 % ([(str(d), s) for d, s in shapes], dev, [(str(o.dtype), tuple(o.shape)) for o in out]))
+    nb = speckle_filter_workspace_bytes(B, H, W)
+    if workspace is None:
+        workspace = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
+    elif workspace.dtype != torch.uint8 or workspace.numel() < nb or workspace.device != dev:
+        raise ValueError('speckle_filter: workspace must be uint8 of at least %d bytes on %s' % (nb, dev))
+    mask, stats = out
+    if B == 0:                                 # no maps (and empty tensors may hold no data pointer)
+        return mask, stats
+    ptr = lambda t: None if t is None else t.data_ptr()
+    tc = (ctypes.c_float * max(T, 1))(*th)
+    rc = _lib.load().s3d_speckle_filter(disp.data_ptr(), B, H, W, ptr(lr_mask), max_size, max_diff, ptr(disp_gt), tc, T,
+                                        0.0 if max_gt is None else max_gt, mask.data_ptr(), stats.data_ptr(),
+                                        workspace.data_ptr(), workspace.numel(), _stream())
+    if rc == -1:                               # S3D_ERR_INVALID: an argument the checks above let through (H W >= 2^31, ...)
+        raise ValueError('speckle_filter: %s' % _lib.load().s3d_last_error().decode('utf-8', 'replace'))
+    _lib.check(rc, 's3d_speckle_filter')
+    _lib.count_launch(4)                       # speckle_local / border / size / finish kernels
+    return mask, stats
