@@ -127,3 +127,10 @@ __C.TEST.CLOUD_MAX_STD = 2.0
 # StereoSGBM's speckleRange in px (filterSpeckles' maxDiff on 1/16-px maps is 16 times it; 1 or 2 recommended), finite and >= 0
 __C.TEST.SPECKLE_MAX_SIZE = 100
 __C.TEST.SPECKLE_MAX_DIFF = 1.0
+# [SPEC] WLS filter (forward(..., wls=True), runner.py --test --wls), OpenCV's DisparityWLSFilter defaults: the fast global
+# smoother of both disparity maps guided by each view's own image, weighted by the confidence (the speckle mask with
+# speckle=True, else the LR mask with lr_check=True, else the finite pixels) and divided by the smoothed confidence.
+# WLS_LAMBDA is the smoothness weight (OpenCV's lambda), WLS_SIGMA the colour scale of the edge weights exp(-|dI| / sigma) in
+# 8-bit colour units (OpenCV's sigmaColor); both finite and > 0
+__C.TEST.WLS_LAMBDA = 8000.0
+__C.TEST.WLS_SIGMA = 1.5

@@ -329,6 +329,43 @@ int64_t s3d_speckle_filter_workspace_bytes(int B, int H, int W);
 int s3d_speckle_filter(const float* disp, int B, int H, int W, const uint8_t* lr_mask, int max_size, float max_diff,
                        const float* gt, const float* thresholds, int T, float max_gt,
                        uint8_t* mask, long long* stats, void* workspace, int64_t workspace_bytes, void* stream);
+/* Confidence-weighted WLS filter of the two disparity maps: the fast global smoother of Min et al. (2014) guided by each
+ * view's own image, run on the map weighted by its confidence and on the confidence, then divided -- the fill that OpenCV's
+ * ximgproc::DisparityWLSFilter applies after StereoSGBM, its LR check and filterSpeckles.  It is not OpenCV's filter bit for
+ * bit: OpenCV also lowers the confidence near depth discontinuities, and here the confidence is 0 or 1.
+ * disp fp32 [2B,H,W] is view-major (map m = v*B + b, as for s3d_disp_cloud); mask, gt are [B,2,H,W].  Per map d, H x W:
+ *   CONFIDENCE: c = 1 where d is finite and, when mask (uint8) is given, mask[b,v,y,x] == 1; else 0.  f = c ? d : 0 (a
+ *     select: NaN and inf never enter).
+ *   GUIDE: the view's own image (left for v = 0, right for v = 1), both uint8 HWC [B,H,W,3] (img_u8 = 1, taken as they are)
+ *     or both fp32 NCHW [B,3,H,W] (img_u8 = 0, each channel rint(clamp(v, 0, 1) * 255) with NaN -> 0, as s3d_disp_cloud).
+ *   EDGE WEIGHT of two 4-neighbours: w = lut[s], s = sum over the 3 channels of the squared colour difference (an integer in
+ *     [0, 3*255^2]).  lut fp32 [3*255^2 + 1] on the device, lut[s] = fp32(exp(-sqrt(s) / sigma)) computed in fp64 (OpenCV's
+ *     table; sigma in 8-bit colour units).
+ *   SCHEDULE: iterations t = 0, 1, 2 with lam_t = fp32(lambda * 0.25^t) (fp64 on the host); each is a horizontal pass over
+ *     every row, then a vertical pass over every column, each pass on the previous pass's output.  U(f) and U(c) go through
+ *     the same passes with the same coefficients.
+ *   ONE LINE u_0 .. u_{n-1} of a pass: k_i = lam_t * w(i, i+1) for i < n-1, kl_i = k_{i-1} (0 for i = 0), kr_i = k_i (0 for
+ *     i = n-1), b_i = (1 + kl_i) + kr_i; b_i u_i - kl_i u_{i-1} - kr_i u_{i+1} = f_i is solved by Thomas elimination with
+ *     g_{-1} = y_{-1} = 0: den_i = b_i - kl_i*g_{i-1}, r_i = 1/den_i, g_i = kr_i*r_i, y_i = (f_i + kl_i*y_{i-1})*r_i, then
+ *     u_{n-1} = y_{n-1} and u_i = y_i + g_i*u_{i+1}.  Every operation is one fp32 round-to-nearest (no FMA contraction,
+ *     denormals kept); k >= 0, so den >= 1 and 0 <= g < 1.
+ * out fp32 [2B,H,W], view-major like disp (s3d_disp_cloud takes it unchanged): U(f) / U(c) (fp32 division) where U(c) > 0,
+ *   NaN where U(c) == 0 (a piece of the map that no confident pixel reaches through non-zero weights); out != disp.
+ * stats int64 [B,2,4+T], ACCUMULATED (the caller zeroes it), per (sample, view):
+ *   [n_finite, n_valid_finite, sum_{valid & finite} q(|out - gt|), count_{valid & finite}(|out - gt| > thresholds[t]) for
+ *    t < T, n_conf (confident input pixels; filled = n_finite - n_conf)]
+ * over the pixels where out is finite: the first 3+T columns have the layout of lr_stats; valid and q as for
+ * s3d_upsample_disp_eval (gt finite and 0 <= gt < max_gt, q(e) = round-half-even(e * 65536)); with gt == NULL the GT columns
+ * are zero.  thresholds: T <= 8 fp32 HOST values.  lambda finite and > 0; max_gt > 0 with gt; H*W < 2^31; 2B < 65536.
+ * workspace: s3d_disp_wls_workspace_bytes(B, H, W) bytes (U(c), g and the two edge weights, 16 bytes per pixel), 4-byte
+ * aligned.
+ * Every output pixel is one fixed sequence of fp32 operations and the counters are integers: out and stats do not depend on
+ * scheduling or batch split.  Six kernels (one per pass, a thread per line). */
+int64_t s3d_disp_wls_workspace_bytes(int B, int H, int W);
+int s3d_disp_wls(const float* disp, int B, int H, int W, const void* left, const void* right, int img_u8,
+                 const uint8_t* mask, const float* lut, float lambda,
+                 const float* gt, const float* thresholds, int T, float max_gt,
+                 float* out, long long* stats, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* --- decoder glue (rows X, D, F, M) ---------------------------------------------------- */
 /* adaptive average pool [N,1,H,W,C] -> [N,1,L,L,C], then the NCHW .view(N,C*L*L/8,2,2,2)

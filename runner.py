@@ -45,6 +45,10 @@ def get_args():
                    help='also remove the small connected regions of each disparity map (OpenCV\'s filterSpeckles with '
                         'TEST.SPECKLE_MAX_SIZE / SPECKLE_MAX_DIFF, after the LR check with --lr-check) and report the kept '
                         'pixels as speckle; with --save-clouds the clouds keep only those pixels')
+    p.add_argument('--wls', action='store_true',
+                   help='also fill each disparity map with the confidence-weighted WLS filter (OpenCV\'s DisparityWLSFilter '
+                        'with TEST.WLS_LAMBDA / WLS_SIGMA; confident where --speckle / --lr-check keep a pixel, else where it '
+                        'is finite) and report it as wls; with --save-clouds the clouds come from the filtered maps')
     p.add_argument('--uncertainty', action='store_true',
                    help='also compute the per-pixel disparity uncertainty and report the confidence-filtered metrics as uncertainty')
     p.add_argument('--surface', action='store_true',
@@ -151,6 +155,8 @@ def main():
         ev.update(eval_cloud=True)
     if args.speckle:
         ev.update(eval_speckle=True)
+    if args.wls:
+        ev.update(eval_wls=True)
     if args.fscore_curves:
         ev.update(eval_fscore_curves=True)
     if args.model == 'Stereo2Voxel':
@@ -170,14 +176,21 @@ def main():
         res['speckle'] = T.speckle_summary(b['speckle'], cfg.TEST.DISP_THRESH, npix, b['disparity'])
         max_size, max_diff = models.speckle_params(cfg)
         res['speckle'].update(max_size=max_size, max_diff=max_diff, after_lr_check=args.lr_check)
+    if 'wls' in b:
+        res['wls'] = T.wls_summary(b['wls'], cfg.TEST.DISP_THRESH, npix, b['disparity'])
+        lam, sigma = models.wls_params(cfg)
+        res['wls'].update({'lambda': lam, 'sigma': sigma,
+                           'confidence': 'speckle' if args.speckle else 'lr_check' if args.lr_check else 'finite'})
     if 'uncertainty' in b:
         res['uncertainty'] = T.unc_summary(b['uncertainty'], cfg.TEST.UNC_THRESH, cfg.TEST.DISP_THRESH, npix, b['disparity'])
     if 'cloud' in b:
         res['cloud'] = T.cloud_summary(b['cloud'], res['n_samples'], cfg.CONST.IMG_H, cfg.CONST.IMG_W)
         res['cloud'].update(camera=models.camera_values(cfg), min_disp=models.cloud_min_disp(cfg),
-                            max_std=models.cloud_max_std(cfg) if args.uncertainty else None)
+                            max_std=models.cloud_max_std(cfg) if args.uncertainty and not args.wls else None)
         if args.speckle:
             res['cloud'].update(speckle=dict(max_size=max_size, max_diff=max_diff))
+        if args.wls:
+            res['cloud'].update(wls={'lambda': lam, 'sigma': sigma})
     if 'surface' in b:
         res['surface'] = T.surface_summary(b['surface'], cfg.TEST.VOXEL_THRESH, cfg.TEST.FSCORE_THRESH, res['n_samples'])
     if 'curves' in b:

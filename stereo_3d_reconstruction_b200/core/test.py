@@ -15,6 +15,10 @@ With eval_speckle=True (needs eval_disp) the speckle-filter counters of the same
 _StereoBase._speckle, after the LR check when eval_lr), per view:
     n_kept, n_valid_kept, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the kept valid pixels, n_speckles,
     n_speckle_px                                                                                     (int64)
+With eval_wls=True (needs eval_disp) the WLS-filter counters of the same forwards follow (models.py, _StereoBase._wls,
+confident where the speckle / LR mask keeps a pixel when eval_speckle / eval_lr, else where it is finite), per view:
+    n_finite, n_valid_finite, sum |wls - gt| in 2^-16 px and count(|wls - gt| > t) over the finite valid pixels, n_conf
+                                                                                                     (int64)
 With eval_unc=True (needs eval_disp) the uncertainty counters of the same forwards follow, per view, then per threshold k in
 TEST.UNC_THRESH (models.py, _StereoBase._upsample_disp):
     n_conf, n_valid_conf, sum |disp - gt| in 2^-16 px and count(|disp - gt| > t) over the confident valid pixels  (int64)
@@ -59,7 +63,7 @@ import torch.distributed as dist
 
 from .. import ops
 from ..models import (Stereo2Point, Stereo2Voxel, camera_values, cloud_max_std, cloud_min_disp, curve_bins, dist_edges,
-                      fscore_thresholds, mesh_thresh, speckle_params, unc_thresholds)
+                      fscore_thresholds, mesh_thresh, speckle_params, unc_thresholds, wls_params)
 from ..utils import synthetic
 
 _FX = float(1 << 40)
@@ -144,6 +148,24 @@ def speckle_summary(stats_block, thresholds, n_pixels, disp_block):
     px = [int(x) for x in v[:, 4 + T].tolist()]
     for name, n, p in (('left', spk[0], px[0]), ('right', spk[1], px[1]), ('all', spk[0] + spk[1], px[0] + px[1])):
         out[name].update(n_speckles=n, speckle_pixels=p, mean_speckle_size=p / n if n else 0.0)
+    return out
+
+
+def wls_summary(stats_block, thresholds, n_pixels, disp_block):
+    """WLS-filter counters [n_finite, n_valid_finite, epe_fx, bad_t..., n_conf] x 2 views (int64 [2 * (4 + T)]) -> dict, per
+    view and over both views: n_finite, density = n_finite / n_pixels (n_pixels: pixels of one view over the run), filled =
+    n_finite - n_conf (the pixels the filter filled in), n_valid_finite, valid_covered = n_valid_finite / n_valid (n_valid
+    from the disparity counters `disp_block`), and EPE / bad-pixel fractions over the finite valid pixels."""
+    T = len(thresholds)
+    v = stats_block.reshape(2, 4 + T)
+    lr = lr_summary(v[:, :3 + T].reshape(-1), thresholds, n_pixels, disp_block)
+    conf = [int(x) for x in v[:, 3 + T].tolist()]
+    out = {'thresholds': list(thresholds)}
+    for name, nc in (('left', conf[0]), ('right', conf[1]), ('all', conf[0] + conf[1])):
+        r = lr[name]
+        out[name] = {'n_finite': r['n_kept'], 'density': r['density'], 'filled': r['n_kept'] - nc,
+                     'n_valid_finite': r['n_valid_kept'], 'valid_covered': r['kept_of_valid'], 'epe': r['epe'],
+                     'bad': r['bad']}
     return out
 
 
@@ -490,9 +512,9 @@ def _disp_gt(pairs, H, W, device):
 
 
 def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eval_surface=False, eval_points=False,
-                 eval_curves=False, eval_fscore_curves=False, eval_cloud=False, eval_speckle=False):
+                 eval_curves=False, eval_fscore_curves=False, eval_cloud=False, eval_speckle=False, eval_wls=False):
     """The driver's int64 stats vector for `model` ('Stereo2Voxel' / 'Stereo2Point') as ordered blocks [(name, length)]: the
-    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'speckle', 'uncertainty', 'cloud' [2],
+    head block ('iou' [2T+1] / 'chamfer' [2]), then 'disparity', 'lr_consistency', 'speckle', 'wls', 'uncertainty', 'cloud' [2],
     then 'surface',
     'curves' and 'surface_curves' (Stereo2Voxel) / 'points' and 'point_curves' (Stereo2Point), each present when its
     evaluation is on (module docstring).  ValueError on an evaluation without the counters it needs or on a bad cfg.TEST
@@ -503,6 +525,8 @@ def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eva
         raise ValueError('eval_unc=True needs eval_disp=True')
     if eval_speckle and not eval_disp:
         raise ValueError('eval_speckle=True needs eval_disp=True')
+    if eval_wls and not eval_disp:
+        raise ValueError('eval_wls=True needs eval_disp=True')
     if eval_fscore_curves and model == 'Stereo2Voxel' and not eval_surface:
         raise ValueError('eval_fscore_curves=True for Stereo2Voxel needs eval_surface=True')
     if eval_fscore_curves and model != 'Stereo2Voxel' and not eval_points:
@@ -516,6 +540,9 @@ def stats_layout(cfg, model, eval_disp=False, eval_lr=False, eval_unc=False, eva
     if eval_speckle:
         speckle_params(cfg)
         blocks.append(('speckle', 2 * (5 + T)))
+    if eval_wls:
+        wls_params(cfg)
+        blocks.append(('wls', 2 * (4 + T)))
     if eval_unc:
         blocks.append(('uncertainty', 2 * len(unc_thresholds(cfg)) * (3 + T)))
     if eval_cloud:
@@ -546,23 +573,25 @@ def split_stats(stats, layout):
 
 
 def _add_disp_blocks(blocks, out):
-    """Adds the batch's disparity, LR-check, speckle-filter, uncertainty and cloud counters of the named forward outputs `out`
-    to their blocks."""
+    """Adds the batch's disparity, LR-check, speckle-filter, WLS-filter, uncertainty and cloud counters of the named forward
+    outputs `out` to their blocks."""
     for block, name in (('disparity', 'disp_stats'), ('lr_consistency', 'lr_stats'), ('speckle', 'speckle_stats'),
-                        ('uncertainty', 'unc_stats'), ('cloud', 'cloud_counts')):
+                        ('wls', 'wls_stats'), ('uncertainty', 'unc_stats'), ('cloud', 'cloud_counts')):
         if block in blocks:
             blocks[block] += out[name].sum(0).flatten()
 
 
 def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
                eval_unc=False, eval_surface=False, mesh_dir=None, eval_curves=False, eval_fscore_curves=False, cloud_dir=None,
-               eval_cloud=False, eval_speckle=False):
+               eval_cloud=False, eval_speckle=False, eval_wls=False):
     """Synthetic StereoShapeNet stand-in: sample i is generated from seed i, so every rank can
     materialise exactly its own shard and the union over ranks is independent of `world`.
     eval_disp: the same forward also evaluates the disparities; their counters follow the IoU ones (module docstring).
     eval_lr: the same forward also runs the left-right consistency check; its counters follow the disparity ones.
     eval_speckle: the same forward also runs the speckle filter (after the LR check with eval_lr); its counters follow the LR
     ones, and with eval_cloud the clouds keep only the pixels it keeps.
+    eval_wls: the same forward also runs the WLS filter (confident where the speckle / LR mask keeps a pixel, else where it
+    is finite); its counters follow the speckle ones, and with eval_cloud the clouds are the WLS maps' (no other filter).
     eval_unc: the same forward also returns the disparity uncertainty; its counters follow the LR ones.
     eval_surface: the same forward also evaluates the voxel surfaces; their block follows the uncertainty one.
     eval_curves: the same forward also returns the occupancy histograms and loss sums; their block follows the surface one.
@@ -573,12 +602,13 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
     uncertainty ones.  cloud_dir (needs eval_cloud): the clouds and the GT disparity's are written there as PLY.
     The vector's blocks: stats_layout(cfg, 'Stereo2Voxel', ...)."""
     layout = stats_layout(cfg, 'Stereo2Voxel', eval_disp, eval_lr, eval_unc, eval_surface, eval_curves=eval_curves,
-                          eval_fscore_curves=eval_fscore_curves, eval_cloud=eval_cloud, eval_speckle=eval_speckle)
+                          eval_fscore_curves=eval_fscore_curves, eval_cloud=eval_cloud, eval_speckle=eval_speckle,
+                          eval_wls=eval_wls)
     _check_cloud(cfg, eval_cloud, eval_unc, cloud_dir)
     if mesh_dir is not None:
         mesh_thresh(cfg)                                # ValueError on a bad TEST.MESH_THRESH, before any forward
         os.makedirs(mesh_dir, exist_ok=True)
-    kw = {k: True for k, on in (('lr_check', eval_lr), ('speckle', eval_speckle), ('uncertainty', eval_unc),
+    kw = {k: True for k, on in (('lr_check', eval_lr), ('speckle', eval_speckle), ('wls', eval_wls), ('uncertainty', eval_unc),
                                 ('surface', eval_surface), ('mesh', mesh_dir is not None), ('curves', eval_curves),
                                 ('fscore_curves', eval_fscore_curves)) if on}    # the options that are on
     names = Stereo2Voxel.output_names(gt=True, disp_gt=eval_disp, camera=eval_cloud, **kw)
@@ -621,17 +651,18 @@ def test_voxel(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda'
 
 def test_point(cfg, model, n_samples, batch_size, rank=0, world=1, device='cuda', eval_disp=False, eval_lr=False,
                eval_points=False, eval_unc=False, eval_fscore_curves=False, cloud_dir=None, eval_cloud=False,
-               eval_speckle=False):
+               eval_speckle=False, eval_wls=False):
     """[sum CD in 2^-40 units, n_samples] (+ the disparity counters with eval_disp, the LR-check counters with eval_lr, the
-    speckle-filter counters with eval_speckle, the uncertainty counters with eval_unc, the stereo-cloud counters with
+    speckle-filter counters with eval_speckle, the WLS-filter counters with eval_wls, the uncertainty counters with eval_unc, the stereo-cloud counters with
     eval_cloud (and the PLY files with cloud_dir), as for test_voxel, + the point-cloud counters with eval_points, + the distance histograms of the same call with
     eval_fscore_curves (needs eval_points): module docstring).
     The vector's blocks: stats_layout(cfg, 'Stereo2Point', ...)."""
     from ..extensions.chamfer_dist import chamfer_per_sample
     layout = stats_layout(cfg, 'Stereo2Point', eval_disp, eval_lr, eval_unc, eval_points=eval_points,
-                          eval_fscore_curves=eval_fscore_curves, eval_cloud=eval_cloud, eval_speckle=eval_speckle)
+                          eval_fscore_curves=eval_fscore_curves, eval_cloud=eval_cloud, eval_speckle=eval_speckle,
+                          eval_wls=eval_wls)
     _check_cloud(cfg, eval_cloud, eval_unc, cloud_dir)
-    kw = {k: True for k, on in (('lr_check', eval_lr), ('speckle', eval_speckle), ('uncertainty', eval_unc),
+    kw = {k: True for k, on in (('lr_check', eval_lr), ('speckle', eval_speckle), ('wls', eval_wls), ('uncertainty', eval_unc),
                                 ('fscore_curves', eval_fscore_curves)) if on}
     names = Stereo2Point.output_names(gt=eval_points, disp_gt=eval_disp, camera=eval_cloud, **kw)
     stats = torch.zeros(sum(n for _, n in layout), dtype=torch.int64, device=device)

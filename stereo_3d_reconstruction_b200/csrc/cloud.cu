@@ -117,11 +117,6 @@ __device__ __forceinline__ int block_sum(int s, int* red) {
   return t;
 }
 
-__device__ __forceinline__ unsigned colour_f32(float c) {
-  const float u = fminf(fmaxf(c, 0.f), 1.f);                             // NaN -> 0 (fmaxf)
-  return (unsigned)__float2int_rn(__fmul_rn(u, 255.f));                  // round half to even
-}
-
 // Colours of pixels x .. x+3 of row y of image `img` of sample b (one row, x % 4 == 0, aligned rows), packed r | g << 8 |
 // b << 16: three 4-byte loads of the uint8 HWC pixels, or one 16-byte load per fp32 channel plane.
 template <bool U8>

@@ -92,6 +92,12 @@ __device__ __forceinline__ float apply_act(float v, int act, float a) {
 // Out-of-line copy for epilogues that must stay small: 16 calls instead of 16 inlined switch bodies.
 static __device__ __noinline__ float apply_act_slow(float v, int act, float a) { return apply_act(v, act, a); }
 
+// 8-bit colour of an fp32 image channel (s3d_disp_cloud, s3d_disp_wls): rint(clamp(c, 0, 1) * 255), NaN -> 0.
+__device__ __forceinline__ unsigned colour_f32(float c) {
+  const float u = fminf(fmaxf(c, 0.f), 1.f);                             // NaN -> 0 (fmaxf)
+  return (unsigned)__float2int_rn(__fmul_rn(u, 255.f));                  // round half to even
+}
+
 // sigma_q = sqrt(var) of a soft-argmin distribution; a non-finite mean gives NaN.
 __device__ __forceinline__ float soft_std(float var, float mu) {
   return isfinite(mu) ? sqrtf(fmaxf(var, 0.f)) : __int_as_float(0x7fffffff);

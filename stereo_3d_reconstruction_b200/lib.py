@@ -78,6 +78,9 @@ SIGNATURES = {
     's3d_disp_cloud': ([_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _f, _vp, _f, _vp, _vp, _vp, _vp, _i64, _vp], _i),
     's3d_speckle_filter_workspace_bytes': ([_i, _i, _i], ctypes.c_int64),
     's3d_speckle_filter': ([_vp, _i, _i, _i, _vp, _i, _f, _vp, ctypes.POINTER(_f), _i, _f, _vp, _vp, _vp, _i64, _vp], _i),
+    's3d_disp_wls_workspace_bytes': ([_i, _i, _i], ctypes.c_int64),
+    's3d_disp_wls': ([_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _f, _vp, ctypes.POINTER(_f), _i, _f, _vp, _vp, _vp, _i64, _vp],
+                     _i),
     's3d_latent_to_vox': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_avg_pool': ([_vp, _vp, _i, _i, _i, _i, _i, _i, _vp], _i),
     's3d_depth_to_space': ([_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp], _i),

@@ -36,6 +36,7 @@ PRECISIONS = ('bf16', 'bf16x3', 'tf32', 'tf32x3', 'fp32')
 OPTIONAL_OUTPUTS = (('disp_gt', ('disp_stats',)),
                     ('lr_check', ('lr_mask', 'lr_stats')),
                     ('speckle', ('speckle_mask', 'speckle_stats')),
+                    ('wls', ('wls_left', 'wls_right', 'wls_stats')),
                     ('uncertainty', ('disp_std', 'unc_stats')),
                     ('camera', ('cloud_xyz', 'cloud_rgb', 'cloud_counts')),
                     ('surface', ('surf_stats',)),
@@ -47,7 +48,8 @@ _VOXEL_ONLY = {'surface': 'surface=True evaluates voxel surfaces: Stereo2Voxel o
                'curves': 'curves=True evaluates the voxel occupancy: Stereo2Voxel only'}
 
 # The options of one forward, checked (_StereoBase._check_args): what the stages branch on and part of the graph key.
-Options = collections.namedtuple('Options', 'gt disp_gt lr_check speckle uncertainty camera surface mesh curves fscore_curves')
+Options = collections.namedtuple('Options', 'gt disp_gt lr_check speckle wls uncertainty camera surface mesh curves '
+                                              'fscore_curves')
 
 
 def _conv_bn2d(cin, cout, k, s, p):
@@ -472,8 +474,8 @@ class _StereoBase(nn.Module):
         return self._conv(layer, x, out=self._bufo(out_name, layer, x))
 
     # ---- CUDA-graph replay (SURVEY.md 8(f) item 3) ---------------------------------------------
-    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, uncertainty=False, camera=None,
-                surface=False, mesh=False, curves=False, fscore_curves=False):
+    def graphed(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, wls=False, uncertainty=False,
+                camera=None, surface=False, mesh=False, curves=False, fscore_curves=False):
         """Same results as forward(), replayed from a CUDA graph captured on first use for this input signature: one
         graph launch instead of ~35 kernel launches + torch glue.  Measured (scripts/graph_latency.py): B = 1 1.23 -> 1.19 ms,
         B = 8 2.40 -> 2.37 ms -- the forward is GPU-bound even at batch 1 (a column of 32 planes is a serial chain of
@@ -481,7 +483,7 @@ class _StereoBase(nn.Module):
         Inputs are copied into the graph's static buffers; the returned tensors are the graph's static outputs and
         are overwritten by the next call with the same signature."""
         left, right, gt, disp_gt, camera, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera,
-                                                                  surface, mesh, curves, fscore_curves, speckle)
+                                                                  surface, mesh, curves, fscore_curves, speckle, wls)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         if mb and left.shape[0] > mb:
             raise ValueError('graphed(): batch %d exceeds CONST.MICRO_BATCH = %d; use forward()' % (left.shape[0], mb))
@@ -496,12 +498,12 @@ class _StereoBase(nn.Module):
     # ---- outputs and their checks --------------------------------------------------------------
     @classmethod
     def output_names(cls, gt=False, disp_gt=False, lr_check=False, uncertainty=False, surface=False, mesh=False,
-                     curves=False, fscore_curves=False, camera=False, speckle=False):
+                     curves=False, fscore_curves=False, camera=False, speckle=False, wls=False):
         """Names of the forward's outputs, in tuple order, for these options (gt / disp_gt / camera: whether the tensor is given):
         the head's outputs, the gt output, then the groups of OPTIONAL_OUTPUTS that are on.  ValueError on an option the
         class does not have."""
-        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'speckle': speckle, 'uncertainty': uncertainty, 'camera': camera,
-              'surface': surface, 'mesh': mesh, 'curves': curves, 'fscore_curves': fscore_curves}
+        on = {'disp_gt': disp_gt, 'lr_check': lr_check, 'speckle': speckle, 'wls': wls, 'uncertainty': uncertainty,
+              'camera': camera, 'surface': surface, 'mesh': mesh, 'curves': curves, 'fscore_curves': fscore_curves}
         names = cls.HEAD_OUTPUTS + ((cls.GT_OUTPUT,) if gt else ())
         for opt, outs in OPTIONAL_OUTPUTS:
             if on[opt]:
@@ -511,12 +513,12 @@ class _StereoBase(nn.Module):
         return names
 
     def _check_args(self, left, right, gt, disp_gt, lr_check, uncertainty, camera, surface, mesh, curves, fscore_curves,
-                    speckle=False):
+                    speckle=False, wls=False):
         """The one check of forward() / graphed()'s arguments, before anything is launched: first the options (which the
         class has, what they need), then the cfg.TEST thresholds of the enabled outputs, then the tensors.
         -> (left, right, gt, disp_gt, camera) as the forward takes them and the options value: an Options of bools."""
-        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(speckle), bool(uncertainty), camera is not None,
-                       bool(surface), bool(mesh), bool(curves), bool(fscore_curves))
+        opts = Options(gt is not None, disp_gt is not None, bool(lr_check), bool(speckle), bool(wls), bool(uncertainty),
+                       camera is not None, bool(surface), bool(mesh), bool(curves), bool(fscore_curves))
         self.output_names(**opts._asdict())                   # ValueError on an option this class does not have
         if opts.surface and not opts.gt:
             raise ValueError('surface=True needs the GT occupancy gt')
@@ -539,6 +541,8 @@ class _StereoBase(nn.Module):
             lr_thresh(self.cfg)
         if opts.speckle:
             speckle_params(self.cfg)
+        if opts.wls:
+            wls_params(self.cfg)
         if opts.fscore_curves:
             dist_edges(self.cfg)
         if opts.camera:
@@ -546,6 +550,8 @@ class _StereoBase(nn.Module):
             if opts.uncertainty:
                 cloud_max_std(self.cfg)
         left, right = self._check_inputs(left, right)
+        if opts.wls:
+            self._wls_lut(wls_params(self.cfg)[1])         # built here, outside the forward (and outside a graph capture)
         return (left, right, self._check_gt(gt, left), self._check_disp_gt(disp_gt, left), self._check_camera(camera, left),
                 opts)
 
@@ -556,6 +562,8 @@ class _StereoBase(nn.Module):
         out.update(disp_left=disp[:B].unsqueeze(1), disp_right=disp[B:].unsqueeze(1))
         if opts.speckle:
             out['speckle_mask'], out['speckle_stats'] = self._speckle(disp, disp_gt, out.get('lr_mask'))
+        if opts.wls:
+            out['wls_left'], out['wls_right'], out['wls_stats'] = self._wls(left, right, disp, disp_gt, out)
         if camera is not None:
             out['cloud_xyz'], out['cloud_rgb'], out['cloud_counts'] = self._cloud(left, right, disp, camera, out)
         self._head(left, right, gt, disp, opts, out)
@@ -627,16 +635,47 @@ class _StereoBase(nn.Module):
                                        self._buf('speckle_stats', (B, 2, 5 + len(th)), torch.int64).zero_()),
                                   workspace=self._buf('speckle_ws', (max(nb, 1),), torch.uint8))
 
+    def _wls_lut(self, sigma):
+        """The edge-weight table of sigma on the module's device (ops.wls_weight_lut), built once per sigma and kept with
+        the workspace."""
+        key = ('wls_lut', sigma)
+        t = self._ws.get(key)
+        if t is None:
+            t = self._ws[key] = torch.from_numpy(ops.wls_weight_lut(sigma)).to(next(self.parameters()).device)
+        return t
+
+    def _wls(self, left, right, disp, disp_gt, ev):
+        """WLS filter of disp [2B,H,W] guided by each view's image (include/s3d.h, s3d_disp_wls; TEST.WLS_LAMBDA / WLS_SIGMA),
+        confident where `ev` holds the speckle mask, else the LR mask, else where d is finite -> (wls_left fp32 [B,1,H,W],
+        wls_right fp32 [B,1,H,W], views of one view-major buffer, wls_stats int64 [B,2,4+T]): the lr_stats counters over
+        the finite output pixels against disp_gt (TEST.DISP_THRESH, valid below 4 * MAX_DISP; zero without it), then n_conf.
+        The stats are zeroed here, so a graph replay starts from zero; the table was built by _check_args and every buffer
+        comes from the workspace: no allocation and no host copy on this path."""
+        B, H, W = disp.shape[0] // 2, disp.shape[1], disp.shape[2]
+        lam, sigma = wls_params(self.cfg)
+        th = list(self.cfg.TEST.DISP_THRESH)
+        mask = ev['speckle_mask'] if 'speckle_mask' in ev else ev.get('lr_mask')
+        nb = ops.disp_wls_workspace_bytes(B, H, W)
+        w, stats = ops.disp_wls(disp, B, left, right, self._wls_lut(sigma), lam, mask=mask, disp_gt=disp_gt, thresholds=th,
+                                max_gt=4.0 * self.cfg.NETWORK.MAX_DISP,
+                                out=(self._buf('wls', (2 * B, H, W), torch.float32),
+                                     self._buf('wls_stats', (B, 2, 4 + len(th)), torch.int64).zero_()),
+                                workspace=self._buf('wls_ws', (max(nb, 1),), torch.uint8))
+        return w[:B].unsqueeze(1), w[B:].unsqueeze(1), stats
+
     def _cloud(self, left, right, disp, camera, ev):
         """Coloured point clouds of disp [2B,H,W] with the camera -> (cloud_xyz fp32 [B,2HW,3], cloud_rgb uint8 [B,2HW,3],
         cloud_counts int32 [B,2]), filtered by the speckle mask (which includes the LR check) or else the LR mask, and by the
         disparity spread (TEST.CLOUD_MAX_STD), when the forward computed them in `ev` (include/s3d.h, s3d_disp_cloud;
-        TEST.CLOUD_MIN_DISP).  The kernels write every output (nothing to zero) into workspace buffers: no allocation on this
-        path."""
+        TEST.CLOUD_MIN_DISP).  When `ev` holds the WLS maps, those are back-projected instead, with no mask and no spread
+        filter: the confidence already went into the filter.  The kernels write every output (nothing to zero) into workspace
+        buffers: no allocation on this path."""
         B, H, W = disp.shape[0] // 2, disp.shape[1], disp.shape[2]
         std = ev.get('disp_std')
         nb = ops.disp_cloud_workspace_bytes(B, H)
         mask = ev['speckle_mask'] if 'speckle_mask' in ev else ev.get('lr_mask')
+        if 'wls_stats' in ev:
+            disp, mask, std = self._buf('wls', (2 * B, H, W), torch.float32), None, None
         return ops.disp_cloud(disp, B, left, right, camera, cloud_min_disp(self.cfg), lr_mask=mask, disp_std=std,
                               max_std=None if std is None else cloud_max_std(self.cfg),
                               out=(self._buf('cloud_xyz', (B, 2 * H * W, 3), torch.float32),
@@ -646,9 +685,10 @@ class _StereoBase(nn.Module):
 
 
 class Stereo2Voxel(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=][, speckle=][, uncertainty=][, camera=]) -> (disp_left [B,1,H,W],
-    disp_right [B,1,H,W], voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask uint8
-    [B,2,H,W], lr_stats int64 [B,2,3+T']][, speckle_mask uint8 [B,2,H,W], speckle_stats int64 [B,2,5+T']][, disp_std fp32
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, speckle=][, wls=][, uncertainty=][, camera=]) -> (disp_left
+    [B,1,H,W], disp_right [B,1,H,W], voxels [B,32,32,32][, iou_counts int64 [B,T,2]][, disp_stats int64 [B,2,2+T']][, lr_mask
+    uint8 [B,2,H,W], lr_stats int64 [B,2,3+T']][, speckle_mask uint8 [B,2,H,W], speckle_stats int64 [B,2,5+T']][, wls_left
+    fp32 [B,1,H,W], wls_right fp32 [B,1,H,W], wls_stats int64 [B,2,4+T']][, disp_std fp32
     [B,2,H,W], unc_stats int64 [B,2,K,3+T']][, cloud_xyz fp32 [B,2HW,3], cloud_rgb
     uint8 [B,2HW,3], cloud_counts int32 [B,2]][, surf_stats int64 [B,T,2,3+F]][, mesh_verts fp32
     [B,max_verts,3], mesh_faces int32 [B,max_faces,3], mesh_counts int32 [B,2]][, occ_hist int64 [B,3,K], occ_loss int64
@@ -662,6 +702,12 @@ class Stereo2Voxel(_StereoBase):
     TEST.SPECKLE_MAX_SIZE pixels; speckle_stats = the lr_stats counters over those pixels, then the number of removed regions
     and their pixels (_StereoBase._speckle; include/s3d.h, s3d_speckle_filter; four more launches).  With camera= as well the
     cloud keeps only the pixels of speckle_mask.
+    wls=True: OpenCV's WLS fill of the two disparity maps, guided by each view's image and weighted by the confidence
+    (speckle_mask with speckle=True, else lr_mask with lr_check=True, else the finite pixels): wls_left / wls_right fp32
+    [B,1,H,W] (NaN where no confident pixel reaches) and wls_stats int64 [B,2,4+T'] = the lr_stats counters over the finite
+    output pixels, then the confident input pixels (_StereoBase._wls; include/s3d.h, s3d_disp_wls; TEST.WLS_LAMBDA /
+    WLS_SIGMA; six more launches), right after the speckle outputs.  With camera= as well the cloud back-projects the WLS
+    maps with no mask and no spread filter.
     camera=(fp32 [B,5] = (f, cx, cy, baseline, doffs) per sample on the images' device, with or without gt): the coloured
     point clouds of the two disparity maps in the left camera's frame, one per sample: the kept pixels of disp_left in raster
     order, then those of disp_right, each at depth f * baseline / (d + doffs) and coloured from its own image; a pixel is kept
@@ -686,7 +732,7 @@ class Stereo2Voxel(_StereoBase):
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'voxels')
     GT_OUTPUT = 'iou_counts'
-    OPTIONS = ('disp_gt', 'lr_check', 'speckle', 'uncertainty', 'camera', 'surface', 'mesh', 'curves', 'fscore_curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'speckle', 'wls', 'uncertainty', 'camera', 'surface', 'mesh', 'curves', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -725,10 +771,10 @@ class Stereo2Voxel(_StereoBase):
             P['mrg%d' % i] = PackedConv.from_conv(seq[0], seq[1], A.ACT_LEAKY, dc, dev,
                                                   act_param=self.cfg.NETWORK.LEAKY_VALUE)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, uncertainty=False, camera=None,
-                surface=False, mesh=False, curves=False, fscore_curves=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, wls=False, uncertainty=False,
+                camera=None, surface=False, mesh=False, curves=False, fscore_curves=False):
         left, right, gt, disp_gt, camera, opts = self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera,
-                                                                  surface, mesh, curves, fscore_curves, speckle)
+                                                                  surface, mesh, curves, fscore_curves, speckle, wls)
         mb = int(self.cfg.CONST.get('MICRO_BATCH', 0) or 0)
         B = left.shape[0]
         if mb and B > mb:
@@ -884,6 +930,24 @@ def speckle_params(cfg):
     return n, t
 
 
+def wls_params(cfg):
+    """(TEST.WLS_LAMBDA, TEST.WLS_SIGMA) of the WLS filter: the smoothness weight lambda and the colour scale sigma of the
+    edge weights exp(-|colour difference| / sigma) in 8-bit colour units (OpenCV's DisparityWLSFilter lambda and
+    sigmaColor), each a number (not a bool), finite and > 0 also in fp32; anything else is a ValueError."""
+    out = []
+    for key in ('WLS_LAMBDA', 'WLS_SIGMA'):
+        v = cfg.TEST.get(key)
+        try:
+            t = float(v)
+        except (TypeError, ValueError):
+            raise ValueError('TEST.%s must be a number, got %r' % (key, v)) from None
+        if isinstance(v, bool) or not (math.isfinite(t) and t > 0) or not (math.isfinite(ctypes.c_float(t).value) and
+                                                                             ctypes.c_float(t).value > 0):
+            raise ValueError('TEST.%s must be finite and > 0, got %r' % (key, v))
+        out.append(t)
+    return tuple(out)
+
+
 def cloud_min_disp(cfg):
     """TEST.CLOUD_MIN_DISP as a float: the smallest disparity + doffs (input px) a stereo cloud back-projects, which bounds
     the depth at f * baseline / CLOUD_MIN_DISP; finite and > 0 (also in fp32); anything else is a ValueError."""
@@ -969,10 +1033,10 @@ def fscore_thresholds(cfg):
 
 
 class Stereo2Point(_StereoBase):
-    """forward(left, right[, gt][, disp_gt=][, lr_check=][, speckle=][, uncertainty=][, camera=]) -> (disp_left, disp_right,
-    points [B,N_POINTS,3][, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats][, speckle_mask,
-    speckle_stats][, disp_std, unc_stats][, cloud_xyz, cloud_rgb, cloud_counts][, dist_hist]) (disp_gt, lr_check, speckle,
-    uncertainty, camera and their outputs as for
+    """forward(left, right[, gt][, disp_gt=][, lr_check=][, speckle=][, wls=][, uncertainty=][, camera=]) -> (disp_left,
+    disp_right, points [B,N_POINTS,3][, point_stats int64 [B,2,3+T]][, disp_stats int64 [B,2,2+T']][, lr_mask, lr_stats]
+    [, speckle_mask, speckle_stats][, wls_left, wls_right, wls_stats][, disp_std, unc_stats][, cloud_xyz, cloud_rgb,
+    cloud_counts][, dist_hist]) (disp_gt, lr_check, speckle, wls, uncertainty, camera and their outputs as for
     Stereo2Voxel: the stereo clouds are the dense counterpart of the decoder's points).  gt: fp32 [B,M,3] GT point cloud; with it the same forward runs the Chamfer search of
     `points` against it and counts, per sample and direction (0: predicted -> GT, 1: GT -> predicted), [sum of squared
     distances and sum of distances in 2^-32 units, points out of range, points closer than t for t in TEST.FSCORE_THRESH]
@@ -982,7 +1046,7 @@ class Stereo2Point(_StereoBase):
 
     HEAD_OUTPUTS = ('disp_left', 'disp_right', 'points')
     GT_OUTPUT = 'point_stats'
-    OPTIONS = ('disp_gt', 'lr_check', 'speckle', 'uncertainty', 'camera', 'fscore_curves')
+    OPTIONS = ('disp_gt', 'lr_check', 'speckle', 'wls', 'uncertainty', 'camera', 'fscore_curves')
 
     def __init__(self, cfg):
         super().__init__(cfg)
@@ -1010,10 +1074,10 @@ class Stereo2Point(_StereoBase):
         P['pt_fc1'] = PackedConv.from_linear_over_map(pd.fc1, 2 * c, L // 2, L // 2, A.ACT_RELU, dc, dev)
         P['pt_fc2'] = PackedConv.from_pointwise(pd.fc2.weight, pd.fc2.bias, None, A.ACT_TANH, dc, dev, act_param=0.5)
 
-    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, uncertainty=False, camera=None,
-                mesh=False, curves=False, fscore_curves=False):
+    def forward(self, left, right, gt=None, *, disp_gt=None, lr_check=False, speckle=False, wls=False, uncertainty=False,
+                camera=None, mesh=False, curves=False, fscore_curves=False):
         return self._forward_impl(*self._check_args(left, right, gt, disp_gt, lr_check, uncertainty, camera, False, mesh,
-                                                    curves, fscore_curves, speckle))
+                                                    curves, fscore_curves, speckle, wls))
 
     def _head(self, left, right, gt, disp, opts, out):
         """The point head: adds points and point_stats (with gt) to `out`."""

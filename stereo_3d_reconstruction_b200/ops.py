@@ -850,3 +850,104 @@ def speckle_filter(disp, B, max_size, max_diff, lr_mask=None, disp_gt=None, thre
     _lib.check(rc, 's3d_speckle_filter')
     _lib.count_launch(4)                       # speckle_local / border / size / finish kernels
     return mask, stats
+
+
+def wls_weight_lut(sigma):
+    """Edge-weight table of disp_wls for the colour scale sigma (finite and > 0, 8-bit colour units): float32 numpy
+    [3 * 255^2 + 1], entry s = fp32(exp(-sqrt(s) / sigma)) computed in fp64, s the summed squared colour difference of two
+    neighbours (OpenCV's DisparityWLSFilter table).  ValueError on a bad sigma."""
+    import numpy as np
+    try:
+        s = float(sigma)
+    except (TypeError, ValueError):
+        raise ValueError('wls_weight_lut: sigma must be a number, got %r' % (sigma,)) from None
+    if isinstance(sigma, bool) or not (math.isfinite(s) and s > 0):
+        raise ValueError('wls_weight_lut: sigma must be finite and > 0, got %r' % (sigma,))
+    return np.exp(-np.sqrt(np.arange(3 * 255 * 255 + 1, dtype=np.float64)) / s).astype(np.float32)
+
+
+def disp_wls_workspace_bytes(B, H, W):
+    """Bytes of the workspace of disp_wls: U(c), the elimination's g and the two edge weights, 16 bytes per pixel of the
+    2B maps."""
+    return int(_lib.load().s3d_disp_wls_workspace_bytes(int(B), int(H), int(W)))
+
+
+def disp_wls(disp, B, left, right, lut, lam, mask=None, disp_gt=None, thresholds=(), max_gt=None, out=None, workspace=None):
+    """Confidence-weighted WLS filter of the two disparity maps (include/s3d.h, s3d_disp_wls), OpenCV's DisparityWLSFilter
+    fill on the GPU.  disp fp32 [2B,H,W], view-major (the forward's buffer: left-referenced maps first); left / right the
+    guides, both fp32 NCHW [B,3,H,W] or both uint8 HWC [B,H,W,3]; lut fp32 [3 * 255^2 + 1] on the device (wls_weight_lut);
+    lam (lambda) finite and > 0.  A pixel is confident where d is finite and, with mask uint8 [B,2,H,W], mask is 1.
+    -> (out fp32 [2B,H,W]: U(d c) / U(c), NaN where no confident pixel reaches, stats int64 [B,2,4+T] ADDED to: [n_finite,
+    n_valid_finite, sum of |out - gt| in 2^-16 px and count(|out - gt| > t) per threshold over the finite pixels with valid
+    GT (disp_gt fp32 [B,2,H,W], valid where finite and 0 <= gt < max_gt; zero without it), n_conf]).  T = len(thresholds)
+    <= 8.  out: (out, stats), else a new map and zeroed stats (out must not be disp); workspace: uint8 of at least
+    disp_wls_workspace_bytes(B, H, W) bytes.  Six kernel launches."""
+    _chk(disp, left, right, lut, mask, disp_gt, workspace)
+    if disp.dtype != torch.float32 or disp.dim() != 3:
+        raise ValueError('disp_wls: expected disp float32 [2B,H,W], got %s %s' % (disp.dtype, tuple(disp.shape)))
+    if not isinstance(B, int) or isinstance(B, bool) or B < 0 or disp.shape[0] != 2 * B:
+        raise ValueError('disp_wls: disp must hold 2B maps for an int B >= 0, got B = %r and %s' % (B, tuple(disp.shape)))
+    H, W = disp.shape[1], disp.shape[2]
+    dev = disp.device
+    if left.dtype == torch.uint8 and right.dtype == torch.uint8:
+        u8, want = 1, (B, H, W, 3)
+    elif left.dtype == torch.float32 and right.dtype == torch.float32:
+        u8, want = 0, (B, 3, H, W)
+    else:
+        raise ValueError('disp_wls: left / right must be both float32 or both uint8, got %s / %s' % (left.dtype, right.dtype))
+    for name, t, d, s in (('left', left, None, want), ('right', right, None, want),
+                          ('lut', lut, torch.float32, (3 * 255 * 255 + 1,)), ('mask', mask, torch.uint8, (B, 2, H, W)),
+                          ('disp_gt', disp_gt, torch.float32, (B, 2, H, W))):
+        if t is not None and ((d is not None and t.dtype != d) or tuple(t.shape) != s or t.device != dev):
+            raise ValueError('disp_wls: expected %s %s %s on %s, got %s %s on %s'
+                             % (name, '' if d is None else d, s, dev, t.dtype, tuple(t.shape), t.device))
+    if lut is None:
+        raise ValueError('disp_wls: lut is required (wls_weight_lut)')
+    try:
+        lam_v = float(lam)
+        th = [float(t) for t in thresholds]
+        max_gt = None if max_gt is None else float(max_gt)
+    except (TypeError, ValueError):
+        raise ValueError('disp_wls: lam, thresholds and max_gt must be numbers, got %r / %r / %r'
+                         % (lam, thresholds, max_gt)) from None
+    if isinstance(lam, bool) or not (math.isfinite(lam_v) and lam_v > 0 and math.isfinite(ctypes.c_float(lam_v).value) and
+                                     ctypes.c_float(lam_v).value > 0):
+        raise ValueError('disp_wls: lam must be finite and > 0 (also in fp32), got %r' % (lam,))
+    if len(th) > 8:
+        raise ValueError('disp_wls: at most 8 thresholds, got %d' % len(th))
+    if disp_gt is not None and not (max_gt is not None and max_gt > 0 and ctypes.c_float(max_gt).value > 0):
+        raise ValueError('disp_wls: disp_gt needs max_gt > 0, got %r' % (max_gt,))
+    T = len(th)
+    shapes = ((torch.float32, (2 * B, H, W)), (torch.int64, (B, 2, 4 + T)))
+    if out is None:
+        out = (torch.empty(shapes[0][1], dtype=torch.float32, device=dev),
+               torch.zeros(shapes[1][1], dtype=torch.int64, device=dev))
+    else:
+        out = tuple(out)
+        if len(out) != 2:
+            raise ValueError('disp_wls: out must hold (out, stats)')
+        _chk(*out)
+        for o, (d, s) in zip(out, shapes):
+            if o.dtype != d or tuple(o.shape) != s or o.device != dev:
+                raise ValueError('disp_wls: out tensors must be %s on %s, got %s'
+                                 % ([(str(d), s) for d, s in shapes], dev, [(str(o.dtype), tuple(o.shape)) for o in out]))
+        if B and out[0].untyped_storage().data_ptr() == disp.untyped_storage().data_ptr():
+            raise ValueError('disp_wls: out must not share memory with disp')
+    nb = disp_wls_workspace_bytes(B, H, W)
+    if workspace is None:
+        workspace = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
+    elif workspace.dtype != torch.uint8 or workspace.numel() < nb or workspace.device != dev:
+        raise ValueError('disp_wls: workspace must be uint8 of at least %d bytes on %s' % (nb, dev))
+    res, stats = out
+    if B == 0:                                 # no maps (and empty tensors may hold no data pointer)
+        return res, stats
+    ptr = lambda t: None if t is None else t.data_ptr()
+    tc = (ctypes.c_float * max(T, 1))(*th)
+    rc = _lib.load().s3d_disp_wls(disp.data_ptr(), B, H, W, left.data_ptr(), right.data_ptr(), u8, ptr(mask), lut.data_ptr(),
+                                  lam_v, ptr(disp_gt), tc, T, 0.0 if max_gt is None else max_gt, res.data_ptr(),
+                                  stats.data_ptr(), workspace.data_ptr(), workspace.numel(), _stream())
+    if rc == -1:                               # S3D_ERR_INVALID: an argument the checks above let through (H W >= 2^31, ...)
+        raise ValueError('disp_wls: %s' % _lib.load().s3d_last_error().decode('utf-8', 'replace'))
+    _lib.check(rc, 's3d_disp_wls')
+    _lib.count_launch(6)                       # wls_row_kernel / wls_col_kernel x 3 iterations
+    return res, stats
